@@ -2,7 +2,7 @@
 """bench.py — the reference's headline metric on B200: Mrays/s and frame ms of `Camera::render`
 (lib/src/camera.rs:76-91), beside the CPU render of the same frame.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3] [--impl ours|reference] [--dump-outputs DIR]
 
 A *step* is one frame of the workload (default c3 = BASELINE.json configs[2]: the soft-shadow scene at
 3840x2160 with a 4x4 = 16-cell jittered area light, reflections, depth 5 — the frame the north-star target is
@@ -232,6 +232,32 @@ class Ctx:
         return self._peak
 
 
+DUMP_PIXELS = 1 << 20  # sampled pixels of a larger frame: 32 bytes each over the three arrays, 32 MiB in all
+
+
+def dump_frame(ctx: Ctx, prepared, depth: int, out_dir: str) -> None:
+    """Writes the frame of the last timed step as a caller of PreparedScene.render receives it: the f32 canvas and its
+    8-bit plane at every pixel, or at a fixed seeded sample of DUMP_PIXELS pixels of a larger frame, plus the ray counts.
+    The timed steps leave the frame on the device, so it is rendered once more with a copy to the host.  A host canvas
+    would otherwise cut the frame into sliced launches in natural tile order.  With RTC_OPT_RENDER_SLICES = 1 the render
+    is the timed steps' single launch, in the tile order they learnt.  Equal ray and launch counts are a sanity check,
+    not a proof."""
+    timed = prepared.last_stats
+    prepared.set_option(4, 1)  # RTC_OPT_RENDER_SLICES
+    frame = prepared.render(depth, shard=ctx.rank, n_shards=ctx.n_shards, fma=ctx.args.fma)
+    st = prepared.last_stats
+    counts = [st.primary_rays, st.secondary_rays, st.shadow_rays]
+    if counts != [timed.primary_rays, timed.secondary_rays, timed.shadow_rays] or st.launches != timed.launches:
+        raise RuntimeError("the frame rendered for --dump-outputs is not the timed one")
+    n = frame.width * frame.height
+    pixel = np.arange(n) if n <= DUMP_PIXELS else np.sort(np.random.default_rng(0).choice(n, DUMP_PIXELS, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "rgb.npy"), frame.data.reshape(n, 3)[pixel])
+    np.save(os.path.join(out_dir, "u8.npy"), frame.to_u8().reshape(n, 3)[pixel].astype(np.float32))
+    np.save(os.path.join(out_dir, "pixel.npy"), pixel.astype(np.float64))
+    np.save(os.path.join(out_dir, "ray_counts.npy"), np.array(counts, np.float64))
+
+
 def measure_device(ctx: Ctx, prepared, depth: int, steps: int, warmup: int, spin_s: float = 0.0) -> dict:
     """Device-resident throughput of one workload: `steps` frames, L2 flushed before each, CUDA-event time of the render
     kernel per frame, max over ranks; rays summed over ranks."""
@@ -373,7 +399,7 @@ def roofline_of(ctx: Ctx, workload: str, detail: dict, ms_frame: float) -> dict:
             "prim_tests_per_ray": round(sum(detail["prim_tests"]) / max(detail["rays"], 1), 2)}
 
 
-def run_workload(ctx: Ctx, workload: str, steps: int, warmup: int, headline: bool) -> dict:
+def run_workload(ctx: Ctx, workload: str, steps: int, warmup: int, headline: bool, dump_dir: str | None = None) -> dict:
     """Everything measured for one workload.  headline: the long form (clock sampling, e2e variants)."""
     a = ctx.args
     cam, world, depth, desc = build_scene(ctx.api, workload)
@@ -393,6 +419,8 @@ def run_workload(ctx: Ctx, workload: str, steps: int, warmup: int, headline: boo
     stop.set()
     if sampler:
         sampler.join(timeout=2)
+    if dump_dir is not None:
+        dump_frame(ctx, prepared, depth, dump_dir)
     # the first frame of a shard, before anything about the frame has been learnt (the reference API is one-shot):
     # a fresh commit, one untimed-by-us render whose own CUDA-event time is read
     first = cam.prepare(world)
@@ -412,15 +440,19 @@ def run_workload(ctx: Ctx, workload: str, steps: int, warmup: int, headline: boo
 def main() -> None:
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed frames of the headline workload")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--workload", default="c3", choices=sorted(WORKLOADS))
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--fma", action="store_true", help="time the FMA-contracted kernel build instead of the IEEE one")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-per-workload", action="store_true", help="skip the short runs of the other BASELINE configs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed frame of the headline workload to DIR as .npy "
+                                                          "(one process only), to compare two builds output for output")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
+    if args.dump_outputs and (args.impl != "ours" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs needs --impl ours and one process (a rank renders only its own bands)")
 
     if args.impl == "reference":
         run_reference(args)
@@ -428,7 +460,7 @@ def main() -> None:
 
     ctx = Ctx(args)
     rank, world_size = ctx.rank, ctx.world_size
-    main_run = run_workload(ctx, args.workload, args.steps, args.warmup, headline=True)
+    main_run = run_workload(ctx, args.workload, args.steps, args.warmup, headline=True, dump_dir=args.dump_outputs)
     dev, detail = main_run["dev"], main_run["detail"]
     w, h = main_run["resolution"]
 
