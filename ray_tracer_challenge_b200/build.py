@@ -1,8 +1,9 @@
 """In-tree build of the native libraries (sm_100a only; nvcc cross-compiles without a GPU).
 
     librtc_b200.so  the C ABI of include/rtc_b200.h: csrc/rtc_api.cu + csrc/rtc_commit.cu (host half of a commit) + csrc/rtc_lbvh.cu (device tree builder) +
-                    csrc/rtc_kernels.cu compiled twice
-                    (FMA-contracting `fast` build and -fmad=false `strict` build)
+                    csrc/rtc_kernels.cu compiled four times
+                    (FMA-contracting `fast` build and -fmad=false `strict` build, each again with csg_sweep's call sites
+                    for scenes holding a CSG beyond csg_eval's limits)
     librtc_host.so  the C++ host mirror of the reference API + flattener (csrc/host/), linked against
                     librtc_b200.so
 
@@ -55,6 +56,9 @@ def build(force: bool = False, verbose: bool = False) -> None:
     objs = {
         os.path.join(BUILD, "kernels_fast.o"): [NVCC, *NVCC_FLAGS, "-c", kernels],
         os.path.join(BUILD, "kernels_strict.o"): [NVCC, *NVCC_FLAGS, "-DRTC_STRICT", "-fmad=false", "-c", kernels],
+        os.path.join(BUILD, "kernels_fast_sweep.o"): [NVCC, *NVCC_FLAGS, "-DRTC_CSG_SWEEP_BUILD", "-c", kernels],
+        os.path.join(BUILD, "kernels_strict_sweep.o"): [NVCC, *NVCC_FLAGS, "-DRTC_STRICT", "-fmad=false", "-DRTC_CSG_SWEEP_BUILD", "-c",
+                                                        kernels],
         os.path.join(BUILD, "api.o"): [NVCC, *NVCC_FLAGS, "-c", api],
         os.path.join(BUILD, "commit.o"): [NVCC, *NVCC_FLAGS, "-c", commit],
         os.path.join(BUILD, "lbvh.o"): [NVCC, *NVCC_FLAGS, "-c", lbvh],
@@ -67,7 +71,7 @@ def build(force: bool = False, verbose: bool = False) -> None:
     if jobs:
         if verbose:
             print(f"compiling {len(jobs)} CUDA translation unit(s) for sm_100a ...", flush=True)
-        with ThreadPoolExecutor(max_workers=5) as pool:
+        with ThreadPoolExecutor(max_workers=7) as pool:
             list(pool.map(_run, jobs))
     if force or jobs or _newer(LIB_DEVICE, list(objs)):
         _run([NVCC, "-gencode", "arch=compute_100a,code=sm_100a", "-shared", "-o", LIB_DEVICE, *objs, "-cudart", "shared"])

@@ -153,6 +153,214 @@ __device__ __noinline__ int csg_eval(const DevScene& S, int pc, V3 wo, V3 wd, fl
     return n;
 }
 
+// ---------------------------------------------------------------------------------------------------
+// csg_sweep's call sites are compiled into the kernel builds for scenes that hold a CSG marked for it
+// (RTC_CSG_SWEEP_BUILD, rtc_kernels.cu) and into host builds of this code; every other kernel build is exactly the
+// csg_eval-only code, so the sweep costs the scenes that do not use it no registers.
+#if defined(RTC_CSG_SWEEP_BUILD) || !defined(__CUDA_ARCH__)
+constexpr bool kWithCsgSweep = true;
+#else
+constexpr bool kWithCsgSweep = false;
+#endif
+
+// csg_sweep: the same filtered hit list as csg_eval, in the same order, delivered one hit at a time in memory that does
+// not depend on the size of the tree (CSGs beyond csg_eval's limits, marked at commit: rtc_types.h, DevCsgOp::pad).
+//
+// Order.  csg.rs:101 stable-sorts at every CSG and groups concatenate, so a CSG's filtered list is ordered by the key
+// (t, position of the leaf's PRIM instruction, index of the hit in the leaf's local_intersect output): key = t and
+// (PRIM position << 2 | index).  t compares as a float (-0 == +0: the tie goes to the rest of the key).
+// Pass.  Walk the program as csg_eval does (same ENTER transforms and box culls, same GROUP culls, same PRIM arithmetic)
+// and keep the kCsgSweepPass (= kCsgHitCap) smallest leaf hits whose key is above a cursor, sorted.
+// Filter by climbing.  Each buffered hit, in order, climbs its chain of CSG ancestors: at each it is tested with
+// intersection_allowed (csg.rs:63-74) against that CSG's in_s1 / in_s2, then the flag of the side it came from toggles
+// (csg.rs:37-58); it stops at the first CSG that does not allow it.  A hit that clears the root is the next output.
+// Every CSG thereby sees its operands' outputs merged in key order, which is what the stable sort gives it.
+// Repeat from the last key of the pass until the consumer stops or no hit is left.  The cursor moves strictly forward
+// (keys are distinct), so every ray ends.  A NaN distance is above no cursor: such a hit is never buffered and never
+// delivered (the reference cannot order it either: its sort panics), where csg_eval would keep it in some position.
+// Hits per pass: kCsgHitCap (a smaller figure is a test aid: every ray then takes several passes).
+#ifndef RTC_CSG_SWEEP_PASS
+#define RTC_CSG_SWEEP_PASS kCsgHitCap
+#endif
+constexpr int kCsgSweepPass = RTC_CSG_SWEEP_PASS;
+static_assert(kCsgSweepPass >= 1 && kCsgSweepPass <= kCsgHitCap, "csg_sweep: 1 .. kCsgHitCap hits per pass");
+__device__ __forceinline__ bool csg_key_less(float ta, int ka, float tb, int kb) { return ta < tb || (ta == tb && ka < kb); }
+
+// One pass: the up to kCsgSweepPass smallest leaf hits above the cursor {bt, bk}[kCsgSweepPass] into bt / bk, sorted;
+// returns the count.  ro[0] / rd[0] hold the world ray.  The world ray and the cursor are read from local memory rather
+// than held in registers through the walk: that keeps the sweep's register footprint, which every caller of
+// test_prim_other, test_small and container_csg in the sweep builds makes room for, near csg_eval's.
+template <bool STATS>
+__device__ __forceinline__ int csg_sweep_pass(const DevScene& S, int root, V3* ro, V3* rd, float* bt, int* bk, Ctr<STATS>& k) {
+    int rsp = 0, n = 0, pc = root;
+    k.prim(T_CSG);
+    const int end = S.csg_ops[root].skip;
+#pragma unroll 1
+    while (pc < end) {
+        DevCsgOp op = S.csg_ops[pc];
+        switch (op.op) {
+            case OP_CSG_ENTER: {
+                const DevNode& nd = S.nodes[op.arg];
+                Xf m{nd.inv[0], nd.inv[1], nd.inv[2]};
+                V3 o2 = xf_point(m, ro[rsp]), d2 = xf_vec(m, rd[rsp]);  // shape.rs:60-70 on the CSG itself
+                k.xform();
+                float lo, hi;
+                k.node();
+                if (!aabb_ref(o2, d2, ld3(nd.bmin), ld3(nd.bmax), lo, hi)) {  // csg.rs:90-93
+                    pc = op.skip;
+                    break;
+                }
+                rsp++;
+                ro[rsp] = o2;
+                rd[rsp] = d2;
+                pc++;
+                break;
+            }
+            case OP_CSG_MID:
+                pc++;
+                break;
+            case OP_CSG_EXIT:
+                rsp--;
+                pc++;
+                break;
+            case OP_GROUP: {
+                const DevNode& nd = S.nodes[op.arg];
+                float lo, hi;
+                k.node();
+                if (!aabb_ref(ro[rsp], rd[rsp], ld3(nd.bmin), ld3(nd.bmax), lo, hi))  // group.rs:122-125
+                    pc = op.skip;
+                else
+                    pc++;
+                break;
+            }
+            default: {  // OP_PRIM
+                int4 h = __ldg(&S.head[op.arg]);
+                Xf m = load_xf(S.xform + 3 * (size_t)h.y);
+                V3 o2 = xf_point(m, ro[rsp]), d2 = xf_vec(m, rd[rsp]);
+                k.xform();
+                float t[4];
+                int type = h.x & 15;
+                k.prim(type);
+                int c = local_intersect(S, type, h.z, load_bound(S, type, h.z), o2, d2, t);
+#pragma unroll 1
+                for (int i = 0; i < c; i++) {
+                    const float ti = t[i];
+                    const int ki = (pc << 2) | i;
+                    const float ct = *(volatile float*)&bt[kCsgSweepPass];
+                    const int ck = *(volatile int*)&bk[kCsgSweepPass];
+                    if (!csg_key_less(ct, ck, ti, ki)) continue;  // not above the cursor (or NaN)
+                    if (n == kCsgSweepPass && !csg_key_less(ti, ki, bt[n - 1], bk[n - 1])) continue;
+                    int j = n < kCsgSweepPass ? n++ : n - 1;  // a full buffer drops its largest key
+                    while (j > 0 && csg_key_less(ti, ki, bt[j - 1], bk[j - 1])) {
+                        bt[j] = bt[j - 1];
+                        bk[j] = bk[j - 1];
+                        j--;
+                    }
+                    bt[j] = ti;
+                    bk[j] = ki;
+                }
+                pc++;
+                break;
+            }
+        }
+    }
+    return n;
+}
+
+// The sweep driver.  Both consumers stop at the first output hit with t >= 0 (nearest hit: it is the answer; container
+// walk: the hits before it are the ones behind the origin), so the driver returns that hit in t_out / pos_out (pos_out
+// -1: none).  NEG: the output hits with t < 0 are compacted, in order, into bt / bk (distance, primitive position) and
+// handed to neg(bt, bk, m) after each pass's climb, so the consumer's state is not live through the climb.
+template <bool STATS, bool NEG, class Neg>
+__device__ __forceinline__ void csg_sweep(const DevScene& S, int root, V3 wo, V3 wd, Neg& neg, float& t_out, int& pos_out,
+                                          Ctr<STATS>& k) {
+    float bt[kCsgSweepPass + 1];  // [kCsgSweepPass]: the cursor
+    int bk[kCsgSweepPass + 1];
+    V3 ro[kCsgSweepDepth], rd[kCsgSweepDepth];
+    ro[0] = wo;
+    rd[0] = wd;
+    unsigned state[2 * kCsgSweepNodes / 32];  // in_s1 / in_s2 of CSG node s: bits 2 s and 2 s + 1
+    const int words = (2 * -S.csg_ops[root].pad + 31) / 32;  // the root ENTER's pad: -(CSG nodes of the program)
+#pragma unroll 1
+    for (int w = 0; w < words; w++) state[w] = 0u;
+    bt[kCsgSweepPass] = -kInfF;
+    bk[kCsgSweepPass] = -1;  // below every key: the first pass takes every hit that is not NaN
+    pos_out = -1;
+#pragma unroll 1
+    for (;;) {
+        const int n = csg_sweep_pass<STATS>(S, root, ro, rd, bt, bk, k);
+        if (n == 0) return;
+        bt[kCsgSweepPass] = bt[n - 1];  // the next pass starts above this one's last key
+        bk[kCsgSweepPass] = bk[n - 1];
+        int m = 0;
+#pragma unroll 1
+        for (int j = 0; j < n && pos_out < 0; j++) {
+            const DevCsgOp leaf = S.csg_ops[bk[j] >> 2];
+            int e = root + (leaf.pad >> 1);
+            bool left = leaf.pad & 1;
+#pragma unroll 1
+            for (;;) {
+                const DevCsgOp enter = S.csg_ops[e];
+                const int sidx = S.csg_ops[enter.skip - 1].pad >> 1;
+                const unsigned word = state[sidx >> 4];
+                const int shift = 2 * (sidx & 15);
+                const bool in1 = (word >> shift) & 1u, in2 = (word >> (shift + 1)) & 1u;
+                const int csg_op = S.nodes[enter.arg].op;
+                bool allowed;  // csg.rs:63-74
+                if (csg_op == 0)
+                    allowed = (left && !in2) || (!left && !in1);
+                else if (csg_op == 1)
+                    allowed = (left && in2) || (!left && in1);
+                else
+                    allowed = (left && !in2) || (!left && in1);
+                state[sidx >> 4] = word ^ (1u << (shift + (left ? 0 : 1)));
+                if (!allowed) break;
+                if (e == root) {  // an output hit
+                    if (bt[j] >= 0.0f) {
+                        t_out = bt[j];
+                        pos_out = leaf.arg;
+                    } else if (NEG) {
+                        bt[m] = bt[j];  // m <= j: the keys still to climb are untouched
+                        bk[m] = leaf.arg;
+                        m++;
+                    }
+                    break;
+                }
+                left = S.csg_ops[enter.skip - 1].pad & 1;
+                e = root + enter.pad;
+            }
+        }
+        if (NEG) neg(bt, bk, m);
+        if (pos_out >= 0 || n < kCsgSweepPass) return;
+    }
+}
+
+// csg_sweep's consumers.  Nearest hit: the first output hit with t >= 0.  Inlined into test_prim_other and test_small,
+// which costs their callers fewer registers than one more level of call.
+struct CsgSweepNoNeg {
+    __device__ __forceinline__ void operator()(const float*, const int*, int) {}
+};
+template <bool STATS>
+__device__ __forceinline__ void csg_sweep_nearest(const DevScene& S, int pc, V3 o, V3 d, Hit& best, Ctr<STATS>& k) {
+    CsgSweepNoNeg none;
+    float t;
+    int pos;
+    csg_sweep<STATS, false>(S, pc, o, d, none, t, pos, k);
+    if (pos >= 0) consider(best, t, pos, __ldg(&S.head[pos]).w);
+}
+
+// Marks a capacity overflow of csg_sweep in the render's DevCounters::overflows, in every kernel build: the render then
+// fails with RTC_ERR_CAPACITY rather than being silently wrong.  A plain store, not an atomic: any nonzero value fails
+// the render (the counters are zeroed before each one), and an atomic here costs every caller of the container walk
+// registers.
+__device__ __forceinline__ void flag_csg_overflow(const DevScene& S) {
+#ifdef __CUDA_ARCH__
+    *S.csg_overflows = 1ull;
+#else
+    if (S.csg_overflows) *S.csg_overflows = 1ull;
+#endif
+}
+
 // Test one stored primitive against the world ray for the nearest-hit search: test_prim, below, does a mesh triangle
 // itself and sends the rest here.
 // Everything but a mesh triangle: CSG trees and the analytic shapes.  Out of line: the traversal loop then holds only
@@ -162,6 +370,12 @@ __device__ __noinline__ void test_prim_other(const DevScene& S, int pos, int4 h,
     const float4* rec = S.rec + 4 * (size_t)pos;
     int type = h.x & 15;
     if (type == T_CSG) {
+        if constexpr (kWithCsgSweep) {
+            if (S.csg_ops[h.z].pad < 0) {  // marked at commit: beyond csg_eval's limits
+                csg_sweep_nearest<STATS>(S, h.z, o, d, best, k);
+                return;
+            }
+        }
         float ht[kCsgHitCap];
         int hp[kCsgHitCap];
         int n = csg_eval<STATS>(S, h.z, o, d, ht, hp, k);
@@ -316,9 +530,63 @@ __device__ __forceinline__ void container_add(Containers& c, int hit_pos, float 
         c.best_pos = pos;
     }
 }
+// container_csg's parity and last negative hit per leaf, from csg_sweep's output hits with t < 0: a plane or triangle has
+// one hit, so an output hit opens it for good and goes to container_add directly; the other leaves toggle in and out of
+// a list of the open ones, which holds their latest hit.  More than kCsgHitCap solids of one CSG open at once along the
+// backward ray is an overflow: counted, so the render fails.
+struct CsgSweepOpen {
+    const DevScene& S;
+    Containers& c;
+    int hit_pos;
+    int n = 0;
+    int pos[kCsgHitCap];
+    float last[kCsgHitCap];
+    __device__ __forceinline__ void operator()(const float* ht, const int* hp, int m) {
+#pragma unroll 1
+        for (int i = 0; i < m; i++) {
+            const int p = hp[i];
+            const int4 h = __ldg(&S.head[p]);
+            const int type = h.x & 15;
+            if (type == T_PLANE || type == T_TRIANGLE) {
+                container_add(c, hit_pos, ht[i], p, h.w);
+                continue;
+            }
+            int j = 0;
+#pragma unroll 1
+            while (j < n && pos[j] != p) j++;
+            if (j < n) {  // an even count: closed again
+                n--;
+                pos[j] = pos[n];
+                last[j] = last[n];
+            } else if (n < kCsgHitCap) {
+                pos[n] = p;
+                last[n] = ht[i];
+                n++;
+            } else {
+                flag_csg_overflow(S);
+            }
+        }
+    }
+};
+template <bool STATS>
+__device__ __noinline__ void csg_sweep_containers(const DevScene& S, int pc, V3 o, V3 d, int hit_pos, Containers& c, Ctr<STATS>& k) {
+    CsgSweepOpen open{S, c, hit_pos};
+    float t;
+    int pos;
+    csg_sweep<STATS, true>(S, pc, o, d, open, t, pos, k);
+#pragma unroll 1
+    for (int j = 0; j < open.n; j++) container_add(c, hit_pos, open.last[j], open.pos[j], __ldg(&S.head[open.pos[j]]).w);
+}
+
 // The CSG case of container_prim, out of line (one copy for both of its call sites; rarely taken).
 template <bool STATS>
 __device__ __noinline__ void container_csg(const DevScene& S, int pc, V3 o, V3 d, int hit_pos, Containers& c, Ctr<STATS>& k) {
+    if constexpr (kWithCsgSweep) {
+        if (S.csg_ops[pc].pad < 0) {  // marked at commit: beyond csg_eval's limits
+            csg_sweep_containers<STATS>(S, pc, o, d, hit_pos, c, k);
+            return;
+        }
+    }
     float ht[kCsgHitCap];
     int hp[kCsgHitCap];
     int n = csg_eval<STATS>(S, pc, o, d, ht, hp, k);

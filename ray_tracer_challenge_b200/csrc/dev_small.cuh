@@ -100,6 +100,12 @@ __device__ __noinline__ void test_small(const Env& E, int i, bool cached, V3 o, 
     const int4 head = *reinterpret_cast<const int4*>(tab + i * kSmallStride);
     const int type = head.x & 15;
     if (type == T_CSG) {
+        if constexpr (kWithCsgSweep) {
+            if (E.S.csg_ops[head.z].pad < 0) {  // marked at commit: beyond csg_eval's limits
+                csg_sweep_nearest<STATS>(E.S, head.z, o, d, best, k);
+                return;
+            }
+        }
         float ht[kCsgHitCap];
         int hp[kCsgHitCap];
         int n = csg_eval<STATS>(E.S, head.z, o, d, ht, hp, k);

@@ -179,6 +179,21 @@ struct ArenaWriter {
     }
 };
 
+// The kernel build a scene renders with: IEEE (strict) or FMA-contracted (fast), with csg_sweep's call sites when the scene
+// holds a CSG beyond csg_eval's limits (rtc_kernels.cu).
+struct KernelBuild {
+    decltype(&fast::launch_render) render;
+    decltype(&fast::launch_trace) trace;
+    decltype(&fast::launch_wave) wave;
+};
+const KernelBuild& kernel_build(bool strict_fp, bool csg_sweep) {
+    static const KernelBuild builds[4] = {{fast::launch_render, fast::launch_trace, fast::launch_wave},
+                                          {strict::launch_render, strict::launch_trace, strict::launch_wave},
+                                          {fast_sweep::launch_render, fast_sweep::launch_trace, fast_sweep::launch_wave},
+                                          {strict_sweep::launch_render, strict_sweep::launch_trace, strict_sweep::launch_wave}};
+    return builds[(strict_fp ? 1 : 0) + (csg_sweep ? 2 : 0)];
+}
+
 int upload_replica(RtcScene* s, const Flattened& f, Replica& r, int device) {
     int rc;
     if ((rc = lease_slot(device, &r.slot))) return rc;
@@ -241,6 +256,8 @@ int upload_replica(RtcScene* s, const Flattened& f, Replica& r, int device) {
     d.bvh_root = f.bvh_root;
     d.n_prims = f.n_pos;
     d.all_cast_shadow = f.all_cast_shadow;
+    d.csg_overflows = &slot->d_counters->overflows;  // reset with the counters before every render / trace
+    r.csg_sweep = f.csg_sweep;
     r.small = f.small;
     r.filter_eligible = f.small.filter_ok;
     r.cell_masks_eligible = f.small.cell_masks;
@@ -516,10 +533,7 @@ int render_impl(RtcScene* s, int depth, int shard0, int n_shards_ext, float* rgb
                 DevFrame F{slot->d_rgb, slot->d_u8, shard, n_shards, depth, b1 - b0, b0, nullptr, nullptr, 1, nullptr, 0};
                 WavePoolRaw pool{slot->d_wave_rays, slot->d_wave_nodes, slot->wave_capacity, slot->d_wave_ints,
                                  reinterpret_cast<unsigned long long*>(slot->d_wave_ints + kWaveInts) + 3 * k};
-                if (s->strict_fp)
-                    strict::launch_wave(r.scene, r.small, F, pool, slot->d_counters, slot->sm_count * 8, slot->stream);
-                else
-                    fast::launch_wave(r.scene, r.small, F, pool, slot->d_counters, slot->sm_count * 8, slot->stream);
+                kernel_build(s->strict_fp, r.csg_sweep).wave(r.scene, r.small, F, pool, slot->d_counters, slot->sm_count * 8, slot->stream);
                 CUDA_TRY(cudaGetLastError());
                 st.launches += 2 + 5 * (depth + 1) + (depth + 1);
                 r.wave_chunks = k + 1;
@@ -559,10 +573,7 @@ int render_impl(RtcScene* s, int depth, int shard0, int n_shards_ext, float* rgb
                 F.stream_blocks = slot->sm_count * 6;
                 F.tile_order = nullptr, F.tile_cost = nullptr;
             }
-            if (s->strict_fp)
-                strict::launch_render(r.scene, r.small, F, slot->d_counters, detailed, lane);
-            else
-                fast::launch_render(r.scene, r.small, F, slot->d_counters, detailed, lane);
+            kernel_build(s->strict_fp, r.csg_sweep).render(r.scene, r.small, F, slot->d_counters, detailed, lane);
             CUDA_TRY(cudaGetLastError());
             st.launches++;
             if (copy_out) {
@@ -618,10 +629,7 @@ int render_impl(RtcScene* s, int depth, int shard0, int n_shards_ext, float* rgb
                 DevFrame F{slot->d_rgb, slot->d_u8, shard, n_shards, depth, b1 - b0, b0, nullptr, nullptr, 1, slot->d_stream_counter + (k % 64),
                            slot->sm_count * 6};
                 CUDA_TRY(cudaMemsetAsync(slot->d_stream_counter + (k % 64), 0, sizeof(unsigned), slot->stream));
-                if (s->strict_fp)
-                    strict::launch_render(rw.scene, rw.small, F, slot->d_counters, false, slot->stream);
-                else
-                    fast::launch_render(rw.scene, rw.small, F, slot->d_counters, false, slot->stream);
+                kernel_build(s->strict_fp, rw.csg_sweep).render(rw.scene, rw.small, F, slot->d_counters, false, slot->stream);
                 CUDA_TRY(cudaGetLastError());
                 st.launches++;
                 CUDA_TRY(cudaStreamSynchronize(slot->stream));  // one chunk at a time: they may share a counter slot
@@ -685,7 +693,7 @@ int render_impl(RtcScene* s, int depth, int shard0, int n_shards_ext, float* rgb
     st.total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
     if (stats) *stats = st;
     if (st.capacity_overflows)
-        return fail(RTC_ERR_CAPACITY, "CSG hit buffer overflowed " + std::to_string(st.capacity_overflows) + " times");
+        return fail(RTC_ERR_CAPACITY, "CSG evaluation overflowed its buffers " + std::to_string(st.capacity_overflows) + " times");
     return 0;
 }
 
@@ -989,16 +997,16 @@ int rtc_trace_rays(RtcScene* s, uint32_t n, const float* origins, const float* d
     CUDA_TRY(cudaMemcpyAsync(b.o, origins, b3, cudaMemcpyHostToDevice, r.stream));
     CUDA_TRY(cudaMemcpyAsync(b.d, directions, b3, cudaMemcpyHostToDevice, r.stream));
     CUDA_TRY(cudaMemsetAsync(r.d_counters, 0, sizeof(DevCounters), r.stream));
-    if (s->strict_fp)
-        strict::launch_trace(r.scene, r.small, (int)n, b.o, b.d, depth, b.rgb, b.t, b.pos, r.d_counters, r.stream);
-    else
-        fast::launch_trace(r.scene, r.small, (int)n, b.o, b.d, depth, b.rgb, b.t, b.pos, r.d_counters, r.stream);
+    kernel_build(s->strict_fp, rep.csg_sweep).trace(r.scene, r.small, (int)n, b.o, b.d, depth, b.rgb, b.t, b.pos, r.d_counters, r.stream);
     CUDA_TRY(cudaGetLastError());
     std::vector<int> pos(n);
     CUDA_TRY(cudaMemcpyAsync(out_rgb, b.rgb, b3, cudaMemcpyDeviceToHost, r.stream));
     if (out_t) CUDA_TRY(cudaMemcpyAsync(out_t, b.t, (size_t)n * sizeof(float), cudaMemcpyDeviceToHost, r.stream));
     CUDA_TRY(cudaMemcpyAsync(pos.data(), b.pos, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, r.stream));
+    unsigned long long overflows = 0;
+    CUDA_TRY(cudaMemcpyAsync(&overflows, &r.d_counters->overflows, sizeof(overflows), cudaMemcpyDeviceToHost, r.stream));
     CUDA_TRY(cudaStreamSynchronize(r.stream));
+    if (overflows) return fail(RTC_ERR_CAPACITY, "CSG evaluation overflowed its buffers " + std::to_string(overflows) + " times");
     if (out_prim)
         for (uint32_t i = 0; i < n; i++) out_prim[i] = pos[i] >= 0 ? s->pos_to_prim[pos[i]] : -1;
     return 0;

@@ -6,6 +6,7 @@
 #include <chrono>
 #include <cmath>
 #include <cstdio>
+#include <cstdlib>
 #include <cstring>
 #include <future>
 #include <map>
@@ -901,7 +902,7 @@ int flatten(RtcScene* s, Flattened& f, TreeBuilderFn tree_builder, void* tree_bu
         RtcScene* s;
         Flattened& f;
         std::vector<int>& prim_pos;
-        int worst_hits = 0, max_depth = 0;
+        int max_depth = 0;  // CSG nesting of the program being emitted
         int emit(int ref, int csg_depth) {  // returns worst-case hit count of the subtree
             if (ref >= 0) {
                 f.ops.push_back(DevCsgOp{OP_PRIM, prim_pos[ref], 0, 0});
@@ -925,25 +926,62 @@ int flatten(RtcScene* s, Flattened& f, TreeBuilderFn tree_builder, void* tree_bu
                 f.ops.push_back(DevCsgOp{OP_CSG_EXIT, node, 0, 0});
                 f.ops[idx].skip = (int)f.ops.size();
             }
-            worst_hits = std::max(worst_hits, total);
             return total;
         }
     } emitter{s, f, prim_pos};
+    // The links csg_sweep climbs (rtc_types.h: DevCsgOp::pad) for the program [start, f.ops.size()); returns its CSG nodes.
+    auto link_for_sweep = [&f](int start) {
+        struct Open {
+            int enter;
+            bool left;
+        };
+        std::vector<Open> open;
+        int n_csg = 0;
+        for (int pc = start; pc < (int)f.ops.size(); pc++) {
+            DevCsgOp& op = f.ops[pc];
+            if (op.op == OP_CSG_ENTER) {
+                if (!open.empty()) op.pad = open.back().enter - start;
+                f.ops[op.skip - 1].pad = (n_csg++ << 1) | (!open.empty() && open.back().left ? 1 : 0);
+                open.push_back(Open{pc, true});
+            } else if (op.op == OP_CSG_MID) {
+                open.back().left = false;
+            } else if (op.op == OP_CSG_EXIT) {
+                open.pop_back();
+            } else if (op.op == OP_PRIM) {
+                op.pad = ((open.back().enter - start) << 1) | (open.back().left ? 1 : 0);
+            }
+        }
+        f.ops[start].pad = -n_csg;
+        return n_csg;
+    };
+    // RTC_CSG_SWEEP=1 (test aid, read on every commit): every CSG goes to csg_sweep, so that scenes csg_eval accepts can
+    // be rendered both ways and compared.
+    const char* sweep_env = getenv("RTC_CSG_SWEEP");
+    const bool sweep_all = sweep_env && atoi(sweep_env) != 0;
     for (int i = 0; i < nn; i++) {
         if (csg_pos[i] < 0) continue;
         int start = (int)f.ops.size();
-        emitter.emit(~i, 0);
+        emitter.max_depth = 0;
+        const int worst = emitter.emit(~i, 0);
+        if (sweep_all || worst > kCsgHitCap || emitter.max_depth > kCsgRayDepth - 1) {
+            // beyond csg_eval's hit buffer or ray stack: the same program, evaluated by csg_sweep
+            if (emitter.max_depth > kCsgSweepDepth - 1)
+                return fail(RTC_ERR_CAPACITY, "CSG nesting depth " + std::to_string(emitter.max_depth) + " exceeds " +
+                                                  std::to_string(kCsgSweepDepth - 1));
+            const int n_csg = link_for_sweep(start);
+            f.csg_sweep = true;
+            if (n_csg > kCsgSweepNodes)
+                return fail(RTC_ERR_CAPACITY, "a CSG holds " + std::to_string(n_csg) + " CSG nodes; at most " +
+                                                  std::to_string(kCsgSweepNodes) + " are supported");
+        }
         int pos = csg_pos[i];
         // order: depth-first index of the CSG's first leaf (ties are resolved with the leaves' own orders)
         f.head[pos] = make_int4(T_CSG | (kFlagCastsShadow << 4), 0, start, 0);
         f.head[f.n_pos + pos] = make_int4(s->nodes[i].parent, -1, 0, 0);
     }
-    if (emitter.worst_hits > kCsgHitCap)
-        return fail(RTC_ERR_CAPACITY, "a CSG subtree can produce " + std::to_string(emitter.worst_hits) +
-                                          " intersections on one ray; the device hit buffer holds " + std::to_string(kCsgHitCap));
-    if (emitter.max_depth > kCsgRayDepth - 1)
-        return fail(RTC_ERR_CAPACITY, "CSG nesting depth " + std::to_string(emitter.max_depth) + " exceeds " + std::to_string(kCsgRayDepth - 1));
 
+    if (f.ops.size() >= (1u << 29))  // csg_sweep's keys hold a PRIM instruction's position << 2
+        return fail(RTC_ERR_CAPACITY, "CSG programs exceed 2^29 instructions");
     lap("nodes + csg programs");
     // ---- traversal records: head + the rows the intersection test needs, one 64 B fetch per primitive
     f.rec.resize(4 * (size_t)f.n_pos);

@@ -91,6 +91,7 @@ struct Replica {
     SmallScene small{};
     int cell_masks_eligible = 0, plane_cells_eligible = 0;
     int filter_eligible = 0;  // SmallScene::filter_ok as computed at commit (RTC_OPT_SHADOW_FILTER masks it per render)
+    bool csg_sweep = false;   // Flattened::csg_sweep
     // Longest-first launch order learnt from the previous render of the same shard (see render_impl)
     int order_shard = -1, order_n_shards = -1, order_depth = -1, order_filter = -1;  // what d_tile_order was learnt for
     // The learnt order is kept only if it wins a timed trial: after the render that records the costs, one more in
@@ -129,6 +130,7 @@ struct Flattened {
     int bvh_root = -1;
     int n_pos = 0;
     int all_cast_shadow = 1;
+    bool csg_sweep = false;  // some CSG is evaluated by csg_sweep: the scene renders with the *_sweep kernel builds
 };
 
 }  // namespace rtc

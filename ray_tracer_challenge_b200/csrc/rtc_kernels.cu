@@ -7,8 +7,14 @@
 //                   RGB canvas and the 8-bit canvas (canvas.rs:39-43) in the same pass.
 // K4 trace_rays   : World::color_at for caller-supplied rays (the unit-test probe).
 // K5 fma_peak     : dependent-FMA micro-benchmark for the measured FP32 roofline denominator.
-#ifdef RTC_STRICT
+// Each is compiled once more with -DRTC_CSG_SWEEP_BUILD, as `fast_sweep` / `strict_sweep`: the builds that evaluate CSGs
+// beyond csg_eval's limits with csg_sweep (dev_bvh.cuh), used only for scenes that hold one.
+#if defined(RTC_STRICT) && defined(RTC_CSG_SWEEP_BUILD)
+#define RTC_NS strict_sweep
+#elif defined(RTC_STRICT)
 #define RTC_NS strict
+#elif defined(RTC_CSG_SWEEP_BUILD)
+#define RTC_NS fast_sweep
 #else
 #define RTC_NS fast
 #endif
@@ -295,7 +301,7 @@ void launch_trace(const DevScene& S, const SmallScene& SS, int n, const float* o
         trace_rays<false, false><<<(n + kBlockThreads - 1) / kBlockThreads, kBlockThreads, 0, stream>>>(S, SS, n, origins, directions, depth, out_rgb, out_t, out_pos, counters);
 }
 
-#ifndef RTC_STRICT
+#if !defined(RTC_STRICT) && !defined(RTC_CSG_SWEEP_BUILD)
 // K5: 8 independent FMA chains per thread, 4096 iterations: 2 * 8 * 4096 flops per thread.
 __global__ void __launch_bounds__(256) fma_peak(float* out, float a, float b, int iters) {
     float x0 = threadIdx.x, x1 = x0 + 1.f, x2 = x0 + 2.f, x3 = x0 + 3.f, x4 = x0 + 4.f, x5 = x0 + 5.f, x6 = x0 + 6.f, x7 = x0 + 7.f;

@@ -1,4 +1,4 @@
-// rtc_launch.h — host-callable launchers of the two kernel builds (see rtc_kernels.cu).
+// rtc_launch.h — host-callable launchers of the kernel builds (see rtc_kernels.cu).
 #pragma once
 #include <cuda_runtime.h>
 
@@ -24,4 +24,21 @@ void launch_trace(const DevScene& S, const SmallScene& SS, int n, const float* o
 void launch_wave(const DevScene& S, const SmallScene& SS, const DevFrame& F, const WavePoolRaw& pool, DevCounters* counters, int blocks,
                  cudaStream_t stream);
 }  // namespace strict
+// the same two builds with csg_sweep's call sites (scenes holding a CSG beyond csg_eval's limits)
+namespace fast_sweep {
+void launch_render(const DevScene& S, const SmallScene& SS, const DevFrame& F, DevCounters* counters, bool detailed,
+                   cudaStream_t stream);
+void launch_trace(const DevScene& S, const SmallScene& SS, int n, const float* origins, const float* directions, int depth,
+                  float* out_rgb, float* out_t, int* out_pos, DevCounters* counters, cudaStream_t stream);
+void launch_wave(const DevScene& S, const SmallScene& SS, const DevFrame& F, const WavePoolRaw& pool, DevCounters* counters, int blocks,
+                 cudaStream_t stream);
+}  // namespace fast_sweep
+namespace strict_sweep {
+void launch_render(const DevScene& S, const SmallScene& SS, const DevFrame& F, DevCounters* counters, bool detailed,
+                   cudaStream_t stream);
+void launch_trace(const DevScene& S, const SmallScene& SS, int n, const float* origins, const float* directions, int depth,
+                  float* out_rgb, float* out_t, int* out_pos, DevCounters* counters, cudaStream_t stream);
+void launch_wave(const DevScene& S, const SmallScene& SS, const DevFrame& F, const WavePoolRaw& pool, DevCounters* counters, int blocks,
+                 cudaStream_t stream);
+}  // namespace strict_sweep
 }  // namespace rtc

@@ -31,8 +31,13 @@ enum : int { T_SPHERE = 0, T_PLANE = 1, T_CUBE = 2, T_CYLINDER = 3, T_CONE = 4, 
 constexpr int kFlagCastsShadow = 1;   // BaseShape::casts_shadow
 constexpr int kFlagHasParent = 2;     // has an enclosing group / CSG whose cull must be honoured exactly
 constexpr int kMaxFrames = 24;        // explicit reflect/refract stack: depth + 1 frames (depth <= 23)
-constexpr int kCsgHitCap = 32;        // hits a CSG evaluation may hold at once
-constexpr int kCsgRayDepth = 6;       // nested CSG transforms
+// A CSG whose worst case stays within kCsgHitCap leaf hits and kCsgRayDepth - 1 nesting levels is evaluated whole by
+// csg_eval (dev_bvh.cuh); any other is marked at commit and evaluated by csg_sweep, whose memory does not depend on the
+// hit count: it holds kCsgHitCap hits at a time and needs nesting <= kCsgSweepDepth - 1 and <= kCsgSweepNodes CSG nodes.
+constexpr int kCsgHitCap = 32;        // csg_eval: leaf hits held at once; csg_sweep: hits per pass, open solids per CSG
+constexpr int kCsgRayDepth = 6;       // csg_eval: nested CSG transforms
+constexpr int kCsgSweepDepth = 64;    // csg_sweep: nested CSG transforms
+constexpr int kCsgSweepNodes = 1024;  // csg_sweep: CSG nodes of one outermost CSG (2 state bits each)
 constexpr int kBvhStack = 48;  // traversal stack entries per thread: one deferred child per level (the builder bounds the depth)
 
 struct DevMaterial {  // 48 B
@@ -62,13 +67,17 @@ struct DevNode {  // group / CSG node of the reference shape tree (cull chain + 
     int kind, parent, op, pad;
 };
 
-// One instruction of a flattened CSG tree (post-order), see csg_eval in dev_bvh.cuh.
+// One instruction of a flattened CSG tree (post-order), see csg_eval and csg_sweep in dev_bvh.cuh.
 enum : int { OP_CSG_ENTER = 0, OP_CSG_MID = 1, OP_CSG_EXIT = 2, OP_GROUP = 3, OP_PRIM = 4 };
 struct DevCsgOp {
     int op;    // OP_*
     int arg;   // node index (ENTER/MID/EXIT/GROUP) or primitive position (PRIM)
     int skip;  // ENTER/GROUP: instruction to jump to when the bounding-box cull rejects the ray
-    int pad;
+    int pad;   // 0, except in a program evaluated by csg_sweep (offsets are from the root ENTER):
+               //   root ENTER  -(number of CSG nodes in the program): < 0 marks the program for csg_sweep
+               //   ENTER       offset of the parent CSG's ENTER
+               //   EXIT        state index << 1 | 1 when the CSG is in its parent's left operand (s1)
+               //   PRIM        offset of the innermost enclosing CSG's ENTER << 1 | 1 when in its left operand
 };
 
 struct DevBvhNode {  // 64 B
@@ -115,6 +124,7 @@ struct DevScene {
     const DevUvPattern* uvs;
     const float4* texels;  // image textures, one float4 {r, g, b, 0} per pixel, all canvases back to back
     int all_cast_shadow;  // every primitive casts a shadow: shadow rays may stop at the first hit
+    unsigned long long* csg_overflows;  // DevCounters::overflows of the render: csg_sweep flags an overflow here in every build
 };
 
 // Small scenes (every BASELINE demo scene: 4..13 primitives) skip the tree: their primitives travel in the

@@ -531,6 +531,102 @@ def csg_gallery(rt, width=320, height=200):
     return camera, world
 
 
+def _union_chain(rt, shapes):
+    """CSG(union, CSG(union, ..., a), b): one more nesting level per shape after the second."""
+    out = shapes[0]
+    for s in shapes[1:]:
+        out = rt.CSG(CSG_UNION, out, s)
+    return out
+
+
+def csg_die(rt, width=320, height=200, glassy=False, area_light=False, surrounded=False):
+    """The book's chapter-16 die: a rounded cube (cube ∩ sphere) minus 21 pip spheres, a worst case of 46 hits per ray.
+    Faces 1-3's pips are a union chain (the die nests 7 CSG levels deep), faces 4-6's pips sit in a group.
+    `surrounded` adds 20 marbles, which puts the die in a tree scene rather than a small one."""
+    if glassy:
+        body = Material(color=(0.1, 0.1, 0.15), transparency=1.0, refractive_index=REFRACTION_GLASS, diffuse=0.1, ambient=0.05,
+                        reflective=0.9, shininess=300.0)
+    else:
+        body = Material(color=(0.95, 0.93, 0.85), specular=0.4, shininess=80.0, reflective=0.05)
+    pip_mat = Material(color=(0.1, 0.1, 0.12), specular=0.2) if not glassy else \
+        Material(color=(0.6, 0.1, 0.1), transparency=0.6, refractive_index=1.2, diffuse=0.4, reflective=0.3)
+    rounded = rt.CSG(CSG_INTERSECTION, rt.Cube.build(rt.identity_4x4(), body),
+                     rt.Sphere.build(rt.scaling(1.45, 1.45, 1.45), body))
+    grid = {1: [(0, 0)], 2: [(-1, -1), (1, 1)], 3: [(-1, -1), (0, 0), (1, 1)], 4: [(-1, -1), (-1, 1), (1, -1), (1, 1)],
+            5: [(-1, -1), (-1, 1), (0, 0), (1, -1), (1, 1)], 6: [(-1, -1), (-1, 0), (-1, 1), (1, -1), (1, 0), (1, 1)]}
+    # face -> (axis, sign); opposite faces add up to 7
+    faces = {1: (2, -1.0), 6: (2, 1.0), 2: (0, 1.0), 5: (0, -1.0), 3: (1, 1.0), 4: (1, -1.0)}
+
+    def pips(face):
+        axis, sign = faces[face]
+        out = []
+        for a, b in grid[face]:
+            c = [0.0, 0.0, 0.0]
+            c[axis] = sign * 1.05
+            c[(axis + 1) % 3], c[(axis + 2) % 3] = 0.5 * a, 0.5 * b
+            out.append(rt.Sphere.build(rt.translation(*c) * rt.scaling(0.2, 0.2, 0.2), pip_mat))
+        return out
+
+    holes = rt.GroupShape()
+    holes.add_child(_union_chain(rt, pips(1) + pips(2) + pips(3)))
+    for face in (4, 5, 6):
+        for p in pips(face):
+            holes.add_child(p)
+    die = rt.CSG(CSG_DIFFERENCE, rounded, holes)
+    die.set_transformation(rt.translation(0.0, 1.0, 0.0) * rt.rotation_y(0.6) * rt.rotation_x(-0.25))
+    floor = rt.Plane.build(rt.identity_4x4(), Material(pattern=rt.Checkers((0.8, 0.8, 0.8), (0.3, 0.35, 0.3)), specular=0.0,
+                                                       reflective=0.1))
+    objects = [floor, die]
+    if surrounded:
+        for i in range(20):
+            a = 2 * math.pi * i / 20
+            objects.append(rt.Sphere.build(rt.translation(3.0 * math.cos(a), 0.3, 3.0 * math.sin(a) + 1.0) * rt.scaling(0.3, 0.3, 0.3),
+                                           Material(color=(0.2 + 0.04 * i, 0.5, 0.9 - 0.04 * i), reflective=0.2)))
+    if area_light:
+        light = RectangleLight((1.2, 1.2, 1.2), (-5.0, 7.0, -6.0), (2.0, 0, 0), 3, (0, 0, 2.0), 3, jitter_table(18))
+    else:
+        light = PointLight((-5.0, 8.0, -7.0), (1, 1, 1))
+    camera = rt.Camera(width, height, PI / 3.0, rt.view_transform((1.0, 3.5, -5.5), (0, 0.9, 0), (0, 1, 0)))
+    return camera, rt.World(objects, light)
+
+
+def csg_carved_mesh(rt, width=320, height=200, n_u=24, n_v=12):
+    """The divided synthetic_obj mesh minus a cylinder (one leaf per triangle: the worst case grows with the mesh), with a
+    glass sphere in front of it."""
+    mesh = rt.parse_obj(synthetic_obj(n_u, n_v))
+    mesh.set_material(Material(color=(0.9, 0.5, 0.2), specular=0.3, shininess=20.0))
+    mesh.divide(4)
+    drill = rt.Cylinder()
+    drill.minimum_y, drill.maximum_y, drill.closed = -3.0, 3.0, True
+    drill.set_transformation(rt.translation(0.8, 0.0, 0.0) * rt.scaling(0.9, 1.0, 0.9))
+    drill.set_material(Material(color=(0.2, 0.6, 0.9)))
+    carved = rt.CSG(CSG_DIFFERENCE, mesh, drill)
+    carved.set_transformation(rt.translation(0.0, 1.5, 0.0) * rt.rotation_x(0.4) * rt.scaling(0.8, 0.8, 0.8))
+    marble = rt.Sphere.build(rt.translation(-0.8, 0.6, -2.2) * rt.scaling(0.6, 0.6, 0.6),
+                             Material(color=(0.05, 0.05, 0.05), transparency=0.9, reflective=0.9, refractive_index=REFRACTION_GLASS,
+                                      diffuse=0.1, ambient=0.05, shininess=300.0))
+    floor = rt.Plane.build(rt.translation(0.0, -0.2, 0.0), Material(pattern=rt.Checkers((0.85, 0.85, 0.85), (0.25, 0.25, 0.3)),
+                                                                    specular=0.0))
+    camera = rt.Camera(width, height, PI / 3.0, rt.view_transform((0.0, 3.0, -6.5), (0, 1.2, 0), (0, 1, 0)))
+    return camera, rt.World([floor, carved, marble], PointLight((-6.0, 9.0, -8.0), (1, 1, 1)))
+
+
+def csg_chain(rt, width=320, height=200, n=40):
+    """A glass union chain of n spheres along a helix (n - 1 nesting levels); every fifth sphere repeats the one before it,
+    so equal distances from different leaves are common."""
+    balls = []
+    for i in range(n):
+        k = i - 1 if i % 5 == 4 else i
+        a = 0.45 * k
+        balls.append(rt.Sphere.build(rt.translation(1.6 * math.cos(a), 0.5 + 0.06 * k, 1.6 * math.sin(a)) * rt.scaling(0.45, 0.45, 0.45),
+                                     Material(color=(0.1, 0.15, 0.2), transparency=0.8, reflective=0.5,
+                                              refractive_index=1.3 + 0.005 * i, diffuse=0.3, shininess=200.0)))
+    chain = _union_chain(rt, balls)
+    floor = rt.Plane.build(rt.identity_4x4(), Material(pattern=rt.Checkers((0.9, 0.9, 0.9), (0.2, 0.3, 0.2)), specular=0.0))
+    camera = rt.Camera(width, height, PI / 3.0, rt.view_transform((0.0, 4.0, -6.0), (0, 1.2, 0), (0, 1, 0)))
+    return camera, rt.World([floor, chain], PointLight((-5.0, 9.0, -6.0), (1, 1, 1)))
+
+
 def synthetic_obj(n_u=48, n_v=24, smooth=False) -> str:
     """A deterministic 'teapot-class' mesh as OBJ text: a torus knot-ish bumpy tube, n_u * n_v quads written as
     4-vertex faces (fan-triangulated by the loader into 2 * n_u * n_v triangles)."""
