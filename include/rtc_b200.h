@@ -231,6 +231,7 @@ typedef struct RtcCommitInfo {
     uint64_t digest;         /* FNV-1a over the arrays a commit would upload for intersection (primitive heads and
                               * records, transforms, triangles, bounds, tree nodes, linear list): equal digests mean
                               * the device would trace the same geometry through the same tree */
+    int32_t lean;            /* cell_masks and no pattern or transparency on the small-scene table: the lean kernel build */
 } RtcCommitInfo;
 int rtc_scene_inspect(RtcScene*, RtcCommitInfo* out);
 

@@ -61,7 +61,7 @@ class RtcCommitInfo(C.Structure):
         ("n_positions", C.c_int32), ("n_bvh_nodes", C.c_int32), ("n_linear", C.c_int32), ("n_xforms", C.c_int32),
         ("bvh_leaf_size", C.c_int32), ("small_n", C.c_int32), ("filter_ok", C.c_int32), ("cell_masks", C.c_int32),
         ("plane_cells", C.c_int32), ("converge", C.c_int32), ("tol_sphere", C.c_float), ("light_ball", C.c_float * 4),
-        ("bvh_depth", C.c_int32), ("host_ms", C.c_double), ("digest", C.c_uint64),
+        ("bvh_depth", C.c_int32), ("host_ms", C.c_double), ("digest", C.c_uint64), ("lean", C.c_int32),
     ]
 
     def as_dict(self) -> dict:

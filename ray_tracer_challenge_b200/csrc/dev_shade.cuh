@@ -2,6 +2,8 @@
 // Part of rtc_device.cuh (include that, not this): compiled once per kernel build inside namespace rtc::RTC_NS.
 #pragma once
 
+#include <type_traits>
+
 namespace rtc {
 namespace RTC_NS {
 
@@ -24,6 +26,20 @@ struct Frame {
     int flags;          // bit 0: waiting for the refraction subtree (stage 2); bit 1: a refraction ray is pending
     float transparency;
     V3 refr_o, refr_d;
+};
+// The frame of the lean build (SmallScene::lean: no transparent material), whose ray trees are reflection chains: every
+// frame waits for its reflection subtree alone and combines with the plain sum.  The path (the jitter key of a child's
+// shadow rays) is kept only where the light draws its samples.
+template <bool PATH>
+struct ReflectFrame {
+    V3 acc;
+    float reflective;
+    unsigned path;
+};
+template <>
+struct ReflectFrame<false> {
+    V3 acc;
+    float reflective;
 };
 
 // world.rs:80-85, first and second addition
@@ -111,12 +127,18 @@ struct PixelStream {
 // Without the vote the compiler's reconvergence points leave lanes that took different exits of the body running
 // their iterations one after the other (c5: 5 of 32 lanes active in the traversal code; 126 -> 64 ms with it).  Scenes
 // whose trees are chains run ~5 % faster without it.
-template <bool STATS, bool SMALL, bool CONVERGE, bool DRAWN = false, class Source = OnePixel>
+//
+// LEAN (small scenes the commit marked SmallScene::lean: no pattern, no transparency, only spheres, planes and
+// axis-aligned cubes, an area light on the cell-mask loops): patterns, the n1 / n2 walk, Schlick and refraction are
+// not compiled, and the stack holds ReflectFrames.  Same arithmetic in the same order: a frame without a refraction
+// child combines with reflectance -1, the plain sum.
+template <bool STATS, bool SMALL, bool CONVERGE, bool DRAWN = false, bool LEAN = false, class Source = OnePixel>
 __device__ __forceinline__ V3 color_at(const Env& E, bool active, V3 ro, V3 rd, int depth, unsigned pixel, Rays& r, Ctr<STATS>& k,
                                        float* out_t, int* out_pos, Source src = Source()) {
     static_assert(!Source::kStream || CONVERGE, "a pixel stream refills at the converged top of the loop");
+    static_assert(!LEAN || (SMALL && !CONVERGE), "the lean build is the chain-order small-scene build");
     const DevScene& S = E.S;
-    Frame stack[kMaxFrames];
+    std::conditional_t<LEAN, ReflectFrame<DRAWN>, Frame> stack[kMaxFrames];
     int sp = 0;
     int remaining = depth;
     unsigned path = 1u;
@@ -132,7 +154,7 @@ __device__ __forceinline__ V3 color_at(const Env& E, bool active, V3 ro, V3 rd, 
             if (!running) continue;
         }
         Hit best{kInfF, -1, 0x7fffffff};
-        find_hit<STATS, SMALL>(E, ro, rd, best, k);
+        find_hit<STATS, SMALL, LEAN>(E, ro, rd, best, k);
         if (primary) {
             if (out_t) *out_t = best.pos >= 0 ? best.t : -1.0f;
             if (out_pos) *out_pos = best.pos;
@@ -156,13 +178,13 @@ __device__ __forceinline__ V3 color_at(const Env& E, bool active, V3 ro, V3 rd, 
                 if (dot(n, -rd) < 0.0f) n = -n;
                 over_point = point + n * kAcne;
                 material_color = ld3(mat.color);
-                if (mat.pattern >= 0) {
+                if (!LEAN && mat.pattern >= 0) {
                     k.pattern();
                     material_color = pattern_color(S, mat.pattern, xf_point(m, over_point));
                 }
             }
             // ---- shade_hit (world.rs:62-86): light intensity first, then Phong (phong_lighting.rs:12-63)
-            const float li = intensity_at<STATS, SMALL, DRAWN>(E, over_point, pixel, path, r, k);
+            const float li = intensity_at<STATS, SMALL, DRAWN, LEAN>(E, over_point, pixel, path, r, k);
             const V3 eye = -rd;
             V3 light_rgb = ld3(S.light_rgb);
             V3 effective = material_color * light_rgb;
@@ -190,7 +212,7 @@ __device__ __forceinline__ V3 color_at(const Env& E, bool active, V3 ro, V3 rd, 
             bool want_refr = false;
             float reflectance = -1.0f;
             V3 refr_d = mk(0.f, 0.f, 0.f);
-            if (mat.transparency != 0.0f) {
+            if (!LEAN && mat.transparency != 0.0f) {
                 float n1, n2;
                 find_containers<STATS>(S, ro, rd, best.pos, n1, n2, k);
                 float cos_i = dot(eye, n);
@@ -226,29 +248,31 @@ __device__ __forceinline__ V3 color_at(const Env& E, bool active, V3 ro, V3 rd, 
                 }
             }
             if ((want_refl || want_refr) && sp < kMaxFrames) {
-                Frame& f = stack[sp++];
-                f.reflectance = reflectance;
-                f.path = path;
+                auto& f = stack[sp++];
+                if constexpr (!LEAN) f.reflectance = reflectance;
+                if constexpr (!LEAN || DRAWN) f.path = path;
                 r.secondary++;
                 remaining = remaining - 1;
                 V3 under_point = over_point;
-                if (want_refr) {
-                    under_point = (ro + rd * best.t) - n * kAcne;  // `point` again: the same expression, the same bits
-                    f.transparency = mat.transparency;
-                    f.refr_o = under_point;
-                    f.refr_d = refr_d;
+                if constexpr (!LEAN) {
+                    if (want_refr) {
+                        under_point = (ro + rd * best.t) - n * kAcne;  // `point` again: the same expression, the same bits
+                        f.transparency = mat.transparency;
+                        f.refr_o = under_point;
+                        f.refr_d = refr_d;
+                    }
                 }
-                if (want_refl) {
+                if (LEAN || want_refl) {
                     f.acc = surface;
                     f.reflective = mat.reflective;
-                    f.flags = want_refr ? 2 : 0;
+                    if constexpr (!LEAN) f.flags = want_refr ? 2 : 0;
                     // reflect(rd, n) (world.rs:225) is bit-for-bit the same for n and -n — every product and every sum
                     // changes sign twice — so it is evaluated here from the flipped normal instead of being kept live
                     // across the light loop
                     ro = over_point;
                     rd = reflect(rd, n);
                     path = path * 3u + 1u;
-                } else {  // no reflection: reflected_color is black (world.rs:126-128)
+                } else if constexpr (!LEAN) {  // no reflection: reflected_color is black (world.rs:126-128)
                     f.acc = add_reflected(surface, mk(0.f, 0.f, 0.f), reflectance);
                     f.flags = 1;
                     ro = under_point;
@@ -268,26 +292,35 @@ __device__ __forceinline__ V3 color_at(const Env& E, bool active, V3 ro, V3 rd, 
                 running = false;
                 break;
             }
-            Frame& f = stack[sp - 1];
-            const int flags = f.flags;
-            const float reflectance = f.reflectance;
-            if (!(flags & 1)) {                        // the reflection subtree is done
-                const V3 reflected = c * f.reflective;  // world.rs:131
-                if (flags & 2) {                        // its refraction sibling is next
-                    f.acc = add_reflected(f.acc, reflected, reflectance);
-                    f.flags = 1;
-                    ro = f.refr_o;
-                    rd = f.refr_d;
-                    remaining = depth - sp;  // the frame's ray had depth - (sp - 1)
-                    path = f.path * 3u + 2u;
-                    r.secondary++;
-                    break;
-                }
-                c = combine(f.acc, reflected, mk(0.f, 0.f, 0.f), reflectance);
+            auto& f = stack[sp - 1];
+            if constexpr (LEAN) {
+                // world.rs:131, 80-85.  The general build rounds `reflected` before the sum (a select on the frame's
+                // reflectance sits between them), so the FMA build must not fuse the two here either
+                const V3 reflected = mk(mul_rn(c.x, f.reflective), mul_rn(c.y, f.reflective), mul_rn(c.z, f.reflective));
+                c = combine(f.acc, reflected, mk(0.f, 0.f, 0.f), -1.0f);
+                sp--;
+                continue;
             } else {
-                c = add_refracted(f.acc, c * f.transparency, reflectance);  // world.rs:159-160
+                const int flags = f.flags;
+                const float reflectance = f.reflectance;
+                if (!(flags & 1)) {                        // the reflection subtree is done
+                    const V3 reflected = c * f.reflective;  // world.rs:131
+                    if (flags & 2) {                        // its refraction sibling is next
+                        f.acc = add_reflected(f.acc, reflected, reflectance);
+                        f.flags = 1;
+                        ro = f.refr_o;
+                        rd = f.refr_d;
+                        remaining = depth - sp;  // the frame's ray had depth - (sp - 1)
+                        path = f.path * 3u + 2u;
+                        r.secondary++;
+                        break;
+                    }
+                    c = combine(f.acc, reflected, mk(0.f, 0.f, 0.f), reflectance);
+                } else {
+                    c = add_refracted(f.acc, c * f.transparency, reflectance);  // world.rs:159-160
+                }
+                sp--;
             }
-            sp--;
         }
     }
     return result;

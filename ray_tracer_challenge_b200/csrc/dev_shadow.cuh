@@ -189,7 +189,7 @@ __device__ __forceinline__ int shadow_filter(const Env& E, bool cached, V3 light
 // the non-casting objects do, and otherwise only a non-casting object NEARER than the nearest caster (same
 // (t, depth-first order) comparison as Intersection::hit) can un-shadow the point.  Same predicate as the
 // reference's, evaluated with fewer intersection tests.
-template <bool STATS>
+template <bool STATS, bool LEAN>
 __device__ __forceinline__ bool shadow_exact_small(const Env& E, bool cached, V3 light_position, V3 p, Ctr<STATS>& k) {
     const DevScene& S = E.S;
     const SmallScene& SS = E.SS;
@@ -198,18 +198,18 @@ __device__ __forceinline__ bool shadow_exact_small(const Env& E, bool cached, V3
     V3 direction = div3(v, distance);
     // order -1: a hit AT the light distance is never accepted (`<`, world.rs:116)
     Hit best{distance, -1, -1};
-    if (!SS.two_pass_shadows || SS.has_cull_chain) {  // a CSG root or a cull chain: plain nearest-hit search
+    if (!LEAN && (!SS.two_pass_shadows || SS.has_cull_chain)) {  // a CSG root or a cull chain: plain nearest-hit search
 #pragma unroll 1
         for (int i = 0; i < SS.n; i++) test_small<STATS>(E, i, cached, p, direction, best, k);
         return best.pos >= 0 && ((__ldg(&S.head[best.pos]).x >> 4) & kFlagCastsShadow);
     }
     if (S.all_cast_shadow)  // every object casts: any hit in [0, distance) shadows the point
-        return scan_small<STATS, true>(E, cached, 0, SS.caster_end, p, direction, best, k);
+        return scan_small<STATS, true, LEAN>(E, cached, 0, SS.caster_end, p, direction, best, k);
     int begin = 0, caster = -1;
     int4 ends = SS.caster_end;
 #pragma unroll 1
     for (int seg = 0; seg < 2; seg++) {  // casters, then non-casters: one copy of the loops
-        scan_small<STATS, false>(E, cached, begin, ends, p, direction, best, k);
+        scan_small<STATS, false, LEAN>(E, cached, begin, ends, p, direction, best, k);
         if (seg == 0) {
             if (best.pos < 0) return false;
             caster = best.pos;
@@ -221,15 +221,17 @@ __device__ __forceinline__ bool shadow_exact_small(const Env& E, bool cached, V3
 }
 // One shadow ray of a small scene, out of line (ONE copy of the filter and of the exact test in the kernel: the
 // kernel's instruction footprint, not its arithmetic, limits the issue rate).  skip_filter: the caller already
-// knows the filter cannot decide this ray.
-template <bool STATS>
+// knows the filter cannot decide this ray.  LEAN: a lean scene is filter-eligible, holds no CSG root, cull chain or
+// "everything else" item, and its cell-mask loops never fill the origin cache.
+template <bool STATS, bool LEAN = false>
 __device__ __noinline__ bool shadow_query_small(const Env& E, bool cached, bool skip_filter, V3 light_position, V3 p, Ctr<STATS>& k) {
-    if (E.SS.filter_ok) {
+    if (LEAN) cached = false;
+    if (LEAN || E.SS.filter_ok) {
         const int f = skip_filter ? 2 : shadow_filter<STATS>(E, cached, light_position, p, k);
         if (f != 2) return f == 1;
         k.refiltered();
     }
-    return shadow_exact_small<STATS>(E, cached, light_position, p, k);
+    return shadow_exact_small<STATS, LEAN>(E, cached, light_position, p, k);
 }
 template <bool STATS, bool SMALL, bool CACHED>
 __device__ __forceinline__ bool is_shadowed(const Env& E, V3 light_position, V3 p, Rays& r, Ctr<STATS>& k) {
@@ -321,7 +323,7 @@ __device__ __forceinline__ void draw_light_samples(const DevScene& S, unsigned p
 // generator) a chunk's sample points are drawn first — two jitter values per cell in the reference's order
 // `for v { for u { j_u, j_v } }`, point_on_light's arithmetic (rectangle_light.rs:60-66) — into a per-thread array,
 // and the same loops read them from there.
-template <bool STATS, bool TABLE>
+template <bool STATS, bool TABLE, bool LEAN>
 __device__ __forceinline__ float intensity_cells(const Env& E, V3 p, unsigned pixel, unsigned path, Rays& r, Ctr<STATS>& k) {
     const DevScene& S = E.S;
     const SmallScene& SS = E.SS;
@@ -475,7 +477,7 @@ __device__ __forceinline__ float intensity_cells(const Env& E, V3 p, unsigned pi
             const int j = __ffs(todo) - 1;
             todo &= todo - 1u;
             const float4 L = smp[j];
-            lit += !shadow_query_small<STATS>(E, false, (unsure >> j) & 1u, mk(L.x, L.y, L.z), p, k);
+            lit += !shadow_query_small<STATS, LEAN>(E, false, (unsure >> j) & 1u, mk(L.x, L.y, L.z), p, k);
         }
     }
     return (float)lit / (float)cells;  // `total += 1.0` per lit cell is exact in f32
@@ -484,12 +486,13 @@ __device__ __forceinline__ float intensity_cells(const Env& E, V3 p, unsigned pi
 
 // Light::intensity_at (point_light.rs:28-34, rectangle_light.rs:76-88).  DRAWN: the kernel build for small scenes whose
 // area light draws its jitter from the counter-based generator (only that build carries intensity_cells<.., false>).
-template <bool STATS, bool SMALL, bool DRAWN>
+// LEAN: the scene's light takes the cell-mask loops (SmallScene::lean implies SmallScene::cell_masks).
+template <bool STATS, bool SMALL, bool DRAWN, bool LEAN = false>
 __device__ __forceinline__ float intensity_at(const Env& E, V3 p, unsigned pixel, unsigned path, Rays& r, Ctr<STATS>& k) {
     const DevScene& S = E.S;
-    if (!S.light_is_rect) return is_shadowed<STATS, SMALL, false>(E, ld3(S.light_pos), p, r, k) ? 0.f : 1.f;
-    if (SMALL && E.SS.cell_masks)
-        return DRAWN ? intensity_cells<STATS, false>(E, p, pixel, path, r, k) : intensity_cells<STATS, true>(E, p, pixel, path, r, k);
+    if (!LEAN && !S.light_is_rect) return is_shadowed<STATS, SMALL, false>(E, ld3(S.light_pos), p, r, k) ? 0.f : 1.f;
+    if (SMALL && (LEAN || E.SS.cell_masks))
+        return DRAWN ? intensity_cells<STATS, false, LEAN>(E, p, pixel, path, r, k) : intensity_cells<STATS, true, LEAN>(E, p, pixel, path, r, k);
     if (SMALL) cache_origins(E, p);
     const unsigned key = S.jitter_len > 0 ? 0u : jitter_key(S.seed, pixel, path);
     float total = 0.f;

@@ -37,16 +37,28 @@ __device__ __forceinline__ const float4* small_samples() {  // table-mode light 
     return rtc_smem + kSmemSamples;
 }
 // A block's staging: three coalesced copies out of the scene's image (L2 / L1 resident after the first blocks), each
-// started by a different warp so that no warp does all of it while the others wait at the barrier.
+// started by a different warp so that no warp does all of it while the others wait at the barrier.  Every kernel that
+// stages runs blocks of kBlockThreads threads: with the block size a constant the start offsets and trip counts are
+// shifts and masks, not the integer divisions a runtime blockDim.x costs every block (the host harness of
+// tests/emu stages with one thread).
 __device__ __forceinline__ void stage_small_scene(const DevScene& S, const SmallScene& SS) {
     extern __shared__ float4 rtc_smem[];
     const float4* img = S.small_image;
-    const int t = threadIdx.x, nt = blockDim.x;
+#ifdef __CUDA_ARCH__
+    constexpr int nt = kBlockThreads;
+#else
+    const int nt = blockDim.x;
+#endif
+    const int t = threadIdx.x;
+    // at most kPlaneCellCap / kBlockThreads iterations each: not unrolled, the prologue stays short
+#pragma unroll 1
     for (int i = t; i < SS.n * kSmallStride; i += nt) rtc_smem[i] = __ldg(img + i);
     if (SS.cell_masks && S.jitter_len > 0) {
+#pragma unroll 1
         for (int i = (t + nt - 32) % nt; i < S.cells; i += nt) rtc_smem[kSmemSamples + i] = __ldg(img + kSmemSamples + i);
         if (SS.plane_cells) {
             const int n = (SS.caster_end.y - SS.caster_end.x) * S.cells;
+#pragma unroll 1
             for (int i = (t + nt - 64) % nt; i < n; i += nt) rtc_smem[kSmemPlaneCells + i] = __ldg(img + kSmemPlaneCells + i);
         }
     }
@@ -130,7 +142,8 @@ __device__ __noinline__ void test_small(const Env& E, int i, bool cached, V3 o, 
 // Nearest hit among the items [begin, ends.w) of a small scene, which are runs of spheres, planes, cubes and
 // "everything else" ending at ends.x / .y / .z / .w: one tight loop per kind, no per-item dispatch.
 // ANY: return true as soon as some item is hit in [0, best.t) (shadow rays when every object casts a shadow).
-template <bool STATS>
+// LEAN: the lean kernel build (render_tiles), for scenes the commit marked SmallScene::lean — no "everything else" run.
+template <bool STATS, bool LEAN>
 __device__ __forceinline__ bool scan_small_impl(const Env& E, bool cached, const bool any, int begin, int4 ends, V3 o, V3 d, Hit& best,
                                                 Ctr<STATS>& k) {
     const float4* tab = small_tab();
@@ -175,7 +188,7 @@ __device__ __forceinline__ bool scan_small_impl(const Env& E, bool cached, const
         consider(best, t, i, __float_as_int(tab[i * kSmallStride].w));
     }
 #pragma unroll 1
-    for (; i < ends.w; i++) {  // cylinders, cones, triangles, CSG roots
+    for (; !LEAN && i < ends.w; i++) {  // cylinders, cones, triangles, CSG roots
         if (ball_missed(tab[i * kSmallStride + 5], tab[i * kSmallStride + 4].w, o, d)) continue;
         const int before = best.pos;
         test_small<STATS>(E, i, cached, o, d, best, k);
@@ -185,14 +198,14 @@ __device__ __forceinline__ bool scan_small_impl(const Env& E, bool cached, const
 }
 #ifdef RTC_SHARED_SCAN
 // One out-of-line copy of the four loops for every caller (nearest hit, both shadow passes); `any` at run time.
-template <bool STATS>
+template <bool STATS, bool LEAN>
 __device__ __noinline__ Hit scan_small_shared(const Env& E, bool cached, bool any, int begin, int4 ends, V3 o, V3 d, Hit best, Ctr<STATS>& k) {
-    if (scan_small_impl<STATS>(E, cached, any, begin, ends, o, d, best, k)) best.pos = -2;  // any: found
+    if (scan_small_impl<STATS, LEAN>(E, cached, any, begin, ends, o, d, best, k)) best.pos = -2;  // any: found
     return best;
 }
-template <bool STATS, bool ANY>
+template <bool STATS, bool ANY, bool LEAN = false>
 __device__ __forceinline__ bool scan_small(const Env& E, bool cached, int begin, int4 ends, V3 o, V3 d, Hit& best, Ctr<STATS>& k) {
-    best = scan_small_shared<STATS>(E, cached, ANY, begin, ends, o, d, best, k);
+    best = scan_small_shared<STATS, LEAN>(E, cached, ANY, begin, ends, o, d, best, k);
     if (ANY && best.pos == -2) {
         best.pos = -1;
         return true;
@@ -200,18 +213,18 @@ __device__ __forceinline__ bool scan_small(const Env& E, bool cached, int begin,
     return false;
 }
 #else
-template <bool STATS, bool ANY>
+template <bool STATS, bool ANY, bool LEAN = false>
 __device__ __forceinline__ bool scan_small(const Env& E, bool cached, int begin, int4 ends, V3 o, V3 d, Hit& best, Ctr<STATS>& k) {
-    return scan_small_impl<STATS>(E, cached, ANY, begin, ends, o, d, best, k);
+    return scan_small_impl<STATS, LEAN>(E, cached, ANY, begin, ends, o, d, best, k);
 }
 #endif
 
 // World::intersect + Intersection::hit for the nearest hit, general (BVH) or small-scene form.
-template <bool STATS, bool SMALL>
+template <bool STATS, bool SMALL, bool LEAN = false>
 __device__ __forceinline__ void find_hit(const Env& E, V3 o, V3 d, Hit& best, Ctr<STATS>& k) {
     if (SMALL) {
         const SmallScene& SS = E.SS;
-        if (SS.has_cull_chain) {
+        if (!LEAN && SS.has_cull_chain) {
 #pragma unroll 1
             for (int i = 0; i < SS.n; i++) test_small<STATS>(E, i, false, o, d, best, k);
         } else {
@@ -219,7 +232,7 @@ __device__ __forceinline__ void find_hit(const Env& E, V3 o, V3 d, Hit& best, Ct
             int4 ends = SS.caster_end;
 #pragma unroll 1
             for (int seg = 0; seg < 2; seg++) {  // casters, then non-casters: one copy of the loops
-                scan_small<STATS, false>(E, false, begin, ends, o, d, best, k);
+                scan_small<STATS, false, LEAN>(E, false, begin, ends, o, d, best, k);
                 begin = ends.w;
                 ends = SS.other_end;
             }

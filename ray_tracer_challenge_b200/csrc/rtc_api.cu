@@ -883,7 +883,7 @@ int rtc_scene_inspect(RtcScene* s, RtcCommitInfo* out) {
     out->n_positions = f.n_pos, out->n_bvh_nodes = (int)f.bvh.size(), out->n_linear = (int)f.linear.size();
     out->n_xforms = (int)f.xform.size() / 3, out->bvh_leaf_size = f.leaf_size, out->bvh_depth = f.bvh_depth;
     out->small_n = f.small.n, out->filter_ok = f.small.filter_ok, out->cell_masks = f.small.cell_masks;
-    out->plane_cells = f.small.plane_cells, out->converge = s->has_branching_materials ? 1 : 0;
+    out->plane_cells = f.small.plane_cells, out->converge = s->has_branching_materials ? 1 : 0, out->lean = f.small.lean;
     out->tol_sphere = f.small.tol_sphere;
     out->light_ball[0] = f.small.light_ball.x, out->light_ball[1] = f.small.light_ball.y;
     out->light_ball[2] = f.small.light_ball.z, out->light_ball[3] = f.small.light_ball.w;

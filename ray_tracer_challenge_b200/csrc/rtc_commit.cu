@@ -448,6 +448,17 @@ void plan_small_scene(const RtcScene* s, Flattened& f, int n_items) {
         const bool table_light = s->light_is_rect && !f.samples.empty() && f.samples.size() <= (size_t)kSampleCap;
         const bool counter_light = s->light_is_rect && s->jitter.empty() && s->u_steps > 0 && s->v_steps > 0;
         f.small.cell_masks = ok && (table_light || counter_light);
+        // the lean kernel build (dev_shade.cuh: color_at<.., LEAN>): cell_masks already rules out CSG roots, cull chains,
+        // kinds other than spheres, planes and axis-aligned cubes, and point lights; no material of the table may have a
+        // pattern or transparency.  RTC_LEAN=0 (test aid, read on every commit) keeps such scenes on the general build,
+        // so that the two builds' frames can be compared.
+        const char* lean_env = getenv("RTC_LEAN");
+        bool lean = f.small.cell_masks && !(lean_env && atoi(lean_env) == 0);
+        for (int i = 0; i < n_items && lean; i++) {
+            const DevMaterial& m = f.materials[f.small.p[i].head.x >> 8];
+            lean = m.pattern < 0 && m.transparency == 0.0f;
+        }
+        f.small.lean = lean ? 1 : 0;
         if (f.small.cell_masks) {
             // the bundle reject (dev_shadow.cuh: bundle_misses): a ball around the light samples, and for every sphere /
             // cube its world-space bounding ball — centre = forward transform of the origin, radius = the largest

@@ -26,6 +26,9 @@
 #ifndef RTC_SMALL_MINBLOCKS
 #define RTC_SMALL_MINBLOCKS 4
 #endif
+#ifndef RTC_SMALL_LEAN_MINBLOCKS
+#define RTC_SMALL_LEAN_MINBLOCKS 6  // the lean build: 6 blocks (77 regs, no spills) beat 4 and 5 on c3 and c3_counter
+#endif
 #ifndef RTC_SMALL_CONVERGE_MINBLOCKS
 #define RTC_SMALL_CONVERGE_MINBLOCKS 3  // the converging small-scene build keeps more state live: 3 blocks (168 regs) win
 #endif
@@ -77,9 +80,11 @@ __device__ __forceinline__ void flush_counters<true>(const Rays& r, const Ctr<tr
 // the RTC_*_MINBLOCKS figures are resident blocks of 128 threads: the same warps per SM for any tile width
 constexpr int min_blocks(int of_128_threads) { return of_128_threads * 128 / kBlockThreads > 0 ? of_128_threads * 128 / kBlockThreads : 1; }
 
-template <bool STATS, bool SMALL, bool CONVERGE, bool DRAWN>
-__global__ void __launch_bounds__(kBlockThreads, min_blocks(SMALL ? (CONVERGE ? RTC_SMALL_CONVERGE_MINBLOCKS : RTC_SMALL_MINBLOCKS)
-                                                                       : (CONVERGE ? RTC_BVH_CONVERGE_MINBLOCKS : RTC_BVH_MINBLOCKS)))
+// LEAN: the build for small scenes marked SmallScene::lean (dev_shade.cuh: color_at), with its own occupancy target.
+template <bool STATS, bool SMALL, bool CONVERGE, bool DRAWN, bool LEAN = false>
+__global__ void __launch_bounds__(kBlockThreads, min_blocks(LEAN ? RTC_SMALL_LEAN_MINBLOCKS
+                                                            : SMALL ? (CONVERGE ? RTC_SMALL_CONVERGE_MINBLOCKS : RTC_SMALL_MINBLOCKS)
+                                                                    : (CONVERGE ? RTC_BVH_CONVERGE_MINBLOCKS : RTC_BVH_MINBLOCKS)))
     render_tiles(const __grid_constant__ DevScene S, const __grid_constant__ SmallScene SS,
                                                     const DevFrame F, DevCounters* counters) {
     // small scenes: primitive table + per-thread shadow-origin cache in dynamic shared memory (kSmallSmemBytes)
@@ -106,7 +111,7 @@ __global__ void __launch_bounds__(kBlockThreads, min_blocks(SMALL ? (CONVERGE ? 
     V3 o = mk(0.f, 0.f, 0.f), d = mk(0.f, 0.f, 1.f);
     if (rendered) ray_for_pixel(S, x, y, o, d);
     if (CONVERGE || rendered)
-        c = color_at<STATS, SMALL, CONVERGE, DRAWN>(E, rendered, o, d, F.depth, (unsigned)(y * S.width + x), r, k, nullptr, nullptr);
+        c = color_at<STATS, SMALL, CONVERGE, DRAWN, LEAN>(E, rendered, o, d, F.depth, (unsigned)(y * S.width + x), r, k, nullptr, nullptr);
     // Canvas::write_pixel + scale_color (canvas.rs:26-43).  A warp owns 8x4 pixels: four canvas rows of 96 B (f32) and
     // 24 B (8-bit).  When the frame's width is a multiple of 8 those row pieces are 16- / 8-byte aligned in global memory,
     // so the warp transposes its colours through shared memory and writes them as 24 STG.128 + 12 STG.64 streaming
@@ -161,7 +166,7 @@ __global__ void __launch_bounds__(kBlockThreads, min_blocks(RTC_STREAM_MINBLOCKS
     PixelStream src{S, F, F.stream_counter, (unsigned)F.n_bands * (unsigned)blocks_x * 2u * 32u, blocks_x};
     Ctr<STATS> k;
     Rays r;
-    color_at<STATS, false, true, false, PixelStream>(E, false, mk(0.f, 0.f, 0.f), mk(0.f, 0.f, 1.f), F.depth, 0u, r, k, nullptr, nullptr, src);
+    color_at<STATS, false, true, false, false, PixelStream>(E, false, mk(0.f, 0.f, 0.f), mk(0.f, 0.f, 1.f), F.depth, 0u, r, k, nullptr, nullptr, src);
     flush_counters<STATS>(r, k, counters);
 }
 
@@ -262,7 +267,19 @@ void launch_render(const DevScene& S, const SmallScene& SS, const DevFrame& F, D
     }
     // small scenes whose area light draws its samples (jitter None) need the build with the drawn-sample cell loop
     const bool drawn = small && SS.cell_masks && S.jitter_len == 0;
-    // the detailed (counting) pass always uses the converging build; the timed kernels pick by DevFrame::converge
+    // the detailed (counting) pass always uses the converging build; the timed kernels pick by DevFrame::converge.
+    // Lean scenes (SmallScene::lean, set only with cell_masks) take the lean build, which does not use the per-thread
+    // shadow-origin cache: the part of kSmallSmemBytes before it is all it stages.
+    // The *_sweep builds have no lean kernel: a scene that needs them holds a CSG, and a lean one holds none.
+#ifndef RTC_CSG_SWEEP_BUILD
+    if (!detailed && !F.converge && small && SS.cell_masks && SS.lean) {
+        if (drawn)
+            render_tiles<false, true, false, true, true><<<grid, kBlockThreads, kSmemOrg * 16, stream>>>(S, SS, F, counters);
+        else
+            render_tiles<false, true, false, false, true><<<grid, kBlockThreads, kSmemOrg * 16, stream>>>(S, SS, F, counters);
+        return;
+    }
+#endif
     if (drawn) {
         if (detailed)
             render_tiles<true, true, true, true><<<grid, kBlockThreads, kSmallSmemBytes, stream>>>(S, SS, F, counters);

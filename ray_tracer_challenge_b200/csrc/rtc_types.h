@@ -152,7 +152,7 @@ struct SmallScene {
     float tol_sphere;           // the filter's relative error bound for spheres (grows with the transforms' condition)
     int cell_masks;             // filter_ok, table-mode area light with <= kSampleCap cells: intensity_cells path
     int plane_cells;            // cell_masks and (caster planes x cells) <= kPlaneCellCap: per-(plane, cell) constants staged
-    int pad;
+    int lean;                   // cell_masks, and no material of the table has a pattern or transparency: the lean kernel build
     float4 light_ball;          // cell_masks: ball around the light samples (centre, radius) for the bundle reject
     float4 plane_bundle[2];     // cell_masks, first two caster planes: over all light cells (table) or the whole light
                                 // rectangle (generated jitter) {min r1.L, max r1.L,

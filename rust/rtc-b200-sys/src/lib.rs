@@ -167,6 +167,7 @@ pub struct RtcCommitInfo {
     pub bvh_depth: i32,
     pub host_ms: f64,
     pub digest: u64,
+    pub lean: i32,
 }
 
 extern "C" {
