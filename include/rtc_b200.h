@@ -202,6 +202,14 @@ enum {
                                   next ray when theirs ends, shading and the post-order combine in kernels of their own —
                                   instead of the streaming kernel.  Same pixels; on B200 it measures ~15 % slower (the walks
                                   are bound by dependent node loads, not by idle lanes), so it is opt-in.  Any time */
+    RTC_OPT_EXACT_GROUPS = 9,  /* default 0.  1: every bounded primitive, and every outermost CSG, inside a GroupShape reports
+                                  a hit only when each enclosing group's cached box passes the forward ray first
+                                  (group.rs:115-133), in tree scenes too; with 0 that chain is checked only for the items
+                                  tested for every ray (small scenes, unbounded shapes).  The two differ where the reference's
+                                  f32 sphere test reports phantom hits at the silhouettes of far, small spheres, and wherever
+                                  a group's box is stale (cached before a later add_child or set_transformation, group.rs:19):
+                                  then the reference clips what lies outside the old box, and only 1 reproduces that.  Other
+                                  values are RTC_ERR_INVALID.  Before commit (it changes the uploaded heads and the digest) */
     RTC_OPT_SHADOW_FILTER = 6   /* default 1: in small scenes of spheres, planes and axis-aligned cubes a shadow ray is
                                   first decided on the un-normalised point->light segment with error bounds; only
                                   undecided rays run the reference's arithmetic.  Changes no pixel (0 = always run
@@ -232,6 +240,9 @@ typedef struct RtcCommitInfo {
                               * records, transforms, triangles, bounds, tree nodes, linear list): equal digests mean
                               * the device would trace the same geometry through the same tree */
     int32_t lean;            /* cell_masks and no pattern or transparency on the small-scene table: the lean kernel build */
+    int32_t exact_groups;    /* RTC_OPT_EXACT_GROUPS as applied */
+    int32_t loose_group_boxes; /* group nodes whose cached box does not contain the box of one of their children (a stale
+                                  box): there the default culls differently from the reference on whole objects */
 } RtcCommitInfo;
 int rtc_scene_inspect(RtcScene*, RtcCommitInfo* out);
 

@@ -62,6 +62,7 @@ class RtcCommitInfo(C.Structure):
         ("bvh_leaf_size", C.c_int32), ("small_n", C.c_int32), ("filter_ok", C.c_int32), ("cell_masks", C.c_int32),
         ("plane_cells", C.c_int32), ("converge", C.c_int32), ("tol_sphere", C.c_float), ("light_ball", C.c_float * 4),
         ("bvh_depth", C.c_int32), ("host_ms", C.c_double), ("digest", C.c_uint64), ("lean", C.c_int32),
+        ("exact_groups", C.c_int32), ("loose_group_boxes", C.c_int32),
     ]
 
     def as_dict(self) -> dict:
@@ -85,6 +86,7 @@ _HOST_EXTRAS = {
     "sg_set_render_options": (_I, [_V, _I, _IP, _I, _I]),
     "sg_last_rtc_stats": (_I, [_V, C.POINTER(RtcStats)]),
     "sg_set_bvh_builder": (_I, [_V, _I]),
+    "sg_set_exact_groups": (_I, [_V, _I]),
     "sg_ppm_from_u8": (C.c_int64, [_V, _I, _I, _U8P, C.c_char_p, C.c_int64]),
     "sg_prepare": (_I, [_V, _I, _I]),
     "sg_camera_render_shard": (_I, [_V, _I, _I, _I, _I, _I, _FP, _U8P, C.POINTER(SgStats)]),
@@ -213,6 +215,11 @@ class HostApi(_api.Api):
         """RTC_OPT_BVH_BUILDER policy of this session: -1 automatic (device LBVH for one-shot renders of >= 10 000
         primitives, the host's binned SAH for prepared scenes), 0 always host, 1 always device."""
         self.check(self.lib.sg_set_bvh_builder(self.ctx, int(mode)))
+
+    def set_exact_groups(self, on: bool = True):
+        """RTC_OPT_EXACT_GROUPS for every later render, prepare and inspect of this session: grouped primitives and CSGs
+        of tree scenes honour the reference's group box culls exactly (default off)."""
+        self.check(self.lib.sg_set_exact_groups(self.ctx, 1 if on else 0))
 
     def last_rtc_stats(self) -> RtcStats:
         st = RtcStats()

@@ -18,6 +18,11 @@ __device__ __forceinline__ void consider(Hit& best, float t, int pos, int order)
     best.pos = better ? pos : best.pos;
     best.order = better ? order : best.order;
 }
+// A candidate with t >= 0 that consider() would take.  The cull-chain walk runs only for such a candidate: one that loses
+// leaves `best` as it was whether its chain passes or not.
+__device__ __forceinline__ bool would_win(const Hit& best, float t, int order) {
+    return t < best.t || (t == best.t && order < best.order);
+}
 
 // The world ray as seen by the primitive being tested; cached by transform id so that a mesh whose
 // triangles share one transform pays for one ray transform per traversal, not one per triangle.
@@ -36,6 +41,23 @@ __device__ __noinline__ bool ancestors_pass(const DevScene& S, int node, V3 o, V
         node = n.parent;
     }
     return true;
+}
+
+// The one-box certificate for a hit at distance t >= 0 of a primitive whose innermost group is `node`: true only when
+// ancestors_pass would be true.  The hit point o + t d lies inside the node's box by the margin 2^-21 (max(|mn|, |mx|) +
+// |o| + |p|) + 2^-100 on every axis, and every ancestor's box contains its child's (DevNode::pad, set at commit), so the
+// reference's aabb_intersection of each box of the chain brackets t on every axis (DESIGN.md §4, "Exact group culls: the
+// certificate's margin").  A direction component below 2^-60, an infinite bound, a non-finite point or an unmarked node
+// never certifies: the chain is then walked.
+__device__ __forceinline__ bool axis_certified(float mn, float mx, float o, float d, float t) {
+    const float p = o + t * d;
+    const float m = 4.76837158203125e-07f * (fmaxf(fabsf(mn), fabsf(mx)) + fabsf(o) + fabsf(p)) + 7.888609052210118e-31f;
+    return fabsf(d) >= 8.673617379884035e-19f && m <= 1e30f && mn + m <= p && p + m <= mx;
+}
+__device__ __forceinline__ bool chain_certified(const DevScene& S, int node, V3 o, V3 d, float t) {
+    const DevNode& n = S.nodes[node];
+    return n.pad == 1 && axis_certified(n.bmin[0], n.bmax[0], o.x, d.x, t) && axis_certified(n.bmin[1], n.bmax[1], o.y, d.y, t) &&
+           axis_certified(n.bmin[2], n.bmax[2], o.z, d.z, t);
 }
 
 // CSG::local_intersect (csg.rs:87-104) for a whole CSG subtree, flattened at commit time into a post-order
@@ -370,6 +392,8 @@ __device__ __noinline__ void test_prim_other(const DevScene& S, int pos, int4 h,
     const float4* rec = S.rec + 4 * (size_t)pos;
     int type = h.x & 15;
     if (type == T_CSG) {
+        // a CSG inside groups (RTC_OPT_EXACT_GROUPS): the enclosing groups cull before it is evaluated (group.rs:122-125)
+        if (((h.x >> 4) & kFlagHasParent) && !ancestors_pass(S, __ldg(&S.head[pos + S.n_prims]).x, o, d)) return;
         if constexpr (kWithCsgSweep) {
             if (S.csg_ops[h.z].pad < 0) {  // marked at commit: beyond csg_eval's limits
                 csg_sweep_nearest<STATS>(S, h.z, o, d, best, k);
@@ -392,7 +416,10 @@ __device__ __noinline__ void test_prim_other(const DevScene& S, int pos, int4 h,
     k.xform();
     float tn = nearest_t(S, type, h.z, load_bound(S, type, h.z), xf_point(m, o), xf_vec(m, d));
     if (!(tn >= 0.0f)) return;
-    if (((h.x >> 4) & kFlagHasParent) && !ancestors_pass(S, __ldg(&S.head[pos + S.n_prims]).x, o, d)) return;
+    if (((h.x >> 4) & kFlagHasParent) && would_win(best, tn, h.w)) {
+        const int parent = __ldg(&S.head[pos + S.n_prims]).x;
+        if (!chain_certified(S, parent, o, d, tn) && !ancestors_pass(S, parent, o, d)) return;
+    }
     consider(best, tn, pos, h.w);
 }
 
@@ -415,7 +442,10 @@ __device__ __forceinline__ void test_prim(const DevScene& S, int pos, V3 o, V3 d
     }
     float tn = nearest_t(S, T_TRIANGLE, h.z, make_float4(0.f, 0.f, 0.f, 0.f), cache.o, cache.d, rec + 1);
     if (!(tn >= 0.0f)) return;
-    if (((h.x >> 4) & kFlagHasParent) && !ancestors_pass(S, __ldg(&S.head[pos + S.n_prims]).x, o, d)) return;
+    if (((h.x >> 4) & kFlagHasParent) && would_win(best, tn, h.w)) {
+        const int parent = __ldg(&S.head[pos + S.n_prims]).x;
+        if (!chain_certified(S, parent, o, d, tn) && !ancestors_pass(S, parent, o, d)) return;
+    }
     consider(best, tn, pos, h.w);
 }
 
@@ -616,6 +646,7 @@ __device__ __forceinline__ void container_prim(const DevScene& S, int pos, V3 o,
     int4 h = __ldg(&S.head[pos]);
     int type = h.x & 15;
     if (type == T_CSG) {
+        if (((h.x >> 4) & kFlagHasParent) && !ancestors_pass(S, __ldg(&S.head[pos + S.n_prims]).x, o, d)) return;
         container_csg<STATS>(S, h.z, o, d, hit_pos, c, k);
         return;
     }

@@ -112,6 +112,7 @@ __device__ __noinline__ void test_small(const Env& E, int i, bool cached, V3 o, 
     const int4 head = *reinterpret_cast<const int4*>(tab + i * kSmallStride);
     const int type = head.x & 15;
     if (type == T_CSG) {
+        if (((head.x >> 4) & kFlagHasParent) && !ancestors_pass(E.S, head.y, o, d)) return;  // RTC_OPT_EXACT_GROUPS
         if constexpr (kWithCsgSweep) {
             if (E.S.csg_ops[head.z].pad < 0) {  // marked at commit: beyond csg_eval's limits
                 csg_sweep_nearest<STATS>(E.S, head.z, o, d, best, k);
@@ -135,7 +136,7 @@ __device__ __noinline__ void test_small(const Env& E, int i, bool cached, V3 o, 
     k.xform();
     k.prim(type);
     float tn = nearest_t(E.S, type, head.z, tab[i * kSmallStride + 4], o2, d2);
-    if (((head.x >> 4) & kFlagHasParent) && tn >= 0.0f && !ancestors_pass(E.S, head.y, o, d)) return;
+    if (((head.x >> 4) & kFlagHasParent) && tn >= 0.0f && would_win(best, tn, head.w) && !ancestors_pass(E.S, head.y, o, d)) return;
     consider(best, tn, i, head.w);
 }
 

@@ -171,6 +171,7 @@ static int commit(sg_ctx* c, RtcScene* scene, bool one_shot, size_t n_prims) {
     if (rtc_set_option(scene, RTC_OPT_FMA_CONTRACTION, o.fma ? 1 : 0)) return fail(rtc_last_error());
     const bool device_tree = o.bvh_builder < 0 ? (one_shot && n_prims >= 10000) : o.bvh_builder != 0;
     if (rtc_set_option(scene, RTC_OPT_BVH_BUILDER, device_tree ? 1 : 0)) return fail(rtc_last_error());
+    if (rtc_set_option(scene, RTC_OPT_EXACT_GROUPS, o.exact_groups ? 1 : 0)) return fail(rtc_last_error());
     const int32_t* ids = o.device_ids.empty() ? nullptr : o.device_ids.data();
     int n = o.device_ids.empty() ? o.n_devices : (int)o.device_ids.size();
     if (rtc_scene_commit(scene, n, ids)) return fail(rtc_last_error());
@@ -409,6 +410,12 @@ int sg_set_bvh_builder(sg_ctx* c, int mode) {
     c->options.bvh_builder = mode < 0 ? -1 : (mode != 0);
     return 0;
 }
+// RTC_OPT_EXACT_GROUPS (0 / 1) for every later commit of this context: one-shot renders, sg_prepare and sg_inspect
+int sg_set_exact_groups(sg_ctx* c, int on) {
+    if (on != 0 && on != 1) return fail("exact groups: 0 or 1");
+    c->options.exact_groups = on != 0;
+    return 0;
+}
 int sg_last_rtc_stats(sg_ctx* c, RtcStats* out) {
     *out = c->last_stats;
     return 0;
@@ -482,7 +489,9 @@ int sg_inspect(sg_ctx* c, int cam, int w, void* info, double* flatten_ms) {
         const auto t0 = std::chrono::steady_clock::now();
         fill_scene(scene, c->graph, c->worlds[w], c->cameras[cam], flat);
         if (flatten_ms) *flatten_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-        if (rtc_scene_inspect(scene, static_cast<RtcCommitInfo*>(info))) rc = fail(rtc_last_error());
+        if (rtc_set_option(scene, RTC_OPT_EXACT_GROUPS, c->options.exact_groups ? 1 : 0) ||
+            rtc_scene_inspect(scene, static_cast<RtcCommitInfo*>(info)))
+            rc = fail(rtc_last_error());
     } catch (const std::exception& e) {
         rc = fail(e.what());
     }

@@ -1008,6 +1008,7 @@ struct RenderOptions {
     bool fma = false;  // RTC_OPT_FMA_CONTRACTION
     bool detailed = false;
     int bvh_builder = -1;  // -1 automatic, 0 host binned SAH, 1 device LBVH (see rtc_host.cpp: commit)
+    bool exact_groups = false;  // RTC_OPT_EXACT_GROUPS
 };
 
 inline void fill_scene(RtcScene* scene, SceneGraph& g, const World& w, const Camera& cam, FlatScene& flat) {

@@ -866,6 +866,11 @@ int rtc_set_option(RtcScene* s, int32_t option, int64_t value) {
             s->bvh_min_prims = (int)std::max<int64_t>(0, value);
             s->committed = false;
             return 0;
+        case RTC_OPT_EXACT_GROUPS:
+            if (value != 0 && value != 1) return fail(RTC_ERR_INVALID, "exact groups: 0 (default) or 1");
+            s->exact_groups = (int)value;
+            s->committed = false;
+            return 0;
     }
     return fail(RTC_ERR_INVALID, "unknown option");
 }
@@ -885,6 +890,7 @@ int rtc_scene_inspect(RtcScene* s, RtcCommitInfo* out) {
     out->small_n = f.small.n, out->filter_ok = f.small.filter_ok, out->cell_masks = f.small.cell_masks;
     out->plane_cells = f.small.plane_cells, out->converge = s->has_branching_materials ? 1 : 0, out->lean = f.small.lean;
     out->tol_sphere = f.small.tol_sphere;
+    out->exact_groups = s->exact_groups, out->loose_group_boxes = f.loose_group_boxes;
     out->light_ball[0] = f.small.light_ball.x, out->light_ball[1] = f.small.light_ball.y;
     out->light_ball[2] = f.small.light_ball.z, out->light_ball[3] = f.small.light_ball.w;
     // FNV-1a over the padding-free geometry arrays (the tree's two unused link lanes are skipped)

@@ -887,8 +887,10 @@ int flatten(RtcScene* s, Flattened& f, TreeBuilderFn tree_builder, void* tree_bu
                 plain++;
             }
             int flags = p.casts_shadow ? kFlagCastsShadow : 0;
+            // the group cull chain (Q6): always for the items tested for every ray; for the tree's primitives too under
+            // RTC_OPT_EXACT_GROUPS (a CSG's own primitives never: csg_eval culls their groups exactly)
             const bool in_linear = pos >= n_tree && pos < n_items;
-            if (in_linear && p.parent >= 0) flags |= kFlagHasParent;
+            if ((in_linear || (s->exact_groups && prim_top_csg[i] < 0)) && p.parent >= 0) flags |= kFlagHasParent;
             f.head[pos] = make_int4(p.type | (flags << 4) | (p.material << 8), xf, aux, (int)i);
             f.head[f.n_pos + pos] = make_int4(prim_top_csg[i] < 0 ? p.parent : -1, (int)i, 0, 0);
             s->pos_to_prim[pos] = (int)i;
@@ -906,6 +908,47 @@ int flatten(RtcScene* s, Flattened& f, TreeBuilderFn tree_builder, void* tree_bu
         d.parent = n.parent;
         d.op = n.op;
         d.pad = 0;
+    }
+    // ---- loose group boxes: a group whose cached box does not contain a child's parent-space box (exact f32 compare; a
+    // NaN bound counts as loose).  The reference caches a group's box on first use and never invalidates it
+    // (group.rs:19), so a later add_child or set_transformation leaves it culling with the old box.
+    {
+        std::atomic<int> loose{0};
+        parallel_for((size_t)nn, 4096, [&](size_t b, size_t e, int) {
+            int count = 0;
+            for (size_t i = b; i < e; i++) {
+                const RtcNode& n = s->nodes[i];
+                if (n.kind != RTC_NODE_GROUP) continue;
+                bool contains = true;
+                for (int c = 0; c < n.child_count && contains; c++) {
+                    const int r = s->refs[n.child_begin + c];
+                    const float* lo = r >= 0 ? s->prims[r].bbox_min : s->nodes[~r].world_bbox_min;
+                    const float* hi = r >= 0 ? s->prims[r].bbox_max : s->nodes[~r].world_bbox_max;
+                    for (int a = 0; a < 3; a++) contains = contains && n.bbox_min[a] <= lo[a] && hi[a] <= n.bbox_max[a];
+                }
+                count += !contains;
+            }
+            loose += count;
+        });
+        f.loose_group_boxes = loose.load();
+        // RTC_OPT_EXACT_GROUPS: DevNode::pad = 1 marks a group whose chain is nested: every box on the way up contains the
+        // box below it (the boxes the culls use, exact f32 compare), so a hit point inside this group's box by the rounding
+        // margin passes every box of the chain (dev_bvh.cuh: chain_certified).  A stale box breaks the chains through it.
+        // RTC_EXACT_GROUPS_CERT=0 (test and timing aid, read on every commit) leaves every node unmarked: every chain walks.
+        const char* cert_env = getenv("RTC_EXACT_GROUPS_CERT");
+        if (s->exact_groups && !(cert_env && atoi(cert_env) == 0))
+            parallel_for((size_t)nn, 4096, [&](size_t b, size_t e, int) {
+                for (size_t i = b; i < e; i++) {
+                    if (s->nodes[i].kind != RTC_NODE_GROUP) continue;
+                    bool ok = true;
+                    for (int c = (int)i, a = s->nodes[i].parent; a >= 0 && ok; c = a, a = s->nodes[a].parent) {
+                        const RtcNode &in = s->nodes[c], &out = s->nodes[a];
+                        ok = out.kind == RTC_NODE_GROUP;
+                        for (int k = 0; k < 3; k++) ok = ok && out.bbox_min[k] <= in.bbox_min[k] && in.bbox_max[k] <= out.bbox_max[k];
+                    }
+                    f.nodes[i].pad = ok ? 1 : 0;
+                }
+            });
     }
 
     // ---- CSG programs
@@ -987,7 +1030,9 @@ int flatten(RtcScene* s, Flattened& f, TreeBuilderFn tree_builder, void* tree_bu
         }
         int pos = csg_pos[i];
         // order: depth-first index of the CSG's first leaf (ties are resolved with the leaves' own orders)
-        f.head[pos] = make_int4(T_CSG | (kFlagCastsShadow << 4), 0, start, 0);
+        // RTC_OPT_EXACT_GROUPS: a CSG inside a group is evaluated only when its chain of group boxes passes
+        const int csg_flags = kFlagCastsShadow | (s->exact_groups && s->nodes[i].parent >= 0 ? kFlagHasParent : 0);
+        f.head[pos] = make_int4(T_CSG | (csg_flags << 4), 0, start, 0);
         f.head[f.n_pos + pos] = make_int4(s->nodes[i].parent, -1, 0, 0);
     }
 

@@ -131,6 +131,7 @@ struct Flattened {
     int n_pos = 0;
     int all_cast_shadow = 1;
     bool csg_sweep = false;  // some CSG is evaluated by csg_sweep: the scene renders with the *_sweep kernel builds
+    int loose_group_boxes = 0;  // group nodes whose cached box does not contain some child's box (RtcCommitInfo)
 };
 
 }  // namespace rtc
@@ -159,6 +160,7 @@ struct RtcScene {
     int strict_fp = 1, leaf_size = 0 /* automatic */, bvh_min_prims = rtc::kSmallCap + 1;
     int bvh_builder = 0;       // RTC_OPT_BVH_BUILDER: 0 host binned SAH, 1 device LBVH (scenes of >= kLbvhMinItems bounded items)
     int built_on_device = 0;   // the last commit's tree came from the device builder
+    int exact_groups = 0;      // RTC_OPT_EXACT_GROUPS: grouped tree primitives and CSG roots carry the cull chain too
     int render_slices = 24;  // kernel / copy pipeline depth when rendering into host memory
     int adaptive_order = 1;  // launch a shard's bands longest-first, learnt from the previous render
     int shadow_filter = 1;   // RTC_OPT_SHADOW_FILTER

@@ -50,6 +50,7 @@ pub const RTC_OPT_ADAPTIVE_ORDER: i32 = 5;
 pub const RTC_OPT_SHADOW_FILTER: i32 = 6;
 pub const RTC_OPT_BVH_BUILDER: i32 = 7;
 pub const RTC_OPT_WAVEFRONT: i32 = 8;
+pub const RTC_OPT_EXACT_GROUPS: i32 = 9;
 
 #[repr(C)]
 #[derive(Clone, Copy)]
@@ -168,6 +169,8 @@ pub struct RtcCommitInfo {
     pub host_ms: f64,
     pub digest: u64,
     pub lean: i32,
+    pub exact_groups: i32,
+    pub loose_group_boxes: i32,
 }
 
 extern "C" {
