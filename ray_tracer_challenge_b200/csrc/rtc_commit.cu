@@ -730,7 +730,8 @@ int flatten(RtcScene* s, Flattened& f, TreeBuilderFn tree_builder, void* tree_bu
             while ((1u << builder.par_depth) < hw && builder.par_depth < 5) builder.par_depth++;  // up to 32 subtree tasks
             f.bvh.reserve(build_items.size());
             root = builder.build(0, (int)build_items.size(), 0);
-            f.bvh_depth = builder.max_depth + 1;
+            // max_depth is the most inner nodes above a leaf; a tree that is one leaf gets the wrapping node below
+            f.bvh_depth = std::max(builder.max_depth, 1);
         }
         if (f.bvh_depth > kBvhStack - 1)  // cannot happen (Builder::build balances before the cap); never silent if it does
             return fail(RTC_ERR_CAPACITY, "BVH depth " + std::to_string(f.bvh_depth) + " exceeds the traversal stack (" +
