@@ -177,14 +177,18 @@ __device__ __forceinline__ V3 color_at(const Env& E, bool active, V3 ro, V3 rd, 
                 n = norm(xf_normal(m, local_normal(S, h.x & 15, h.z, object_point)));  // shape.rs:148-154,130-145
                 if (dot(n, -rd) < 0.0f) n = -n;
                 over_point = point + n * kAcne;
-                material_color = ld3(mat.color);
-                if (!LEAN && mat.pattern >= 0) {
-                    k.pattern();
-                    material_color = pattern_color(S, mat.pattern, xf_point(m, over_point));
+                if constexpr (!LEAN) {
+                    material_color = ld3(mat.color);
+                    if (mat.pattern >= 0) {
+                        k.pattern();
+                        material_color = pattern_color(S, mat.pattern, xf_point(m, over_point));
+                    }
                 }
             }
             // ---- shade_hit (world.rs:62-86): light intensity first, then Phong (phong_lighting.rs:12-63)
             const float li = intensity_at<STATS, SMALL, DRAWN, LEAN>(E, over_point, pixel, path, r, k);
+            // without patterns the colour is loaded after the light loop instead of held in registers across it
+            if constexpr (LEAN) material_color = ld3(mat.color);
             const V3 eye = -rd;
             V3 light_rgb = ld3(S.light_rgb);
             V3 effective = material_color * light_rgb;

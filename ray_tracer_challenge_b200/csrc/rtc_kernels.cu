@@ -27,7 +27,7 @@
 #define RTC_SMALL_MINBLOCKS 4
 #endif
 #ifndef RTC_SMALL_LEAN_MINBLOCKS
-#define RTC_SMALL_LEAN_MINBLOCKS 6  // the lean build: 6 blocks (77 regs, no spills) beat 4 and 5 on c3 and c3_counter
+#define RTC_SMALL_LEAN_MINBLOCKS 8  // the lean build: 8 blocks (64 regs, 36 / 8 B spill) beat 7 on c3_counter, 6 on both
 #endif
 #ifndef RTC_SMALL_CONVERGE_MINBLOCKS
 #define RTC_SMALL_CONVERGE_MINBLOCKS 3  // the converging small-scene build keeps more state live: 3 blocks (168 regs) win
@@ -80,7 +80,22 @@ __device__ __forceinline__ void flush_counters<true>(const Rays& r, const Ctr<tr
 // the RTC_*_MINBLOCKS figures are resident blocks of 128 threads: the same warps per SM for any tile width
 constexpr int min_blocks(int of_128_threads) { return of_128_threads * 128 / kBlockThreads > 0 ? of_128_threads * 128 / kBlockThreads : 1; }
 
+// Block -> tile of 16x8 pixels: natural order = (tile column bx, band `shard + by * n_shards`), or the learnt
+// longest-first list.
+__device__ __forceinline__ void tile_of(const DevFrame& F, int& band, int& bx) {
+    band = F.shard + (F.band_begin + blockIdx.y) * F.n_shards, bx = blockIdx.x;
+    if (F.tile_order) {
+        const int id = F.tile_order[blockIdx.y * gridDim.x + blockIdx.x];
+        band = id / (int)gridDim.x;
+        bx = id - band * (int)gridDim.x;
+    }
+}
+
 // LEAN: the build for small scenes marked SmallScene::lean (dev_shade.cuh: color_at), with its own occupancy target.
+// It holds nothing of the epilogue across color_at — the tile coordinates are evaluated again after it (one more
+// tile_order load per thread) and the tile-cost probe's start is one shared word per warp — which lets it run more
+// resident blocks.  The other builds keep both in registers: the same change made c4 1 % and c2 0.5 % slower
+// (profiles/README.md).
 template <bool STATS, bool SMALL, bool CONVERGE, bool DRAWN, bool LEAN = false>
 __global__ void __launch_bounds__(kBlockThreads, min_blocks(LEAN ? RTC_SMALL_LEAN_MINBLOCKS
                                                             : SMALL ? (CONVERGE ? RTC_SMALL_CONVERGE_MINBLOCKS : RTC_SMALL_MINBLOCKS)
@@ -90,28 +105,31 @@ __global__ void __launch_bounds__(kBlockThreads, min_blocks(LEAN ? RTC_SMALL_LEA
     // small scenes: primitive table + per-thread shadow-origin cache in dynamic shared memory (kSmallSmemBytes)
     if (SMALL) stage_small_scene(S, SS);
     const Env E{S, SS};
-    // block -> tile of 16x8 pixels: natural order = (tile column bx, band `shard + by * n_shards`), or the learnt
-    // longest-first list; warp w -> 8x4 sub-tile
-    const long long t_start = F.tile_cost ? clock64() : 0;
+    const long long t_start = !LEAN && F.tile_cost ? clock64() : 0;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    int band = F.shard + (F.band_begin + blockIdx.y) * F.n_shards, bx = blockIdx.x;
-    if (F.tile_order) {
-        const int id = F.tile_order[blockIdx.y * gridDim.x + blockIdx.x];
-        band = id / (int)gridDim.x;
-        bx = id - band * (int)gridDim.x;
-    }
-    const int x = bx * kTileW + (warp % kWarpsX) * 8 + (lane & 7);
-    const int y = band * kBandRows + (warp / kWarpsX) * 4 + (lane >> 3);
+    __shared__ long long s_t_start[LEAN ? kBlockThreads / 32 : 1];
+    if (LEAN && F.tile_cost && lane == 0) s_t_start[warp] = clock64();
+    // warp w -> 8x4 sub-tile
+    int band, bx;
+    tile_of(F, band, bx);
+    int x = bx * kTileW + (warp % kWarpsX) * 8 + (lane & 7);
+    int y = band * kBandRows + (warp / kWarpsX) * 4 + (lane >> 3);
     Ctr<STATS> k;
     Rays r;
     V3 c = mk(0.f, 0.f, 0.f);
-    const bool inside = x < S.width && y < S.height;
+    bool inside = x < S.width && y < S.height;
     // camera.rs:80-81 — the last row and the last column are never rendered and stay black (canvas.rs:23)
     const bool rendered = inside && x < S.width - 1 && y < S.height - 1;
     V3 o = mk(0.f, 0.f, 0.f), d = mk(0.f, 0.f, 1.f);
     if (rendered) ray_for_pixel(S, x, y, o, d);
     if (CONVERGE || rendered)
         c = color_at<STATS, SMALL, CONVERGE, DRAWN, LEAN>(E, rendered, o, d, F.depth, (unsigned)(y * S.width + x), r, k, nullptr, nullptr);
+    if (LEAN) {
+        tile_of(F, band, bx);
+        x = bx * kTileW + (warp % kWarpsX) * 8 + (lane & 7);
+        y = band * kBandRows + (warp / kWarpsX) * 4 + (lane >> 3);
+        inside = x < S.width && y < S.height;
+    }
     // Canvas::write_pixel + scale_color (canvas.rs:26-43).  A warp owns 8x4 pixels: four canvas rows of 96 B (f32) and
     // 24 B (8-bit).  When the frame's width is a multiple of 8 those row pieces are 16- / 8-byte aligned in global memory,
     // so the warp transposes its colours through shared memory and writes them as 24 STG.128 + 12 STG.64 streaming
@@ -150,7 +168,7 @@ __global__ void __launch_bounds__(kBlockThreads, min_blocks(LEAN ? RTC_SMALL_LEA
     }
     flush_counters<STATS>(r, k, counters);
     if (F.tile_cost && lane == 0)  // a block lasts as long as its slowest warp
-        atomicMax(&F.tile_cost[band * gridDim.x + bx], (unsigned)min(clock64() - t_start, 0xffffffffLL));
+        atomicMax(&F.tile_cost[band * gridDim.x + bx], (unsigned)min(clock64() - (LEAN ? s_t_start[warp] : t_start), 0xffffffffLL));
 }
 
 // K1b render_stream: Camera::render for tree scenes with branching ray trees — a persistent grid whose lanes draw
