@@ -201,7 +201,8 @@ enum {
                                   wavefront — per bounce level a queue of rays, tree walks in a kernel whose lanes draw the
                                   next ray when theirs ends, shading and the post-order combine in kernels of their own —
                                   instead of the streaming kernel.  Same pixels; on B200 it measures ~15 % slower (the walks
-                                  are bound by dependent node loads, not by idle lanes), so it is opt-in.  Any time */
+                                  are bound by dependent node loads, not by idle lanes), so it is opt-in.  Any time.
+                                  rtc_render_views does not use it: a batch takes the streaming kernel */
     RTC_OPT_EXACT_GROUPS = 9,  /* default 0.  1: every bounded primitive, and every outermost CSG, inside a GroupShape reports
                                   a hit only when each enclosing group's cached box passes the forward ray first
                                   (group.rs:115-133), in tree scenes too; with 0 that chain is checked only for the items
@@ -266,6 +267,43 @@ int rtc_render_shard(RtcScene*, int32_t depth, int32_t shard, int32_t n_shards, 
 int rtc_shard_bands(uint32_t height, int32_t shard, int32_t n_shards, uint32_t* first_rows);
 /* As rtc_render but with the detailed work counters (node visits, primitive tests, flops). */
 int rtc_render_detailed(RtcScene*, int32_t depth, float* rgb_f32, uint8_t* rgb_u8, RtcStats* stats);
+
+/* One camera view of a batch: Camera::new's derived fields (camera.rs:23-56), as rtc_set_camera takes them. */
+typedef struct RtcView {
+    float half_width, half_height, pixel_size;
+    float transform_inverse[16];
+} RtcView;
+/* Render n_views camera views of the committed scene, at the committed canvas size, in one batch: the scene stays committed,
+ * and the pixels of every view come from one launch per device (per chunk, below), not one launch per view.
+ * rgb_f32 / rgb_u8: n_views * height * width * 3 each, view-major (view v at offset v * height * width * 3); either may be
+ * NULL (NULL, NULL = leave the frames on the device: kernel timing).  Pinned and pageable destinations both work.
+ *   - View v's planes are bit-identical, in f32 and in 8 bits, to rtc_render of the scene committed with that camera, for
+ *     every kernel build and option.  With generated jitter a pixel's generator key is its index within its own view
+ *     (y * width + x), as in a single-view render.
+ *   - The arguments are checked before the scene's state, all with RTC_ERR_INVALID: n_views == 0 or views == NULL; a
+ *     non-finite field or pixel_size <= 0; a depth outside [0, 23] (rtc_render's rule).  Then an uncommitted scene is
+ *     RTC_ERR_STATE.
+ *   - Reach: a scene with a tree pads its boxes for coordinates up to the commit's reach — the largest of the bounded items'
+ *     coordinates, the light's reach and the committed camera's origin.  A view whose camera origin (the translation column
+ *     of transform_inverse) has a coordinate beyond it is refused with RTC_ERR_INVALID: commit with the farthest camera of
+ *     the batch.  Small and tree-less scenes take any finite view.
+ *   - With several committed devices each renders its interleaved bands of every view (rtc_shard_bands' rule); copies are
+ *     queued after every device has its kernels.  Copied to host memory, the batch is cut into runs of whole views by
+ *     rtc_render's slice rule applied to the whole batch (one slice per MiB copied, at most RTC_OPT_RENDER_SLICES); a view
+ *     bigger than a slice is cut by bands as rtc_render cuts a frame.  The frames live in a device arena of 2 GiB per
+ *     device (environment RTC_VIEW_ARENA_BYTES overrides it); a bigger batch is rendered chunk by chunk through it.  A
+ *     pageable destination is staged through pinned host frames of at most 256 MiB per device (one view's planes when
+ *     a view alone is bigger), kept with the device for later calls; a chunk then holds no more views than they fit.
+ *   - A tree scene whose ray trees branch renders each chunk with one persistent streaming launch, whatever
+ *     RTC_OPT_WAVEFRONT says.
+ *   - stats: primary_rays = n_views * (width - 1) * (height - 1) over the devices' shares, launches = the launches made,
+ *     kernel_ms from the first launch to the last.  With several chunks and a host destination a chunk's launches wait
+ *     for the previous chunk's copies, so kernel_ms then includes that copy time; a batch that fits one chunk, or stays
+ *     on the device, measures its kernels alone.  There is no detailed variant.
+ *   - Nothing of rtc_render's state changes: the committed camera, its frame on the device and its learnt tile order.
+ *     rtc_set_camera keeps its meaning (it invalidates the commit). */
+int rtc_render_views(RtcScene*, int32_t depth, uint32_t n_views, const RtcView* views, float* rgb_f32, uint8_t* rgb_u8,
+                     RtcStats* stats);
 /* World::color_at (world.rs:88-101) for caller-supplied rays: origins / directions are n*3 f32; out_rgb n*3;
  * out_t (optional) the hit distance or -1; out_prim (optional) the hit primitive index or -1. */
 int rtc_trace_rays(RtcScene*, uint32_t n, const float* origins, const float* directions, int32_t depth,

@@ -81,6 +81,13 @@ class RtcNode(C.Structure):
                 ("bbox_max", C.c_float * 3), ("world_bbox_min", C.c_float * 3), ("world_bbox_max", C.c_float * 3)]
 
 
+class RtcView(C.Structure):
+    """include/rtc_b200.h: RtcView — one camera of rtc_render_views (Camera::new's derived fields)"""
+
+    _fields_ = [("half_width", C.c_float), ("half_height", C.c_float), ("pixel_size", C.c_float),
+                ("transform_inverse", C.c_float * 16)]
+
+
 _V, _I, _FP, _IP, _U8P = C.c_void_p, C.c_int, _api.FP, _api.IP, _api.U8P
 _HOST_EXTRAS = {
     "sg_set_render_options": (_I, [_V, _I, _IP, _I, _I]),
@@ -98,7 +105,33 @@ _HOST_EXTRAS = {
     "sg_set_prepared_option": (_I, [_V, _I, _I, C.c_int64]),
     "sg_trace_rays": (_I, [_V, _I, C.c_uint32, _FP, _FP, _I, _I, _FP, _FP, _IP]),
     "sg_flatten": (_I, [_V, _I, _IP, C.POINTER(RtcPrim), C.POINTER(RtcNode), C.POINTER(C.c_int32), _IP]),
+    "sg_render_prepared_views": (_I, [_V, _I, _I, _I, _IP, _I, _FP, _U8P, C.POINTER(SgStats)]),
+    "sg_camera_render_views": (_I, [_V, _IP, _I, _I, _I, _FP, _U8P, C.POINTER(SgStats)]),
+    "sg_camera_view": (_I, [_V, _I, C.POINTER(RtcView)]),
+    "sg_farthest_camera": (_I, [_V, _IP, _I]),
 }
+
+
+def _handles(cameras):
+    return (C.c_int * len(cameras))(*[c.handle for c in cameras])
+
+
+def _view_planes(n, h, w, want_rgb, want_u8, out_rgb, out_u8):
+    """The (n, h, w, 3) planes of a batch: the caller's (checked) or new ones; None where not wanted."""
+    rgb = u8 = None
+    if want_rgb:
+        rgb = out_rgb if out_rgb is not None else np.zeros((n, h, w, 3), np.float32)
+        if rgb.shape != (n, h, w, 3) or rgb.dtype != np.float32 or not rgb.flags.c_contiguous:
+            raise ValueError(f"out_rgb must be a C-contiguous float32 array of shape {(n, h, w, 3)}")
+    if want_u8:
+        u8 = out_u8 if out_u8 is not None else np.zeros((n, h, w, 3), np.uint8)
+        if u8.shape != (n, h, w, 3) or u8.dtype != np.uint8 or not u8.flags.c_contiguous:
+            raise ValueError(f"out_u8 must be a C-contiguous uint8 array of shape {(n, h, w, 3)}")
+    return rgb, u8
+
+
+def _canvases(api, n, h, w, rgb, u8):
+    return [Canvas(w, h, rgb[i] if rgb is not None else None, u8[i] if u8 is not None else None, api=api) for i in range(n)]
 
 
 class PreparedScene:
@@ -126,6 +159,22 @@ class PreparedScene:
             C.byref(stats)))
         self.last_stats = api.last_rtc_stats()
         return Canvas(w, h, out_rgb if want_rgb else None, out_u8 if want_u8 else None, api=api)
+
+    def render_views(self, cameras, depth=DEFAULT_RAY_RECURSION_DEPTH, want_rgb=True, want_u8=True, out_rgb=None, out_u8=None,
+                     fma=False):
+        """rtc_render_views: every camera (of this scene's canvas size) rendered from the committed scene in one batch.
+        Returns one Canvas per camera, views into one (n, h, w, 3) array per plane; want_* = False leaves the frames on the
+        device.  In a scene with a tree a camera farther out than the committed one is refused (commit with the farthest)."""
+        cameras = list(cameras)
+        n, w, h = len(cameras), self.camera.width_pixels, self.camera.height_pixels
+        rgb, u8 = _view_planes(n, h, w, want_rgb, want_u8, out_rgb, out_u8)
+        stats = SgStats()
+        api = self.api
+        api.check(api.lib.sg_render_prepared_views(
+            api.ctx, self.handle, int(depth), n, _handles(cameras), int(fma), _api.fptr(rgb) if rgb is not None else None,
+            u8.ctypes.data_as(_U8P) if u8 is not None else None, C.byref(stats)))
+        self.last_stats = api.last_rtc_stats()
+        return _canvases(api, n, h, w, rgb, u8)
 
     def trace_rays(self, origins, directions, depth=DEFAULT_RAY_RECURSION_DEPTH, fma=False):
         """World::color_at (world.rs:88-101) for arbitrary rays: returns (rgb[n,3], t[n], shape_handle[n])."""
@@ -225,6 +274,31 @@ class HostApi(_api.Api):
         st = RtcStats()
         self.lib.sg_last_rtc_stats(self.ctx, C.byref(st))
         return st
+
+    def render_views(self, world, cameras, depth=DEFAULT_RAY_RECURSION_DEPTH, want_u8=True):
+        """The one-shot batch (Camera::render_b200 for several cameras of one canvas size): flatten the world once, commit it
+        with the camera farthest out, render every view, release.  Returns one Canvas per camera."""
+        cameras = list(cameras)
+        if not cameras:
+            raise ValueError("render_views needs at least one camera")
+        n, w, h = len(cameras), cameras[0].width_pixels, cameras[0].height_pixels
+        rgb, u8 = _view_planes(n, h, w, True, want_u8, None, None)
+        stats = SgStats()
+        self.check(self.lib.sg_camera_render_views(self.ctx, _handles(cameras), n, world.handle, int(depth), _api.fptr(rgb),
+                                                   u8.ctypes.data_as(_U8P) if u8 is not None else None, C.byref(stats)))
+        self.last_views_stats = self.last_rtc_stats()
+        return _canvases(self, n, h, w, rgb, u8)
+
+    def camera_view(self, camera) -> RtcView:
+        """The RtcView a batch hands the device library for `camera` (the fields rtc_set_camera receives for it)."""
+        v = RtcView()
+        self.check(self.lib.sg_camera_view(self.ctx, camera.handle, C.byref(v)))
+        return v
+
+    def farthest_camera(self, cameras) -> int:
+        """Index of the camera the one-shot batch commits with: the origin farthest out."""
+        cameras = list(cameras)
+        return self.check(self.lib.sg_farthest_camera(self.ctx, _handles(cameras), len(cameras)))
 
     def inspect(self, camera, world) -> dict:
         """rtc_scene_inspect: what a commit of (camera, world) would build — tree size, leaf size, small-scene path and

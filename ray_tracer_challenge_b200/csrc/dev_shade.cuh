@@ -67,6 +67,7 @@ struct OnePixel {
 
 __device__ __forceinline__ unsigned char scale_color(float c);
 __device__ __forceinline__ void ray_for_pixel(const DevScene& S, int x, int y, V3& o, V3& d);
+__device__ __forceinline__ void ray_for_pixel(const DevView& V, int x, int y, V3& o, V3& d);
 
 // Pixels of a launch in stream order: 32 consecutive indices are one 8x4 block (so a warp that refills all its lanes at
 // once gets coherent primary rays), blocks run along a band (kBandRows rows: two block rows), bands in the order of
@@ -110,6 +111,55 @@ struct PixelStream {
     }
     __device__ __forceinline__ void finish(unsigned pixel, V3 c) {  // Canvas::write_pixel + scale_color (canvas.rs:26-43)
         const size_t i = (size_t)pixel * 3;
+        if (F.rgb) F.rgb[i] = c.x, F.rgb[i + 1] = c.y, F.rgb[i + 2] = c.z;
+        if (F.u8) F.u8[i] = scale_color(c.x), F.u8[i + 1] = scale_color(c.y), F.u8[i + 2] = scale_color(c.z);
+    }
+};
+
+// The pixel stream of a batch of views (rtc_render_views): the view is the outermost term of the stream index, so the
+// pixels a warp draws in one refill lie in one view but at a view's end; view v's frame follows view v - 1's.  The
+// arithmetic of PixelStream with the view split off first (a separate type: PixelStream's code stays as it is).
+struct ViewPixelStream {
+    static constexpr bool kStream = true;
+    const DevScene& S;
+    const DevFrame& F;
+    unsigned* counter;      // next unclaimed stream index of this launch
+    unsigned total;         // stream indices of this launch
+    int blocks_x;           // 8-pixel blocks across the frame
+    const DevView* views;   // the launch's cameras
+    unsigned view_blocks;   // 8x4 blocks of one view in this launch
+    bool done = false;      // warp-uniform: the counter has run past the end
+    size_t out = 0;         // where this lane's view starts in the frame planes (elements)
+    __device__ __forceinline__ bool exhausted() const { return done; }
+    __device__ __forceinline__ bool refill(bool& running, V3& ro, V3& rd, unsigned& pixel) {
+        const unsigned idle = __ballot_sync(0xffffffffu, !running);
+        if (done || (__popc(idle) < kRefillLanes && idle != 0xffffffffu)) return false;
+        const int lane = threadIdx.x & 31, leader = __ffs(idle) - 1;
+        unsigned base = 0;
+        if (lane == leader) base = atomicAdd(counter, (unsigned)__popc(idle));
+        base = __shfl_sync(0xffffffffu, base, leader);
+        if (base + (unsigned)__popc(idle) >= total) done = true;
+        if (running) return false;
+        const unsigned idx = base + (unsigned)__popc(idle & ((1u << lane) - 1u));
+        if (idx >= total) return false;
+        const unsigned within = idx & 31u, view = (idx >> 5) / view_blocks, block = (idx >> 5) - view * view_blocks;
+        const unsigned per_band = (unsigned)blocks_x * 2u;
+        const unsigned band_i = block / per_band, b = block - band_i * per_band;
+        const int band = F.shard + (F.band_begin + (int)band_i) * F.n_shards;
+        const int x = (int)(b >> 1) * 8 + (int)(within & 7u), y = band * kBandRows + (int)(b & 1u) * 4 + (int)(within >> 3);
+        if (x >= S.width || y >= S.height) return false;
+        pixel = (unsigned)(y * S.width + x);  // within its view: the jitter generator's key, as in a single-view render
+        out = (size_t)view * ((size_t)S.width * S.height * 3);
+        if (x >= S.width - 1 || y >= S.height - 1) {  // camera.rs:80-81: never rendered, stays black (canvas.rs:23)
+            finish(pixel, mk(0.f, 0.f, 0.f));
+            return false;
+        }
+        ray_for_pixel(views[view], x, y, ro, rd);
+        running = true;
+        return true;
+    }
+    __device__ __forceinline__ void finish(unsigned pixel, V3 c) {  // Canvas::write_pixel + scale_color (canvas.rs:26-43)
+        const size_t i = out + (size_t)pixel * 3;
         if (F.rgb) F.rgb[i] = c.x, F.rgb[i + 1] = c.y, F.rgb[i + 2] = c.z;
         if (F.u8) F.u8[i] = scale_color(c.x), F.u8[i + 1] = scale_color(c.y), F.u8[i + 2] = scale_color(c.z);
     }
@@ -333,8 +383,10 @@ __device__ __forceinline__ V3 color_at(const Env& E, bool active, V3 ro, V3 rd, 
 // is_shadowed calls of a thread's shades (see Rays)
 __device__ __forceinline__ void finish_rays(const DevScene& S, Rays& r) { r.shadow = r.shades * (unsigned)(S.light_is_rect ? S.cells : 1); }
 
-// Camera::ray_for_pixel (camera.rs:60-74)
-__device__ __forceinline__ void ray_for_pixel(const DevScene& S, int x, int y, V3& o, V3& d) {
+// Camera::ray_for_pixel (camera.rs:60-74), for the committed camera (DevScene) or one view of a batch (DevView): the
+// same arithmetic in the same order
+template <class Camera>
+__device__ __forceinline__ void camera_ray(const Camera& S, int x, int y, V3& o, V3& d) {
     float x_offset = ((float)x + 0.5f) * S.pixel_size;
     float y_offset = ((float)y + 0.5f) * S.pixel_size;
     float world_x = S.half_w - x_offset;
@@ -344,6 +396,8 @@ __device__ __forceinline__ void ray_for_pixel(const DevScene& S, int x, int y, V
     o = xf_point(m, mk(0.f, 0.f, 0.f));
     d = norm(pixel - o);
 }
+__device__ __forceinline__ void ray_for_pixel(const DevScene& S, int x, int y, V3& o, V3& d) { camera_ray(S, x, y, o, d); }
+__device__ __forceinline__ void ray_for_pixel(const DevView& V, int x, int y, V3& o, V3& d) { camera_ray(V, x, y, o, d); }
 
 // Canvas::scale_color (canvas.rs:39-43): clamp, then truncate; NaN -> 255 because f32::min returns the
 // non-NaN operand (fminf does the same) and `as u8` saturates.

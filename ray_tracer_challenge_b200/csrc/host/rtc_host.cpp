@@ -126,6 +126,7 @@ int fail(const std::string& m) {
 struct Prepared {
     RtcScene* scene = nullptr;
     FlatScene flat;
+    uint32_t width = 0, height = 0;  // the committed canvas
 };
 }  // namespace
 
@@ -476,6 +477,34 @@ int sg_camera_render_shard(sg_ctx* c, int cam, int w, int depth, int shard, int 
     return camera_render(c, cam, w, depth, shard, n_shards, out_rgb, out_u8, stats);
 }
 
+// A batch of views: the cameras' RtcViews, every camera of the committed canvas size (or the call fails)
+static int camera_views(sg_ctx* c, const int* cams, int n, uint32_t width, uint32_t height, std::vector<RtcView>& out) {
+    if (n < 1 || !cams) return fail("a batch needs at least one camera");
+    out.clear();
+    for (int i = 0; i < n; i++) {
+        if (cams[i] < 0 || cams[i] >= (int)c->cameras.size()) return fail("bad camera handle");
+        const Camera& k = c->cameras[cams[i]];
+        if (k.width != width || k.height != height)
+            return fail("camera " + std::to_string(i) + " of the batch is " + std::to_string(k.width) + "x" + std::to_string(k.height) +
+                        ", the scene's canvas is " + std::to_string(width) + "x" + std::to_string(height) +
+                        ": every view of a batch has the committed canvas size");
+        out.push_back(camera_view(k));
+    }
+    return 0;
+}
+// The camera of a batch whose origin lies farthest out (largest coordinate magnitude; the first of equals): committing with
+// it gives the tree the reach every view of the batch needs (rtc_render_views)
+static int farthest_camera(const sg_ctx* c, const int* cams, int n) {
+    int best = 0;
+    float far = -1.f;
+    for (int i = 0; i < n; i++) {
+        const Mat4& m = c->cameras[cams[i]].transform_inverse;
+        const float r = std::max(std::fabs(m.m[3]), std::max(std::fabs(m.m[7]), std::fabs(m.m[11])));
+        if (r > far) far = r, best = i;
+    }
+    return best;
+}
+
 // rtc_scene_inspect for (camera, world): flatten + the host half of the commit, no device needed.  `info` is an
 // RtcCommitInfo (include/rtc_b200.h); flatten_ms receives the time of the scene-graph flattening itself.
 int sg_inspect(sg_ctx* c, int cam, int w, void* info, double* flatten_ms) {
@@ -535,6 +564,7 @@ int sg_prepare(sg_ctx* c, int cam, int w) {
         rtc_scene_destroy(p->scene);
         return -1;
     }
+    p->width = c->cameras[cam].width, p->height = c->cameras[cam].height;
     c->prepared.push_back(std::move(p));
     return (int)c->prepared.size() - 1;
 }
@@ -559,6 +589,58 @@ int sg_render_prepared(sg_ctx* c, int h, int depth, int shard, int n_shards, int
         rc = rtc_render(scene, depth, out_rgb, out_u8, &c->last_stats);
     to_sg_stats(c->last_stats, stats);
     return rc ? fail(rtc_last_error()) : 0;
+}
+// rtc_render_views on a prepared scene: n cameras (handles) of its canvas size, frames view-major in out_rgb / out_u8
+int sg_render_prepared_views(sg_ctx* c, int h, int depth, int n, const int* cams, int fma, float* out_rgb, uint8_t* out_u8,
+                             sg_stats* stats) {
+    if (h < 0 || h >= (int)c->prepared.size() || !c->prepared[h]) return fail("bad prepared handle");
+    RtcScene* scene = c->prepared[h]->scene;
+    std::vector<RtcView> views;
+    if (camera_views(c, cams, n, c->prepared[h]->width, c->prepared[h]->height, views)) return -1;
+    if (rtc_set_option(scene, RTC_OPT_FMA_CONTRACTION, fma ? 1 : 0)) return fail(rtc_last_error());
+    const int rc = rtc_render_views(scene, depth, (uint32_t)n, views.data(), out_rgb, out_u8, &c->last_stats);
+    to_sg_stats(c->last_stats, stats);
+    return rc ? fail(rtc_last_error()) : 0;
+}
+// The one-shot form (Camera::render_b200 for a batch of cameras): flatten, commit with the camera whose origin is farthest
+// out, render every view, release.  The world is consumed once and n canvases come out.
+int sg_camera_render_views(sg_ctx* c, const int* cams, int n, int w, int depth, float* out_rgb, uint8_t* out_u8, sg_stats* stats) {
+    if (n < 1 || !cams) return fail("a batch needs at least one camera");
+    for (int i = 0; i < n; i++)
+        if (cams[i] < 0 || cams[i] >= (int)c->cameras.size()) return fail("bad camera handle");
+    if (w < 0 || w >= (int)c->worlds.size()) return fail("bad world handle");
+    const Camera& first = c->cameras[cams[farthest_camera(c, cams, n)]];
+    std::vector<RtcView> views;
+    if (camera_views(c, cams, n, first.width, first.height, views)) return -1;
+    RtcScene* scene = nullptr;
+    if (rtc_scene_create(&scene)) return fail(rtc_last_error());
+    int rc = 0;
+    try {
+        const auto t0 = std::chrono::steady_clock::now();
+        FlatScene flat;
+        fill_scene(scene, c->graph, c->worlds[w], first, flat);
+        rc = commit(c, scene, true, flat.n_prims);
+        if (!rc && rtc_render_views(scene, depth, (uint32_t)n, views.data(), out_rgb, out_u8, &c->last_stats)) rc = fail(rtc_last_error());
+        c->last_stats.total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+        to_sg_stats(c->last_stats, stats);
+    } catch (const std::exception& e) {
+        rc = fail(e.what());
+    }
+    rtc_scene_destroy(scene);
+    return rc ? -1 : 0;
+}
+// What a batch hands the device library for a camera (the fields fill_scene passes to rtc_set_camera), and which camera of a
+// batch the one-shot form commits with — host arithmetic, no device
+int sg_camera_view(sg_ctx* c, int cam, RtcView* out) {
+    if (cam < 0 || cam >= (int)c->cameras.size() || !out) return fail("bad camera handle");
+    *out = camera_view(c->cameras[cam]);
+    return 0;
+}
+int sg_farthest_camera(sg_ctx* c, const int* cams, int n) {
+    if (n < 1 || !cams) return fail("a batch needs at least one camera");
+    for (int i = 0; i < n; i++)
+        if (cams[i] < 0 || cams[i] >= (int)c->cameras.size()) return fail("bad camera handle");
+    return farthest_camera(c, cams, n);
 }
 // rtc_set_option on a prepared scene (RTC_OPT_* of include/rtc_b200.h)
 int sg_set_prepared_option(sg_ctx* c, int h, int option, int64_t value) {

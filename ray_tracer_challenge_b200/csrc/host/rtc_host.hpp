@@ -1011,6 +1011,14 @@ struct RenderOptions {
     bool exact_groups = false;  // RTC_OPT_EXACT_GROUPS
 };
 
+// The camera as the device library takes it: what fill_scene hands rtc_set_camera, and one view of rtc_render_views
+inline RtcView camera_view(const Camera& cam) {
+    RtcView v;
+    v.half_width = cam.half_width, v.half_height = cam.half_height, v.pixel_size = cam.pixel_size;
+    memcpy(v.transform_inverse, cam.transform_inverse.m, sizeof(v.transform_inverse));
+    return v;
+}
+
 inline void fill_scene(RtcScene* scene, SceneGraph& g, const World& w, const Camera& cam, FlatScene& flat) {
     auto ck = [](int rc) {
         if (rc) throw Error(rtc_last_error());
@@ -1023,7 +1031,8 @@ inline void fill_scene(RtcScene* scene, SceneGraph& g, const World& w, const Cam
     if (timing)
         fprintf(stderr, "[rtc host]   %-28s %8.3f ms\n", "scene graph -> flat arrays",
                 std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count());
-    ck(rtc_set_camera(scene, cam.width, cam.height, cam.half_width, cam.half_height, cam.pixel_size, cam.transform_inverse.m));
+    const RtcView view = camera_view(cam);
+    ck(rtc_set_camera(scene, cam.width, cam.height, view.half_width, view.half_height, view.pixel_size, view.transform_inverse));
     ck(rtc_set_materials(scene, (uint32_t)flat.materials.size(), flat.materials.data()));
     ck(rtc_set_patterns(scene, (uint32_t)flat.patterns.size(), flat.patterns.data(), (uint32_t)flat.uvs.size(), flat.uvs.data()));
     ck(rtc_set_textures(scene, (uint32_t)flat.textures.size(), flat.textures.data()));

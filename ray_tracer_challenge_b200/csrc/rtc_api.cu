@@ -185,12 +185,14 @@ struct KernelBuild {
     decltype(&fast::launch_render) render;
     decltype(&fast::launch_trace) trace;
     decltype(&fast::launch_wave) wave;
+    decltype(&fast::launch_views) views;
 };
 const KernelBuild& kernel_build(bool strict_fp, bool csg_sweep) {
-    static const KernelBuild builds[4] = {{fast::launch_render, fast::launch_trace, fast::launch_wave},
-                                          {strict::launch_render, strict::launch_trace, strict::launch_wave},
-                                          {fast_sweep::launch_render, fast_sweep::launch_trace, fast_sweep::launch_wave},
-                                          {strict_sweep::launch_render, strict_sweep::launch_trace, strict_sweep::launch_wave}};
+    static const KernelBuild builds[4] = {{fast::launch_render, fast::launch_trace, fast::launch_wave, fast::launch_views},
+                                          {strict::launch_render, strict::launch_trace, strict::launch_wave, strict::launch_views},
+                                          {fast_sweep::launch_render, fast_sweep::launch_trace, fast_sweep::launch_wave, fast_sweep::launch_views},
+                                          {strict_sweep::launch_render, strict_sweep::launch_trace, strict_sweep::launch_wave,
+                                           strict_sweep::launch_views}};
     return builds[(strict_fp ? 1 : 0) + (csg_sweep ? 2 : 0)];
 }
 
@@ -350,6 +352,123 @@ int ensure_stage(DeviceSlot* d, char** stage, size_t* have, size_t bytes) {
     return 0;
 }
 
+// Device frames -> the caller's canvases, for rtc_render and rtc_render_views.  A piece is bands [b0, b1) of a shard's
+// band list in views [v0, v1) of the canvases (rtc_render: the one view 0); the device holds view v0's frame at d_rgb / d_u8
+// and the following views' frames after it.  With several devices the pieces wait in `pending` until every device has its
+// kernels: a device-to-host copy into pageable memory blocks the calling thread, and queued inside the device loop it would
+// make the devices run one after the other (ADVICE r1).  One device: a piece's copy is queued right behind its kernel.
+// A pageable destination (the reference's Canvas is a Vec): cudaMemcpyAsync into it would block the calling thread slice
+// after slice at the driver's single-threaded staging rate (~10 GB/s).  Instead the pieces land in a pinned frame kept
+// with the device slot (view v at stage index v - stage_v0), and the host's threads move each one on as soon as its copy
+// event has fired, while the device renders and copies the next (c3's 24.9 MB 8-bit canvas into a heap array: 0.71 ms
+// end to end instead of 3.07; into pinned memory 0.66).
+struct CanvasCopy {
+    struct Piece {
+        DeviceSlot* slot;
+        int shard, b0, b1, v0, v1;
+        const float* d_rgb;
+        const unsigned char* d_u8;
+    };
+    RtcScene* s;
+    int n_shards;
+    float* rgb;
+    uint8_t* u8;
+    bool stage_rgb, stage_u8;
+    int stage_views, stage_v0 = 0;  // views the pinned staging frames hold, and the first of them
+    std::vector<Piece> pending;
+    struct Unstage {
+        cudaEvent_t done;
+        Piece p;
+    };
+    std::vector<Unstage> unstage;
+    size_t unstaged = 0;
+    std::vector<int> events_used;
+    CanvasCopy(RtcScene* s_, int n_shards_, float* rgb_, uint8_t* u8_, bool stage_rgb_, bool stage_u8_, int stage_views_)
+        : s(s_), n_shards(n_shards_), rgb(rgb_), u8(u8_), stage_rgb(stage_rgb_), stage_u8(stage_u8_), stage_views(stage_views_),
+          events_used(s_->replicas.size(), 0) {}
+    size_t frame_px() const { return (size_t)s->width * s->height; }
+    int slot_index(DeviceSlot* slot) const {
+        for (size_t i = 0; i < s->replicas.size(); i++)
+            if (s->replicas[i].slot == slot) return (int)i;
+        return 0;
+    }
+    int nb(int shard) const {
+        const int total = ((int)s->height + kBandRows - 1) / kBandRows;
+        return shard < total ? (total - shard + n_shards - 1) / n_shards : 0;
+    }
+    // one plane of a piece: whole views of a one-shard frame are one contiguous copy, anything else goes band by band
+    int copy_plane(const Piece& p, const char* src, char* dst, size_t px_bytes) {
+        const size_t fb = frame_px() * px_bytes;
+        if (p.v1 - p.v0 > 1 && n_shards == 1 && p.b0 == 0 && p.b1 == nb(p.shard)) {
+            CUDA_TRY(cudaMemcpyAsync(dst, src, (size_t)(p.v1 - p.v0) * fb, cudaMemcpyDeviceToHost, p.slot->copy_stream));
+            return 0;
+        }
+        for (int v = 0; v < p.v1 - p.v0; v++)
+            if (int rc = copy_bands(p.slot, s, p.shard, n_shards, p.b0, p.b1, src + v * fb, dst + v * fb, px_bytes)) return rc;
+        return 0;
+    }
+    int copy_out(const Piece& p) {  // device frames -> canvas or staging frame
+        int rc;
+        const size_t px = frame_px();
+        DeviceSlot* slot = p.slot;
+        if (stage_rgb && (rc = ensure_stage(slot, &slot->h_stage_rgb, &slot->h_stage_rgb_bytes, px * 12 * stage_views))) return rc;
+        if (stage_u8 && (rc = ensure_stage(slot, &slot->h_stage_u8, &slot->h_stage_u8_bytes, px * 3 * stage_views))) return rc;
+        if (rgb && (rc = copy_plane(p, (const char*)p.d_rgb,
+                                    stage_rgb ? slot->h_stage_rgb + (p.v0 - stage_v0) * px * 12 : (char*)(rgb + p.v0 * px * 3), 12)))
+            return rc;
+        if (u8 && (rc = copy_plane(p, (const char*)p.d_u8,
+                                   stage_u8 ? slot->h_stage_u8 + (p.v0 - stage_v0) * px * 3 : (char*)(u8 + p.v0 * px * 3), 3)))
+            return rc;
+        if (stage_rgb || stage_u8) {
+            int& used = events_used[slot_index(slot)];
+            while ((int)slot->copy_done.size() <= used) {
+                cudaEvent_t e;
+                CUDA_TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+                slot->copy_done.push_back(e);
+            }
+            CUDA_TRY(cudaEventRecord(slot->copy_done[used], slot->copy_stream));
+            unstage.push_back({slot->copy_done[used], p});
+            used++;
+        }
+        return 0;
+    }
+    int queue(const Piece& p) {
+        if (s->replicas.size() > 1) {
+            pending.push_back(p);
+            return 0;
+        }
+        return copy_out(p);
+    }
+    int flush_pending() {  // the copy stream of each device already waits for the piece's event
+        for (const Piece& p : pending) {
+            CUDA_TRY(cudaSetDevice(p.slot->device));
+            if (int rc = copy_out(p)) return rc;
+        }
+        pending.clear();
+        return 0;
+    }
+    void host_plane(const Piece& p, const char* stage, char* dst, size_t px_bytes) {
+        const size_t fb = frame_px() * px_bytes;
+        const char* src = stage + (p.v0 - stage_v0) * fb;
+        dst += p.v0 * fb;
+        if (p.v1 - p.v0 > 1 && n_shards == 1 && p.b0 == 0 && p.b1 == nb(p.shard)) {
+            parallel_copy(dst, src, (size_t)(p.v1 - p.v0) * fb, (size_t)96 << 10);
+            return;
+        }
+        for (int v = 0; v < p.v1 - p.v0; v++) host_copy_bands(s, p.shard, n_shards, p.b0, p.b1, src + v * fb, dst + v * fb, px_bytes);
+    }
+    int drain() {  // the host half of the staged copies queued so far
+        for (; unstaged < unstage.size(); unstaged++) {
+            const Unstage& u = unstage[unstaged];
+            CUDA_TRY(cudaSetDevice(u.p.slot->device));
+            CUDA_TRY(cudaEventSynchronize(u.done));
+            if (stage_rgb) host_plane(u.p, u.p.slot->h_stage_rgb, (char*)rgb, 12);
+            if (stage_u8) host_plane(u.p, u.p.slot->h_stage_u8, (char*)u8, 3);
+        }
+        return 0;
+    }
+};
+
 // The wavefront renderer's chunking: about a million pixels of the shard at a time (whole bands).
 int wave_chunk_bands(int width, int nb) {
     const int per_band = std::max(1, width) * kBandRows;
@@ -391,73 +510,18 @@ int render_impl(RtcScene* s, int depth, int shard0, int n_shards_ext, float* rgb
     memset(&st, 0, sizeof(st));
     st.n_devices = ndev;
     st.detailed = detailed;
-    // With several devices in one process the copies are queued only after every device has all its kernels: a
-    // device-to-host copy into pageable memory blocks the calling thread, and queued inside the loop it would make the
-    // devices run one after the other (ADVICE r1).  One device: the copy of a slice is queued right behind its kernel.
-    struct PendingCopy {
-        DeviceSlot* slot;
-        int shard, b0, b1;
-    };
-    std::vector<PendingCopy> pending;
-    // A pageable destination (the reference's Canvas is a Vec): cudaMemcpyAsync into it would block the calling thread
-    // slice after slice at the driver's single-threaded staging rate (~10 GB/s).  Instead the slices land in a pinned
-    // frame kept with the device slot, and the host's threads move each one on as soon as its copy event has fired,
-    // while the device renders and copies the next (c3's 24.9 MB 8-bit canvas into a heap array: 0.71 ms end to end instead of
-    // 3.07; into pinned memory 0.66).
     // (small planes are left to the driver: waking the worker threads costs more than its pageable path loses — c1's 1.2 MB:
     // 0.28 ms through the driver, 0.40 ms staged)
     const size_t frame_px = (size_t)s->width * s->height;
     const bool stage_rgb = rgb && frame_px * 12 >= ((size_t)4 << 20) && is_pageable(rgb);
     const bool stage_u8 = u8 && frame_px * 3 >= ((size_t)4 << 20) && is_pageable(u8);
-    struct Unstage {
-        cudaEvent_t done;
-        DeviceSlot* slot;
-        int shard, b0, b1;
-    };
-    std::vector<Unstage> unstage;
-    std::vector<int> events_used(ndev, 0);
-    auto slot_index = [&](DeviceSlot* slot) {
-        for (int i = 0; i < ndev; i++)
-            if (s->replicas[i].slot == slot) return i;
-        return 0;
-    };
+    CanvasCopy cc(s, n_shards, rgb, u8, stage_rgb, stage_u8, 1);
     auto copy_out_bands = [&](DeviceSlot* slot, int shard, int b0, int b1) -> int {  // device frame -> canvas or staging frame
-        int rc;
-        const size_t px = (size_t)s->width * s->height;
-        if (stage_rgb && (rc = ensure_stage(slot, &slot->h_stage_rgb, &slot->h_stage_rgb_bytes, px * 12))) return rc;
-        if (stage_u8 && (rc = ensure_stage(slot, &slot->h_stage_u8, &slot->h_stage_u8_bytes, px * 3))) return rc;
-        if (rgb && (rc = copy_bands(slot, s, shard, n_shards, b0, b1, slot->d_rgb, stage_rgb ? (void*)slot->h_stage_rgb : (void*)rgb, 12))) return rc;
-        if (u8 && (rc = copy_bands(slot, s, shard, n_shards, b0, b1, slot->d_u8, stage_u8 ? (void*)slot->h_stage_u8 : (void*)u8, 3))) return rc;
-        if (stage_rgb || stage_u8) {
-            int& used = events_used[slot_index(slot)];
-            while ((int)slot->copy_done.size() <= used) {
-                cudaEvent_t e;
-                CUDA_TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-                slot->copy_done.push_back(e);
-            }
-            CUDA_TRY(cudaEventRecord(slot->copy_done[used], slot->copy_stream));
-            unstage.push_back({slot->copy_done[used], slot, shard, b0, b1});
-            used++;
-        }
-        return 0;
+        return cc.copy_out({slot, shard, b0, b1, 0, 1, slot->d_rgb, slot->d_u8});
     };
-    size_t unstaged = 0;
-    auto drain_unstage = [&]() -> int {  // the host half of the staged copies queued so far
-        for (; unstaged < unstage.size(); unstaged++) {
-            const Unstage& u = unstage[unstaged];
-            CUDA_TRY(cudaSetDevice(u.slot->device));
-            CUDA_TRY(cudaEventSynchronize(u.done));
-            if (stage_rgb) host_copy_bands(s, u.shard, n_shards, u.b0, u.b1, u.slot->h_stage_rgb, (char*)rgb, 12);
-            if (stage_u8) host_copy_bands(s, u.shard, n_shards, u.b0, u.b1, u.slot->h_stage_u8, (char*)u8, 3);
-        }
-        return 0;
-    };
+    auto drain_unstage = [&]() -> int { return cc.drain(); };
     auto queue_copy = [&](DeviceSlot* slot, int shard, int b0, int b1) -> int {
-        if (ndev > 1) {
-            pending.push_back({slot, shard, b0, b1});
-            return 0;
-        }
-        return copy_out_bands(slot, shard, b0, b1);
+        return cc.queue({slot, shard, b0, b1, 0, 1, slot->d_rgb, slot->d_u8});
     };
     for (int i = 0; i < ndev; i++) {
         Replica& r = s->replicas[i];
@@ -588,10 +652,7 @@ int render_impl(RtcScene* s, int depth, int shard0, int n_shards_ext, float* rgb
         CUDA_TRY(cudaEventRecord(slot->ev1, slot->stream));
         CUDA_TRY(cudaMemcpyAsync(slot->h_counters, slot->d_counters, sizeof(DevCounters), cudaMemcpyDeviceToHost, slot->stream));
     }
-    for (const PendingCopy& c : pending) {  // the copy stream of each device already waits for the slice's event
-        CUDA_TRY(cudaSetDevice(c.slot->device));
-        if (int rc = copy_out_bands(c.slot, c.shard, c.b0, c.b1)) return rc;
-    }
+    if (int rc = cc.flush_pending()) return rc;
     if (int rc = drain_unstage()) return rc;
     const bool timing = getenv("RTC_TIMING") != nullptr;  // tuning aid
     auto since = [&] { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count(); };
@@ -690,6 +751,234 @@ int render_impl(RtcScene* s, int depth, int shard0, int n_shards_ext, float* rgb
         }
     }
     st.flops = detailed ? flops_of(st, st.primary_rays) : 0.0;
+    st.total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    if (stats) *stats = st;
+    if (st.capacity_overflows)
+        return fail(RTC_ERR_CAPACITY, "CSG evaluation overflowed its buffers " + std::to_string(st.capacity_overflows) + " times");
+    return 0;
+}
+
+// rtc_render_views: the device frames of a batch live in a per-device arena of this many bytes (both planes of a chunk of
+// whole views); a bigger batch is rendered chunk by chunk through it.  RTC_VIEW_ARENA_BYTES (read at every call) lowers or
+// raises it: a test aid that forces several chunks.
+constexpr size_t kViewArenaBytes = (size_t)2 << 30;
+// ... and a pageable destination is staged through pinned host frames of at most this many bytes per device (or one view's
+// planes, when a view alone is bigger): a chunk holds no more views than its staged planes fit in.  Page-locked host memory
+// is taken from the whole system and the frames are kept with the pooled device slot, so they are bounded apart from the
+// device arena.
+constexpr size_t kViewStageBytes = (size_t)256 << 20;
+constexpr int kMaxViewsPerLaunch = 65535;  // gridDim.z
+
+int ensure_views(DeviceSlot* d, uint32_t n, size_t frame_bytes) {
+    CUDA_TRY(cudaSetDevice(d->device));
+    if (n > d->views_capacity) {
+        if (d->d_views) cudaFree(d->d_views);
+        if (d->h_views) cudaFreeHost(d->h_views);
+        d->d_views = nullptr, d->h_views = nullptr, d->views_capacity = 0;
+        const uint32_t cap = std::max<uint32_t>(n, 64);
+        CUDA_TRY(cudaMalloc(&d->d_views, cap * sizeof(DevView)));
+        CUDA_TRY(cudaHostAlloc(&d->h_views, cap * sizeof(DevView), cudaHostAllocDefault));
+        d->views_capacity = cap;
+    }
+    if (frame_bytes > d->view_frames_bytes) {
+        if (d->d_view_frames) cudaFree(d->d_view_frames);
+        d->d_view_frames = nullptr, d->view_frames_bytes = 0;
+        CUDA_TRY(cudaMalloc(&d->d_view_frames, frame_bytes));
+        d->view_frames_bytes = frame_bytes;
+    }
+    return 0;
+}
+
+int render_views_impl(RtcScene* s, int depth, uint32_t n_views, const RtcView* views, float* rgb, uint8_t* u8, RtcStats* stats) {
+    // the arguments first (no device needed), then the scene's state
+    if (!s) return fail(RTC_ERR_INVALID, "null scene");
+    if (n_views == 0 || !views) return fail(RTC_ERR_INVALID, "rtc_render_views: n_views must be >= 1 and views non-null");
+    for (uint32_t v = 0; v < n_views; v++) {
+        const RtcView& w = views[v];
+        bool finite = std::isfinite(w.half_width) && std::isfinite(w.half_height) && std::isfinite(w.pixel_size);
+        for (float x : w.transform_inverse) finite = finite && std::isfinite(x);
+        if (!finite) return fail(RTC_ERR_INVALID, "rtc_render_views: view " + std::to_string(v) + " has a non-finite field");
+        if (!(w.pixel_size > 0.f)) return fail(RTC_ERR_INVALID, "rtc_render_views: view " + std::to_string(v) + " has pixel_size <= 0");
+    }
+    if (depth < 0 || depth > kMaxFrames - 1)
+        return fail(RTC_ERR_INVALID, "reflection_recursion_depth must be in [0, " + std::to_string(kMaxFrames - 1) + "]");
+    if (!s->committed) return fail(RTC_ERR_STATE, "rtc_render_views before rtc_scene_commit");
+    // The tree's boxes are padded for ray origins up to the commit's reach (rtc_commit.cu: "pad"): a camera farther out
+    // could lose hits the reference reports.  Small and tree-less scenes test every item exactly: any view goes.
+    if (s->replicas[0].scene.bvh_root >= 0)
+        for (uint32_t v = 0; v < n_views; v++)
+            for (int a = 0; a < 3; a++) {
+                const float c = views[v].transform_inverse[a * 4 + 3];
+                if (std::fabs(c) > s->reach) {
+                    char msg[320];
+                    snprintf(msg, sizeof(msg),
+                             "rtc_render_views: view %u's camera origin has a coordinate %g beyond the scene's reach %g (the tree is "
+                             "padded for coordinates up to it); commit the scene with the farthest camera of the batch",
+                             v, (double)c, (double)s->reach);
+                    return fail(RTC_ERR_INVALID, msg);
+                }
+            }
+    auto t0 = std::chrono::steady_clock::now();
+    const int ndev = (int)s->replicas.size(), n_shards = ndev;
+    const int total_bands = ((int)s->height + kBandRows - 1) / kBandRows;
+    const bool copy_out = rgb || u8;
+    const size_t frame_px = (size_t)s->width * s->height;
+    RtcStats st;
+    memset(&st, 0, sizeof(st));
+    st.n_devices = ndev;
+    // both planes of every view of a chunk, as rtc_render's frame holds both
+    size_t budget = kViewArenaBytes;
+    if (const char* env = getenv("RTC_VIEW_ARENA_BYTES")) budget = (size_t)std::max(1LL, atoll(env));
+    const bool stream_scene = s->replicas[0].small.n == 0 && (s->stream < 0 ? s->has_branching_materials : s->stream != 0);
+    const int blocks_x = ((int)s->width + 7) / 8;
+    const int nb_max = (total_bands + n_shards - 1) / n_shards;
+    uint32_t chunk = (uint32_t)std::max<size_t>(1, std::min<size_t>(budget / (frame_px * 15), n_views));
+    chunk = std::min<uint32_t>(chunk, kMaxViewsPerLaunch);
+    if (stream_scene)  // the pixel stream's index (views x bands x 8x4 blocks x 32) is 32-bit
+        chunk = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(chunk, 0xffffffffull / ((uint64_t)nb_max * blocks_x * 64)));
+    const bool stage_rgb = rgb && frame_px * 12 * n_views >= ((size_t)4 << 20) && is_pageable(rgb);
+    const bool stage_u8 = u8 && frame_px * 3 * n_views >= ((size_t)4 << 20) && is_pageable(u8);
+    const size_t staged_per_view = frame_px * ((stage_rgb ? 12 : 0) + (stage_u8 ? 3 : 0));
+    if (staged_per_view) chunk = (uint32_t)std::max<size_t>(1, std::min<size_t>(chunk, kViewStageBytes / staged_per_view));
+    CanvasCopy cc(s, n_shards, rgb, u8, stage_rgb, stage_u8, (int)chunk);
+    static const bool rotate = [] {
+        const char* env = getenv("RTC_SLICE_STREAMS");  // tuning aid: 0 = all slices on one stream
+        return !env || atoi(env) != 0;
+    }();
+    static const int slice_shift = [] {
+        const char* env = getenv("RTC_SLICE_BYTES_LOG2");  // tuning aid
+        return env ? std::max(16, std::min(30, atoi(env))) : 20;
+    }();
+    std::vector<int> launches_on(ndev, 0);  // slice events used per device
+    std::vector<cudaEvent_t> chunk_copied(ndev, nullptr);  // the previous chunk's copies: the arena is free after them
+    for (int i = 0; i < ndev; i++) {
+        Replica& r = s->replicas[i];
+        DeviceSlot* slot = r.slot;
+        r.small.filter_ok = r.filter_eligible && s->shadow_filter;
+        r.small.cell_masks = r.cell_masks_eligible && s->shadow_filter;
+        r.small.plane_cells = r.plane_cells_eligible && r.small.cell_masks;
+        if (int rc = ensure_views(slot, n_views, frame_px * 15 * chunk)) return rc;
+        for (uint32_t v = 0; v < n_views; v++) {  // the view table, uploaded once per call on the render stream
+            DevView& d = slot->h_views[v];
+            rows3(views[v].transform_inverse, d.cam_inv);
+            d.half_w = views[v].half_width, d.half_h = views[v].half_height, d.pixel_size = views[v].pixel_size, d.pad = 0.f;
+        }
+        CUDA_TRY(cudaMemcpyAsync(slot->d_views, slot->h_views, n_views * sizeof(DevView), cudaMemcpyHostToDevice, slot->stream));
+        CUDA_TRY(cudaMemsetAsync(slot->d_counters, 0, sizeof(DevCounters), slot->stream));
+        CUDA_TRY(cudaEventRecord(slot->ev0, slot->stream));
+    }
+    auto slice_event = [&](DeviceSlot* slot, int& used) -> cudaEvent_t {
+        while ((int)slot->slice_done.size() <= used) {
+            cudaEvent_t e;
+            if (cudaEventCreateWithFlags(&e, cudaEventDisableTiming) != cudaSuccess) return nullptr;
+            slot->slice_done.push_back(e);
+        }
+        return slot->slice_done[used++];
+    };
+    for (uint32_t c0 = 0; c0 < n_views; c0 += chunk) {
+        const uint32_t c1 = std::min(n_views, c0 + chunk);
+        cc.stage_v0 = (int)c0;
+        for (int i = 0; i < ndev; i++) {
+            Replica& r = s->replicas[i];
+            DeviceSlot* slot = r.slot;
+            const int shard = i;
+            const int nb = shard < total_bands ? (total_bands - shard + n_shards - 1) / n_shards : 0;
+            CUDA_TRY(cudaSetDevice(slot->device));
+            float* d_rgb = reinterpret_cast<float*>(slot->d_view_frames);
+            unsigned char* d_u8 = reinterpret_cast<unsigned char*>(slot->d_view_frames + frame_px * 12 * chunk);
+            // The launches of a chunk: left on the device, one.  Copied to host memory, rtc_render's slice rule applied to the
+            // whole batch — one slice per MiB copied, at most RTC_OPT_RENDER_SLICES — as runs of whole views, or, when a view
+            // is bigger than a slice, that view cut by bands as rtc_render cuts it.  A branching tree scene renders a chunk as
+            // one pixel stream (rtc_render does not slice it either).
+            struct Launch {
+                uint32_t v0, v1;
+                int b0, b1;
+            };
+            std::vector<Launch> plan;
+            const size_t view_copy = (size_t)s->width * kBandRows * nb * ((rgb ? 12 : 0) + (u8 ? 3 : 0));
+            const int want = copy_out && !stream_scene
+                                 ? std::max(1, (int)std::min<size_t>((size_t)s->render_slices, (view_copy * n_views) >> slice_shift))
+                                 : 1;
+            if (nb == 0) {
+            } else if (want <= (int)n_views) {
+                const uint32_t per_run = (n_views + want - 1) / want;
+                for (uint32_t v = c0; v < c1; v += per_run) plan.push_back({v, std::min(c1, v + per_run), 0, nb});
+            } else {
+                const int per_view = std::max(1, std::min(std::min(s->render_slices, nb), (int)(view_copy >> slice_shift)));
+                for (uint32_t v = c0; v < c1; v++)
+                    for (int k = 0; k < per_view; k++) {
+                        const int b0 = (int)((int64_t)nb * k / per_view), b1 = (int)((int64_t)nb * (k + 1) / per_view);
+                        if (b1 > b0) plan.push_back({v, v + 1, b0, b1});
+                    }
+            }
+            cudaStream_t lanes[3] = {slot->stream, slot->slice_stream[0], slot->slice_stream[1]};
+            const int n_lanes = rotate && plan.size() > 1 ? std::min<int>(3, (int)plan.size()) : 1;
+            // every lane starts behind the table upload and the counter reset, and behind the previous chunk's copies
+            for (int l = 1; l < n_lanes; l++) CUDA_TRY(cudaStreamWaitEvent(lanes[l], slot->ev0, 0));
+            if (chunk_copied[i])
+                for (int l = 0; l < n_lanes; l++) CUDA_TRY(cudaStreamWaitEvent(lanes[l], chunk_copied[i], 0));
+            int last_on_lane[3] = {-1, -1, -1};
+            for (size_t k = 0; k < plan.size(); k++) {
+                const Launch& L = plan[k];
+                cudaStream_t lane = lanes[k % n_lanes];
+                const size_t off = (size_t)(L.v0 - c0) * frame_px * 3;
+                DevFrame F{d_rgb + off, d_u8 + off, shard, n_shards, depth, L.b1 - L.b0, L.b0, nullptr, nullptr,
+                           s->converge < 0 ? (int)s->has_branching_materials : s->converge, nullptr, 0};
+                if (stream_scene) {  // one launch at a time on the render stream: one counter does
+                    F.stream_counter = slot->d_stream_counter, F.stream_blocks = slot->sm_count * 6;
+                    CUDA_TRY(cudaMemsetAsync(slot->d_stream_counter, 0, sizeof(unsigned), lane));
+                }
+                kernel_build(s->strict_fp, r.csg_sweep).views(r.scene, r.small, F, slot->d_views + L.v0, (int)(L.v1 - L.v0), slot->d_counters, lane);
+                CUDA_TRY(cudaGetLastError());
+                st.launches++;
+                const int idx = launches_on[i];
+                cudaEvent_t done = slice_event(slot, launches_on[i]);
+                if (!done) return fail(RTC_ERR_CUDA, "cudaEventCreateWithFlags failed");
+                CUDA_TRY(cudaEventRecord(done, lane));
+                last_on_lane[k % n_lanes] = idx;
+                if (copy_out) {
+                    CUDA_TRY(cudaStreamWaitEvent(slot->copy_stream, done, 0));
+                    if (int rc = cc.queue({slot, shard, L.b0, L.b1, (int)L.v0, (int)L.v1, d_rgb + off, d_u8 + off})) return rc;
+                }
+            }
+            for (int l = 0; l < n_lanes; l++)
+                if (l > 0 && last_on_lane[l] >= 0) CUDA_TRY(cudaStreamWaitEvent(slot->stream, slot->slice_done[last_on_lane[l]], 0));
+        }
+        if (int rc = cc.flush_pending()) return rc;
+        if (c1 < n_views) {  // the next chunk reuses the arena (and the staging frames): it waits for this chunk's copies
+            if (int rc = cc.drain()) return rc;
+            for (int i = 0; i < ndev; i++) {
+                DeviceSlot* slot = s->replicas[i].slot;
+                CUDA_TRY(cudaSetDevice(slot->device));
+                int& used = launches_on[i];
+                cudaEvent_t e = slice_event(slot, used);
+                if (!e) return fail(RTC_ERR_CUDA, "cudaEventCreateWithFlags failed");
+                CUDA_TRY(cudaEventRecord(e, copy_out ? slot->copy_stream : slot->stream));
+                chunk_copied[i] = e;
+            }
+        }
+    }
+    if (int rc = cc.drain()) return rc;
+    for (int i = 0; i < ndev; i++) {
+        DeviceSlot* slot = s->replicas[i].slot;
+        CUDA_TRY(cudaSetDevice(slot->device));
+        CUDA_TRY(cudaEventRecord(slot->ev1, slot->stream));
+        CUDA_TRY(cudaMemcpyAsync(slot->h_counters, slot->d_counters, sizeof(DevCounters), cudaMemcpyDeviceToHost, slot->stream));
+    }
+    for (int i = 0; i < ndev; i++) {
+        DeviceSlot* slot = s->replicas[i].slot;
+        CUDA_TRY(cudaSetDevice(slot->device));
+        CUDA_TRY(cudaStreamSynchronize(slot->stream));
+        CUDA_TRY(cudaStreamSynchronize(slot->copy_stream));
+        float ms = 0.f;
+        CUDA_TRY(cudaEventElapsedTime(&ms, slot->ev0, slot->ev1));
+        st.kernel_ms = std::max(st.kernel_ms, (double)ms);
+        uint64_t rows = 0;  // camera.rs:80-81, per view, of this device's bands
+        for (int b = i; b < total_bands; b += n_shards)
+            rows += (uint64_t)std::max(0, std::min<int>((int)s->height - 1, (b + 1) * kBandRows) - b * kBandRows);
+        add_counters(st, *slot->h_counters, (uint64_t)n_views * rows * (uint64_t)(s->width - 1),
+                     s->light_is_rect ? (uint64_t)s->u_steps * s->v_steps : 1);
+    }
     st.total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
     if (stats) *stats = st;
     if (st.capacity_overflows)
@@ -946,6 +1235,7 @@ int rtc_scene_commit(RtcScene* s, int32_t n_devices, const int32_t* device_ids) 
             return rc;
         }
     }
+    s->reach = f.reach;
     s->committed = true;
     return 0;
 }
@@ -969,6 +1259,9 @@ int rtc_render_shard(RtcScene* s, int32_t depth, int32_t shard, int32_t n_shards
 }
 int rtc_render_detailed(RtcScene* s, int32_t depth, float* rgb, uint8_t* u8, RtcStats* stats) {
     return render_impl(s, depth, 0, 0, rgb, u8, stats, true);
+}
+int rtc_render_views(RtcScene* s, int32_t depth, uint32_t n_views, const RtcView* views, float* rgb, uint8_t* u8, RtcStats* stats) {
+    return render_views_impl(s, depth, n_views, views, rgb, u8, stats);
 }
 
 int rtc_trace_rays(RtcScene* s, uint32_t n, const float* origins, const float* directions, int32_t depth, float* out_rgb,

@@ -669,6 +669,7 @@ int flatten(RtcScene* s, Flattened& f, TreeBuilderFn tree_builder, void* tree_bu
                 l = std::max(l, std::fabs(s->corner[a]) + std::fabs(s->u_cell[a]) * s->u_steps + std::fabs(s->v_cell[a]) * s->v_steps);
             if (std::isfinite(l)) extent = std::max(extent, l);
         }
+        f.reach = extent;
     }
     RawVector<BuildItem> build_items(bounded.size());
     parallel_for(bounded.size(), kGrain, [&](size_t begin, size_t end, int) {

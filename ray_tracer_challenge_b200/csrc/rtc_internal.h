@@ -82,6 +82,13 @@ struct DeviceSlot {
     unsigned* d_stream_counter = nullptr;  // render_stream's pixel counters, one per slice of a render
     void* d_flush = nullptr;
     size_t flush_bytes = 0;
+    // rtc_render_views: the batch's view table (device, and its pinned staging) and the frames of one chunk of views, apart
+    // from d_rgb / d_u8 so that a batch leaves rtc_render's frame alone (all grow-only)
+    DevView* d_views = nullptr;
+    DevView* h_views = nullptr;
+    uint32_t views_capacity = 0;
+    char* d_view_frames = nullptr;
+    size_t view_frames_bytes = 0;
 };
 
 // One committed replica of the scene on one device.
@@ -132,6 +139,7 @@ struct Flattened {
     int all_cast_shadow = 1;
     bool csg_sweep = false;  // some CSG is evaluated by csg_sweep: the scene renders with the *_sweep kernel builds
     int loose_group_boxes = 0;  // group nodes whose cached box does not contain some child's box (RtcCommitInfo)
+    float reach = 0.f;  // the largest coordinate the tree's box padding allows for (bounded items, light, camera origin)
 };
 
 }  // namespace rtc
@@ -176,6 +184,7 @@ struct RtcScene {
     rtc::RawVector<int> pos_to_prim;  // device position -> API primitive index (-1 for CSG pseudo-primitives)
     // commit statistics
     int n_bvh_nodes = 0, n_linear = 0, n_xforms = 0;
+    float reach = 0.f;  // Flattened::reach of the commit: rtc_render_views refuses camera origins beyond it in tree scenes
 };
 
 namespace rtc {

@@ -96,10 +96,13 @@ __device__ __forceinline__ void tile_of(const DevFrame& F, int& band, int& bx) {
 // tile_order load per thread) and the tile-cost probe's start is one shared word per warp — which lets it run more
 // resident blocks.  The other builds keep both in registers: the same change made c4 1 % and c2 0.5 % slower
 // (profiles/README.md).
+constexpr int tile_min_blocks(bool SMALL, bool CONVERGE, bool LEAN) {
+    return min_blocks(LEAN ? RTC_SMALL_LEAN_MINBLOCKS
+                           : SMALL ? (CONVERGE ? RTC_SMALL_CONVERGE_MINBLOCKS : RTC_SMALL_MINBLOCKS)
+                                   : (CONVERGE ? RTC_BVH_CONVERGE_MINBLOCKS : RTC_BVH_MINBLOCKS));
+}
 template <bool STATS, bool SMALL, bool CONVERGE, bool DRAWN, bool LEAN = false>
-__global__ void __launch_bounds__(kBlockThreads, min_blocks(LEAN ? RTC_SMALL_LEAN_MINBLOCKS
-                                                            : SMALL ? (CONVERGE ? RTC_SMALL_CONVERGE_MINBLOCKS : RTC_SMALL_MINBLOCKS)
-                                                                    : (CONVERGE ? RTC_BVH_CONVERGE_MINBLOCKS : RTC_BVH_MINBLOCKS)))
+__global__ void __launch_bounds__(kBlockThreads, tile_min_blocks(SMALL, CONVERGE, LEAN))
     render_tiles(const __grid_constant__ DevScene S, const __grid_constant__ SmallScene SS,
                                                     const DevFrame F, DevCounters* counters) {
     // small scenes: primitive table + per-thread shadow-origin cache in dynamic shared memory (kSmallSmemBytes)
@@ -171,6 +174,63 @@ __global__ void __launch_bounds__(kBlockThreads, min_blocks(LEAN ? RTC_SMALL_LEA
         atomicMax(&F.tile_cost[band * gridDim.x + bx], (unsigned)min(clock64() - (LEAN ? s_t_start[warp] : t_start), 0xffffffffLL));
 }
 
+// K1c render_tiles_views: render_tiles for a batch of views of the committed scene (rtc_render_views).  blockIdx.z is a view
+// of the launch: the block takes its camera from the view table instead of DevScene and writes view z's frame, which
+// follows view z - 1's in the frame planes.  There is no learnt tile order and no tile-cost probe.  The body restates
+// render_tiles' instead of sharing it: with render_tiles made a wrapper over a shared inlined body, ptxas allocated the
+// existing builds differently (4 B more spill in the lean and the tree builds).
+template <bool SMALL, bool CONVERGE, bool DRAWN, bool LEAN>
+__global__ void __launch_bounds__(kBlockThreads, tile_min_blocks(SMALL, CONVERGE, LEAN))
+    render_tiles_views(const __grid_constant__ DevScene S, const __grid_constant__ SmallScene SS, const DevFrame F,
+                       DevCounters* counters, const DevView* views) {
+    if (SMALL) stage_small_scene(S, SS);
+    const Env E{S, SS};
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int band = F.shard + (F.band_begin + (int)blockIdx.y) * F.n_shards, bx = blockIdx.x;
+    // warp w -> 8x4 sub-tile (the lean build evaluates these again after color_at, as render_tiles does)
+    auto px_x = [&] { return bx * kTileW + (warp % kWarpsX) * 8 + (lane & 7); };
+    auto px_y = [&] { return band * kBandRows + (warp / kWarpsX) * 4 + (lane >> 3); };
+    int x = px_x(), y = px_y();
+    Ctr<false> k;
+    Rays r;
+    V3 c = mk(0.f, 0.f, 0.f);
+    const bool rendered = x < S.width - 1 && y < S.height - 1;  // camera.rs:80-81
+    V3 o = mk(0.f, 0.f, 0.f), d = mk(0.f, 0.f, 1.f);
+    {
+        const DevView& V = views[blockIdx.z];  // warp-uniform
+        if (rendered) ray_for_pixel(V, x, y, o, d);
+    }
+    if (CONVERGE || rendered)
+        c = color_at<false, SMALL, CONVERGE, DRAWN, LEAN>(E, rendered, o, d, F.depth, (unsigned)(y * S.width + x), r, k, nullptr, nullptr);
+    if (LEAN) x = px_x(), y = px_y();
+    // Canvas::write_pixel + scale_color as in render_tiles: warp-transposed streaming stores where the rows allow them
+    const size_t view0 = (size_t)blockIdx.z * ((size_t)S.width * S.height * 3);
+    __shared__ __align__(16) float s_rgb[kBlockThreads * 3];
+    __shared__ __align__(16) unsigned char s_u8[kBlockThreads * 3];
+    const int wx0 = bx * kTileW + (warp % kWarpsX) * 8, wy0 = band * kBandRows + (warp / kWarpsX) * 4;  // warp-uniform
+    if ((S.width & 7) == 0 && wx0 + 8 <= S.width && wy0 + 4 <= S.height) {
+        float* w_rgb = s_rgb + warp * 96;
+        unsigned char* w_u8 = s_u8 + warp * 96;
+        w_rgb[lane * 3] = c.x, w_rgb[lane * 3 + 1] = c.y, w_rgb[lane * 3 + 2] = c.z;
+        w_u8[lane * 3] = scale_color(c.x), w_u8[lane * 3 + 1] = scale_color(c.y), w_u8[lane * 3 + 2] = scale_color(c.z);
+        __syncwarp();
+        const size_t px0 = (size_t)wy0 * S.width + wx0;
+        if (F.rgb && lane < 24) {
+            const int row = lane / 6, q = lane - row * 6;
+            __stcs(reinterpret_cast<float4*>(F.rgb + view0 + (px0 + (size_t)row * S.width) * 3) + q, reinterpret_cast<const float4*>(w_rgb)[lane]);
+        }
+        if (F.u8 && lane >= 20) {
+            const int u = lane - 20, row = u / 3, q = u - row * 3;
+            __stcs(reinterpret_cast<uint2*>(F.u8 + view0 + (px0 + (size_t)row * S.width) * 3) + q, reinterpret_cast<const uint2*>(w_u8)[u]);
+        }
+    } else if (x < S.width && y < S.height) {
+        const size_t idx = view0 + ((size_t)y * S.width + x) * 3;
+        if (F.rgb) F.rgb[idx] = c.x, F.rgb[idx + 1] = c.y, F.rgb[idx + 2] = c.z;
+        if (F.u8) F.u8[idx] = scale_color(c.x), F.u8[idx + 1] = scale_color(c.y), F.u8[idx + 2] = scale_color(c.z);
+    }
+    flush_counters<false>(r, k, counters);
+}
+
 // K1b render_stream: Camera::render for tree scenes with branching ray trees — a persistent grid whose lanes draw
 // pixels from a counter as their ray trees finish (dev_shade.cuh: PixelStream) instead of owning one pixel each.
 #ifndef RTC_STREAM_MINBLOCKS
@@ -186,6 +246,21 @@ __global__ void __launch_bounds__(kBlockThreads, min_blocks(RTC_STREAM_MINBLOCKS
     Rays r;
     color_at<STATS, false, true, false, false, PixelStream>(E, false, mk(0.f, 0.f, 0.f), mk(0.f, 0.f, 1.f), F.depth, 0u, r, k, nullptr, nullptr, src);
     flush_counters<STATS>(r, k, counters);
+}
+
+// The same for a batch of views: the stream covers views x bands x 8x4 blocks, the view outermost
+__global__ void __launch_bounds__(kBlockThreads, min_blocks(RTC_STREAM_MINBLOCKS))
+    render_stream_views(const __grid_constant__ DevScene S, const __grid_constant__ SmallScene SS, const DevFrame F, DevCounters* counters,
+                        const DevView* views, int n_views) {
+    const Env E{S, SS};
+    const int blocks_x = (S.width + 7) / 8;
+    const unsigned view_blocks = (unsigned)F.n_bands * (unsigned)blocks_x * 2u;
+    ViewPixelStream src{S, F, F.stream_counter, (unsigned)n_views * view_blocks * 32u, blocks_x, views, view_blocks};
+    Ctr<false> k;
+    Rays r;
+    color_at<false, false, true, false, false, ViewPixelStream>(E, false, mk(0.f, 0.f, 0.f), mk(0.f, 0.f, 1.f), F.depth, 0u, r, k, nullptr,
+                                                                    nullptr, src);
+    flush_counters<false>(r, k, counters);
 }
 
 // ---- the wavefront renderer's kernels (dev_wave.cuh) --------------------------------------------------------------------
@@ -320,6 +395,42 @@ void launch_render(const DevScene& S, const SmallScene& SS, const DevFrame& F, D
             render_tiles<false, false, true, false><<<grid, kBlockThreads, 0, stream>>>(S, SS, F, counters);
         else
             render_tiles<false, false, false, false><<<grid, kBlockThreads, 0, stream>>>(S, SS, F, counters);
+    }
+}
+
+// A batch of views (rtc_render_views): the kernel choice of launch_render without its detailed pass
+void launch_views(const DevScene& S, const SmallScene& SS, const DevFrame& F, const DevView* views, int n_views, DevCounters* counters,
+                  cudaStream_t stream) {
+    dim3 grid((S.width + kTileW - 1) / kTileW, F.n_bands, n_views);
+    if (grid.x == 0 || grid.y == 0 || grid.z == 0) return;
+    const bool small = SS.n > 0;
+    if (!small && F.stream_counter) {
+        render_stream_views<<<F.stream_blocks, kBlockThreads, 0, stream>>>(S, SS, F, counters, views, n_views);
+        return;
+    }
+    const bool drawn = small && SS.cell_masks && S.jitter_len == 0;
+#ifndef RTC_CSG_SWEEP_BUILD
+    if (!F.converge && small && SS.cell_masks && SS.lean) {
+        if (drawn)
+            render_tiles_views<true, false, true, true><<<grid, kBlockThreads, kSmemOrg * 16, stream>>>(S, SS, F, counters, views);
+        else
+            render_tiles_views<true, false, false, true><<<grid, kBlockThreads, kSmemOrg * 16, stream>>>(S, SS, F, counters, views);
+        return;
+    }
+#endif
+    if (small) {
+        if (drawn && F.converge)
+            render_tiles_views<true, true, true, false><<<grid, kBlockThreads, kSmallSmemBytes, stream>>>(S, SS, F, counters, views);
+        else if (drawn)
+            render_tiles_views<true, false, true, false><<<grid, kBlockThreads, kSmallSmemBytes, stream>>>(S, SS, F, counters, views);
+        else if (F.converge)
+            render_tiles_views<true, true, false, false><<<grid, kBlockThreads, kSmallSmemBytes, stream>>>(S, SS, F, counters, views);
+        else
+            render_tiles_views<true, false, false, false><<<grid, kBlockThreads, kSmallSmemBytes, stream>>>(S, SS, F, counters, views);
+    } else if (F.converge) {
+        render_tiles_views<false, true, false, false><<<grid, kBlockThreads, 0, stream>>>(S, SS, F, counters, views);
+    } else {
+        render_tiles_views<false, false, false, false><<<grid, kBlockThreads, 0, stream>>>(S, SS, F, counters, views);
     }
 }
 

@@ -8,6 +8,10 @@ namespace rtc {
 namespace fast {
 void launch_render(const DevScene& S, const SmallScene& SS, const DevFrame& F, DevCounters* counters, bool detailed,
                    cudaStream_t stream);
+// A batch of views of the committed scene (rtc_render_views): F's bands of `n_views` views, view v's camera views[v] and its
+// frame at F.rgb / F.u8 + v * width * height * 3; a tree scene with F.stream_counter set renders them as one pixel stream.
+void launch_views(const DevScene& S, const SmallScene& SS, const DevFrame& F, const DevView* views, int n_views, DevCounters* counters,
+                  cudaStream_t stream);
 void launch_trace(const DevScene& S, const SmallScene& SS, int n, const float* origins, const float* directions, int depth,
                   float* out_rgb, float* out_t, int* out_pos, DevCounters* counters, cudaStream_t stream);
 void launch_fma_peak(float* out, int blocks, int iters, cudaStream_t stream);
@@ -19,6 +23,8 @@ void launch_wave(const DevScene& S, const SmallScene& SS, const DevFrame& F, con
 namespace strict {
 void launch_render(const DevScene& S, const SmallScene& SS, const DevFrame& F, DevCounters* counters, bool detailed,
                    cudaStream_t stream);
+void launch_views(const DevScene& S, const SmallScene& SS, const DevFrame& F, const DevView* views, int n_views, DevCounters* counters,
+                  cudaStream_t stream);
 void launch_trace(const DevScene& S, const SmallScene& SS, int n, const float* origins, const float* directions, int depth,
                   float* out_rgb, float* out_t, int* out_pos, DevCounters* counters, cudaStream_t stream);
 void launch_wave(const DevScene& S, const SmallScene& SS, const DevFrame& F, const WavePoolRaw& pool, DevCounters* counters, int blocks,
@@ -28,6 +34,8 @@ void launch_wave(const DevScene& S, const SmallScene& SS, const DevFrame& F, con
 namespace fast_sweep {
 void launch_render(const DevScene& S, const SmallScene& SS, const DevFrame& F, DevCounters* counters, bool detailed,
                    cudaStream_t stream);
+void launch_views(const DevScene& S, const SmallScene& SS, const DevFrame& F, const DevView* views, int n_views, DevCounters* counters,
+                  cudaStream_t stream);
 void launch_trace(const DevScene& S, const SmallScene& SS, int n, const float* origins, const float* directions, int depth,
                   float* out_rgb, float* out_t, int* out_pos, DevCounters* counters, cudaStream_t stream);
 void launch_wave(const DevScene& S, const SmallScene& SS, const DevFrame& F, const WavePoolRaw& pool, DevCounters* counters, int blocks,
@@ -36,6 +44,8 @@ void launch_wave(const DevScene& S, const SmallScene& SS, const DevFrame& F, con
 namespace strict_sweep {
 void launch_render(const DevScene& S, const SmallScene& SS, const DevFrame& F, DevCounters* counters, bool detailed,
                    cudaStream_t stream);
+void launch_views(const DevScene& S, const SmallScene& SS, const DevFrame& F, const DevView* views, int n_views, DevCounters* counters,
+                  cudaStream_t stream);
 void launch_trace(const DevScene& S, const SmallScene& SS, int n, const float* origins, const float* directions, int depth,
                   float* out_rgb, float* out_t, int* out_pos, DevCounters* counters, cudaStream_t stream);
 void launch_wave(const DevScene& S, const SmallScene& SS, const DevFrame& F, const WavePoolRaw& pool, DevCounters* counters, int blocks,

@@ -207,6 +207,14 @@ struct DevFrame {  // where a render writes
     unsigned* stream_counter;  // render_stream: next unclaimed pixel of the launch (zeroed by the host), or null
     int stream_blocks;         // render_stream: resident blocks to launch (a persistent grid)
 };
+// One camera of a batch of views (rtc_render_views): Camera::new's derived fields (camera.rs:23-56), read by
+// ray_for_pixel in place of DevScene's.  The batch's table lives in device memory, one entry per view of the call.
+struct DevView {  // 64 B
+    float4 cam_inv[3];
+    float half_w, half_h, pixel_size, pad;
+};
+static_assert(sizeof(DevView) == 64, "DevView: 64 B per view");
+
 #ifndef RTC_REFILL_LANES
 #define RTC_REFILL_LANES 8
 #endif

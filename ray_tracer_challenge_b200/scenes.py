@@ -823,3 +823,23 @@ def stress(rt, width=3840, height=2160, n_spheres=100_000, n_each=64, n_csg=16, 
     camera = rt.Camera(width, height, PI / 3.0,
                        rt.view_transform((0, extent * 0.4, -extent * 2.2), (0, 0, 0), (0, 1, 0)))
     return camera, world
+
+
+def orbit_cameras(rt, camera, n, degrees=360.0, field_of_view=None):
+    """`n` cameras of `camera`'s canvas size (a host session's camera) whose eyes turn about the vertical axis through the
+    look-at point: the point of the camera's forward ray nearest that axis — the turntable of rtc_render_views.  View i is
+    at i * degrees / n (view 0 is the camera's own eye); field_of_view defaults to the camera's."""
+    inv = np.asarray(rt.camera_view(camera).transform_inverse, np.float64).reshape(4, 4)
+    eye, fwd = inv[:3, 3], -inv[:3, 2]
+    h2 = fwd[0] ** 2 + fwd[2] ** 2
+    t = -(eye[0] * fwd[0] + eye[2] * fwd[2]) / h2 if h2 > 1e-12 else 1.0
+    pivot = eye + t * fwd
+    fov = camera.field_of_view if field_of_view is None else field_of_view
+    out = []
+    for i in range(n):
+        a = math.radians(degrees * i / n)
+        dx, dz = eye[0] - pivot[0], eye[2] - pivot[2]
+        e = (pivot[0] + dx * math.cos(a) + dz * math.sin(a), eye[1], pivot[2] - dx * math.sin(a) + dz * math.cos(a))
+        out.append(rt.Camera(camera.width_pixels, camera.height_pixels, fov,
+                             rt.view_transform(tuple(float(c) for c in e), tuple(float(c) for c in pivot), (0, 1, 0))))
+    return out

@@ -555,4 +555,54 @@ impl Camera {
         }
         out
     }
+
+    /// `Camera::render` for several cameras of one canvas size (a turntable, a stereo pair): the world is flattened and
+    /// committed once — with the camera whose origin is farthest out, so that the tree's reach covers every view — and all
+    /// views come from one `rtc_render_views` batch.  Canvas i is what `cameras[i].render(world, depth)` returns.
+    pub fn render_b200_views(cameras: &[Camera], world: World, reflection_recursion_depth: i16) -> Vec<Canvas> {
+        assert!(!cameras.is_empty(), "render_b200_views needs at least one camera");
+        let reach = |c: &Camera| {
+            let m = mat16(&c.transform_inverse);
+            m[3].abs().max(m[7].abs()).max(m[11].abs())
+        };
+        let mut far = 0;
+        for (i, c) in cameras.iter().enumerate() {
+            if reach(c) > reach(&cameras[far]) {
+                far = i;
+            }
+        }
+        let (w, h) = (cameras[far].width_pixels as usize, cameras[far].height_pixels as usize);
+        let views: Vec<sys::RtcView> = cameras
+            .iter()
+            .map(|c| {
+                assert!(c.width_pixels as usize == w && c.height_pixels as usize == h, "every view of a batch has one canvas size");
+                sys::RtcView {
+                    half_width: c.half_width_world,
+                    half_height: c.half_height_world,
+                    pixel_size: c.pixel_size,
+                    transform_inverse: mat16(&c.transform_inverse),
+                }
+            })
+            .collect();
+        let mut rgb = vec![0f32; views.len() * w * h * 3];
+        unsafe {
+            let scene = cameras[far].commit_b200(&world);
+            let mut stats: sys::RtcStats = std::mem::zeroed();
+            check(sys::rtc_render_views(scene, reflection_recursion_depth as i32, views.len() as u32, views.as_ptr(), rgb.as_mut_ptr(),
+                                        std::ptr::null_mut(), &mut stats));
+            sys::rtc_scene_destroy(scene);
+        }
+        rgb.chunks(w * h * 3)
+            .map(|frame| {
+                let mut canvas = Canvas::new(w, h);
+                for y in 0..h {
+                    for x in 0..w {
+                        let i = (y * w + x) * 3;
+                        canvas.write_pixel(x, y, Color::new(frame[i], frame[i + 1], frame[i + 2]));
+                    }
+                }
+                canvas
+            })
+            .collect()
+    }
 }

@@ -149,6 +149,16 @@ pub struct RtcStats {
     pub wave_overflows: i32,
 }
 
+/// One camera view of `rtc_render_views`: `Camera::new`'s derived fields (camera.rs:23-56), as `rtc_set_camera` takes them.
+#[repr(C)]
+#[derive(Clone, Copy, Default)]
+pub struct RtcView {
+    pub half_width: f32,
+    pub half_height: f32,
+    pub pixel_size: f32,
+    pub transform_inverse: [f32; 16],
+}
+
 /// What `rtc_scene_commit` would build, computed without a device (`rtc_scene_inspect`).
 #[repr(C)]
 #[derive(Clone, Copy, Default)]
@@ -199,6 +209,8 @@ extern "C" {
     pub fn rtc_render_shard(scene: *mut RtcScene, depth: i32, shard: i32, n_shards: i32, rgb_f32: *mut f32,
                             rgb_u8: *mut u8, stats: *mut RtcStats) -> c_int;
     pub fn rtc_render_detailed(scene: *mut RtcScene, depth: i32, rgb_f32: *mut f32, rgb_u8: *mut u8, stats: *mut RtcStats) -> c_int;
+    pub fn rtc_render_views(scene: *mut RtcScene, depth: i32, n_views: u32, views: *const RtcView, rgb_f32: *mut f32, rgb_u8: *mut u8,
+                            stats: *mut RtcStats) -> c_int;
     pub fn rtc_trace_rays(scene: *mut RtcScene, n: u32, origins: *const f32, directions: *const f32, depth: i32,
                           out_rgb: *mut f32, out_t: *mut f32, out_prim: *mut i32) -> c_int;
     pub fn rtc_shard_bands(height: u32, shard: i32, n_shards: i32, first_rows: *mut u32) -> c_int;
