@@ -64,6 +64,24 @@ struct WavePool {
     unsigned long long* shades;
 };
 
+// the pool as the host hands it to the launchers (rtc_types.h), typed
+__device__ __forceinline__ WavePool wave_pool(const WavePoolRaw& raw) {
+    WavePool P;
+    P.rays = static_cast<WaveRay*>(raw.rays), P.nodes = static_cast<WaveNode*>(raw.nodes), P.capacity = raw.capacity;
+    P.base = raw.ints, P.count = raw.ints + kWaveLevels, P.cursor = raw.ints + 2 * kWaveLevels;
+    P.overflow = raw.record, P.secondary = raw.record + 1, P.shades = raw.record + 2;
+    return P;
+}
+
+// between the appends to a level and its first walk (one thread): the level keeps the rays that were written, and the
+// next level starts where it ends.  wave_append counts every ray, also those that did not fit (the overflow record has
+// them and the chunk is rendered again); left in the count they would send the level's kernels past the pool's end.
+__device__ __forceinline__ void wave_next_level(const WavePool& P, int level) {
+    const int n = min(P.count[level], P.capacity - P.base[level]);
+    P.count[level] = n;
+    P.base[level + 1] = P.base[level] + n;
+}
+
 // ---- chunk start: the primary rays of bands [band_begin, band_begin + n_bands) of the shard ------------------------
 __device__ __forceinline__ int wave_append(const WavePool& P, int level, bool want) {
     // warp-aggregated: one atomic per warp, lanes in order

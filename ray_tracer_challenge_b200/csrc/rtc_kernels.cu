@@ -267,40 +267,27 @@ __global__ void __launch_bounds__(kBlockThreads, min_blocks(RTC_STREAM_MINBLOCKS
 #ifndef RTC_WAVE_TRACE_MINBLOCKS
 #define RTC_WAVE_TRACE_MINBLOCKS 8
 #endif
-__device__ __forceinline__ WavePool wave_pool(const WavePoolRaw& raw, DevCounters* counters) {
-    WavePool P;
-    P.rays = static_cast<WaveRay*>(raw.rays), P.nodes = static_cast<WaveNode*>(raw.nodes), P.capacity = raw.capacity;
-    P.base = raw.ints, P.count = raw.ints + kWaveLevels, P.cursor = raw.ints + 2 * kWaveLevels;
-    P.overflow = raw.record, P.secondary = raw.record + 1, P.shades = raw.record + 2;
-    (void)counters;
-    return P;
-}
 __global__ void __launch_bounds__(128) wave_primary_kernel(const __grid_constant__ DevScene S, const DevFrame F, const WavePoolRaw raw,
                                                           DevCounters* counters) {
-    wave_primary(S, F, wave_pool(raw, counters));
+    wave_primary(S, F, wave_pool(raw));
 }
-// the next level starts where this one ends
-__global__ void wave_next_level_kernel(const WavePoolRaw raw, int level) {
-    int* base = raw.ints;
-    int* count = raw.ints + kWaveLevels;
-    base[level + 1] = min(base[level] + count[level], raw.capacity);
-}
+__global__ void wave_next_level_kernel(const WavePoolRaw raw, int level) { wave_next_level(wave_pool(raw), level); }
 template <bool SHADOW>
 __global__ void __launch_bounds__(128, RTC_WAVE_TRACE_MINBLOCKS) wave_trace_kernel(const __grid_constant__ DevScene S, const WavePoolRaw raw,
                                                                                  DevCounters* counters, int level) {
-    wave_trace<SHADOW>(S, wave_pool(raw, counters), level);
+    wave_trace<SHADOW>(S, wave_pool(raw), level);
 }
 __global__ void __launch_bounds__(128) wave_hit_kernel(const __grid_constant__ DevScene S, const WavePoolRaw raw, DevCounters* counters,
                                                       int level) {
-    wave_hit(S, wave_pool(raw, counters), level);
+    wave_hit(S, wave_pool(raw), level);
 }
 __global__ void __launch_bounds__(128) wave_shade_kernel(const __grid_constant__ DevScene S, const WavePoolRaw raw, DevCounters* counters,
                                                         int level, int depth) {
-    wave_shade(S, wave_pool(raw, counters), level, depth);
+    wave_shade(S, wave_pool(raw), level, depth);
 }
 __global__ void __launch_bounds__(128) wave_combine_kernel(const __grid_constant__ DevScene S, const DevFrame F, const WavePoolRaw raw,
                                                           DevCounters* counters, int level) {
-    wave_combine(S, F, wave_pool(raw, counters), level);
+    wave_combine(S, F, wave_pool(raw), level);
 }
 
 void launch_wave(const DevScene& S, const SmallScene&, const DevFrame& F, const WavePoolRaw& pool, DevCounters* counters, int blocks,

@@ -228,7 +228,7 @@ struct WavePoolRaw {
     void* rays;    // capacity x 96 B
     void* nodes;   // capacity x 64 B
     int capacity;
-    int* ints;     // base[L], count[L], cursor[2 L] for L <= kMaxFrames: see rtc_kernels.cu: wave_pool
+    int* ints;     // base[L], count[L], cursor[2 L] for L <= kMaxFrames: see dev_wave.cuh: wave_pool
     unsigned long long* record;  // this chunk's {rays that did not fit the pool, secondary rays, shades}
 };
 constexpr int kWaveLevels = kMaxFrames + 1;

@@ -4,13 +4,18 @@
 // "thread" per "block".  It runs World::color_at for caller-supplied rays over the arrays rtc::flatten() — the host half
 // of rtc_scene_commit — would upload, so kernel logic can be compared with the oracle on a machine without a GPU.
 // With -ffp-contract=off the host evaluates the strict build's IEEE expression order; libm is glibc's on both sides.
+// It also runs the wavefront renderer's kernel sequence (dev_wave.cuh) over one chunk of a frame, one lane per "warp".
 #include <math.h>
 #include <string.h>
 
 #include <cmath>
 #include <cstdlib>
 #include <cstring>
+#include <vector>
 
+// one lane per "warp": wave_trace refills as soon as that lane is idle (with the default of 8 idle lanes it never
+// would); of the rest of the device code only PixelStream reads this, and it is compiled here but never run
+#define RTC_REFILL_LANES 1
 #include "rtc_internal.h"  // Flattened, RtcScene, rtc::flatten (exported by librtc_b200.so)
 
 #undef __device__
@@ -70,8 +75,11 @@ static inline int __any_sync(unsigned, int p) { return p; }
 // PixelStream (dev_shade.cuh) is compiled but never run here: one lane per "warp"
 static inline unsigned __ballot_sync(unsigned, int p) { return p ? 1u : 0u; }
 static inline unsigned __shfl_sync(unsigned, unsigned v, int) { return v; }
-static inline unsigned atomicAdd(unsigned* p, unsigned v) {
-    unsigned old = *p;
+static inline unsigned __activemask() { return 1u; }
+static inline unsigned __reduce_add_sync(unsigned, unsigned v) { return v; }
+template <typename T>
+static inline T atomicAdd(T* p, T v) {  // unsigned, int, unsigned long long
+    T old = *p;
     *p += v;
     return old;
 }
@@ -91,6 +99,7 @@ float4 rtc_smem[kSmallSmemBytes / sizeof(float4) + 64];  // the block's dynamic 
 #include "dev_small.cuh"
 #include "dev_shadow.cuh"
 #include "dev_shade.cuh"
+#include "dev_wave.cuh"
 
 namespace {
 // upload_replica (rtc_api.cu) with host pointers
@@ -162,5 +171,39 @@ extern "C" int emu_color_at(RtcScene* s, uint32_t n, const float* origins, const
         out_rgb[3 * (size_t)i] = c.x, out_rgb[3 * (size_t)i + 1] = c.y, out_rgb[3 * (size_t)i + 2] = c.z;
         if (out_t) out_t[i] = t;
     }
+    return 0;
+}
+
+// One chunk of a frame through the wavefront renderer: launch_wave's kernel sequence (rtc_kernels.cu) over bands
+// [band_begin, band_begin + n_bands) of the shard, into the caller's w x h x 3 f32 frame.  The pool holds exactly
+// `capacity` rays and nodes (heap arrays: AddressSanitizer guards their ends).  out_ints: base[L], count[L] and the two
+// cursors of every level after the render (4 * kWaveLevels); out_record: {rays that did not fit, secondary rays, shades}.
+extern "C" int emu_wave_chunk(RtcScene* s, int depth, int shard, int n_shards, int band_begin, int n_bands, int capacity,
+                              float* out_rgb, int32_t* out_ints, unsigned long long* out_record) {
+    using namespace rtc;
+    if (s->light_is_rect) return fail(RTC_ERR_INVALID, "the wavefront renderer takes point lights only");
+    if (depth < 0 || depth > kMaxFrames - 1 || capacity < 1 || n_shards < 1 || shard < 0 || shard >= n_shards)
+        return fail(RTC_ERR_INVALID, "bad wavefront chunk");
+    Flattened f;
+    if (int rc = flatten(s, f)) return rc;
+    DevScene S;
+    host_scene(s, f, S);
+    std::vector<emu::WaveRay> rays((size_t)capacity);
+    std::vector<emu::WaveNode> nodes((size_t)capacity);
+    std::vector<int> ints(kWaveInts, 0);
+    std::vector<unsigned long long> record(3, 0ull);
+    const DevFrame F{out_rgb, nullptr, shard, n_shards, depth, n_bands, band_begin, nullptr, nullptr, 1, nullptr, 0};
+    const emu::WavePool P = emu::wave_pool(WavePoolRaw{rays.data(), nodes.data(), capacity, ints.data(), record.data()});
+    emu::wave_primary(S, F, P);
+    for (int level = 0; level <= depth; level++) {
+        emu::wave_next_level(P, level);
+        emu::wave_trace<false>(S, P, level);
+        emu::wave_hit(S, P, level);
+        emu::wave_trace<true>(S, P, level);
+        emu::wave_shade(S, P, level, depth);
+    }
+    for (int level = depth; level >= 0; level--) emu::wave_combine(S, F, P, level);
+    memcpy(out_ints, ints.data(), ints.size() * sizeof(int));
+    memcpy(out_record, record.data(), record.size() * sizeof(unsigned long long));
     return 0;
 }

@@ -12,6 +12,7 @@ import numpy as np
 import pytest
 
 from ray_tracer_challenge_b200 import scenes
+from tests.wave_child import tight_glass_die
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CUDA_INCLUDE = "/usr/local/cuda/include"
@@ -52,6 +53,8 @@ def emu(tmp_path_factory):
 def emu_color(tmp_path_factory):
     device, lib = _build(tmp_path_factory, "emu_color.cpp")
     lib.emu_color_at.argtypes = [C.c_void_p, C.c_uint32, FP, FP, C.c_int, C.c_int, C.c_int, FP, FP, C.POINTER(C.c_int32)]
+    lib.emu_wave_chunk.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, FP, C.POINTER(C.c_int32),
+                                   C.POINTER(C.c_ulonglong)]
     return device, lib
 
 
@@ -332,6 +335,141 @@ def test_shadow_filter_at_scale_extremes_through_the_device_code(emu_color, host
         finally:
             device.rtc_scene_destroy(scene)
     assert eligible >= (2 if extreme == "stretched" else 4), (extreme, eligible)
+
+
+# ---- the wavefront renderer (dev_wave.cuh) through the device code ------------------------------------------------------
+BAND_ROWS = 8                 # rtc_types.h: kBandRows
+WAVE_LEVELS = 25              # rtc_types.h: kWaveLevels = kMaxFrames + 1
+UNWRITTEN = 0x7FBADBAD        # a NaN no render writes: marks the pixels a chunk must leave alone
+
+WAVE_SCENES = {
+    "sphere_field": (scenes.stress, dict(width=64, height=36, n_spheres=1500, n_each=6, n_csg=6)),
+    "mesh": (scenes.dragon_element, dict(width=64, height=36, n_u=24, n_v=12)),
+    "csg": (scenes.csg_gallery, dict(width=64, height=40)),
+    "csg_chain": (scenes.csg_chain, dict(width=61, height=37)),  # ragged last band and last 8-pixel column
+    "reflect_refract_csg": (scenes.reflect_refract, dict(width=64, height=32, with_csg=True)),
+    "tight_glass_die": (tight_glass_die, dict(width=40, height=26)),  # 26 rays per pixel at depth 5, 260 at depth 9
+}
+
+
+def _shard_bands(h, shard, n_shards):
+    return [b for b in range((h + BAND_ROWS - 1) // BAND_ROWS) if b % n_shards == shard]
+
+
+def _wave_chunk(emu_color, scene, w, h, depth, capacity, shard=0, n_shards=1, band_begin=0, n_bands=None):
+    """One chunk through launch_wave's kernel sequence: (frame, base[L], count[L], (overflow, secondary, shades))."""
+    device, lib = emu_color
+    if n_bands is None:
+        n_bands = len(_shard_bands(h, shard, n_shards)) - band_begin
+    frame = np.full((h, w, 3), UNWRITTEN, np.uint32).view(np.float32)
+    ints = np.zeros(4 * WAVE_LEVELS, np.int32)
+    record = (C.c_ulonglong * 3)()
+    rc = lib.emu_wave_chunk(scene, depth, shard, n_shards, band_begin, n_bands, capacity, frame.ctypes.data_as(FP),
+                            ints.ctypes.data_as(C.POINTER(C.c_int32)), record)
+    assert rc == 0, device.rtc_last_error()
+    return frame, ints[:WAVE_LEVELS].astype(np.int64), ints[WAVE_LEVELS:2 * WAVE_LEVELS].astype(np.int64), tuple(record)
+
+
+def _same_bits(a, b):
+    return (a.view(np.uint32) == b.view(np.uint32)).all(axis=-1)
+
+
+@pytest.mark.parametrize("depth", [0, 1, 5, 9])
+@pytest.mark.parametrize("name", sorted(WAVE_SCENES))
+def test_wavefront_of_the_device_code_matches_oracle_bit_for_bit(name, depth, emu_color, host, oracle):
+    """The wavefront renderer's kernels (primary rays, per level the nearest-hit walk, hit record, shadow walk and shade,
+    then the post-order combine) over the whole frame as one chunk with an ample pool: the frame is the oracle's
+    Camera::render, bit for bit, black last row and column included; the chunk record counts the oracle's secondary rays
+    and shades; and the levels lie end to end in the pool, holding exactly the primary plus secondary rays."""
+    device, _ = emu_color
+    make, kw = WAVE_SCENES[name]
+    cam, world = make(host, **kw)
+    ocam, oworld = make(oracle, **kw)
+    want = np.asarray(ocam.render(oworld, depth).data, np.float32)
+    st = ocam.last_stats
+    rays = st.primary_rays + st.secondary_rays
+    h, w = want.shape[:2]
+    scene = host.export_scene(cam, world)
+    try:
+        frame, base, count, (overflow, secondary, shades) = _wave_chunk(emu_color, scene, w, h, depth, 2 * rays)
+    finally:
+        device.rtc_scene_destroy(scene)
+    same = _same_bits(frame, want)
+    assert same.all(), (name, depth, int((~same).sum()), np.argwhere(~same)[:3], frame[~same][:2], want[~same][:2])
+    assert (overflow, secondary, shades) == (0, st.secondary_rays, st.shades), (name, depth, st.as_dict())
+    assert base[0] == 0 and (base[1:depth + 2] == base[:depth + 1] + count[:depth + 1]).all(), (base, count)
+    assert count[:depth + 1].sum() == rays and not count[depth + 1:].any(), (count, rays)
+    assert count[0] == st.primary_rays
+
+
+def test_wavefront_chunks_and_shards_of_the_device_code_match_oracle(emu_color, host, oracle):
+    """A frame rendered as chunks of bands (band_begin, n_bands) and as three interleaved shards, one of them in two
+    chunks: every part writes exactly the oracle's pixels of its bands and nothing outside them, and the parts' records
+    add up to the oracle's secondary rays and shades."""
+    device, _ = emu_color
+    kw = dict(width=64, height=44, with_csg=True)  # six bands, the last of four rows
+    cam, world = scenes.reflect_refract(host, **kw)
+    ocam, oworld = scenes.reflect_refract(oracle, **kw)
+    depth = 5
+    want = np.asarray(ocam.render(oworld, depth).data, np.float32)
+    st = ocam.last_stats
+    h, w = want.shape[:2]
+    partitions = {
+        "chunks": [(0, 1, 0, 2), (0, 1, 2, 3), (0, 1, 5, 1)],               # (shard, n_shards, band_begin, n_bands)
+        "shards": [(0, 3, 0, 2), (1, 3, 0, 1), (1, 3, 1, 1), (2, 3, 0, 2)],
+    }
+    scene = host.export_scene(cam, world)
+    try:
+        for label, parts in partitions.items():
+            whole = np.full((h, w, 3), UNWRITTEN, np.uint32).view(np.float32)
+            secondary = shades = 0
+            for shard, n_shards, band_begin, n_bands in parts:
+                frame, _, _, rec = _wave_chunk(emu_color, scene, w, h, depth, 6 * w * h, shard, n_shards, band_begin, n_bands)
+                assert rec[0] == 0
+                secondary, shades = secondary + rec[1], shades + rec[2]
+                rows = np.zeros(h, bool)
+                for band in _shard_bands(h, shard, n_shards)[band_begin:band_begin + n_bands]:
+                    rows[band * BAND_ROWS:(band + 1) * BAND_ROWS] = True
+                part = (label, shard, band_begin, n_bands)
+                assert _same_bits(frame[rows], want[rows]).all(), part
+                assert (frame[~rows].view(np.uint32) == UNWRITTEN).all(), part
+                assert (whole[rows].view(np.uint32) == UNWRITTEN).all(), part  # the parts do not overlap ...
+                whole[rows] = frame[rows]
+            assert _same_bits(whole, want).all(), label  # ... and cover the frame
+            assert (secondary, shades) == (st.secondary_rays, st.shades), label
+    finally:
+        device.rtc_scene_destroy(scene)
+
+
+def test_overflowing_wavefront_pool_stays_in_bounds(emu_color, host, oracle):
+    """A chunk whose rays do not fit the pool is rendered again by render_stream, but first its own kernels must stay
+    inside the pool: every level keeps only the rays that were written (base + count <= capacity), the overflow record
+    is non-zero exactly when the pool holds fewer than the chunk's primary plus secondary rays, and a pool of exactly
+    that many renders the oracle's frame.  Under AddressSanitizer (test_device_code_under_address_sanitizer) the
+    pool's arrays end in red zones, so a ray or node read or written past the end aborts the run."""
+    device, _ = emu_color
+    kw = dict(width=64, height=40)
+    cam, world = tight_glass_die(host, **kw)
+    ocam, oworld = tight_glass_die(oracle, **kw)
+    depth = 5
+    want = np.asarray(ocam.render(oworld, depth).data, np.float32)
+    st = ocam.last_stats
+    rays = st.primary_rays + st.secondary_rays
+    h, w = want.shape[:2]
+    chunk_px = len(_shard_bands(h, 0, 1)) * BAND_ROWS * ((w + 7) // 8 * 8)
+    assert rays > 6 * chunk_px  # the product's first pool (kWaveRaysPerPixel = 6) overflows on this frame
+    scene = host.export_scene(cam, world)
+    try:
+        for capacity in (rays, rays - 1, 6 * chunk_px, st.primary_rays - 1, 5):
+            frame, base, count, (overflow, _, _) = _wave_chunk(emu_color, scene, w, h, depth, capacity)
+            assert (base + count <= capacity).all(), (capacity, base[:depth + 2], count[:depth + 2])
+            assert (base[1:depth + 2] == base[:depth + 1] + count[:depth + 1]).all(), (capacity, base, count)
+            assert (overflow == 0) == (capacity >= rays), (capacity, overflow)
+            assert count.sum() == min(capacity, rays), (capacity, count)
+            if capacity >= rays:
+                assert _same_bits(frame, want).all()
+    finally:
+        device.rtc_scene_destroy(scene)
 
 
 def test_device_code_under_address_sanitizer():
