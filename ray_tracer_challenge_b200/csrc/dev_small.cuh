@@ -2,6 +2,12 @@
 // Part of rtc_device.cuh (include that, not this): compiled once per kernel build inside namespace rtc::RTC_NS.
 #pragma once
 
+// The declaration of the dynamic shared-memory block.  The host harness of the device code (tests/emu/simt.h) turns
+// __shared__ into `static` for the static arrays, so it spells this one as a plain `extern` array instead.
+#ifndef RTC_EXTERN_SHARED
+#define RTC_EXTERN_SHARED extern __shared__
+#endif
+
 namespace rtc {
 namespace RTC_NS {
 
@@ -21,28 +27,28 @@ struct Env {
 //             primitives (element (i, c) of thread t at org[(i * 3 + c) * kBlockThreads + t]) — the per-cell shadow loop.
 // The first three are the same for every block: stage_small_scene copies them from the scene's image.
 __device__ __forceinline__ const float4* small_tab() {
-    extern __shared__ float4 rtc_smem[];
+    RTC_EXTERN_SHARED float4 rtc_smem[];
     return rtc_smem;
 }
 __device__ __forceinline__ float* small_org() {
-    extern __shared__ float4 rtc_smem[];
+    RTC_EXTERN_SHARED float4 rtc_smem[];
     return reinterpret_cast<float*>(rtc_smem + kSmemOrg) + threadIdx.x;
 }
 __device__ __forceinline__ const float4* small_plane_cells() {
-    extern __shared__ float4 rtc_smem[];
+    RTC_EXTERN_SHARED float4 rtc_smem[];
     return rtc_smem + kSmemPlaneCells;
 }
 __device__ __forceinline__ const float4* small_samples() {  // table-mode light samples (SmallScene::cell_masks)
-    extern __shared__ float4 rtc_smem[];
+    RTC_EXTERN_SHARED float4 rtc_smem[];
     return rtc_smem + kSmemSamples;
 }
 // A block's staging: three coalesced copies out of the scene's image (L2 / L1 resident after the first blocks), each
 // started by a different warp so that no warp does all of it while the others wait at the barrier.  Every kernel that
 // stages runs blocks of kBlockThreads threads: with the block size a constant the start offsets and trip counts are
-// shifts and masks, not the integer divisions a runtime blockDim.x costs every block (the host harness of
-// tests/emu stages with one thread).
+// shifts and masks, not the integer divisions a runtime blockDim.x costs every block (the host harnesses of
+// tests/emu stage with one thread, emu_color.cpp, or with kBlockThreads, emu_kernels.cpp).
 __device__ __forceinline__ void stage_small_scene(const DevScene& S, const SmallScene& SS) {
-    extern __shared__ float4 rtc_smem[];
+    RTC_EXTERN_SHARED float4 rtc_smem[];
     const float4* img = S.small_image;
 #ifdef __CUDA_ARCH__
     constexpr int nt = kBlockThreads;

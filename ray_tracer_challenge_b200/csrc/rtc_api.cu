@@ -546,7 +546,7 @@ int render_impl(RtcScene* s, int depth, int shard0, int n_shards_ext, float* rgb
         // tree scenes whose ray trees branch: the streaming kernel (lanes draw pixels from a per-launch counter).  A
         // persistent launch pays its tail once per launch and such frames take far longer than their copy, so they
         // are not sliced
-        const bool stream_scene = r.small.n == 0 && (s->stream < 0 ? s->has_branching_materials : s->stream != 0);
+        const bool stream_scene = streams_pixels(s, r.small);
         // a frame is cut only as finely as its copy is long: one slice per MiB that leaves the device, at most
         // `render_slices` (c3's 24.9 MB 8-bit canvas: 23 slices, 0.67 ms end to end against 1.10 in one piece; c1's 1.2 MB:
         // 1 slice, 0.22 ms against 0.43 in six).  Slices on one stream cost ~15 us each of launch ramp and tail (6 slices
@@ -630,11 +630,11 @@ int render_impl(RtcScene* s, int depth, int shard0, int n_shards_ext, float* rgb
             if (b1 <= b0) continue;
             cudaStream_t lane = lanes[k % n_lanes];
             DevFrame F{slot->d_rgb, slot->d_u8, shard, n_shards, depth, b1 - b0, b0, use_order ? slot->d_tile_order : nullptr,
-                       r.learning ? slot->d_tile_cost : nullptr, s->converge < 0 ? (int)s->has_branching_materials : s->converge,
+                       r.learning ? slot->d_tile_cost : nullptr, frame_converge(s),
                        nullptr, 0};
             if (use_stream) {
                 F.stream_counter = slot->d_stream_counter + k;
-                F.stream_blocks = slot->sm_count * 6;
+                F.stream_blocks = stream_blocks(slot->sm_count);
                 F.tile_order = nullptr, F.tile_cost = nullptr;
             }
             kernel_build(s->strict_fp, r.csg_sweep).render(r.scene, r.small, F, slot->d_counters, detailed, lane);
@@ -688,7 +688,7 @@ int render_impl(RtcScene* s, int depth, int shard0, int n_shards_ext, float* rgb
                 st.wave_overflows++;
                 const int b0 = k * chunk_bands, b1 = std::min(nb, b0 + chunk_bands);
                 DevFrame F{slot->d_rgb, slot->d_u8, shard, n_shards, depth, b1 - b0, b0, nullptr, nullptr, 1, slot->d_stream_counter + (k % 64),
-                           slot->sm_count * 6};
+                           stream_blocks(slot->sm_count)};
                 CUDA_TRY(cudaMemsetAsync(slot->d_stream_counter + (k % 64), 0, sizeof(unsigned), slot->stream));
                 kernel_build(s->strict_fp, rw.csg_sweep).render(rw.scene, rw.small, F, slot->d_counters, false, slot->stream);
                 CUDA_TRY(cudaGetLastError());
@@ -829,7 +829,7 @@ int render_views_impl(RtcScene* s, int depth, uint32_t n_views, const RtcView* v
     // both planes of every view of a chunk, as rtc_render's frame holds both
     size_t budget = kViewArenaBytes;
     if (const char* env = getenv("RTC_VIEW_ARENA_BYTES")) budget = (size_t)std::max(1LL, atoll(env));
-    const bool stream_scene = s->replicas[0].small.n == 0 && (s->stream < 0 ? s->has_branching_materials : s->stream != 0);
+    const bool stream_scene = streams_pixels(s, s->replicas[0].small);
     const int blocks_x = ((int)s->width + 7) / 8;
     const int nb_max = (total_bands + n_shards - 1) / n_shards;
     uint32_t chunk = (uint32_t)std::max<size_t>(1, std::min<size_t>(budget / (frame_px * 15), n_views));
@@ -923,9 +923,9 @@ int render_views_impl(RtcScene* s, int depth, uint32_t n_views, const RtcView* v
                 cudaStream_t lane = lanes[k % n_lanes];
                 const size_t off = (size_t)(L.v0 - c0) * frame_px * 3;
                 DevFrame F{d_rgb + off, d_u8 + off, shard, n_shards, depth, L.b1 - L.b0, L.b0, nullptr, nullptr,
-                           s->converge < 0 ? (int)s->has_branching_materials : s->converge, nullptr, 0};
+                           frame_converge(s), nullptr, 0};
                 if (stream_scene) {  // one launch at a time on the render stream: one counter does
-                    F.stream_counter = slot->d_stream_counter, F.stream_blocks = slot->sm_count * 6;
+                    F.stream_counter = slot->d_stream_counter, F.stream_blocks = stream_blocks(slot->sm_count);
                     CUDA_TRY(cudaMemsetAsync(slot->d_stream_counter, 0, sizeof(unsigned), lane));
                 }
                 kernel_build(s->strict_fp, r.csg_sweep).views(r.scene, r.small, F, slot->d_views + L.v0, (int)(L.v1 - L.v0), slot->d_counters, lane);

@@ -188,6 +188,17 @@ struct RtcScene {
 };
 
 namespace rtc {
+// What a render of the scene decides before it picks a kernel (rtc_launch.h: frame_variant), shared with the host harness
+// of the kernels (tests/emu/emu_kernels.cpp).  Tree scenes stream pixels (render_stream) when their ray trees branch,
+// unless RTC_STREAM forces it; `small` is the replica's small-scene table.
+inline bool streams_pixels(const RtcScene* s, const SmallScene& small) {
+    return small.n == 0 && (s->stream < 0 ? s->has_branching_materials : s->stream != 0);
+}
+// DevFrame::converge: the warp vote before every ray when the ray trees branch, unless RTC_CONVERGE forces it
+inline int frame_converge(const RtcScene* s) { return s->converge < 0 ? (int)s->has_branching_materials : s->converge; }
+// DevFrame::stream_blocks: render_stream's persistent grid, the resident blocks of its launch bounds (RTC_STREAM_MINBLOCKS)
+inline int stream_blocks(int sm_count) { return sm_count * 6; }
+
 // A tree builder other than the host's binned SAH (rtc_lbvh.cu: the device LBVH).  In: the padded boxes of the bounded
 // items (6 floats each: lo.xyz, hi.xyz), their "closed primitive" flags, the leaf size.  Out: the items' leaf order, the
 // binary nodes, the root link (>= 0 node, < 0 a leaf code: the whole tree is one leaf) and the tree's depth.  A non-zero

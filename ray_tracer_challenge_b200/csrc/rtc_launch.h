@@ -5,6 +5,40 @@
 #include "rtc_types.h"
 
 namespace rtc {
+// The kernel a launch function runs for its inputs.  launch_render, launch_views and launch_trace (rtc_kernels.cu) switch
+// on it, and so does the host harness of the kernels (tests/emu/emu_kernels.cpp), which thus runs the kernel the GPU runs.
+struct KernelVariant {
+    bool stream;  // render_stream / render_stream_views: a tree scene whose lanes draw pixels from F.stream_counter
+    // otherwise the template flags of render_tiles / render_tiles_views / trace_rays
+    bool stats, small, converge, drawn, lean;
+};
+constexpr int variant_code(bool stats, bool small, bool converge, bool drawn, bool lean) {
+    return (stats ? 16 : 0) | (small ? 8 : 0) | (converge ? 4 : 0) | (drawn ? 2 : 0) | (lean ? 1 : 0);
+}
+constexpr int variant_code(const KernelVariant& v) { return variant_code(v.stats, v.small, v.converge, v.drawn, v.lean); }
+
+// A frame or a batch of views.  detailed: the counting pass (launch_render only), which always uses the converging build;
+// the timed kernels pick by DevFrame::converge.  Small scenes whose area light draws its samples (jitter None) need the
+// build with the drawn-sample cell loop.  Lean scenes (SmallScene::lean, set only with cell_masks) take the lean build,
+// which does not use the per-thread shadow-origin cache: the part of kSmallSmemBytes before it is all it stages.
+// has_lean: the build has the lean kernel (the *_sweep builds have none: a scene that needs them holds a CSG, and a lean
+// one holds none).
+inline KernelVariant frame_variant(const DevScene& S, const SmallScene& SS, const DevFrame& F, bool detailed, bool has_lean) {
+    const bool small = SS.n > 0;
+    if (!small && F.stream_counter) return {true, detailed, false, true, false, false};  // the host zeroed the counter
+    const bool drawn = small && SS.cell_masks && S.jitter_len == 0;
+    const bool lean = has_lean && !detailed && !F.converge && small && SS.cell_masks && SS.lean;
+    return {false, detailed, small, detailed || F.converge != 0, drawn, lean};
+}
+// Caller-supplied rays: always the converging build, drawn by the predicate of frame_variant
+inline KernelVariant trace_variant(const DevScene& S, const SmallScene& SS) {
+    const bool small = SS.n > 0;
+    return {false, false, small, true, small && SS.cell_masks && S.jitter_len == 0, false};
+}
+// The dynamic shared memory of a tile or trace kernel: small scenes stage their table (dev_small.cuh); the lean build
+// stages only the part of kSmallSmemBytes before the shadow-origin cache
+inline int dynamic_smem(const KernelVariant& v) { return v.lean ? kSmemOrg * 16 : v.small ? kSmallSmemBytes : 0; }
+
 namespace fast {
 void launch_render(const DevScene& S, const SmallScene& SS, const DevFrame& F, DevCounters* counters, bool detailed,
                    cudaStream_t stream);

@@ -5,12 +5,6 @@
 // of rtc_scene_commit — would upload, so kernel logic can be compared with the oracle on a machine without a GPU.
 // With -ffp-contract=off the host evaluates the strict build's IEEE expression order; libm is glibc's on both sides.
 // It also runs the wavefront renderer's kernel sequence (dev_wave.cuh) over one chunk of a frame, one lane per "warp".
-#include <math.h>
-#include <string.h>
-
-#include <cmath>
-#include <cstdlib>
-#include <cstring>
 #include <vector>
 
 // one lane per "warp": wave_trace refills as soon as that lane is idle (with the default of 8 idle lanes it never
@@ -18,13 +12,8 @@
 #define RTC_REFILL_LANES 1
 #include "rtc_internal.h"  // Flattened, RtcScene, rtc::flatten (exported by librtc_b200.so)
 
-#undef __device__
-#undef __forceinline__
-#undef __noinline__
+#include "shim.h"
 #undef __shared__
-#define __device__
-#define __forceinline__ inline
-#define __noinline__ __attribute__((noinline))
 #define __shared__
 
 namespace {
@@ -35,44 +24,8 @@ struct EmuDim {
 static EmuDim threadIdx, blockIdx;
 static EmuDim blockDim{1, 1, 1}, gridDim{1, 1, 1};
 
-template <typename T>
-static inline T __ldg(const T* p) {
-    return *p;
-}
-static inline float __fmaf_rn(float a, float b, float c) { return std::fmaf(a, b, c); }
-static inline float __fdividef(float a, float b) { return a / b; }
-static inline float rsqrtf(float a) { return 1.0f / std::sqrt(a); }
-static inline int __float_as_int(float f) {
-    int i;
-    memcpy(&i, &f, 4);
-    return i;
-}
-static inline float __int_as_float(int i) {
-    float f;
-    memcpy(&f, &i, 4);
-    return f;
-}
-static inline unsigned __float_as_uint(float f) {
-    unsigned i;
-    memcpy(&i, &f, 4);
-    return i;
-}
-static inline float __uint_as_float(unsigned i) {
-    float f;
-    memcpy(&f, &i, 4);
-    return f;
-}
-static inline int __float2int_rz(float f) { return (int)f; }
-static inline unsigned __float2uint_rz(float f) { return f > 0.0f ? (unsigned)f : 0u; }
-static inline int min(int a, int b) { return a < b ? a : b; }
-static inline unsigned min(unsigned a, unsigned b) { return a < b ? a : b; }
-static inline unsigned max(unsigned a, unsigned b) { return a > b ? a : b; }
-[[noreturn]] static inline void __trap() { abort(); }
-static inline int max(int a, int b) { return a > b ? a : b; }
-static inline int __popc(unsigned v) { return __builtin_popcount(v); }
-static inline int __ffs(int v) { return __builtin_ffs(v); }
 static inline int __any_sync(unsigned, int p) { return p; }
-// PixelStream (dev_shade.cuh) is compiled but never run here: one lane per "warp"
+// PixelStream (dev_shade.cuh) is compiled but never run here: one lane per "warp" (simt.h runs it with 32)
 static inline unsigned __ballot_sync(unsigned, int p) { return p ? 1u : 0u; }
 static inline unsigned __shfl_sync(unsigned, unsigned v, int) { return v; }
 static inline unsigned __activemask() { return 1u; }
@@ -101,30 +54,7 @@ float4 rtc_smem[kSmallSmemBytes / sizeof(float4) + 64];  // the block's dynamic 
 #include "dev_shade.cuh"
 #include "dev_wave.cuh"
 
-namespace {
-// upload_replica (rtc_api.cu) with host pointers
-void host_scene(const RtcScene* s, const rtc::Flattened& f, rtc::DevScene& d) {
-    memset(&d, 0, sizeof(d));
-    rtc::rows3(s->cam_inv, d.cam_inv);
-    d.half_w = s->half_w, d.half_h = s->half_h, d.pixel_size = s->pixel_size;
-    d.width = (int)s->width, d.height = (int)s->height;
-    d.light_is_rect = s->light_is_rect;
-    memcpy(d.light_pos, s->light_pos, 12);
-    memcpy(d.light_rgb, s->light_rgb, 12);
-    memcpy(d.corner, s->corner, 12);
-    memcpy(d.u_vec, s->u_cell, 12);
-    memcpy(d.v_vec, s->v_cell, 12);
-    d.u_steps = s->u_steps, d.v_steps = s->v_steps, d.cells = s->u_steps * s->v_steps;
-    d.jitter_len = (int)s->jitter.size();
-    d.seed = s->seed;
-    auto at = [](const auto& v) { return v.empty() ? nullptr : v.data(); };
-    d.jitter = at(s->jitter), d.samples = at(f.samples), d.head = at(f.head), d.rec = at(f.rec), d.xform = at(f.xform);
-    d.tri = at(f.tri), d.bound = at(f.bound), d.bvh = at(f.bvh), d.linear = at(f.linear), d.nodes = at(f.nodes);
-    d.csg_ops = at(f.ops), d.materials = at(f.materials), d.patterns = at(f.patterns), d.uvs = at(f.uvs), d.texels = at(f.texels);
-    d.small_image = at(f.small_image);
-    d.n_linear = (int)f.linear.size(), d.bvh_root = f.bvh_root, d.n_prims = f.n_pos, d.all_cast_shadow = f.all_cast_shadow;
-}
-}  // namespace
+#include "host_scene.h"
 
 static unsigned long long g_rays[4];  // primary, secondary, shadow rays and shades of the last emu_color_at call
 extern "C" void emu_last_rays(unsigned long long out[4]) { memcpy(out, g_rays, sizeof(g_rays)); }
@@ -170,6 +100,39 @@ extern "C" int emu_color_at(RtcScene* s, uint32_t n, const float* origins, const
         g_rays[0] += r.primary, g_rays[1] += r.secondary, g_rays[2] += r.shadow, g_rays[3] += r.shades;
         out_rgb[3 * (size_t)i] = c.x, out_rgb[3 * (size_t)i + 1] = c.y, out_rgb[3 * (size_t)i + 2] = c.z;
         if (out_t) out_t[i] = t;
+    }
+    return 0;
+}
+
+// The detailed pass's work counters of every ray, one lane at a time: color_at<STATS = true> in the converging build, as
+// render_tiles<true, ...> runs it.  out: n x kRayCounts, in the order of the fields below.
+constexpr int kRayCounts = 19;
+extern "C" int emu_color_at_counts(RtcScene* s, uint32_t n, const float* origins, const float* directions, int depth,
+                                   unsigned* out) {
+    using namespace rtc;
+    Flattened f;
+    if (int rc = flatten(s, f)) return rc;
+    DevScene S;
+    host_scene(s, f, S);
+    const SmallScene SS = f.small;
+    const bool small = SS.n > 0, drawn = small && SS.cell_masks && S.jitter_len == 0;
+    const emu::Env E{S, SS};
+    for (uint32_t i = 0; i < n; i++) {
+        if (small) emu::stage_small_scene(S, SS);
+        const emu::V3 o = emu::ld3(origins + 3 * (size_t)i), d = emu::ld3(directions + 3 * (size_t)i);
+        emu::Ctr<true> k;
+        emu::Rays r;
+        if (drawn)
+            emu::color_at<true, true, true, true>(E, true, o, d, depth, i, r, k, nullptr, nullptr);
+        else if (small)
+            emu::color_at<true, true, true, false>(E, true, o, d, depth, i, r, k, nullptr, nullptr);
+        else
+            emu::color_at<true, false, true, false>(E, true, o, d, depth, i, r, k, nullptr, nullptr);
+        unsigned* c = out + (size_t)i * kRayCounts;
+        c[0] = k.nodes;
+        for (int j = 0; j < 8; j++) c[1 + j] = k.prims[j];
+        c[9] = k.xforms, c[10] = k.patterns, c[11] = k.cells, c[12] = k.schlicks, c[13] = k.refr_dirs, c[14] = k.overflows;
+        c[15] = k.refilters, c[16] = r.secondary, c[17] = r.shades, c[18] = r.primary;
     }
     return 0;
 }

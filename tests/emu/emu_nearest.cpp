@@ -9,29 +9,7 @@
 
 #include "rtc_internal.h"  // Flattened, RtcScene, rtc::flatten (exported by librtc_b200.so)
 
-#undef __device__
-#undef __forceinline__
-#undef __noinline__
-#define __device__
-#define __forceinline__ inline
-#define __noinline__ __attribute__((noinline))
-
-template <typename T>
-static inline T __ldg(const T* p) {
-    return *p;
-}
-static inline float __fmaf_rn(float a, float b, float c) { return std::fmaf(a, b, c); }
-static inline float __fdividef(float a, float b) { return a / b; }
-static inline int __float_as_int(float f) {
-    int i;
-    memcpy(&i, &f, 4);
-    return i;
-}
-static inline float __int_as_float(int i) {
-    float f;
-    memcpy(&f, &i, 4);
-    return f;
-}
+#include "shim.h"
 
 #define RTC_NS emu
 #include "dev_math.cuh"

@@ -18,7 +18,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CUDA_INCLUDE = "/usr/local/cuda/include"
 
 
-def _build(tmp_path_factory, source):
+def _build(tmp_path_factory, source, defines=()):
     import ray_tracer_challenge_b200 as rt
 
     if shutil.which("g++") is None or not os.path.isdir(CUDA_INCLUDE):
@@ -30,7 +30,12 @@ def _build(tmp_path_factory, source):
     # under AddressSanitizer + UBSan — the memcheck pass a host can give CUDA code
     sanitize = ["-fsanitize=address,undefined", "-fno-omit-frame-pointer", "-fno-sanitize-recover=undefined"] \
         if os.environ.get("RTC_EMU_SANITIZE") else []
-    subprocess.run(["g++", "-std=c++17", "-O1", "-ffp-contract=off", "-fPIC", "-shared", *sanitize, "-I", CUDA_INCLUDE,
+    # RTC_EMU_TSAN=1 (test_kernels_under_thread_sanitizer, libtsan preloaded): the host threads of emu_kernels.cpp's
+    # blocks under ThreadSanitizer — the racecheck pass
+    if os.environ.get("RTC_EMU_TSAN"):
+        sanitize = ["-fsanitize=thread", "-fno-omit-frame-pointer"]
+    subprocess.run(["g++", "-std=c++17", "-O1", "-ffp-contract=off", "-fPIC", "-shared", "-pthread", *sanitize, *defines,
+                    "-I", CUDA_INCLUDE,
                     "-I", os.path.join(ROOT, "ray_tracer_challenge_b200", "csrc"), os.path.join(ROOT, "tests", "emu", source),
                     "-o", str(out), "-L", lib_dir, "-lrtc_b200", f"-Wl,-rpath,{lib_dir}"], check=True)
     device = rt.device_library()  # the raw C ABI; RTLD_GLOBAL, so the harness binds rtc::flatten from it
