@@ -304,6 +304,30 @@ typedef struct RtcView {
  *     rtc_set_camera keeps its meaning (it invalidates the commit). */
 int rtc_render_views(RtcScene*, int32_t depth, uint32_t n_views, const RtcView* views, float* rgb_f32, uint8_t* rgb_u8,
                      RtcStats* stats);
+/* Camera::render followed by Canvas::to_ppm (canvas.rs:58-96), the last step of every demo, with the text written on the
+ * device.  rtc_ppm_bound is host arithmetic: the header's length plus width * height * 3 * 4 bytes (three digits and a
+ * separator per value), an upper bound on the text of any frame of that size.
+ *   - ppm receives exactly the bytes Canvas::to_ppm returns for the rendered canvas: "P3\n{w} {h}\n255\n", then every row's
+ *     values in decimal without padding, each followed by a space while the line is shorter than 70 - 3 columns and by a
+ *     newline otherwise, and by a newline after the row's last value.  The rows and columns the reference does not render
+ *     (camera.rs:80-81) are zeros.  *ppm_bytes receives the length; no terminating NUL is written.
+ *   - The arguments are checked before the scene's state, all with RTC_ERR_INVALID: ppm or ppm_bytes NULL; a capacity below
+ *     rtc_ppm_bound of the committed canvas; a depth outside [0, 23] (rtc_render's rule).  Then an uncommitted scene is
+ *     RTC_ERR_STATE.
+ *   - The render is rtc_render's with the frame left on the device; stats are rtc_render's (kernel_ms: the render kernels),
+ *     except total_ms, which covers the whole call.  The text is written from the device's 8-bit plane: the value bytes of a
+ *     row do not depend on the line breaks, so each device first computes the byte length of each of its rows, the host
+ *     scans the lengths of all rows (one small device-to-host copy and a synchronize per call), and each device then writes
+ *     its bands' text and copies each band to its offset in ppm.
+ *   - Pinned and pageable destinations both work.  A pageable one receives texts of 4 MiB or more through the pinned staging
+ *     frame that rtc_render uses for its 8-bit plane, grown to the device's share of the text and kept with the device.
+ *   - Device memory kept with each device for later calls: the text of its rows (up to 12 bytes per pixel, 89 MB for a
+ *     3840x2160 frame) and 16 bytes per row.
+ *   - Not provided: a shard of a frame shared by several processes (rtc_render_shard) — a process cannot know the offsets of
+ *     rows other processes render; batches of views (rtc_render_views); encoding a plane that is not the committed scene's
+ *     frame. */
+size_t rtc_ppm_bound(uint32_t width, uint32_t height);
+int rtc_render_ppm(RtcScene*, int32_t depth, char* ppm, size_t capacity, size_t* ppm_bytes, RtcStats* stats);
 /* World::color_at (world.rs:88-101) for caller-supplied rays: origins / directions are n*3 f32; out_rgb n*3;
  * out_t (optional) the hit distance or -1; out_prim (optional) the hit primitive index or -1. */
 int rtc_trace_rays(RtcScene*, uint32_t n, const float* origins, const float* directions, int32_t depth,

@@ -109,6 +109,9 @@ _HOST_EXTRAS = {
     "sg_camera_render_views": (_I, [_V, _IP, _I, _I, _I, _FP, _U8P, C.POINTER(SgStats)]),
     "sg_camera_view": (_I, [_V, _I, C.POINTER(RtcView)]),
     "sg_farthest_camera": (_I, [_V, _IP, _I]),
+    "sg_camera_render_ppm": (C.c_int64, [_V, _I, _I, _I, C.c_void_p, C.c_int64, C.POINTER(SgStats)]),
+    "sg_render_prepared_ppm": (C.c_int64, [_V, _I, _I, _I, C.c_void_p, C.c_int64, C.POINTER(SgStats)]),
+    "rtc_ppm_bound": (C.c_size_t, [C.c_uint32, C.c_uint32]),  # librtc_b200.so, reached through the host library
 }
 
 
@@ -128,6 +131,16 @@ def _view_planes(n, h, w, want_rgb, want_u8, out_rgb, out_u8):
         if u8.shape != (n, h, w, 3) or u8.dtype != np.uint8 or not u8.flags.c_contiguous:
             raise ValueError(f"out_u8 must be a C-contiguous uint8 array of shape {(n, h, w, 3)}")
     return rgb, u8
+
+
+def _ppm_buffer(api, w, h, out):
+    """The bytes rtc_render_ppm writes into: the caller's C-contiguous uint8 array (e.g. over pinned memory) or a new one,
+    at least rtc_ppm_bound bytes."""
+    bound = api.lib.rtc_ppm_bound(w, h)
+    buf = out if out is not None else np.empty(bound, np.uint8)
+    if buf.dtype != np.uint8 or not buf.flags.c_contiguous or not buf.flags.writeable or buf.nbytes < bound:
+        raise ValueError(f"out must be a writable C-contiguous uint8 array of at least rtc_ppm_bound = {bound} bytes")
+    return buf
 
 
 def _canvases(api, n, h, w, rgb, u8):
@@ -175,6 +188,19 @@ class PreparedScene:
             u8.ctypes.data_as(_U8P) if u8 is not None else None, C.byref(stats)))
         self.last_stats = api.last_rtc_stats()
         return _canvases(api, n, h, w, rgb, u8)
+
+    def render_ppm(self, depth=DEFAULT_RAY_RECURSION_DEPTH, out=None, fma=False) -> str:
+        """rtc_render_ppm: the committed scene rendered and its frame's `Canvas::to_ppm` text (canvas.rs:58-96) written on the
+        device.  `out`: where the bytes land (a writable uint8 array of at least rtc_ppm_bound bytes, e.g. over pinned memory);
+        a new pageable one by default."""
+        w, h = self.camera.width_pixels, self.camera.height_pixels
+        api = self.api
+        buf = _ppm_buffer(api, w, h, out)
+        stats = SgStats()
+        n = api.check(api.lib.sg_render_prepared_ppm(api.ctx, self.handle, int(depth), int(fma), buf.ctypes.data, buf.nbytes,
+                                                     C.byref(stats)))
+        self.last_stats = api.last_rtc_stats()
+        return buf[:n].tobytes().decode("ascii")
 
     def trace_rays(self, origins, directions, depth=DEFAULT_RAY_RECURSION_DEPTH, fma=False):
         """World::color_at (world.rs:88-101) for arbitrary rays: returns (rgb[n,3], t[n], shape_handle[n])."""
@@ -248,8 +274,21 @@ class HostApi(_api.Api):
             camera.last_rtc_stats = api.last_rtc_stats()
             return CanvasU8(w, h, u8, api)
 
+        def render_b200_ppm(camera, world, reflection_recursion_depth=DEFAULT_RAY_RECURSION_DEPTH, out=None) -> str:
+            """The demos' flow, `camera.render(world, depth).to_ppm()`, in one call: flatten, commit, render, and the frame's
+            PPM text written on the device (rtc_render_ppm).  `out` as PreparedScene.render_ppm's."""
+            w, h = camera.width_pixels, camera.height_pixels
+            buf = _ppm_buffer(api, w, h, out)
+            stats = SgStats()
+            n = api.check(api.lib.sg_camera_render_ppm(api.ctx, camera.handle, world.handle, int(reflection_recursion_depth),
+                                                       buf.ctypes.data, buf.nbytes, C.byref(stats)))
+            camera.last_stats = stats
+            camera.last_rtc_stats = api.last_rtc_stats()
+            return buf[:n].tobytes().decode("ascii")
+
         self.Camera.render_b200 = render_b200
         self.Camera.render_b200_u8 = render_b200_u8
+        self.Camera.render_b200_ppm = render_b200_ppm
         self.Camera.render = render_b200
         self.Camera.prepare = lambda camera, world: PreparedScene(api, camera, world)
 

@@ -1,6 +1,7 @@
 """In-tree build of the native libraries (sm_100a only; nvcc cross-compiles without a GPU).
 
     librtc_b200.so  the C ABI of include/rtc_b200.h: csrc/rtc_api.cu + csrc/rtc_commit.cu (host half of a commit) + csrc/rtc_lbvh.cu (device tree builder) +
+                    csrc/rtc_ppm.cu (PPM text kernels) +
                     csrc/rtc_kernels.cu compiled four times
                     (FMA-contracting `fast` build and -fmad=false `strict` build, each again with csg_sweep's call sites
                     for scenes holding a CSG beyond csg_eval's limits)
@@ -53,6 +54,7 @@ def build(force: bool = False, verbose: bool = False) -> None:
     api = os.path.join(CSRC, "rtc_api.cu")
     commit = os.path.join(CSRC, "rtc_commit.cu")
     lbvh = os.path.join(CSRC, "rtc_lbvh.cu")
+    ppm = os.path.join(CSRC, "rtc_ppm.cu")
     objs = {
         os.path.join(BUILD, "kernels_fast.o"): [NVCC, *NVCC_FLAGS, "-c", kernels],
         os.path.join(BUILD, "kernels_strict.o"): [NVCC, *NVCC_FLAGS, "-DRTC_STRICT", "-fmad=false", "-c", kernels],
@@ -62,6 +64,7 @@ def build(force: bool = False, verbose: bool = False) -> None:
         os.path.join(BUILD, "api.o"): [NVCC, *NVCC_FLAGS, "-c", api],
         os.path.join(BUILD, "commit.o"): [NVCC, *NVCC_FLAGS, "-c", commit],
         os.path.join(BUILD, "lbvh.o"): [NVCC, *NVCC_FLAGS, "-c", lbvh],
+        os.path.join(BUILD, "ppm.o"): [NVCC, *NVCC_FLAGS, "-c", ppm],
     }
     jobs = []
     for obj, cmd in objs.items():

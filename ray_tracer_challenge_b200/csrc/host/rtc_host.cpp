@@ -179,6 +179,49 @@ static int commit(sg_ctx* c, RtcScene* scene, bool one_shot, size_t n_prims) {
     return 0;
 }
 
+// Camera::render_b200 — one call: flatten, commit, render, copy back, release.  With n_shards > 1 the call renders
+// and copies only the bands of `shard` (one process per GPU, every process making the same one-shot call on its own
+// device for one shared frame); either plane may be null (not copied: the reference's demos only ever serialise the
+// 8-bit values, canvas.rs:58-96).  `render` makes the render call on the committed scene.
+template <class Render>
+static int one_shot(sg_ctx* c, int cam, int w, sg_stats* stats, Render render) {
+    if (cam < 0 || cam >= (int)c->cameras.size()) return fail("bad camera handle");
+    if (w < 0 || w >= (int)c->worlds.size()) return fail("bad world handle");
+    RtcScene* scene = nullptr;
+    if (rtc_scene_create(&scene)) return fail(rtc_last_error());
+    int rc = 0;
+    try {
+        auto t0 = std::chrono::steady_clock::now();
+        const bool timing = getenv("RTC_TIMING") != nullptr;  // tuning aid: where a one-shot render spends its time
+        auto mark = [&, last = t0](const char* what) mutable {
+            if (!timing) return;
+            const auto now = std::chrono::steady_clock::now();
+            fprintf(stderr, "[rtc one-shot] %-28s %8.3f ms\n", what, std::chrono::duration<double, std::milli>(now - last).count());
+            last = now;
+        };
+        FlatScene flat;
+        fill_scene(scene, c->graph, c->worlds[w], c->cameras[cam], flat);
+        mark("fill_scene");
+        rc = commit(c, scene, true, flat.n_prims);
+        mark("commit (host half + upload)");
+        if (!rc) {
+            rc = render(scene);
+            if (rc) fail(rtc_last_error());
+            mark("render + copies");
+        }
+        c->last_stats.total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+        to_sg_stats(c->last_stats, stats);
+    } catch (const std::exception& e) {
+        rc = fail(e.what());
+    }
+    const auto t1 = std::chrono::steady_clock::now();
+    rtc_scene_destroy(scene);
+    if (getenv("RTC_TIMING"))
+        fprintf(stderr, "[rtc one-shot] %-28s %8.3f ms\n", "scene destroy",
+                std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t1).count());
+    return rc ? -1 : 0;
+}
+
 extern "C" {
 
 const char* sg_last_error(void) { return g_err.c_str(); }
@@ -422,51 +465,13 @@ int sg_last_rtc_stats(sg_ctx* c, RtcStats* out) {
     return 0;
 }
 
-// Camera::render_b200 — one call: flatten, commit, render, copy back, release.  With n_shards > 1 the call renders
-// and copies only the bands of `shard` (one process per GPU, every process making the same one-shot call on its own
-// device for one shared frame); either plane may be null (not copied: the reference's demos only ever serialise the
-// 8-bit values, canvas.rs:58-96).
 static int camera_render(sg_ctx* c, int cam, int w, int depth, int shard, int n_shards, float* out_rgb, uint8_t* out_u8,
                          sg_stats* stats) {
-    if (cam < 0 || cam >= (int)c->cameras.size()) return fail("bad camera handle");
-    if (w < 0 || w >= (int)c->worlds.size()) return fail("bad world handle");
-    RtcScene* scene = nullptr;
-    if (rtc_scene_create(&scene)) return fail(rtc_last_error());
-    int rc = 0;
-    try {
-        auto t0 = std::chrono::steady_clock::now();
-        const bool timing = getenv("RTC_TIMING") != nullptr;  // tuning aid: where a one-shot render spends its time
-        auto mark = [&, last = t0](const char* what) mutable {
-            if (!timing) return;
-            const auto now = std::chrono::steady_clock::now();
-            fprintf(stderr, "[rtc one-shot] %-28s %8.3f ms\n", what, std::chrono::duration<double, std::milli>(now - last).count());
-            last = now;
-        };
-        FlatScene flat;
-        fill_scene(scene, c->graph, c->worlds[w], c->cameras[cam], flat);
-        mark("fill_scene");
-        rc = commit(c, scene, true, flat.n_prims);
-        mark("commit (host half + upload)");
-        if (!rc) {
-            if (n_shards > 1)
-                rc = rtc_render_shard(scene, depth, shard, n_shards, out_rgb, out_u8, &c->last_stats);
-            else
-                rc = c->options.detailed ? rtc_render_detailed(scene, depth, out_rgb, out_u8, &c->last_stats)
-                                         : rtc_render(scene, depth, out_rgb, out_u8, &c->last_stats);
-            if (rc) fail(rtc_last_error());
-            mark("render + copies");
-        }
-        c->last_stats.total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-        to_sg_stats(c->last_stats, stats);
-    } catch (const std::exception& e) {
-        rc = fail(e.what());
-    }
-    const auto t1 = std::chrono::steady_clock::now();
-    rtc_scene_destroy(scene);
-    if (getenv("RTC_TIMING"))
-        fprintf(stderr, "[rtc one-shot] %-28s %8.3f ms\n", "scene destroy",
-                std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t1).count());
-    return rc ? -1 : 0;
+    return one_shot(c, cam, w, stats, [&](RtcScene* scene) {
+        if (n_shards > 1) return rtc_render_shard(scene, depth, shard, n_shards, out_rgb, out_u8, &c->last_stats);
+        return c->options.detailed ? rtc_render_detailed(scene, depth, out_rgb, out_u8, &c->last_stats)
+                                   : rtc_render(scene, depth, out_rgb, out_u8, &c->last_stats);
+    });
 }
 int sg_camera_render(sg_ctx* c, int cam, int w, int depth, float* out_rgb, uint8_t* out_u8, sg_stats* stats) {
     return camera_render(c, cam, w, depth, 0, 1, out_rgb, out_u8, stats);
@@ -475,6 +480,17 @@ int sg_camera_render_shard(sg_ctx* c, int cam, int w, int depth, int shard, int 
                            sg_stats* stats) {
     if (n_shards < 1 || shard < 0 || shard >= n_shards) return fail("bad shard index");
     return camera_render(c, cam, w, depth, shard, n_shards, out_rgb, out_u8, stats);
+}
+
+// Camera::render_b200_ppm — the demos' `camera.render(world, depth).to_ppm()` in one call: flatten, commit, render, the
+// frame's PPM text written on the device into `out` (capacity >= rtc_ppm_bound of the camera's canvas).  Returns the
+// text's length, or -1.
+int64_t sg_camera_render_ppm(sg_ctx* c, int cam, int w, int depth, char* out, int64_t capacity, sg_stats* stats) {
+    if (capacity < 0) return fail("negative capacity");
+    size_t bytes = 0;
+    const int rc = one_shot(c, cam, w, stats,
+                            [&](RtcScene* scene) { return rtc_render_ppm(scene, depth, out, (size_t)capacity, &bytes, &c->last_stats); });
+    return rc ? -1 : (int64_t)bytes;
 }
 
 // A batch of views: the cameras' RtcViews, every camera of the committed canvas size (or the call fails)
@@ -589,6 +605,17 @@ int sg_render_prepared(sg_ctx* c, int h, int depth, int shard, int n_shards, int
         rc = rtc_render(scene, depth, out_rgb, out_u8, &c->last_stats);
     to_sg_stats(c->last_stats, stats);
     return rc ? fail(rtc_last_error()) : 0;
+}
+// rtc_render_ppm on a prepared scene: returns the text's length, or -1
+int64_t sg_render_prepared_ppm(sg_ctx* c, int h, int depth, int fma, char* out, int64_t capacity, sg_stats* stats) {
+    if (h < 0 || h >= (int)c->prepared.size() || !c->prepared[h]) return fail("bad prepared handle");
+    if (capacity < 0) return fail("negative capacity");
+    RtcScene* scene = c->prepared[h]->scene;
+    if (rtc_set_option(scene, RTC_OPT_FMA_CONTRACTION, fma ? 1 : 0)) return fail(rtc_last_error());
+    size_t bytes = 0;
+    const int rc = rtc_render_ppm(scene, depth, out, (size_t)capacity, &bytes, &c->last_stats);
+    to_sg_stats(c->last_stats, stats);
+    return rc ? fail(rtc_last_error()) : (int64_t)bytes;
 }
 // rtc_render_views on a prepared scene: n cameras (handles) of its canvas size, frames view-major in out_rgb / out_u8
 int sg_render_prepared_views(sg_ctx* c, int h, int depth, int n, const int* cams, int fma, float* out_rgb, uint8_t* out_u8,

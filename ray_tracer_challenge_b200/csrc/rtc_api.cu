@@ -986,6 +986,146 @@ int render_views_impl(RtcScene* s, int depth, uint32_t n_views, const RtcView* v
     return 0;
 }
 
+// rtc_render_ppm ---------------------------------------------------------------------------------------------------------
+int ensure_ppm_rows(DeviceSlot* d, size_t rows) {
+    if (rows <= d->ppm_rows) return 0;
+    CUDA_TRY(cudaSetDevice(d->device));
+    if (d->d_ppm_rows) cudaFree(d->d_ppm_rows);
+    if (d->h_ppm_rows) cudaFreeHost(d->h_ppm_rows);
+    d->d_ppm_rows = nullptr, d->h_ppm_rows = nullptr, d->ppm_rows = 0;
+    CUDA_TRY(cudaMalloc(&d->d_ppm_rows, rows * sizeof(unsigned long long)));
+    CUDA_TRY(cudaHostAlloc(&d->h_ppm_rows, rows * sizeof(unsigned long long), cudaHostAllocDefault));
+    d->ppm_rows = rows;
+    return 0;
+}
+int ensure_ppm_text(DeviceSlot* d, size_t bytes) {
+    if (bytes <= d->ppm_bytes) return 0;
+    CUDA_TRY(cudaSetDevice(d->device));
+    if (d->d_ppm) cudaFree(d->d_ppm);
+    d->d_ppm = nullptr, d->ppm_bytes = 0;
+    const size_t cap = bytes + bytes / 8;  // a slightly busier frame of the same size does not reallocate
+    CUDA_TRY(cudaMalloc(&d->d_ppm, cap));
+    d->ppm_bytes = cap;
+    return 0;
+}
+
+// Render, then on every device: the byte lengths of its rows' text, one copy back and a synchronize, the host's scan over
+// all rows (ppm_layout), the text of its rows into d_ppm, and the copies of its bands to their offsets in `ppm`.
+int render_ppm_impl(RtcScene* s, int depth, char* ppm, size_t capacity, size_t* ppm_bytes, RtcStats* stats) {
+    // the arguments first (no device needed), then the scene's state
+    if (!s) return fail(RTC_ERR_INVALID, "null scene");
+    if (!ppm || !ppm_bytes) return fail(RTC_ERR_INVALID, "rtc_render_ppm: ppm and ppm_bytes must be non-null");
+    const size_t bound = rtc_ppm_bound(s->width, s->height);
+    if (capacity < bound)
+        return fail(RTC_ERR_INVALID, "rtc_render_ppm: capacity " + std::to_string(capacity) + " is below rtc_ppm_bound = " +
+                                         std::to_string(bound));
+    if (depth < 0 || depth > kMaxFrames - 1)
+        return fail(RTC_ERR_INVALID, "reflection_recursion_depth must be in [0, " + std::to_string(kMaxFrames - 1) + "]");
+    if (!s->committed) return fail(RTC_ERR_STATE, "rtc_render_ppm before rtc_scene_commit");
+    const auto t0 = std::chrono::steady_clock::now();
+    RtcStats st;
+    memset(&st, 0, sizeof(st));
+    if (int rc = render_impl(s, depth, 0, 0, nullptr, nullptr, &st, false)) {  // the frame stays on the device
+        if (stats) *stats = st;
+        return rc;
+    }
+    const int ndev = (int)s->replicas.size();
+    const int total_bands = ((int)s->height + kBandRows - 1) / kBandRows;
+    std::vector<PpmRows> rows(ndev);
+    std::vector<unsigned long long*> lengths(ndev);
+    for (int i = 0; i < ndev; i++) {
+        DeviceSlot* slot = s->replicas[i].slot;
+        CUDA_TRY(cudaSetDevice(slot->device));
+        rows[i] = PpmRows{slot->d_u8, (int)s->width, i, ndev, ppm_device_rows(s->height, i, ndev)};
+        if (int rc = ensure_ppm_rows(slot, std::max(rows[i].n_rows, 1))) return rc;
+        lengths[i] = slot->h_ppm_rows;
+        launch_ppm_row_bytes(rows[i], slot->d_ppm_rows, slot->sm_count, slot->stream);
+        CUDA_TRY(cudaGetLastError());
+        CUDA_TRY(cudaMemcpyAsync(slot->h_ppm_rows, slot->d_ppm_rows, rows[i].n_rows * sizeof(unsigned long long), cudaMemcpyDeviceToHost,
+                                 slot->stream));
+    }
+    for (int i = 0; i < ndev; i++) {
+        CUDA_TRY(cudaSetDevice(s->replicas[i].slot->device));
+        CUDA_TRY(cudaStreamSynchronize(s->replicas[i].slot->stream));
+    }
+    const std::string header = ppm_header(s->width, s->height);
+    PpmLayout L;
+    ppm_layout(s->height, ndev, header.size(), lengths.data(), L);
+    if (L.total > capacity) return fail(RTC_ERR_CAPACITY, "rtc_render_ppm: the text outgrew rtc_ppm_bound");  // cannot happen
+    memcpy(ppm, header.data(), header.size());
+    // A pageable destination (a String, a NumPy array): as rtc_render's planes, the text lands in the pinned staging frame of
+    // the device slot piece by piece, and the host's threads move each piece on as soon as its copy has arrived.
+    const bool staged = L.total >= ((size_t)4 << 20) && is_pageable(ppm);
+    struct Piece {
+        DeviceSlot* slot;
+        int dev, j0, j1;  // bands [j0, j1) of the device's band list
+        cudaEvent_t done;
+    };
+    std::vector<Piece> pieces;
+    for (int i = 0; i < ndev; i++) {
+        DeviceSlot* slot = s->replicas[i].slot;
+        CUDA_TRY(cudaSetDevice(slot->device));
+        if (int rc = ensure_ppm_text(slot, std::max<size_t>(L.device_bytes[i], 16))) return rc;
+        CUDA_TRY(cudaMemcpyAsync(slot->d_ppm_rows, slot->h_ppm_rows, rows[i].n_rows * sizeof(unsigned long long), cudaMemcpyHostToDevice,
+                                 slot->stream));
+        launch_ppm_write(rows[i], slot->d_ppm_rows, slot->d_ppm, slot->sm_count, slot->stream);
+        CUDA_TRY(cudaGetLastError());
+        const int nb = i < total_bands ? (total_bands - i + ndev - 1) / ndev : 0;
+        if (nb == 0) continue;
+        // pieces of about 4 MiB (whole bands) when staged, so that the host's copies overlap the device's; else one
+        const int n_pieces = staged ? (int)std::max<size_t>(1, std::min<size_t>((size_t)nb, L.device_bytes[i] >> 22)) : 1;
+        if (staged)
+            if (int rc = ensure_stage(slot, &slot->h_stage_u8, &slot->h_stage_u8_bytes, L.device_bytes[i])) return rc;
+        for (int k = 0; k < n_pieces; k++) {
+            const int j0 = (int)((int64_t)nb * k / n_pieces), j1 = (int)((int64_t)nb * (k + 1) / n_pieces);
+            const size_t local = L.band_local[i + j0 * ndev];
+            const size_t bytes = L.band_local[i + (j1 - 1) * ndev] + L.band_bytes[i + (j1 - 1) * ndev] - local;
+            if (staged) {
+                CUDA_TRY(cudaMemcpyAsync(slot->h_stage_u8 + local, slot->d_ppm + local, bytes, cudaMemcpyDeviceToHost, slot->stream));
+                const size_t used = pieces.size();
+                while (slot->copy_done.size() <= used) {
+                    cudaEvent_t e;
+                    CUDA_TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+                    slot->copy_done.push_back(e);
+                }
+                CUDA_TRY(cudaEventRecord(slot->copy_done[used], slot->stream));
+                pieces.push_back({slot, i, j0, j1, slot->copy_done[used]});
+            } else if (ndev == 1) {  // the device's text is the frame's
+                CUDA_TRY(cudaMemcpyAsync(ppm + L.band_at[j0], slot->d_ppm + local, bytes, cudaMemcpyDeviceToHost, slot->stream));
+            } else {
+                for (int j = j0; j < j1; j++) {
+                    const int b = i + j * ndev;
+                    CUDA_TRY(cudaMemcpyAsync(ppm + L.band_at[b], slot->d_ppm + L.band_local[b], L.band_bytes[b], cudaMemcpyDeviceToHost,
+                                             slot->stream));
+                }
+            }
+        }
+    }
+    for (const Piece& p : pieces) {
+        CUDA_TRY(cudaSetDevice(p.slot->device));
+        CUDA_TRY(cudaEventSynchronize(p.done));
+        if (ndev == 1) {
+            const size_t at = L.band_at[p.j0], bytes = L.band_at[p.j1 - 1] + L.band_bytes[p.j1 - 1] - at;
+            parallel_copy(ppm + at, p.slot->h_stage_u8 + L.band_local[p.j0], bytes, (size_t)96 << 10);
+            continue;
+        }
+        parallel_for((size_t)(p.j1 - p.j0), 1, [&](size_t jb, size_t je, int) {
+            for (size_t j = jb; j < je; j++) {
+                const int b = p.dev + (p.j0 + (int)j) * ndev;
+                memcpy(ppm + L.band_at[b], p.slot->h_stage_u8 + L.band_local[b], L.band_bytes[b]);
+            }
+        });
+    }
+    for (int i = 0; i < ndev; i++) {
+        CUDA_TRY(cudaSetDevice(s->replicas[i].slot->device));
+        CUDA_TRY(cudaStreamSynchronize(s->replicas[i].slot->stream));
+    }
+    *ppm_bytes = L.total;
+    st.total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    if (stats) *stats = st;
+    return 0;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1262,6 +1402,12 @@ int rtc_render_detailed(RtcScene* s, int32_t depth, float* rgb, uint8_t* u8, Rtc
 }
 int rtc_render_views(RtcScene* s, int32_t depth, uint32_t n_views, const RtcView* views, float* rgb, uint8_t* u8, RtcStats* stats) {
     return render_views_impl(s, depth, n_views, views, rgb, u8, stats);
+}
+size_t rtc_ppm_bound(uint32_t width, uint32_t height) {
+    return ppm_header(width, height).size() + (size_t)width * height * 3 * 4;
+}
+int rtc_render_ppm(RtcScene* s, int32_t depth, char* ppm, size_t capacity, size_t* ppm_bytes, RtcStats* stats) {
+    return render_ppm_impl(s, depth, ppm, capacity, ppm_bytes, stats);
 }
 
 int rtc_trace_rays(RtcScene* s, uint32_t n, const float* origins, const float* directions, int32_t depth, float* out_rgb,

@@ -1,6 +1,7 @@
 // rtc_internal.h — structures shared by the two host translation units of librtc_b200.so: rtc_api.cu (C ABI, device
 // resources, upload, render) and rtc_commit.cu (the host half of a commit: validation, BVH, CSG programs, tables).
 #pragma once
+#include <algorithm>
 #include <cmath>
 #include <cstdint>
 #include <string>
@@ -89,6 +90,13 @@ struct DeviceSlot {
     uint32_t views_capacity = 0;
     char* d_view_frames = nullptr;
     size_t view_frames_bytes = 0;
+    // rtc_render_ppm (grow-only): the text of this device's rows, and their byte lengths, then offsets, on the device and
+    // pinned on the host.  A pageable destination is staged through h_stage_u8.
+    char* d_ppm = nullptr;
+    size_t ppm_bytes = 0;
+    unsigned long long* d_ppm_rows = nullptr;
+    unsigned long long* h_ppm_rows = nullptr;
+    size_t ppm_rows = 0;
 };
 
 // One committed replica of the scene on one device.
@@ -198,6 +206,45 @@ inline bool streams_pixels(const RtcScene* s, const SmallScene& small) {
 inline int frame_converge(const RtcScene* s) { return s->converge < 0 ? (int)s->has_branching_materials : s->converge; }
 // DevFrame::stream_blocks: render_stream's persistent grid, the resident blocks of its launch bounds (RTC_STREAM_MINBLOCKS)
 inline int stream_blocks(int sm_count) { return sm_count * 6; }
+
+// rtc_render_ppm's host scan.  In: for each of n_dev devices, the byte lengths of the text of its rows, in its band order
+// (PpmRows); out: the same arrays holding each row's offset in that device's text, and where every band of the frame goes.
+// Shared with the host harness of the PPM kernels (tests/emu/emu_ppm.cpp).
+struct PpmLayout {
+    std::vector<size_t> band_at;       // frame band b: its offset in the whole text (after the header)
+    std::vector<size_t> band_local;    // ... and in its device's text
+    std::vector<size_t> band_bytes;
+    std::vector<size_t> device_bytes;  // each device's text
+    size_t total = 0;                  // the whole text, header included
+};
+inline std::string ppm_header(uint32_t width, uint32_t height) {  // canvas.rs:60-64
+    return "P3\n" + std::to_string(width) + " " + std::to_string(height) + "\n255\n";
+}
+inline int ppm_device_rows(uint32_t height, int device, int n_dev) {
+    const int total_bands = ((int)height + kBandRows - 1) / kBandRows;
+    int rows = 0;
+    for (int b = device; b < total_bands; b += n_dev) rows += std::min<int>(kBandRows, (int)height - b * kBandRows);
+    return rows;
+}
+inline void ppm_layout(uint32_t height, int n_dev, size_t header, unsigned long long* const* rows, PpmLayout& L) {
+    const int total_bands = ((int)height + kBandRows - 1) / kBandRows;
+    L.band_at.assign(total_bands, 0), L.band_local.assign(total_bands, 0), L.band_bytes.assign(total_bands, 0);
+    L.device_bytes.assign(n_dev, 0);
+    size_t at = header;
+    for (int b = 0; b < total_bands; b++) {
+        const int dev = b % n_dev, j0 = b / n_dev * kBandRows;
+        const int n_rows = std::min<int>(kBandRows, (int)height - b * kBandRows);
+        size_t& local = L.device_bytes[dev];
+        L.band_at[b] = at, L.band_local[b] = local;
+        for (int k = 0; k < n_rows; k++) {
+            const size_t len = rows[dev][j0 + k];
+            rows[dev][j0 + k] = local;
+            local += len, at += len;
+        }
+        L.band_bytes[b] = at - L.band_at[b];
+    }
+    L.total = at;
+}
 
 // A tree builder other than the host's binned SAH (rtc_lbvh.cu: the device LBVH).  In: the padded boxes of the bounded
 // items (6 floats each: lo.xyz, hi.xyz), their "closed primitive" flags, the leaf size.  Out: the items' leaf order, the

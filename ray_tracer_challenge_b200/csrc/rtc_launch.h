@@ -85,4 +85,8 @@ void launch_trace(const DevScene& S, const SmallScene& SS, int n, const float* o
 void launch_wave(const DevScene& S, const SmallScene& SS, const DevFrame& F, const WavePoolRaw& pool, DevCounters* counters, int blocks,
                  cudaStream_t stream);
 }  // namespace strict_sweep
+// rtc_render_ppm (rtc_ppm.cu; one build: no floating point): out[j] = the byte length of the PPM text of R's row j; then
+// that text written at out + row_at[j]
+void launch_ppm_row_bytes(const PpmRows& R, unsigned long long* out, int sm_count, cudaStream_t stream);
+void launch_ppm_write(const PpmRows& R, const unsigned long long* row_at, char* out, int sm_count, cudaStream_t stream);
 }  // namespace rtc

@@ -222,6 +222,16 @@ constexpr int kRefillLanes = RTC_REFILL_LANES;  // render_stream: idle lanes of 
 
 constexpr int kBandRows = kTileH;
 
+// The rows one device writes as PPM text (rtc_render_ppm, dev_ppm.cuh): the bands b of its frame with b % n_shards == shard
+// (rtc_shard_bands' rule), in that order; its j-th row is frame row (shard + j / kBandRows * n_shards) * kBandRows +
+// j % kBandRows.
+struct PpmRows {
+    const unsigned char* u8;  // the frame's 8-bit plane, width * height * 3
+    int width;
+    int shard, n_shards;
+    int n_rows;               // rows of those bands
+};
+
 // The wavefront renderer's per-chunk ray pool as the host hands it to the launchers (dev_wave.cuh: WavePool holds the
 // same pointers, typed).
 struct WavePoolRaw {

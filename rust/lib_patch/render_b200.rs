@@ -556,6 +556,24 @@ impl Camera {
         out
     }
 
+    /// The demos' whole flow in one call: `println!("{}", camera.render_b200_ppm(world, 5))` prints exactly what
+    /// `camera.render(world, 5).to_ppm()` prints (canvas.rs:58-96), with the text written on the device (`rtc_render_ppm`)
+    /// and copied straight into the String's bytes.
+    pub fn render_b200_ppm(&self, world: World, reflection_recursion_depth: i16) -> String {
+        let bound = unsafe { sys::rtc_ppm_bound(self.width_pixels, self.height_pixels) };
+        let mut text = vec![0u8; bound];
+        let mut n = 0usize;
+        unsafe {
+            let scene = self.commit_b200(&world);
+            let mut stats: sys::RtcStats = std::mem::zeroed();
+            check(sys::rtc_render_ppm(scene, reflection_recursion_depth as i32, text.as_mut_ptr() as *mut std::os::raw::c_char, bound,
+                                      &mut n, &mut stats));
+            sys::rtc_scene_destroy(scene);
+        }
+        text.truncate(n);
+        String::from_utf8(text).expect("PPM text is ASCII")
+    }
+
     /// `Camera::render` for several cameras of one canvas size (a turntable, a stereo pair): the world is flattened and
     /// committed once — with the camera whose origin is farthest out, so that the tree's reach covers every view — and all
     /// views come from one `rtc_render_views` batch.  Canvas i is what `cameras[i].render(world, depth)` returns.

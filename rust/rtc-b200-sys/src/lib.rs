@@ -211,6 +211,10 @@ extern "C" {
     pub fn rtc_render_detailed(scene: *mut RtcScene, depth: i32, rgb_f32: *mut f32, rgb_u8: *mut u8, stats: *mut RtcStats) -> c_int;
     pub fn rtc_render_views(scene: *mut RtcScene, depth: i32, n_views: u32, views: *const RtcView, rgb_f32: *mut f32, rgb_u8: *mut u8,
                             stats: *mut RtcStats) -> c_int;
+    /// `Canvas::to_ppm` of the rendered frame, its text written on the device; `capacity >= rtc_ppm_bound(w, h)`.
+    pub fn rtc_ppm_bound(width: u32, height: u32) -> usize;
+    pub fn rtc_render_ppm(scene: *mut RtcScene, depth: i32, ppm: *mut c_char, capacity: usize, ppm_bytes: *mut usize,
+                          stats: *mut RtcStats) -> c_int;
     pub fn rtc_trace_rays(scene: *mut RtcScene, n: u32, origins: *const f32, directions: *const f32, depth: i32,
                           out_rgb: *mut f32, out_t: *mut f32, out_prim: *mut i32) -> c_int;
     pub fn rtc_shard_bands(height: u32, shard: i32, n_shards: i32, first_rows: *mut u32) -> c_int;
