@@ -324,10 +324,33 @@ int rtc_render_views(RtcScene*, int32_t depth, uint32_t n_views, const RtcView* 
  *   - Device memory kept with each device for later calls: the text of its rows (up to 12 bytes per pixel, 89 MB for a
  *     3840x2160 frame) and 16 bytes per row.
  *   - Not provided: a shard of a frame shared by several processes (rtc_render_shard) — a process cannot know the offsets of
- *     rows other processes render; batches of views (rtc_render_views); encoding a plane that is not the committed scene's
- *     frame. */
+ *     rows other processes render; encoding a plane that is not the committed scene's frame. */
 size_t rtc_ppm_bound(uint32_t width, uint32_t height);
 int rtc_render_ppm(RtcScene*, int32_t depth, char* ppm, size_t capacity, size_t* ppm_bytes, RtcStats* stats);
+/* rtc_render_views followed by Canvas::to_ppm of every view, with the text written on the device.
+ *   - ppm receives the views' texts one after the other, no terminating NUL: view v's text is ppm[view_offsets[v] ..
+ *     view_offsets[v + 1]).  view_offsets has n_views + 1 entries: view_offsets[0] = 0, view_offsets[n_views] the total.
+ *   - View v's text is byte for byte what rtc_render_ppm returns for the scene committed with that camera — Canvas::to_ppm
+ *     of rtc_render_views' 8-bit plane of that view — for every kernel build and option.
+ *   - The arguments are checked before the scene's state, all with RTC_ERR_INVALID: ppm or view_offsets NULL; every check
+ *     rtc_render_views makes on n_views and views; a capacity below n_views * rtc_ppm_bound of the committed canvas (a
+ *     product that overflows size_t too); a depth outside [0, 23].  Then an uncommitted scene is RTC_ERR_STATE, and a view
+ *     beyond the committed reach of a tree scene is refused as rtc_render_views refuses it.
+ *   - The render is rtc_render_views' with the frames left on the device: the same chunks through the same arena
+ *     (RTC_VIEW_ARENA_BYTES), one render launch per chunk per device (a branching tree scene: one pixel stream per chunk).
+ *     A pageable destination of 4 MiB or more also caps a chunk at as many views as fit 256 MiB of text bound.  Then, per
+ *     chunk and device: one launch computes the byte length of every row the device owns in every view of the chunk, one
+ *     copy of those lengths to the host and a synchronize, the host's scan, one launch writes the text, and the copies into
+ *     ppm, queued once every device has its kernels.  Several devices each write only their own bands of every view.
+ *   - Pinned and pageable destinations both work.  A pageable one receives a chunk's text of 4 MiB or more through the
+ *     pinned staging frame kept with each device, in pieces of about 4 MiB that the host's threads move on as they arrive.
+ *   - stats are rtc_render_views' (primary_rays = n_views * (width - 1) * (height - 1), launches = the render launches,
+ *     kernel_ms = the render kernels), except total_ms, which covers the whole call.
+ *   - Nothing of rtc_render's state changes: the committed camera, its frame on the device and its learnt tile order.
+ *   - Device memory kept with each device for later calls, grow-only: rtc_render_ppm's buffers, grown to the text of the
+ *     largest chunk and 16 bytes per row of a chunk (its row lengths, on the device and pinned on the host). */
+int rtc_render_views_ppm(RtcScene*, int32_t depth, uint32_t n_views, const RtcView* views, char* ppm, size_t capacity,
+                         size_t* view_offsets, RtcStats* stats);
 /* World::color_at (world.rs:88-101) for caller-supplied rays: origins / directions are n*3 f32; out_rgb n*3;
  * out_t (optional) the hit distance or -1; out_prim (optional) the hit primitive index or -1. */
 int rtc_trace_rays(RtcScene*, uint32_t n, const float* origins, const float* directions, int32_t depth,

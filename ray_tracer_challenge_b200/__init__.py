@@ -111,6 +111,10 @@ _HOST_EXTRAS = {
     "sg_farthest_camera": (_I, [_V, _IP, _I]),
     "sg_camera_render_ppm": (C.c_int64, [_V, _I, _I, _I, C.c_void_p, C.c_int64, C.POINTER(SgStats)]),
     "sg_render_prepared_ppm": (C.c_int64, [_V, _I, _I, _I, C.c_void_p, C.c_int64, C.POINTER(SgStats)]),
+    "sg_render_prepared_views_ppm": (C.c_int64, [_V, _I, _I, _I, _IP, _I, C.c_void_p, C.c_int64, C.POINTER(C.c_size_t),
+                                                 C.POINTER(SgStats)]),
+    "sg_camera_render_views_ppm": (C.c_int64, [_V, _IP, _I, _I, _I, C.c_void_p, C.c_int64, C.POINTER(C.c_size_t),
+                                               C.POINTER(SgStats)]),
     "rtc_ppm_bound": (C.c_size_t, [C.c_uint32, C.c_uint32]),  # librtc_b200.so, reached through the host library
 }
 
@@ -133,14 +137,21 @@ def _view_planes(n, h, w, want_rgb, want_u8, out_rgb, out_u8):
     return rgb, u8
 
 
-def _ppm_buffer(api, w, h, out):
-    """The bytes rtc_render_ppm writes into: the caller's C-contiguous uint8 array (e.g. over pinned memory) or a new one,
-    at least rtc_ppm_bound bytes."""
+def _ppm_buffer(api, w, h, out, n=1):
+    """The bytes rtc_render_ppm (n = 1) or rtc_render_views_ppm (n views) writes into: the caller's C-contiguous uint8 array
+    (e.g. over pinned memory) or a new one, at least n * rtc_ppm_bound bytes."""
     bound = api.lib.rtc_ppm_bound(w, h)
-    buf = out if out is not None else np.empty(bound, np.uint8)
-    if buf.dtype != np.uint8 or not buf.flags.c_contiguous or not buf.flags.writeable or buf.nbytes < bound:
-        raise ValueError(f"out must be a writable C-contiguous uint8 array of at least rtc_ppm_bound = {bound} bytes")
+    buf = out if out is not None else np.empty(n * bound, np.uint8)
+    if not isinstance(buf, np.ndarray) or buf.dtype != np.uint8 or not buf.flags.c_contiguous or not buf.flags.writeable \
+            or buf.nbytes < n * bound:
+        need = f"rtc_ppm_bound = {bound}" if n == 1 else f"{n} * rtc_ppm_bound = {n * bound}"
+        raise ValueError(f"out must be a writable C-contiguous uint8 array of at least {need} bytes")
     return buf
+
+
+def _ppm_texts(buf, offsets):
+    """The views' texts of rtc_render_views_ppm: view i's is buf[offsets[i]:offsets[i + 1]]."""
+    return [buf[offsets[i]:offsets[i + 1]].tobytes().decode("ascii") for i in range(len(offsets) - 1)]
 
 
 def _canvases(api, n, h, w, rgb, u8):
@@ -201,6 +212,22 @@ class PreparedScene:
                                                      C.byref(stats)))
         self.last_stats = api.last_rtc_stats()
         return buf[:n].tobytes().decode("ascii")
+
+    def render_views_ppm(self, cameras, depth=DEFAULT_RAY_RECURSION_DEPTH, out=None, fma=False) -> list:
+        """rtc_render_views_ppm: every camera (of this scene's canvas size) rendered from the committed scene in one batch,
+        and each view's `Canvas::to_ppm` text written on the device.  Returns one str per camera.  `out`: where the bytes
+        land (a writable uint8 array of at least len(cameras) * rtc_ppm_bound bytes, e.g. over pinned memory); a new
+        pageable one by default.  The reach rule is render_views'."""
+        cameras = list(cameras)
+        n, w, h = len(cameras), self.camera.width_pixels, self.camera.height_pixels
+        api = self.api
+        buf = _ppm_buffer(api, w, h, out, max(n, 1))
+        offsets = (C.c_size_t * (n + 1))()
+        stats = SgStats()
+        api.check(api.lib.sg_render_prepared_views_ppm(api.ctx, self.handle, int(depth), n, _handles(cameras), int(fma),
+                                                       buf.ctypes.data, buf.nbytes, offsets, C.byref(stats)))
+        self.last_stats = api.last_rtc_stats()
+        return _ppm_texts(buf, list(offsets))
 
     def trace_rays(self, origins, directions, depth=DEFAULT_RAY_RECURSION_DEPTH, fma=False):
         """World::color_at (world.rs:88-101) for arbitrary rays: returns (rgb[n,3], t[n], shape_handle[n])."""
@@ -327,6 +354,21 @@ class HostApi(_api.Api):
                                                    u8.ctypes.data_as(_U8P) if u8 is not None else None, C.byref(stats)))
         self.last_views_stats = self.last_rtc_stats()
         return _canvases(self, n, h, w, rgb, u8)
+
+    def render_views_ppm(self, world, cameras, depth=DEFAULT_RAY_RECURSION_DEPTH, out=None) -> list:
+        """The one-shot batch in text: render_views' flatten and commit, then rtc_render_views_ppm.  Returns
+        `camera.render(world, depth).to_ppm()` for each camera; `out` as PreparedScene.render_views_ppm's."""
+        cameras = list(cameras)
+        if not cameras:
+            raise ValueError("render_views_ppm needs at least one camera")
+        n, w, h = len(cameras), cameras[0].width_pixels, cameras[0].height_pixels
+        buf = _ppm_buffer(self, w, h, out, n)
+        offsets = (C.c_size_t * (n + 1))()
+        stats = SgStats()
+        self.check(self.lib.sg_camera_render_views_ppm(self.ctx, _handles(cameras), n, world.handle, int(depth), buf.ctypes.data,
+                                                       buf.nbytes, offsets, C.byref(stats)))
+        self.last_views_stats = self.last_rtc_stats()
+        return _ppm_texts(buf, list(offsets))
 
     def camera_view(self, camera) -> RtcView:
         """The RtcView a batch hands the device library for `camera` (the fields rtc_set_camera receives for it)."""

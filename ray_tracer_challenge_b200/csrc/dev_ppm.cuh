@@ -1,6 +1,7 @@
 // dev_ppm.cuh — Canvas::to_ppm (canvas.rs:58-96) of the frame's 8-bit plane, written on the device: the kernels of
-// rtc_ppm.cu (rtc_render_ppm), apart from their launch functions so that the host harness (tests/emu/emu_ppm.cpp) compiles
-// the same bodies.  Like the other device parts it opens namespace rtc::RTC_NS itself.
+// rtc_ppm.cu (rtc_render_ppm, rtc_render_views_ppm), apart from their launch functions so that the host harness
+// (tests/emu/emu_ppm.cpp) compiles the same bodies.  A launch covers the rows of one device's bands in each of n_views
+// frames (PpmRows); a single frame is one view.  Like the other device parts it opens namespace rtc::RTC_NS itself.
 //
 // A row's text is its 3 * width values in decimal, each followed by exactly one separator byte: after the row's last value
 // a newline, after any other a space, or a newline where the line has reached 70 - 3 columns (canvas.rs:47-55).  So a
@@ -17,9 +18,11 @@ constexpr int kPpmPerLane = 4;    // consecutive values per lane: a warp steps t
 constexpr unsigned kPpmNoValue = 256u;
 
 __device__ __forceinline__ unsigned ppm_digits(unsigned v) { return 1u + (v >= 10u) + (v >= 100u); }
+__device__ __forceinline__ long long ppm_launch_rows(const PpmRows& R) { return (long long)R.n_rows * R.n_views; }
 __device__ __forceinline__ const unsigned char* ppm_row(const PpmRows& R, long long j) {
-    const size_t row = (size_t)(R.shard + j / kBandRows * R.n_shards) * kBandRows + (size_t)(j % kBandRows);
-    return R.u8 + row * (size_t)R.width * 3;
+    const long long v = j / R.n_rows, r = j - v * R.n_rows;  // view v's row r
+    const size_t row = (size_t)(R.shard + r / kBandRows * R.n_shards) * kBandRows + (size_t)(r % kBandRows);
+    return R.u8 + (size_t)v * R.view_stride + row * (size_t)R.width * 3;
 }
 
 // out[j] = the byte length of the text of R's row j
@@ -27,7 +30,7 @@ __global__ void __launch_bounds__(kPpmThreads) ppm_row_bytes(PpmRows R, unsigned
     const int lane = threadIdx.x & 31;
     const size_t n = (size_t)R.width * 3;
     const long long warps = (long long)gridDim.x * (kPpmThreads / 32);
-    for (long long j = (long long)blockIdx.x * (kPpmThreads / 32) + (threadIdx.x >> 5); j < R.n_rows; j += warps) {
+    for (long long j = (long long)blockIdx.x * (kPpmThreads / 32) + (threadIdx.x >> 5); j < ppm_launch_rows(R); j += warps) {
         const unsigned char* src = ppm_row(R, j);
         unsigned sum = 0;  // at most 16 bytes per 128 values of the row: below 2^32 for every canvas rtc_set_camera accepts
         for (size_t c = (size_t)lane * kPpmPerLane; c < n; c += 32 * kPpmPerLane)
@@ -47,7 +50,7 @@ __global__ void __launch_bounds__(kPpmThreads) ppm_write(PpmRows R, const unsign
     const int lane = threadIdx.x & 31;
     const size_t n = (size_t)R.width * 3;
     const long long warps = (long long)gridDim.x * (kPpmThreads / 32);
-    for (long long j = (long long)blockIdx.x * (kPpmThreads / 32) + (threadIdx.x >> 5); j < R.n_rows; j += warps) {
+    for (long long j = (long long)blockIdx.x * (kPpmThreads / 32) + (threadIdx.x >> 5); j < ppm_launch_rows(R); j += warps) {
         const unsigned char* src = ppm_row(R, j);
         char* dst = text + row_at[j];
         unsigned long long base = 0;  // row offset of the step's first value

@@ -5,6 +5,7 @@
 #include "rtc_host.hpp"
 
 #include <chrono>
+#include <functional>
 #include <memory>
 #include <sstream>
 
@@ -629,9 +630,24 @@ int sg_render_prepared_views(sg_ctx* c, int h, int depth, int n, const int* cams
     to_sg_stats(c->last_stats, stats);
     return rc ? fail(rtc_last_error()) : 0;
 }
-// The one-shot form (Camera::render_b200 for a batch of cameras): flatten, commit with the camera whose origin is farthest
-// out, render every view, release.  The world is consumed once and n canvases come out.
-int sg_camera_render_views(sg_ctx* c, const int* cams, int n, int w, int depth, float* out_rgb, uint8_t* out_u8, sg_stats* stats) {
+// rtc_render_views_ppm on a prepared scene: n cameras (handles) of its canvas size, their texts one after the other in out,
+// view i's at offsets[i] (n + 1 offsets).  Returns the total length, or -1.
+int64_t sg_render_prepared_views_ppm(sg_ctx* c, int h, int depth, int n, const int* cams, int fma, char* out, int64_t capacity,
+                                     size_t* offsets, sg_stats* stats) {
+    if (h < 0 || h >= (int)c->prepared.size() || !c->prepared[h]) return fail("bad prepared handle");
+    if (capacity < 0) return fail("negative capacity");
+    RtcScene* scene = c->prepared[h]->scene;
+    std::vector<RtcView> views;
+    if (camera_views(c, cams, n, c->prepared[h]->width, c->prepared[h]->height, views)) return -1;
+    if (rtc_set_option(scene, RTC_OPT_FMA_CONTRACTION, fma ? 1 : 0)) return fail(rtc_last_error());
+    const int rc = rtc_render_views_ppm(scene, depth, (uint32_t)n, views.data(), out, (size_t)capacity, offsets, &c->last_stats);
+    to_sg_stats(c->last_stats, stats);
+    return rc ? fail(rtc_last_error()) : (int64_t)offsets[n];
+}
+// The one-shot batch: flatten, commit with the camera whose origin is farthest out, run `render` on the scene and the
+// cameras' views, release.  The world is consumed once.
+static int views_one_shot(sg_ctx* c, const int* cams, int n, int w, sg_stats* stats,
+                          const std::function<int(RtcScene*, const std::vector<RtcView>&)>& render) {
     if (n < 1 || !cams) return fail("a batch needs at least one camera");
     for (int i = 0; i < n; i++)
         if (cams[i] < 0 || cams[i] >= (int)c->cameras.size()) return fail("bad camera handle");
@@ -647,7 +663,7 @@ int sg_camera_render_views(sg_ctx* c, const int* cams, int n, int w, int depth, 
         FlatScene flat;
         fill_scene(scene, c->graph, c->worlds[w], first, flat);
         rc = commit(c, scene, true, flat.n_prims);
-        if (!rc && rtc_render_views(scene, depth, (uint32_t)n, views.data(), out_rgb, out_u8, &c->last_stats)) rc = fail(rtc_last_error());
+        if (!rc && render(scene, views)) rc = fail(rtc_last_error());
         c->last_stats.total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
         to_sg_stats(c->last_stats, stats);
     } catch (const std::exception& e) {
@@ -655,6 +671,22 @@ int sg_camera_render_views(sg_ctx* c, const int* cams, int n, int w, int depth, 
     }
     rtc_scene_destroy(scene);
     return rc ? -1 : 0;
+}
+// The one-shot form (Camera::render_b200 for a batch of cameras): n canvases come out.
+int sg_camera_render_views(sg_ctx* c, const int* cams, int n, int w, int depth, float* out_rgb, uint8_t* out_u8, sg_stats* stats) {
+    return views_one_shot(c, cams, n, w, stats, [&](RtcScene* scene, const std::vector<RtcView>& views) {
+        return rtc_render_views(scene, depth, (uint32_t)n, views.data(), out_rgb, out_u8, &c->last_stats);
+    });
+}
+// ... and its text form (`camera.render(world, depth).to_ppm()` for each camera): the texts one after the other in out, view
+// i's at offsets[i] (n + 1 offsets).  Returns the total length, or -1.
+int64_t sg_camera_render_views_ppm(sg_ctx* c, const int* cams, int n, int w, int depth, char* out, int64_t capacity, size_t* offsets,
+                                   sg_stats* stats) {
+    if (capacity < 0) return fail("negative capacity");
+    const int rc = views_one_shot(c, cams, n, w, stats, [&](RtcScene* scene, const std::vector<RtcView>& views) {
+        return rtc_render_views_ppm(scene, depth, (uint32_t)n, views.data(), out, (size_t)capacity, offsets, &c->last_stats);
+    });
+    return rc ? -1 : (int64_t)offsets[n];
 }
 // What a batch hands the device library for a camera (the fields fill_scene passes to rtc_set_camera), and which camera of a
 // batch the one-shot form commits with — host arithmetic, no device

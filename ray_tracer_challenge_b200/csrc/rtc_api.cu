@@ -789,20 +789,38 @@ int ensure_views(DeviceSlot* d, uint32_t n, size_t frame_bytes) {
     return 0;
 }
 
-int render_views_impl(RtcScene* s, int depth, uint32_t n_views, const RtcView* views, float* rgb, uint8_t* u8, RtcStats* stats) {
-    // the arguments first (no device needed), then the scene's state
-    if (!s) return fail(RTC_ERR_INVALID, "null scene");
-    if (n_views == 0 || !views) return fail(RTC_ERR_INVALID, "rtc_render_views: n_views must be >= 1 and views non-null");
+// rtc_render_views' checks of n_views and views (no device needed); fn names the entry point in the messages
+int check_views(uint32_t n_views, const RtcView* views, const char* fn) {
+    if (n_views == 0 || !views) return fail(RTC_ERR_INVALID, std::string(fn) + ": n_views must be >= 1 and views non-null");
     for (uint32_t v = 0; v < n_views; v++) {
         const RtcView& w = views[v];
         bool finite = std::isfinite(w.half_width) && std::isfinite(w.half_height) && std::isfinite(w.pixel_size);
         for (float x : w.transform_inverse) finite = finite && std::isfinite(x);
-        if (!finite) return fail(RTC_ERR_INVALID, "rtc_render_views: view " + std::to_string(v) + " has a non-finite field");
-        if (!(w.pixel_size > 0.f)) return fail(RTC_ERR_INVALID, "rtc_render_views: view " + std::to_string(v) + " has pixel_size <= 0");
+        if (!finite) return fail(RTC_ERR_INVALID, std::string(fn) + ": view " + std::to_string(v) + " has a non-finite field");
+        if (!(w.pixel_size > 0.f)) return fail(RTC_ERR_INVALID, std::string(fn) + ": view " + std::to_string(v) + " has pixel_size <= 0");
     }
+    return 0;
+}
+int check_depth(int depth) {
     if (depth < 0 || depth > kMaxFrames - 1)
         return fail(RTC_ERR_INVALID, "reflection_recursion_depth must be in [0, " + std::to_string(kMaxFrames - 1) + "]");
-    if (!s->committed) return fail(RTC_ERR_STATE, "rtc_render_views before rtc_scene_commit");
+    return 0;
+}
+
+int write_ppm_text(RtcScene* s, const unsigned char* const* frames, int n_views, size_t view_stride, char* out, size_t capacity,
+                   size_t* view_at, size_t* bytes);
+
+// rtc_render_views_ppm's destination: the texts of the views one after the other, view v's at view_offsets[v]
+struct ViewsText {
+    char* ppm;
+    size_t capacity;
+    size_t* view_offsets;
+};
+
+// rtc_render_views (text == nullptr) and rtc_render_views_ppm, from the scene's state on: the arguments are checked
+int render_views_body(RtcScene* s, int depth, uint32_t n_views, const RtcView* views, float* rgb, uint8_t* u8, RtcStats* stats,
+                      const ViewsText* text, const char* fn) {
+    if (!s->committed) return fail(RTC_ERR_STATE, std::string(fn) + " before rtc_scene_commit");
     // The tree's boxes are padded for ray origins up to the commit's reach (rtc_commit.cu: "pad"): a camera farther out
     // could lose hits the reference reports.  Small and tree-less scenes test every item exactly: any view goes.
     if (s->replicas[0].scene.bvh_root >= 0)
@@ -840,6 +858,12 @@ int render_views_impl(RtcScene* s, int depth, uint32_t n_views, const RtcView* v
     const bool stage_u8 = u8 && frame_px * 3 * n_views >= ((size_t)4 << 20) && is_pageable(u8);
     const size_t staged_per_view = frame_px * ((stage_rgb ? 12 : 0) + (stage_u8 ? 3 : 0));
     if (staged_per_view) chunk = (uint32_t)std::max<size_t>(1, std::min<size_t>(chunk, kViewStageBytes / staged_per_view));
+    // the text of a chunk is staged through pinned frames as well (write_ppm_text): its bound must fit them
+    const size_t text_bound = rtc_ppm_bound(s->width, s->height);
+    if (text && text_bound * n_views >= ((size_t)4 << 20) && is_pageable(text->ppm))
+        chunk = (uint32_t)std::max<size_t>(1, std::min<size_t>(chunk, kViewStageBytes / text_bound));
+    size_t text_at = 0;         // the texts of the chunks so far
+    double render_ms = 0.0;     // text: the render kernels of every chunk
     CanvasCopy cc(s, n_shards, rgb, u8, stage_rgb, stage_u8, (int)chunk);
     static const bool rotate = [] {
         const char* env = getenv("RTC_SLICE_STREAMS");  // tuning aid: 0 = all slices on one stream
@@ -918,6 +942,7 @@ int render_views_impl(RtcScene* s, int depth, uint32_t n_views, const RtcView* v
             if (chunk_copied[i])
                 for (int l = 0; l < n_lanes; l++) CUDA_TRY(cudaStreamWaitEvent(lanes[l], chunk_copied[i], 0));
             int last_on_lane[3] = {-1, -1, -1};
+            if (text) CUDA_TRY(cudaEventRecord(slot->ev0, slot->stream));  // one lane: the chunk's launch
             for (size_t k = 0; k < plan.size(); k++) {
                 const Launch& L = plan[k];
                 cudaStream_t lane = lanes[k % n_lanes];
@@ -943,8 +968,29 @@ int render_views_impl(RtcScene* s, int depth, uint32_t n_views, const RtcView* v
             }
             for (int l = 0; l < n_lanes; l++)
                 if (l > 0 && last_on_lane[l] >= 0) CUDA_TRY(cudaStreamWaitEvent(slot->stream, slot->slice_done[last_on_lane[l]], 0));
+            if (text) CUDA_TRY(cudaEventRecord(slot->ev1, slot->stream));
         }
         if (int rc = cc.flush_pending()) return rc;
+        if (text) {  // the chunk's text, behind its render on each device's render stream
+            std::vector<const unsigned char*> frames(ndev);
+            for (int i = 0; i < ndev; i++) frames[i] = reinterpret_cast<const unsigned char*>(s->replicas[i].slot->d_view_frames + frame_px * 12 * chunk);
+            size_t bytes = 0;
+            if (int rc = write_ppm_text(s, frames.data(), (int)(c1 - c0), frame_px * 3, text->ppm + text_at, text->capacity - text_at,
+                                        text->view_offsets + c0, &bytes))
+                return rc;
+            for (uint32_t v = c0; v < c1; v++) text->view_offsets[v] += text_at;
+            text_at += bytes;
+            double ms_max = 0.0;
+            for (int i = 0; i < ndev; i++) {
+                DeviceSlot* slot = s->replicas[i].slot;
+                CUDA_TRY(cudaSetDevice(slot->device));
+                CUDA_TRY(cudaEventSynchronize(slot->ev1));
+                float ms = 0.f;
+                CUDA_TRY(cudaEventElapsedTime(&ms, slot->ev0, slot->ev1));
+                ms_max = std::max(ms_max, (double)ms);
+            }
+            render_ms += ms_max;
+        }
         if (c1 < n_views) {  // the next chunk reuses the arena (and the staging frames): it waits for this chunk's copies
             if (int rc = cc.drain()) return rc;
             for (int i = 0; i < ndev; i++) {
@@ -962,16 +1008,17 @@ int render_views_impl(RtcScene* s, int depth, uint32_t n_views, const RtcView* v
     for (int i = 0; i < ndev; i++) {
         DeviceSlot* slot = s->replicas[i].slot;
         CUDA_TRY(cudaSetDevice(slot->device));
-        CUDA_TRY(cudaEventRecord(slot->ev1, slot->stream));
+        if (!text) CUDA_TRY(cudaEventRecord(slot->ev1, slot->stream));
         CUDA_TRY(cudaMemcpyAsync(slot->h_counters, slot->d_counters, sizeof(DevCounters), cudaMemcpyDeviceToHost, slot->stream));
     }
+    st.kernel_ms = render_ms;
     for (int i = 0; i < ndev; i++) {
         DeviceSlot* slot = s->replicas[i].slot;
         CUDA_TRY(cudaSetDevice(slot->device));
         CUDA_TRY(cudaStreamSynchronize(slot->stream));
         CUDA_TRY(cudaStreamSynchronize(slot->copy_stream));
         float ms = 0.f;
-        CUDA_TRY(cudaEventElapsedTime(&ms, slot->ev0, slot->ev1));
+        if (!text) CUDA_TRY(cudaEventElapsedTime(&ms, slot->ev0, slot->ev1));
         st.kernel_ms = std::max(st.kernel_ms, (double)ms);
         uint64_t rows = 0;  // camera.rs:80-81, per view, of this device's bands
         for (int b = i; b < total_bands; b += n_shards)
@@ -979,11 +1026,20 @@ int render_views_impl(RtcScene* s, int depth, uint32_t n_views, const RtcView* v
         add_counters(st, *slot->h_counters, (uint64_t)n_views * rows * (uint64_t)(s->width - 1),
                      s->light_is_rect ? (uint64_t)s->u_steps * s->v_steps : 1);
     }
+    if (text) text->view_offsets[n_views] = text_at;
     st.total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
     if (stats) *stats = st;
     if (st.capacity_overflows)
         return fail(RTC_ERR_CAPACITY, "CSG evaluation overflowed its buffers " + std::to_string(st.capacity_overflows) + " times");
     return 0;
+}
+
+int render_views_impl(RtcScene* s, int depth, uint32_t n_views, const RtcView* views, float* rgb, uint8_t* u8, RtcStats* stats) {
+    // the arguments first (no device needed), then the scene's state
+    if (!s) return fail(RTC_ERR_INVALID, "null scene");
+    if (int rc = check_views(n_views, views, "rtc_render_views")) return rc;
+    if (int rc = check_depth(depth)) return rc;
+    return render_views_body(s, depth, n_views, views, rgb, u8, stats, nullptr, "rtc_render_views");
 }
 
 // rtc_render_ppm ---------------------------------------------------------------------------------------------------------
@@ -1009,8 +1065,121 @@ int ensure_ppm_text(DeviceSlot* d, size_t bytes) {
     return 0;
 }
 
-// Render, then on every device: the byte lengths of its rows' text, one copy back and a synchronize, the host's scan over
-// all rows (ppm_layout), the text of its rows into d_ppm, and the copies of its bands to their offsets in `ppm`.
+// The (view, band) texts [e0, e1) of device i's text (view-major; nb own bands per view), as runs contiguous in the whole text
+// too: a whole view of a one-device frame is one run.
+struct PpmRun {
+    size_t at, local, bytes;  // offset in the whole text, offset in the device's text, length
+};
+std::vector<PpmRun> ppm_runs(const PpmLayout& L, int i, int ndev, int nb, int e0, int e1) {
+    auto vb = [&](int e) { return (size_t)(e / nb) * L.total_bands + i + (size_t)(e % nb) * ndev; };
+    std::vector<PpmRun> runs;
+    for (int e = e0; e < e1;) {
+        const size_t first = vb(e);
+        PpmRun r{L.band_at[first], L.band_local[first], L.band_bytes[first]};
+        for (e++; e < e1 && L.band_at[vb(e)] == r.at + r.bytes; e++) r.bytes += L.band_bytes[vb(e)];
+        runs.push_back(r);
+    }
+    return runs;
+}
+
+// The PPM text of n_views frames of s's canvas size, each device i holding view v's 8-bit plane (its own bands of it) at
+// frames[i] + v * view_stride.  On every device: one ppm_row_bytes launch over its rows of every view, one copy of the
+// lengths back and a synchronize; the host's scan over all of them (ppm_layout, which writes the headers into out); one
+// ppm_write launch into d_ppm; and once every device has its kernels, the copies of its texts to their offsets in out.
+// view_at[v] receives view v's offset in out, *bytes the whole length.  The copies into a pinned destination may still be
+// in flight on the devices' render streams when this returns; a staged one has arrived.
+int write_ppm_text(RtcScene* s, const unsigned char* const* frames, int n_views, size_t view_stride, char* out, size_t capacity,
+                   size_t* view_at, size_t* bytes) {
+    const int ndev = (int)s->replicas.size();
+    const int total_bands = ((int)s->height + kBandRows - 1) / kBandRows;
+    std::vector<PpmRows> rows(ndev);
+    std::vector<unsigned long long*> lengths(ndev);
+    for (int i = 0; i < ndev; i++) {
+        DeviceSlot* slot = s->replicas[i].slot;
+        CUDA_TRY(cudaSetDevice(slot->device));
+        rows[i] = PpmRows{frames[i], (int)s->width, i, ndev, ppm_device_rows(s->height, i, ndev), n_views, view_stride};
+        const size_t n_rows = (size_t)rows[i].n_rows * n_views;
+        if (int rc = ensure_ppm_rows(slot, std::max<size_t>(n_rows, 1))) return rc;
+        lengths[i] = slot->h_ppm_rows;
+        launch_ppm_row_bytes(rows[i], slot->d_ppm_rows, slot->sm_count, slot->stream);
+        CUDA_TRY(cudaGetLastError());
+        CUDA_TRY(cudaMemcpyAsync(slot->h_ppm_rows, slot->d_ppm_rows, n_rows * sizeof(unsigned long long), cudaMemcpyDeviceToHost,
+                                 slot->stream));
+    }
+    for (int i = 0; i < ndev; i++) {
+        CUDA_TRY(cudaSetDevice(s->replicas[i].slot->device));
+        CUDA_TRY(cudaStreamSynchronize(s->replicas[i].slot->stream));
+    }
+    PpmLayout L;
+    const std::string header = ppm_header(s->width, s->height);
+    ppm_layout(s->height, ndev, header.size(), lengths.data(), L, n_views, header.data(), out);
+    if (L.total > capacity) return fail(RTC_ERR_CAPACITY, "the PPM text outgrew rtc_ppm_bound");  // cannot happen
+    for (int v = 0; v < n_views; v++) view_at[v] = L.view_at[v];
+    for (int i = 0; i < ndev; i++) {
+        DeviceSlot* slot = s->replicas[i].slot;
+        CUDA_TRY(cudaSetDevice(slot->device));
+        if (int rc = ensure_ppm_text(slot, std::max<size_t>(L.device_bytes[i], 16))) return rc;
+        CUDA_TRY(cudaMemcpyAsync(slot->d_ppm_rows, slot->h_ppm_rows, (size_t)rows[i].n_rows * n_views * sizeof(unsigned long long),
+                                 cudaMemcpyHostToDevice, slot->stream));
+        launch_ppm_write(rows[i], slot->d_ppm_rows, slot->d_ppm, slot->sm_count, slot->stream);
+        CUDA_TRY(cudaGetLastError());
+    }
+    // A pageable destination (a String, a NumPy array): as rtc_render's planes, the text lands in the pinned staging frame of
+    // the device slot piece by piece, and the host's threads move each piece on as soon as its copy has arrived.
+    const bool staged = L.total >= ((size_t)4 << 20) && is_pageable(out);
+    struct Piece {
+        DeviceSlot* slot;
+        int dev, nb, e0, e1;  // (view, band) texts [e0, e1) of the device's text
+        cudaEvent_t done;
+    };
+    std::vector<Piece> pieces;
+    for (int i = 0; i < ndev; i++) {  // the copies, queued once every device has its kernels
+        DeviceSlot* slot = s->replicas[i].slot;
+        CUDA_TRY(cudaSetDevice(slot->device));
+        const int nb = i < total_bands ? (total_bands - i + ndev - 1) / ndev : 0, entries = nb * n_views;
+        if (entries == 0) continue;
+        // pieces of about 4 MiB (whole bands) when staged, so that the host's copies overlap the device's; else one
+        const int n_pieces = staged ? (int)std::max<size_t>(1, std::min<size_t>((size_t)entries, L.device_bytes[i] >> 22)) : 1;
+        if (staged)
+            if (int rc = ensure_stage(slot, &slot->h_stage_u8, &slot->h_stage_u8_bytes, L.device_bytes[i])) return rc;
+        for (int k = 0; k < n_pieces; k++) {
+            const int e0 = (int)((int64_t)entries * k / n_pieces), e1 = (int)((int64_t)entries * (k + 1) / n_pieces);
+            if (!staged) {
+                for (const PpmRun& r : ppm_runs(L, i, ndev, nb, e0, e1))
+                    CUDA_TRY(cudaMemcpyAsync(out + r.at, slot->d_ppm + r.local, r.bytes, cudaMemcpyDeviceToHost, slot->stream));
+                continue;
+            }
+            const size_t first = (size_t)(e0 / nb) * total_bands + i + (size_t)(e0 % nb) * ndev;
+            const size_t last = (size_t)((e1 - 1) / nb) * total_bands + i + (size_t)((e1 - 1) % nb) * ndev;
+            const size_t local = L.band_local[first], n = L.band_local[last] + L.band_bytes[last] - local;
+            CUDA_TRY(cudaMemcpyAsync(slot->h_stage_u8 + local, slot->d_ppm + local, n, cudaMemcpyDeviceToHost, slot->stream));
+            const size_t used = pieces.size();
+            while (slot->copy_done.size() <= used) {
+                cudaEvent_t e;
+                CUDA_TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+                slot->copy_done.push_back(e);
+            }
+            CUDA_TRY(cudaEventRecord(slot->copy_done[used], slot->stream));
+            pieces.push_back({slot, i, nb, e0, e1, slot->copy_done[used]});
+        }
+    }
+    for (const Piece& p : pieces) {
+        CUDA_TRY(cudaSetDevice(p.slot->device));
+        CUDA_TRY(cudaEventSynchronize(p.done));
+        const std::vector<PpmRun> runs = ppm_runs(L, p.dev, ndev, p.nb, p.e0, p.e1);
+        if (runs.size() == 1) {
+            parallel_copy(out + runs[0].at, p.slot->h_stage_u8 + runs[0].local, runs[0].bytes, (size_t)96 << 10);
+            continue;
+        }
+        parallel_for(runs.size(), 1, [&](size_t rb, size_t re, int) {
+            for (size_t r = rb; r < re; r++) memcpy(out + runs[r].at, p.slot->h_stage_u8 + runs[r].local, runs[r].bytes);
+        });
+    }
+    *bytes = L.total;
+    return 0;
+}
+
+// Render, then the frame's text (write_ppm_text, one view).
 int render_ppm_impl(RtcScene* s, int depth, char* ppm, size_t capacity, size_t* ppm_bytes, RtcStats* stats) {
     // the arguments first (no device needed), then the scene's state
     if (!s) return fail(RTC_ERR_INVALID, "null scene");
@@ -1030,100 +1199,39 @@ int render_ppm_impl(RtcScene* s, int depth, char* ppm, size_t capacity, size_t* 
         return rc;
     }
     const int ndev = (int)s->replicas.size();
-    const int total_bands = ((int)s->height + kBandRows - 1) / kBandRows;
-    std::vector<PpmRows> rows(ndev);
-    std::vector<unsigned long long*> lengths(ndev);
-    for (int i = 0; i < ndev; i++) {
-        DeviceSlot* slot = s->replicas[i].slot;
-        CUDA_TRY(cudaSetDevice(slot->device));
-        rows[i] = PpmRows{slot->d_u8, (int)s->width, i, ndev, ppm_device_rows(s->height, i, ndev)};
-        if (int rc = ensure_ppm_rows(slot, std::max(rows[i].n_rows, 1))) return rc;
-        lengths[i] = slot->h_ppm_rows;
-        launch_ppm_row_bytes(rows[i], slot->d_ppm_rows, slot->sm_count, slot->stream);
-        CUDA_TRY(cudaGetLastError());
-        CUDA_TRY(cudaMemcpyAsync(slot->h_ppm_rows, slot->d_ppm_rows, rows[i].n_rows * sizeof(unsigned long long), cudaMemcpyDeviceToHost,
-                                 slot->stream));
-    }
+    std::vector<const unsigned char*> frames(ndev);
+    for (int i = 0; i < ndev; i++) frames[i] = s->replicas[i].slot->d_u8;
+    size_t view_at = 0, bytes = 0;
+    if (int rc = write_ppm_text(s, frames.data(), 1, 0, ppm, capacity, &view_at, &bytes)) return rc;
     for (int i = 0; i < ndev; i++) {
         CUDA_TRY(cudaSetDevice(s->replicas[i].slot->device));
         CUDA_TRY(cudaStreamSynchronize(s->replicas[i].slot->stream));
     }
-    const std::string header = ppm_header(s->width, s->height);
-    PpmLayout L;
-    ppm_layout(s->height, ndev, header.size(), lengths.data(), L);
-    if (L.total > capacity) return fail(RTC_ERR_CAPACITY, "rtc_render_ppm: the text outgrew rtc_ppm_bound");  // cannot happen
-    memcpy(ppm, header.data(), header.size());
-    // A pageable destination (a String, a NumPy array): as rtc_render's planes, the text lands in the pinned staging frame of
-    // the device slot piece by piece, and the host's threads move each piece on as soon as its copy has arrived.
-    const bool staged = L.total >= ((size_t)4 << 20) && is_pageable(ppm);
-    struct Piece {
-        DeviceSlot* slot;
-        int dev, j0, j1;  // bands [j0, j1) of the device's band list
-        cudaEvent_t done;
-    };
-    std::vector<Piece> pieces;
-    for (int i = 0; i < ndev; i++) {
-        DeviceSlot* slot = s->replicas[i].slot;
-        CUDA_TRY(cudaSetDevice(slot->device));
-        if (int rc = ensure_ppm_text(slot, std::max<size_t>(L.device_bytes[i], 16))) return rc;
-        CUDA_TRY(cudaMemcpyAsync(slot->d_ppm_rows, slot->h_ppm_rows, rows[i].n_rows * sizeof(unsigned long long), cudaMemcpyHostToDevice,
-                                 slot->stream));
-        launch_ppm_write(rows[i], slot->d_ppm_rows, slot->d_ppm, slot->sm_count, slot->stream);
-        CUDA_TRY(cudaGetLastError());
-        const int nb = i < total_bands ? (total_bands - i + ndev - 1) / ndev : 0;
-        if (nb == 0) continue;
-        // pieces of about 4 MiB (whole bands) when staged, so that the host's copies overlap the device's; else one
-        const int n_pieces = staged ? (int)std::max<size_t>(1, std::min<size_t>((size_t)nb, L.device_bytes[i] >> 22)) : 1;
-        if (staged)
-            if (int rc = ensure_stage(slot, &slot->h_stage_u8, &slot->h_stage_u8_bytes, L.device_bytes[i])) return rc;
-        for (int k = 0; k < n_pieces; k++) {
-            const int j0 = (int)((int64_t)nb * k / n_pieces), j1 = (int)((int64_t)nb * (k + 1) / n_pieces);
-            const size_t local = L.band_local[i + j0 * ndev];
-            const size_t bytes = L.band_local[i + (j1 - 1) * ndev] + L.band_bytes[i + (j1 - 1) * ndev] - local;
-            if (staged) {
-                CUDA_TRY(cudaMemcpyAsync(slot->h_stage_u8 + local, slot->d_ppm + local, bytes, cudaMemcpyDeviceToHost, slot->stream));
-                const size_t used = pieces.size();
-                while (slot->copy_done.size() <= used) {
-                    cudaEvent_t e;
-                    CUDA_TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-                    slot->copy_done.push_back(e);
-                }
-                CUDA_TRY(cudaEventRecord(slot->copy_done[used], slot->stream));
-                pieces.push_back({slot, i, j0, j1, slot->copy_done[used]});
-            } else if (ndev == 1) {  // the device's text is the frame's
-                CUDA_TRY(cudaMemcpyAsync(ppm + L.band_at[j0], slot->d_ppm + local, bytes, cudaMemcpyDeviceToHost, slot->stream));
-            } else {
-                for (int j = j0; j < j1; j++) {
-                    const int b = i + j * ndev;
-                    CUDA_TRY(cudaMemcpyAsync(ppm + L.band_at[b], slot->d_ppm + L.band_local[b], L.band_bytes[b], cudaMemcpyDeviceToHost,
-                                             slot->stream));
-                }
-            }
-        }
-    }
-    for (const Piece& p : pieces) {
-        CUDA_TRY(cudaSetDevice(p.slot->device));
-        CUDA_TRY(cudaEventSynchronize(p.done));
-        if (ndev == 1) {
-            const size_t at = L.band_at[p.j0], bytes = L.band_at[p.j1 - 1] + L.band_bytes[p.j1 - 1] - at;
-            parallel_copy(ppm + at, p.slot->h_stage_u8 + L.band_local[p.j0], bytes, (size_t)96 << 10);
-            continue;
-        }
-        parallel_for((size_t)(p.j1 - p.j0), 1, [&](size_t jb, size_t je, int) {
-            for (size_t j = jb; j < je; j++) {
-                const int b = p.dev + (p.j0 + (int)j) * ndev;
-                memcpy(ppm + L.band_at[b], p.slot->h_stage_u8 + L.band_local[b], L.band_bytes[b]);
-            }
-        });
-    }
-    for (int i = 0; i < ndev; i++) {
-        CUDA_TRY(cudaSetDevice(s->replicas[i].slot->device));
-        CUDA_TRY(cudaStreamSynchronize(s->replicas[i].slot->stream));
-    }
-    *ppm_bytes = L.total;
+    *ppm_bytes = bytes;
     st.total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
     if (stats) *stats = st;
     return 0;
+}
+
+int render_views_ppm_impl(RtcScene* s, int depth, uint32_t n_views, const RtcView* views, char* ppm, size_t capacity,
+                          size_t* view_offsets, RtcStats* stats) {
+    // the arguments first (no device needed), then the scene's state
+    if (!s) return fail(RTC_ERR_INVALID, "null scene");
+    if (!ppm || !view_offsets) return fail(RTC_ERR_INVALID, "rtc_render_views_ppm: ppm and view_offsets must be non-null");
+    // the capacity before the views' fields: a count the capacity cannot hold is refused without reading that many views
+    const size_t bound = rtc_ppm_bound(s->width, s->height);
+    if (n_views > 0 && bound > SIZE_MAX / n_views)
+        return fail(RTC_ERR_INVALID, "rtc_render_views_ppm: n_views * rtc_ppm_bound overflows size_t");
+    if (n_views > 0 && capacity < bound * n_views)
+        return fail(RTC_ERR_INVALID, "rtc_render_views_ppm: capacity " + std::to_string(capacity) + " is below n_views * rtc_ppm_bound = " +
+                                         std::to_string(bound * n_views));
+    if (int rc = check_views(n_views, views, "rtc_render_views_ppm")) return rc;
+    if (int rc = check_depth(depth)) return rc;
+    const auto t0 = std::chrono::steady_clock::now();
+    const ViewsText text{ppm, capacity, view_offsets};
+    const int rc = render_views_body(s, depth, n_views, views, nullptr, nullptr, stats, &text, "rtc_render_views_ppm");
+    if (!rc && stats) stats->total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    return rc;
 }
 
 }  // namespace
@@ -1408,6 +1516,10 @@ size_t rtc_ppm_bound(uint32_t width, uint32_t height) {
 }
 int rtc_render_ppm(RtcScene* s, int32_t depth, char* ppm, size_t capacity, size_t* ppm_bytes, RtcStats* stats) {
     return render_ppm_impl(s, depth, ppm, capacity, ppm_bytes, stats);
+}
+int rtc_render_views_ppm(RtcScene* s, int32_t depth, uint32_t n_views, const RtcView* views, char* ppm, size_t capacity,
+                         size_t* view_offsets, RtcStats* stats) {
+    return render_views_ppm_impl(s, depth, n_views, views, ppm, capacity, view_offsets, stats);
 }
 
 int rtc_trace_rays(RtcScene* s, uint32_t n, const float* origins, const float* directions, int32_t depth, float* out_rgb,

@@ -4,6 +4,7 @@
 #include <algorithm>
 #include <cmath>
 #include <cstdint>
+#include <cstring>
 #include <string>
 #include <vector>
 
@@ -90,8 +91,9 @@ struct DeviceSlot {
     uint32_t views_capacity = 0;
     char* d_view_frames = nullptr;
     size_t view_frames_bytes = 0;
-    // rtc_render_ppm (grow-only): the text of this device's rows, and their byte lengths, then offsets, on the device and
-    // pinned on the host.  A pageable destination is staged through h_stage_u8.
+    // rtc_render_ppm and rtc_render_views_ppm (grow-only): the text of this device's rows (of a frame, or of every view of a
+    // chunk), and their byte lengths, then offsets, on the device and pinned on the host.  A pageable destination is staged
+    // through h_stage_u8.
     char* d_ppm = nullptr;
     size_t ppm_bytes = 0;
     unsigned long long* d_ppm_rows = nullptr;
@@ -207,15 +209,21 @@ inline int frame_converge(const RtcScene* s) { return s->converge < 0 ? (int)s->
 // DevFrame::stream_blocks: render_stream's persistent grid, the resident blocks of its launch bounds (RTC_STREAM_MINBLOCKS)
 inline int stream_blocks(int sm_count) { return sm_count * 6; }
 
-// rtc_render_ppm's host scan.  In: for each of n_dev devices, the byte lengths of the text of its rows, in its band order
-// (PpmRows); out: the same arrays holding each row's offset in that device's text, and where every band of the frame goes.
-// Shared with the host harness of the PPM kernels (tests/emu/emu_ppm.cpp).
+// The host scan of rtc_render_ppm (one view) and rtc_render_views_ppm (n_views).  In: for each of n_dev devices, the byte
+// lengths of the text of its rows, view after view and in its band order within a view (PpmRows); header: the length of a
+// view's header.  Out: the same arrays holding each row's offset in that device's text (view-major as well), and where
+// every view and every (view, band) goes; the texts of the views follow each other.  With `text`, each view's header
+// (header_text, `header` bytes: ppm_header) is written at its offset there; text must hold the whole (a view's text is at
+// most rtc_ppm_bound).  Shared with the host harnesses of the PPM kernels (tests/emu/emu_ppm.cpp: one frame, the header
+// left to the caller; tests/emu/emu_ppm_views.cpp).
 struct PpmLayout {
-    std::vector<size_t> band_at;       // frame band b: its offset in the whole text (after the header)
+    int total_bands = 0;               // bands of one frame
+    std::vector<size_t> view_at;       // view v: the offset of its text (its header) in the whole text
+    std::vector<size_t> band_at;       // band b of view v (index v * total_bands + b): its offset in the whole text
     std::vector<size_t> band_local;    // ... and in its device's text
     std::vector<size_t> band_bytes;
     std::vector<size_t> device_bytes;  // each device's text
-    size_t total = 0;                  // the whole text, header included
+    size_t total = 0;                  // the whole text, headers included
 };
 inline std::string ppm_header(uint32_t width, uint32_t height) {  // canvas.rs:60-64
     return "P3\n" + std::to_string(width) + " " + std::to_string(height) + "\n255\n";
@@ -226,22 +234,34 @@ inline int ppm_device_rows(uint32_t height, int device, int n_dev) {
     for (int b = device; b < total_bands; b += n_dev) rows += std::min<int>(kBandRows, (int)height - b * kBandRows);
     return rows;
 }
-inline void ppm_layout(uint32_t height, int n_dev, size_t header, unsigned long long* const* rows, PpmLayout& L) {
+inline void ppm_layout(uint32_t height, int n_dev, size_t header, unsigned long long* const* rows, PpmLayout& L, int n_views = 1,
+                       const char* header_text = nullptr, char* text = nullptr) {
     const int total_bands = ((int)height + kBandRows - 1) / kBandRows;
-    L.band_at.assign(total_bands, 0), L.band_local.assign(total_bands, 0), L.band_bytes.assign(total_bands, 0);
+    std::vector<size_t> dev_rows(n_dev);
+    for (int i = 0; i < n_dev; i++) dev_rows[i] = (size_t)ppm_device_rows(height, i, n_dev);
+    L.total_bands = total_bands;
+    L.view_at.assign(n_views, 0);
+    L.band_at.assign((size_t)n_views * total_bands, 0), L.band_local.assign((size_t)n_views * total_bands, 0);
+    L.band_bytes.assign((size_t)n_views * total_bands, 0);
     L.device_bytes.assign(n_dev, 0);
-    size_t at = header;
-    for (int b = 0; b < total_bands; b++) {
-        const int dev = b % n_dev, j0 = b / n_dev * kBandRows;
-        const int n_rows = std::min<int>(kBandRows, (int)height - b * kBandRows);
-        size_t& local = L.device_bytes[dev];
-        L.band_at[b] = at, L.band_local[b] = local;
-        for (int k = 0; k < n_rows; k++) {
-            const size_t len = rows[dev][j0 + k];
-            rows[dev][j0 + k] = local;
-            local += len, at += len;
+    size_t at = 0;
+    for (int v = 0; v < n_views; v++) {
+        L.view_at[v] = at;
+        if (text) memcpy(text + at, header_text, header);
+        at += header;
+        for (int b = 0; b < total_bands; b++) {
+            const int dev = b % n_dev;
+            const size_t j0 = (size_t)v * dev_rows[dev] + (size_t)(b / n_dev * kBandRows), vb = (size_t)v * total_bands + b;
+            const int n_rows = std::min<int>(kBandRows, (int)height - b * kBandRows);
+            size_t& local = L.device_bytes[dev];
+            L.band_at[vb] = at, L.band_local[vb] = local;
+            for (int k = 0; k < n_rows; k++) {
+                const size_t len = rows[dev][j0 + k];
+                rows[dev][j0 + k] = local;
+                local += len, at += len;
+            }
+            L.band_bytes[vb] = at - L.band_at[vb];
         }
-        L.band_bytes[b] = at - L.band_at[b];
     }
     L.total = at;
 }

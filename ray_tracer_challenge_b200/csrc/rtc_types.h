@@ -222,14 +222,16 @@ constexpr int kRefillLanes = RTC_REFILL_LANES;  // render_stream: idle lanes of 
 
 constexpr int kBandRows = kTileH;
 
-// The rows one device writes as PPM text (rtc_render_ppm, dev_ppm.cuh): the bands b of its frame with b % n_shards == shard
-// (rtc_shard_bands' rule), in that order; its j-th row is frame row (shard + j / kBandRows * n_shards) * kBandRows +
-// j % kBandRows.
+// The rows one device writes as PPM text (rtc_render_ppm, rtc_render_views_ppm, dev_ppm.cuh): in each of n_views frames, the
+// bands b with b % n_shards == shard (rtc_shard_bands' rule), in that order.  Row j of a launch is row r = j % n_rows of
+// view j / n_rows, frame row (shard + r / kBandRows * n_shards) * kBandRows + r % kBandRows; one frame is n_views = 1.
 struct PpmRows {
-    const unsigned char* u8;  // the frame's 8-bit plane, width * height * 3
+    const unsigned char* u8;  // view 0's 8-bit plane, width * height * 3
     int width;
     int shard, n_shards;
-    int n_rows;               // rows of those bands
+    int n_rows;               // rows of those bands, in one view
+    int n_views = 1;
+    size_t view_stride = 0;   // bytes from one view's plane to the next
 };
 
 // The wavefront renderer's per-chunk ray pool as the host hands it to the launchers (dev_wave.cuh: WavePool holds the

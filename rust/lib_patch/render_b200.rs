@@ -578,7 +578,54 @@ impl Camera {
     /// committed once — with the camera whose origin is farthest out, so that the tree's reach covers every view — and all
     /// views come from one `rtc_render_views` batch.  Canvas i is what `cameras[i].render(world, depth)` returns.
     pub fn render_b200_views(cameras: &[Camera], world: World, reflection_recursion_depth: i16) -> Vec<Canvas> {
-        assert!(!cameras.is_empty(), "render_b200_views needs at least one camera");
+        let (far, w, h, views) = Camera::batch_views(cameras);
+        let mut rgb = vec![0f32; views.len() * w * h * 3];
+        unsafe {
+            let scene = cameras[far].commit_b200(&world);
+            let mut stats: sys::RtcStats = std::mem::zeroed();
+            check(sys::rtc_render_views(scene, reflection_recursion_depth as i32, views.len() as u32, views.as_ptr(), rgb.as_mut_ptr(),
+                                        std::ptr::null_mut(), &mut stats));
+            sys::rtc_scene_destroy(scene);
+        }
+        rgb.chunks(w * h * 3)
+            .map(|frame| {
+                let mut canvas = Canvas::new(w, h);
+                for y in 0..h {
+                    for x in 0..w {
+                        let i = (y * w + x) * 3;
+                        canvas.write_pixel(x, y, Color::new(frame[i], frame[i + 1], frame[i + 2]));
+                    }
+                }
+                canvas
+            })
+            .collect()
+    }
+
+    /// `Camera::render` then `Canvas::to_ppm` for several cameras of one canvas size, committed once as `render_b200_views`
+    /// commits them, with every view's text written on the device (`rtc_render_views_ppm`).  String i is what
+    /// `cameras[i].render(world, depth).to_ppm()` returns.
+    pub fn render_b200_views_ppm(cameras: &[Camera], world: World, reflection_recursion_depth: i16) -> Vec<String> {
+        let (far, w, h, views) = Camera::batch_views(cameras);
+        let capacity = views.len() * unsafe { sys::rtc_ppm_bound(w as u32, h as u32) };
+        let mut text = vec![0u8; capacity];
+        let mut offsets = vec![0usize; views.len() + 1];
+        unsafe {
+            let scene = cameras[far].commit_b200(&world);
+            let mut stats: sys::RtcStats = std::mem::zeroed();
+            check(sys::rtc_render_views_ppm(scene, reflection_recursion_depth as i32, views.len() as u32, views.as_ptr(),
+                                            text.as_mut_ptr() as *mut std::os::raw::c_char, capacity, offsets.as_mut_ptr(), &mut stats));
+            sys::rtc_scene_destroy(scene);
+        }
+        offsets
+            .windows(2)
+            .map(|o| String::from_utf8(text[o[0]..o[1]].to_vec()).expect("PPM text is ASCII"))
+            .collect()
+    }
+
+    /// A batch's views and the camera it commits with: the one whose origin is farthest out, so that the tree's reach
+    /// covers every view.  Every camera must have one canvas size.
+    fn batch_views(cameras: &[Camera]) -> (usize, usize, usize, Vec<sys::RtcView>) {
+        assert!(!cameras.is_empty(), "a batch needs at least one camera");
         let reach = |c: &Camera| {
             let m = mat16(&c.transform_inverse);
             m[3].abs().max(m[7].abs()).max(m[11].abs())
@@ -602,25 +649,6 @@ impl Camera {
                 }
             })
             .collect();
-        let mut rgb = vec![0f32; views.len() * w * h * 3];
-        unsafe {
-            let scene = cameras[far].commit_b200(&world);
-            let mut stats: sys::RtcStats = std::mem::zeroed();
-            check(sys::rtc_render_views(scene, reflection_recursion_depth as i32, views.len() as u32, views.as_ptr(), rgb.as_mut_ptr(),
-                                        std::ptr::null_mut(), &mut stats));
-            sys::rtc_scene_destroy(scene);
-        }
-        rgb.chunks(w * h * 3)
-            .map(|frame| {
-                let mut canvas = Canvas::new(w, h);
-                for y in 0..h {
-                    for x in 0..w {
-                        let i = (y * w + x) * 3;
-                        canvas.write_pixel(x, y, Color::new(frame[i], frame[i + 1], frame[i + 2]));
-                    }
-                }
-                canvas
-            })
-            .collect()
+        (far, w, h, views)
     }
 }

@@ -215,6 +215,10 @@ extern "C" {
     pub fn rtc_ppm_bound(width: u32, height: u32) -> usize;
     pub fn rtc_render_ppm(scene: *mut RtcScene, depth: i32, ppm: *mut c_char, capacity: usize, ppm_bytes: *mut usize,
                           stats: *mut RtcStats) -> c_int;
+    /// `rtc_render_views` then `Canvas::to_ppm` of every view, the texts written on the device one after the other: view v's
+    /// is `ppm[view_offsets[v]..view_offsets[v + 1]]`; `capacity >= n_views * rtc_ppm_bound(w, h)`, `n_views + 1` offsets.
+    pub fn rtc_render_views_ppm(scene: *mut RtcScene, depth: i32, n_views: u32, views: *const RtcView, ppm: *mut c_char,
+                                capacity: usize, view_offsets: *mut usize, stats: *mut RtcStats) -> c_int;
     pub fn rtc_trace_rays(scene: *mut RtcScene, n: u32, origins: *const f32, directions: *const f32, depth: i32,
                           out_rgb: *mut f32, out_t: *mut f32, out_prim: *mut i32) -> c_int;
     pub fn rtc_shard_bands(height: u32, shard: i32, n_shards: i32, first_rows: *mut u32) -> c_int;
