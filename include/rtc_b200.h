@@ -323,10 +323,40 @@ int rtc_render_views(RtcScene*, int32_t depth, uint32_t n_views, const RtcView* 
  *     frame that rtc_render uses for its 8-bit plane, grown to the device's share of the text and kept with the device.
  *   - Device memory kept with each device for later calls: the text of its rows (up to 12 bytes per pixel, 89 MB for a
  *     3840x2160 frame) and 16 bytes per row.
- *   - Not provided: a shard of a frame shared by several processes (rtc_render_shard) — a process cannot know the offsets of
- *     rows other processes render; encoding a plane that is not the committed scene's frame. */
+ *   - Not provided: encoding a plane that is not the committed scene's frame. */
 size_t rtc_ppm_bound(uint32_t width, uint32_t height);
 int rtc_render_ppm(RtcScene*, int32_t depth, char* ppm, size_t capacity, size_t* ppm_bytes, RtcStats* stats);
+/* rtc_render_ppm for one shard of a frame shared by several processes (rtc_render_shard's split), in two phases with the
+ * callers' exchange of row lengths in between: a row's text length depends only on its values, so once every row's length is
+ * known each process can place its own bands.  The library has no communicator: the exchange is the callers' (shared memory
+ * and a barrier on one node; an all-reduce of zeroed arrays across nodes).
+ *   - Phase 1, rtc_render_shard_ppm_rows: rtc_render_shard with the frame left on the device, then the byte length of the text
+ *     of every row the shard owns.  row_bytes has height entries in frame-row order; only the entries of the shard's rows
+ *     (rtc_shard_bands) are written, the others are not touched — so the ranks can write into one shared array, or into zeroed
+ *     private ones summed by an all-reduce.  stats are rtc_render_shard's, with total_ms covering the whole phase.
+ *   - Phase 2, rtc_write_shard_ppm: given every row's length (all shards' entries), writes the text of the shard's bands at
+ *     their offsets in ppm; shard 0 also writes the header.  *ppm_bytes receives the whole text's length, the same on every
+ *     shard.  A shard writes only [band_at, band_at + band_bytes) of each of its bands (and shard 0 the header): no other byte
+ *     of ppm, so the ranks can write into one shared buffer without locking.  No stats.
+ *   - The bytes: the union of every shard's writes is byte for byte rtc_render_ppm's text of the same scene — Canvas::to_ppm of
+ *     rtc_render's 8-bit plane — for every kernel build and option.
+ *   - The arguments are checked before the scene's state, all with RTC_ERR_INVALID: a NULL pointer (stats may be NULL);
+ *     n_shards < 1 or shard outside [0, n_shards); in phase 1 a depth outside [0, 23]; in phase 2 a capacity below
+ *     rtc_ppm_bound of the committed canvas, and any row_bytes[r] outside [6 * width, 12 * width] (every value takes 2 to 4
+ *     bytes with its separator, so an array in range never lays out a text longer than the bound).  Then an uncommitted scene
+ *     is RTC_ERR_STATE, and so is a scene committed on more than one device (rtc_render_shard's rule).
+ *   - Phase state: phase 2 needs a phase 1 on the same scene with the same shard and n_shards, and no render (of any kind),
+ *     rtc_set_* / rtc_map_* or commit in between; otherwise it is RTC_ERR_STATE.  Phase 2 may be repeated (into a second
+ *     destination, say).  A failed phase 2 changes nothing.
+ *   - The own-row check: phase 2 compares the shard's own entries of row_bytes with the lengths its phase 1 computed (kept
+ *     with the scene); a mismatch is a broken exchange and RTC_ERR_INVALID, naming the first such row.  A wrong entry for
+ *     another shard's row cannot be detected here: that is the callers' exchange.
+ *   - Pinned and pageable destinations both work, as in rtc_render_ppm: a pageable one of 4 MiB or more (the whole text's
+ *     length) receives the shard's bands through the device's pinned staging frame, piece by piece.
+ *   - Device memory kept with the device for later calls: rtc_render_ppm's buffers (the text of its rows, 16 bytes per row). */
+int rtc_render_shard_ppm_rows(RtcScene*, int32_t depth, int32_t shard, int32_t n_shards, uint64_t* row_bytes, RtcStats* stats);
+int rtc_write_shard_ppm(RtcScene*, int32_t shard, int32_t n_shards, const uint64_t* row_bytes, char* ppm, size_t capacity,
+                        size_t* ppm_bytes);
 /* rtc_render_views followed by Canvas::to_ppm of every view, with the text written on the device.
  *   - ppm receives the views' texts one after the other, no terminating NUL: view v's text is ppm[view_offsets[v] ..
  *     view_offsets[v + 1]).  view_offsets has n_views + 1 entries: view_offsets[0] = 0, view_offsets[n_views] the total.

@@ -111,6 +111,8 @@ _HOST_EXTRAS = {
     "sg_farthest_camera": (_I, [_V, _IP, _I]),
     "sg_camera_render_ppm": (C.c_int64, [_V, _I, _I, _I, C.c_void_p, C.c_int64, C.POINTER(SgStats)]),
     "sg_render_prepared_ppm": (C.c_int64, [_V, _I, _I, _I, C.c_void_p, C.c_int64, C.POINTER(SgStats)]),
+    "sg_render_prepared_shard_ppm_rows": (_I, [_V, _I, _I, _I, _I, _I, C.c_void_p, C.POINTER(SgStats)]),
+    "sg_write_prepared_shard_ppm": (C.c_int64, [_V, _I, _I, _I, C.c_void_p, C.c_void_p, C.c_int64]),
     "sg_render_prepared_views_ppm": (C.c_int64, [_V, _I, _I, _I, _IP, _I, C.c_void_p, C.c_int64, C.POINTER(C.c_size_t),
                                                  C.POINTER(SgStats)]),
     "sg_camera_render_views_ppm": (C.c_int64, [_V, _IP, _I, _I, _I, C.c_void_p, C.c_int64, C.POINTER(C.c_size_t),
@@ -147,6 +149,15 @@ def _ppm_buffer(api, w, h, out, n=1):
         need = f"rtc_ppm_bound = {bound}" if n == 1 else f"{n} * rtc_ppm_bound = {n * bound}"
         raise ValueError(f"out must be a writable C-contiguous uint8 array of at least {need} bytes")
     return buf
+
+
+def _row_bytes(row_bytes, h):
+    """The row lengths of a shard's text (rtc_render_shard_ppm_rows / rtc_write_shard_ppm): a writable C-contiguous uint64
+    array of one entry per frame row."""
+    if not isinstance(row_bytes, np.ndarray) or row_bytes.dtype != np.uint64 or row_bytes.shape != (h,) \
+            or not row_bytes.flags.c_contiguous or not row_bytes.flags.writeable:
+        raise ValueError(f"row_bytes must be a writable C-contiguous uint64 array of shape ({h},)")
+    return row_bytes
 
 
 def _ppm_texts(buf, offsets):
@@ -212,6 +223,33 @@ class PreparedScene:
                                                      C.byref(stats)))
         self.last_stats = api.last_rtc_stats()
         return buf[:n].tobytes().decode("ascii")
+
+    def render_shard_ppm_rows(self, shard, n_shards, row_bytes, depth=DEFAULT_RAY_RECURSION_DEPTH, fma=False):
+        """rtc_render_shard_ppm_rows, the first phase of one shard's text of a frame shared by several processes: renders the
+        shard's bands (rtc_render_shard, the frame left on the device) and writes the byte length of each of their rows'
+        text into `row_bytes` (a uint64 array of one entry per frame row; the other shards' entries are not touched).  The
+        callers then exchange the entries (multi.render_ppm_shared does it through shared memory) and call write_shard_ppm."""
+        h = self.camera.height_pixels
+        api = self.api
+        row_bytes = _row_bytes(row_bytes, h)
+        stats = SgStats()
+        api.check(api.lib.sg_render_prepared_shard_ppm_rows(api.ctx, self.handle, int(depth), int(shard), int(n_shards), int(fma),
+                                                            row_bytes.ctypes.data, C.byref(stats)))
+        self.last_stats = api.last_rtc_stats()
+
+    def write_shard_ppm(self, shard, n_shards, row_bytes, out) -> int:
+        """rtc_write_shard_ppm, the second phase: given every row's length (all shards' entries of `row_bytes`), writes the
+        text of this shard's bands at their offsets in `out` (a writable uint8 array of at least rtc_ppm_bound bytes, shared
+        by the ranks); shard 0 also writes the header.  Returns the whole text's length; once every shard has written,
+        out[:length] is render_ppm's text."""
+        w, h = self.camera.width_pixels, self.camera.height_pixels
+        api = self.api
+        row_bytes = _row_bytes(row_bytes, h)
+        if out is None:
+            raise ValueError("write_shard_ppm needs out: the buffer every shard writes its bands into")
+        buf = _ppm_buffer(api, w, h, out)
+        return api.check(api.lib.sg_write_prepared_shard_ppm(api.ctx, self.handle, int(shard), int(n_shards), row_bytes.ctypes.data,
+                                                             buf.ctypes.data, buf.nbytes))
 
     def render_views_ppm(self, cameras, depth=DEFAULT_RAY_RECURSION_DEPTH, out=None, fma=False) -> list:
         """rtc_render_views_ppm: every camera (of this scene's canvas size) rendered from the committed scene in one batch,

@@ -618,6 +618,26 @@ int64_t sg_render_prepared_ppm(sg_ctx* c, int h, int depth, int fma, char* out, 
     to_sg_stats(c->last_stats, stats);
     return rc ? fail(rtc_last_error()) : (int64_t)bytes;
 }
+// The two phases of one shard's text of a frame shared by several processes (rtc_render_shard_ppm_rows, rtc_write_shard_ppm)
+// on a prepared scene.  No one-shot form: the callers exchange the row lengths between the two calls.
+int sg_render_prepared_shard_ppm_rows(sg_ctx* c, int h, int depth, int shard, int n_shards, int fma, uint64_t* row_bytes,
+                                      sg_stats* stats) {
+    if (h < 0 || h >= (int)c->prepared.size() || !c->prepared[h]) return fail("bad prepared handle");
+    RtcScene* scene = c->prepared[h]->scene;
+    if (rtc_set_option(scene, RTC_OPT_FMA_CONTRACTION, fma ? 1 : 0)) return fail(rtc_last_error());
+    const int rc = rtc_render_shard_ppm_rows(scene, depth, shard, n_shards, row_bytes, &c->last_stats);
+    to_sg_stats(c->last_stats, stats);
+    return rc ? fail(rtc_last_error()) : 0;
+}
+// ... returns the whole text's length, or -1
+int64_t sg_write_prepared_shard_ppm(sg_ctx* c, int h, int shard, int n_shards, const uint64_t* row_bytes, char* out,
+                                    int64_t capacity) {
+    if (h < 0 || h >= (int)c->prepared.size() || !c->prepared[h]) return fail("bad prepared handle");
+    if (capacity < 0) return fail("negative capacity");
+    size_t bytes = 0;
+    const int rc = rtc_write_shard_ppm(c->prepared[h]->scene, shard, n_shards, row_bytes, out, (size_t)capacity, &bytes);
+    return rc ? fail(rtc_last_error()) : (int64_t)bytes;
+}
 // rtc_render_views on a prepared scene: n cameras (handles) of its canvas size, frames view-major in out_rgb / out_u8
 int sg_render_prepared_views(sg_ctx* c, int h, int depth, int n, const int* cams, int fma, float* out_rgb, uint8_t* out_u8,
                              sg_stats* stats) {

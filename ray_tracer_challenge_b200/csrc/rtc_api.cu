@@ -504,6 +504,7 @@ int render_impl(RtcScene* s, int depth, int shard0, int n_shards_ext, float* rgb
     if (external && ndev != 1) return fail(RTC_ERR_STATE, "rtc_render_shard needs a scene committed on exactly one device");
     if (external && (shard0 < 0 || shard0 >= n_shards_ext)) return fail(RTC_ERR_INVALID, "bad shard index");
     const int n_shards = external ? n_shards_ext : ndev;
+    s->shard_ppm = {};  // a new frame: a pending rtc_write_shard_ppm is void
     const int total_bands = ((int)s->height + kBandRows - 1) / kBandRows;
     const bool copy_out = rgb || u8;
     RtcStats st;
@@ -836,6 +837,7 @@ int render_views_body(RtcScene* s, int depth, uint32_t n_views, const RtcView* v
                     return fail(RTC_ERR_INVALID, msg);
                 }
             }
+    s->shard_ppm = {};  // any render voids a pending rtc_write_shard_ppm (include/rtc_b200.h)
     auto t0 = std::chrono::steady_clock::now();
     const int ndev = (int)s->replicas.size(), n_shards = ndev;
     const int total_bands = ((int)s->height + kBandRows - 1) / kBandRows;
@@ -1082,25 +1084,24 @@ std::vector<PpmRun> ppm_runs(const PpmLayout& L, int i, int ndev, int nb, int e0
     return runs;
 }
 
-// The PPM text of n_views frames of s's canvas size, each device i holding view v's 8-bit plane (its own bands of it) at
-// frames[i] + v * view_stride.  On every device: one ppm_row_bytes launch over its rows of every view, one copy of the
-// lengths back and a synchronize; the host's scan over all of them (ppm_layout, which writes the headers into out); one
-// ppm_write launch into d_ppm; and once every device has its kernels, the copies of its texts to their offsets in out.
-// view_at[v] receives view v's offset in out, *bytes the whole length.  The copies into a pinned destination may still be
-// in flight on the devices' render streams when this returns; a staged one has arrived.
-int write_ppm_text(RtcScene* s, const unsigned char* const* frames, int n_views, size_t view_stride, char* out, size_t capacity,
-                   size_t* view_at, size_t* bytes) {
+// The PPM text is written in three steps: (a) ppm_row_lengths, (b) a host scan (ppm_layout from the devices' own lengths, or
+// ppm_layout_frame_rows from every row's), (c) ppm_write_copy.  Device i encodes the rows of its PpmRows: its interleaved bands
+// of the committed devices' split (shard i of ndev), or, for a shard of a frame shared by several processes (one device),
+// the bands of shard0 of n_shards_ext.
+
+// (a) On every device: one ppm_row_bytes launch over its rows of every view, each device i holding view v's 8-bit plane (its
+// own bands of it) at frames[i] + v * view_stride; the lengths copied back to the slot's h_ppm_rows, and a synchronize.
+int ppm_row_lengths(RtcScene* s, const unsigned char* const* frames, int n_views, size_t view_stride, int shard0, int n_shards_ext,
+                    std::vector<PpmRows>& rows) {
     const int ndev = (int)s->replicas.size();
-    const int total_bands = ((int)s->height + kBandRows - 1) / kBandRows;
-    std::vector<PpmRows> rows(ndev);
-    std::vector<unsigned long long*> lengths(ndev);
+    rows.resize(ndev);
     for (int i = 0; i < ndev; i++) {
         DeviceSlot* slot = s->replicas[i].slot;
         CUDA_TRY(cudaSetDevice(slot->device));
-        rows[i] = PpmRows{frames[i], (int)s->width, i, ndev, ppm_device_rows(s->height, i, ndev), n_views, view_stride};
+        const int shard = n_shards_ext > 0 ? shard0 : i, n_shards = n_shards_ext > 0 ? n_shards_ext : ndev;
+        rows[i] = PpmRows{frames[i], (int)s->width, shard, n_shards, ppm_device_rows(s->height, shard, n_shards), n_views, view_stride};
         const size_t n_rows = (size_t)rows[i].n_rows * n_views;
         if (int rc = ensure_ppm_rows(slot, std::max<size_t>(n_rows, 1))) return rc;
-        lengths[i] = slot->h_ppm_rows;
         launch_ppm_row_bytes(rows[i], slot->d_ppm_rows, slot->sm_count, slot->stream);
         CUDA_TRY(cudaGetLastError());
         CUDA_TRY(cudaMemcpyAsync(slot->h_ppm_rows, slot->d_ppm_rows, n_rows * sizeof(unsigned long long), cudaMemcpyDeviceToHost,
@@ -1110,15 +1111,20 @@ int write_ppm_text(RtcScene* s, const unsigned char* const* frames, int n_views,
         CUDA_TRY(cudaSetDevice(s->replicas[i].slot->device));
         CUDA_TRY(cudaStreamSynchronize(s->replicas[i].slot->stream));
     }
-    PpmLayout L;
-    const std::string header = ppm_header(s->width, s->height);
-    ppm_layout(s->height, ndev, header.size(), lengths.data(), L, n_views, header.data(), out);
-    if (L.total > capacity) return fail(RTC_ERR_CAPACITY, "the PPM text outgrew rtc_ppm_bound");  // cannot happen
-    for (int v = 0; v < n_views; v++) view_at[v] = L.view_at[v];
+    return 0;
+}
+
+// (c) On every device: its rows' offsets in its text (the slot's h_ppm_rows, as the scan left them) up, one ppm_write launch
+// into d_ppm, and once every device has its kernels, the copies of its (view, band) texts to their offsets in out (L).  The
+// copies into a pinned destination may still be in flight on the devices' render streams when this returns; a staged one
+// has arrived.
+int ppm_write_copy(RtcScene* s, const std::vector<PpmRows>& rows, const PpmLayout& L, char* out) {
+    const int ndev = (int)s->replicas.size(), n_shards = rows[0].n_shards, n_views = rows[0].n_views;
+    const int total_bands = L.total_bands;
     for (int i = 0; i < ndev; i++) {
         DeviceSlot* slot = s->replicas[i].slot;
         CUDA_TRY(cudaSetDevice(slot->device));
-        if (int rc = ensure_ppm_text(slot, std::max<size_t>(L.device_bytes[i], 16))) return rc;
+        if (int rc = ensure_ppm_text(slot, std::max<size_t>(L.device_bytes[rows[i].shard], 16))) return rc;
         CUDA_TRY(cudaMemcpyAsync(slot->d_ppm_rows, slot->h_ppm_rows, (size_t)rows[i].n_rows * n_views * sizeof(unsigned long long),
                                  cudaMemcpyHostToDevice, slot->stream));
         launch_ppm_write(rows[i], slot->d_ppm_rows, slot->d_ppm, slot->sm_count, slot->stream);
@@ -1129,28 +1135,29 @@ int write_ppm_text(RtcScene* s, const unsigned char* const* frames, int n_views,
     const bool staged = L.total >= ((size_t)4 << 20) && is_pageable(out);
     struct Piece {
         DeviceSlot* slot;
-        int dev, nb, e0, e1;  // (view, band) texts [e0, e1) of the device's text
+        int part, nb, e0, e1;  // (view, band) texts [e0, e1) of the device's text
         cudaEvent_t done;
     };
     std::vector<Piece> pieces;
     for (int i = 0; i < ndev; i++) {  // the copies, queued once every device has its kernels
         DeviceSlot* slot = s->replicas[i].slot;
         CUDA_TRY(cudaSetDevice(slot->device));
-        const int nb = i < total_bands ? (total_bands - i + ndev - 1) / ndev : 0, entries = nb * n_views;
+        const int part = rows[i].shard;  // the device's bands: b % n_shards == part
+        const int nb = part < total_bands ? (total_bands - part + n_shards - 1) / n_shards : 0, entries = nb * n_views;
         if (entries == 0) continue;
         // pieces of about 4 MiB (whole bands) when staged, so that the host's copies overlap the device's; else one
-        const int n_pieces = staged ? (int)std::max<size_t>(1, std::min<size_t>((size_t)entries, L.device_bytes[i] >> 22)) : 1;
+        const int n_pieces = staged ? (int)std::max<size_t>(1, std::min<size_t>((size_t)entries, L.device_bytes[part] >> 22)) : 1;
         if (staged)
-            if (int rc = ensure_stage(slot, &slot->h_stage_u8, &slot->h_stage_u8_bytes, L.device_bytes[i])) return rc;
+            if (int rc = ensure_stage(slot, &slot->h_stage_u8, &slot->h_stage_u8_bytes, L.device_bytes[part])) return rc;
         for (int k = 0; k < n_pieces; k++) {
             const int e0 = (int)((int64_t)entries * k / n_pieces), e1 = (int)((int64_t)entries * (k + 1) / n_pieces);
             if (!staged) {
-                for (const PpmRun& r : ppm_runs(L, i, ndev, nb, e0, e1))
+                for (const PpmRun& r : ppm_runs(L, part, n_shards, nb, e0, e1))
                     CUDA_TRY(cudaMemcpyAsync(out + r.at, slot->d_ppm + r.local, r.bytes, cudaMemcpyDeviceToHost, slot->stream));
                 continue;
             }
-            const size_t first = (size_t)(e0 / nb) * total_bands + i + (size_t)(e0 % nb) * ndev;
-            const size_t last = (size_t)((e1 - 1) / nb) * total_bands + i + (size_t)((e1 - 1) % nb) * ndev;
+            const size_t first = (size_t)(e0 / nb) * total_bands + part + (size_t)(e0 % nb) * n_shards;
+            const size_t last = (size_t)((e1 - 1) / nb) * total_bands + part + (size_t)((e1 - 1) % nb) * n_shards;
             const size_t local = L.band_local[first], n = L.band_local[last] + L.band_bytes[last] - local;
             CUDA_TRY(cudaMemcpyAsync(slot->h_stage_u8 + local, slot->d_ppm + local, n, cudaMemcpyDeviceToHost, slot->stream));
             const size_t used = pieces.size();
@@ -1160,13 +1167,13 @@ int write_ppm_text(RtcScene* s, const unsigned char* const* frames, int n_views,
                 slot->copy_done.push_back(e);
             }
             CUDA_TRY(cudaEventRecord(slot->copy_done[used], slot->stream));
-            pieces.push_back({slot, i, nb, e0, e1, slot->copy_done[used]});
+            pieces.push_back({slot, part, nb, e0, e1, slot->copy_done[used]});
         }
     }
     for (const Piece& p : pieces) {
         CUDA_TRY(cudaSetDevice(p.slot->device));
         CUDA_TRY(cudaEventSynchronize(p.done));
-        const std::vector<PpmRun> runs = ppm_runs(L, p.dev, ndev, p.nb, p.e0, p.e1);
+        const std::vector<PpmRun> runs = ppm_runs(L, p.part, n_shards, p.nb, p.e0, p.e1);
         if (runs.size() == 1) {
             parallel_copy(out + runs[0].at, p.slot->h_stage_u8 + runs[0].local, runs[0].bytes, (size_t)96 << 10);
             continue;
@@ -1175,6 +1182,25 @@ int write_ppm_text(RtcScene* s, const unsigned char* const* frames, int n_views,
             for (size_t r = rb; r < re; r++) memcpy(out + runs[r].at, p.slot->h_stage_u8 + runs[r].local, runs[r].bytes);
         });
     }
+    return 0;
+}
+
+// The PPM text of n_views frames of s's canvas size on the committed devices: (a), the host's scan over the lengths of every
+// device (ppm_layout, which writes the headers into out), (c).  view_at[v] receives view v's offset in out, *bytes the whole
+// length.
+int write_ppm_text(RtcScene* s, const unsigned char* const* frames, int n_views, size_t view_stride, char* out, size_t capacity,
+                   size_t* view_at, size_t* bytes) {
+    std::vector<PpmRows> rows;
+    if (int rc = ppm_row_lengths(s, frames, n_views, view_stride, 0, 0, rows)) return rc;
+    const int ndev = (int)s->replicas.size();
+    std::vector<unsigned long long*> lengths(ndev);
+    for (int i = 0; i < ndev; i++) lengths[i] = s->replicas[i].slot->h_ppm_rows;
+    PpmLayout L;
+    const std::string header = ppm_header(s->width, s->height);
+    ppm_layout(s->height, ndev, header.size(), lengths.data(), L, n_views, header.data(), out);
+    if (L.total > capacity) return fail(RTC_ERR_CAPACITY, "the PPM text outgrew rtc_ppm_bound");  // cannot happen
+    for (int v = 0; v < n_views; v++) view_at[v] = L.view_at[v];
+    if (int rc = ppm_write_copy(s, rows, L, out)) return rc;
     *bytes = L.total;
     return 0;
 }
@@ -1234,6 +1260,100 @@ int render_views_ppm_impl(RtcScene* s, int depth, uint32_t n_views, const RtcVie
     return rc;
 }
 
+// rtc_render_shard_ppm_rows / rtc_write_shard_ppm: one shard of a frame shared by several processes.  The argument checks
+// of both phases (no device needed), then the scene's state.
+int check_shard(int shard, int n_shards, const char* fn) {
+    if (n_shards < 1 || shard < 0 || shard >= n_shards)
+        return fail(RTC_ERR_INVALID, std::string(fn) + ": shard " + std::to_string(shard) + " of n_shards " + std::to_string(n_shards) +
+                                         ": n_shards must be >= 1 and shard in [0, n_shards)");
+    return 0;
+}
+int check_shard_scene(const RtcScene* s, const char* fn) {
+    if (!s->committed) return fail(RTC_ERR_STATE, std::string(fn) + " before rtc_scene_commit");
+    if (s->replicas.size() != 1) return fail(RTC_ERR_STATE, std::string(fn) + " needs a scene committed on exactly one device");
+    return 0;
+}
+
+// Phase 1: rtc_render_shard with the frame left on the device, then (a) for the shard's rows.  Their lengths go to row_bytes
+// (frame-row order; no other entry is touched) and are kept for phase 2's own-row check.
+int render_shard_ppm_rows_impl(RtcScene* s, int depth, int shard, int n_shards, uint64_t* row_bytes, RtcStats* stats) {
+    const char* fn = "rtc_render_shard_ppm_rows";
+    if (!s) return fail(RTC_ERR_INVALID, "null scene");
+    if (!row_bytes) return fail(RTC_ERR_INVALID, std::string(fn) + ": row_bytes must be non-null");
+    if (int rc = check_shard(shard, n_shards, fn)) return rc;
+    if (int rc = check_depth(depth)) return rc;
+    if (int rc = check_shard_scene(s, fn)) return rc;
+    const auto t0 = std::chrono::steady_clock::now();
+    RtcStats st;
+    memset(&st, 0, sizeof(st));
+    if (int rc = render_impl(s, depth, shard, n_shards, nullptr, nullptr, &st, false)) {  // the frame stays on the device
+        if (stats) *stats = st;
+        return rc;
+    }
+    const unsigned char* frame = s->replicas[0].slot->d_u8;
+    std::vector<PpmRows> rows;
+    if (int rc = ppm_row_lengths(s, &frame, 1, 0, shard, n_shards, rows)) return rc;
+    const unsigned long long* lengths = s->replicas[0].slot->h_ppm_rows;
+    s->shard_ppm.rows.assign(lengths, lengths + rows[0].n_rows);  // band order: the shard's frame rows in increasing order
+    s->shard_ppm.shard = shard, s->shard_ppm.n_shards = n_shards;
+    for (uint32_t y = 0, k = 0; y < s->height; y++)
+        if ((int)(y / kBandRows % n_shards) == shard) row_bytes[y] = lengths[k++];
+    st.total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    if (stats) *stats = st;
+    return 0;
+}
+
+// Phase 2: the own-row check, the scan over every row's length (ppm_layout_frame_rows; shard 0 writes the header), then (c)
+// for the shard's bands.
+int write_shard_ppm_impl(RtcScene* s, int shard, int n_shards, const uint64_t* row_bytes, char* ppm, size_t capacity,
+                         size_t* ppm_bytes) {
+    const char* fn = "rtc_write_shard_ppm";
+    if (!s) return fail(RTC_ERR_INVALID, "null scene");
+    if (!row_bytes || !ppm || !ppm_bytes) return fail(RTC_ERR_INVALID, std::string(fn) + ": row_bytes, ppm and ppm_bytes must be non-null");
+    if (int rc = check_shard(shard, n_shards, fn)) return rc;
+    const size_t bound = rtc_ppm_bound(s->width, s->height);
+    if (capacity < bound)
+        return fail(RTC_ERR_INVALID, std::string(fn) + ": capacity " + std::to_string(capacity) + " is below rtc_ppm_bound = " +
+                                         std::to_string(bound));
+    // every value takes 2 to 4 bytes with its separator: an array in range never lays out a text longer than the bound
+    const uint64_t lo = 6 * (uint64_t)s->width, hi = 12 * (uint64_t)s->width;
+    for (uint32_t y = 0; y < s->height; y++)
+        if (row_bytes[y] < lo || row_bytes[y] > hi)
+            return fail(RTC_ERR_INVALID, std::string(fn) + ": row_bytes[" + std::to_string(y) + "] = " + std::to_string(row_bytes[y]) +
+                                             " is outside [6 * width, 12 * width] = [" + std::to_string(lo) + ", " + std::to_string(hi) + "]");
+    if (int rc = check_shard_scene(s, fn)) return rc;
+    if (s->shard_ppm.n_shards != n_shards || s->shard_ppm.shard != shard)
+        return fail(RTC_ERR_STATE, std::string(fn) + ": shard " + std::to_string(shard) + " of " + std::to_string(n_shards) +
+                                       " needs rtc_render_shard_ppm_rows of the same shard and n_shards first, with no render, "
+                                       "rtc_set_* or commit since");
+    // the entries of the shard's own rows must be the lengths phase 1 computed: anything else is a broken exchange (a wrong
+    // entry of another shard's row cannot be told from a right one here)
+    for (uint32_t y = 0, k = 0; y < s->height; y++) {
+        if ((int)(y / kBandRows % n_shards) != shard) continue;
+        if (row_bytes[y] != s->shard_ppm.rows[k])
+            return fail(RTC_ERR_INVALID, std::string(fn) + ": row_bytes[" + std::to_string(y) + "] = " + std::to_string(row_bytes[y]) +
+                                             ", but shard " + std::to_string(shard) + "'s rtc_render_shard_ppm_rows measured " +
+                                             std::to_string(s->shard_ppm.rows[k]) + " bytes for that row: the exchange of row lengths is broken");
+        k++;
+    }
+    const std::string header = ppm_header(s->width, s->height);
+    std::vector<std::vector<unsigned long long>> shard_rows;
+    PpmLayout L;
+    ppm_layout_frame_rows(s->height, n_shards, header.size(), row_bytes, shard_rows, L, shard == 0 ? header.data() : nullptr,
+                          shard == 0 ? ppm : nullptr);
+    if (L.total > capacity) return fail(RTC_ERR_CAPACITY, "the PPM text outgrew rtc_ppm_bound");  // cannot happen
+    DeviceSlot* slot = s->replicas[0].slot;
+    const std::vector<unsigned long long>& own = shard_rows[shard];
+    if (int rc = ensure_ppm_rows(slot, std::max<size_t>(own.size(), 1))) return rc;
+    if (!own.empty()) memcpy(slot->h_ppm_rows, own.data(), own.size() * sizeof(unsigned long long));
+    const std::vector<PpmRows> rows{PpmRows{slot->d_u8, (int)s->width, shard, n_shards, (int)own.size()}};
+    if (int rc = ppm_write_copy(s, rows, L, ppm)) return rc;
+    CUDA_TRY(cudaSetDevice(slot->device));
+    CUDA_TRY(cudaStreamSynchronize(slot->stream));
+    *ppm_bytes = L.total;
+    return 0;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1273,6 +1393,7 @@ int rtc_set_camera(RtcScene* s, uint32_t w, uint32_t h, float half_w, float half
     memcpy(s->cam_inv, inv, sizeof(s->cam_inv));
     s->have_camera = true;
     s->committed = false;
+    s->shard_ppm = {};
     return 0;
 }
 int rtc_set_primitives(RtcScene* s, uint32_t n, const RtcPrim* prims) {
@@ -1281,6 +1402,7 @@ int rtc_set_primitives(RtcScene* s, uint32_t n, const RtcPrim* prims) {
     s->prims.resize(n);
     parallel_copy(s->prims.data(), prims, (size_t)n * sizeof(RtcPrim));
     s->committed = false;
+    s->shard_ppm = {};
     return 0;
 }
 int rtc_set_nodes(RtcScene* s, uint32_t n_nodes, const RtcNode* nodes, uint32_t n_refs, const int32_t* refs) {
@@ -1289,6 +1411,7 @@ int rtc_set_nodes(RtcScene* s, uint32_t n_nodes, const RtcNode* nodes, uint32_t 
     parallel_copy(s->nodes.data(), nodes, (size_t)n_nodes * sizeof(RtcNode));
     s->refs.assign(refs, refs + n_refs);
     s->committed = false;
+    s->shard_ppm = {};
     return 0;
 }
 int rtc_map_primitives(RtcScene* s, uint32_t n, RtcPrim** prims) {
@@ -1297,6 +1420,7 @@ int rtc_map_primitives(RtcScene* s, uint32_t n, RtcPrim** prims) {
     s->prims.resize(n);
     *prims = s->prims.data();
     s->committed = false;
+    s->shard_ppm = {};
     return 0;
 }
 int rtc_map_nodes(RtcScene* s, uint32_t n_nodes, uint32_t n_refs, RtcNode** nodes, int32_t** refs) {
@@ -1305,6 +1429,7 @@ int rtc_map_nodes(RtcScene* s, uint32_t n_nodes, uint32_t n_refs, RtcNode** node
     s->refs.resize(n_refs);
     *nodes = s->nodes.data(), *refs = s->refs.data();
     s->committed = false;
+    s->shard_ppm = {};
     return 0;
 }
 int rtc_set_materials(RtcScene* s, uint32_t n, const RtcMaterial* m) {
@@ -1312,6 +1437,7 @@ int rtc_set_materials(RtcScene* s, uint32_t n, const RtcMaterial* m) {
     if (n >= (1u << 23)) return fail(RTC_ERR_CAPACITY, "too many materials");
     s->materials.assign(m, m + n);
     s->committed = false;
+    s->shard_ppm = {};
     return 0;
 }
 int rtc_set_patterns(RtcScene* s, uint32_t n, const RtcPattern* p, uint32_t n_uv, const RtcUvPattern* uv) {
@@ -1319,6 +1445,7 @@ int rtc_set_patterns(RtcScene* s, uint32_t n, const RtcPattern* p, uint32_t n_uv
     s->patterns.assign(p, p + n);
     s->uvs.assign(uv, uv + n_uv);
     s->committed = false;
+    s->shard_ppm = {};
     return 0;
 }
 int rtc_set_textures(RtcScene* s, uint32_t n, const RtcTexture* t) {
@@ -1332,6 +1459,7 @@ int rtc_set_textures(RtcScene* s, uint32_t n, const RtcTexture* t) {
         s->textures.push_back(std::move(x));
     }
     s->committed = false;
+    s->shard_ppm = {};
     return 0;
 }
 int rtc_set_point_light(RtcScene* s, const float position[3], const float intensity[3]) {
@@ -1344,6 +1472,7 @@ int rtc_set_point_light(RtcScene* s, const float position[3], const float intens
     s->jitter.clear();
     s->have_light = true;
     s->committed = false;
+    s->shard_ppm = {};
     return 0;
 }
 int rtc_set_rect_light(RtcScene* s, const float intensity[3], const float corner[3], const float u_cell[3], int32_t u_steps,
@@ -1370,10 +1499,12 @@ int rtc_set_rect_light(RtcScene* s, const float intensity[3], const float corner
     s->seed = seed;
     s->have_light = true;
     s->committed = false;
+    s->shard_ppm = {};
     return 0;
 }
 int rtc_set_option(RtcScene* s, int32_t option, int64_t value) {
     if (!s) return fail(RTC_ERR_INVALID, "null scene");
+    s->shard_ppm = {};
     switch (option) {
         case RTC_OPT_FMA_CONTRACTION: s->strict_fp = value == 0; return 0;  // may change between renders
         case RTC_OPT_BVH_LEAF_SIZE:
@@ -1455,6 +1586,7 @@ int rtc_scene_commit(RtcScene* s, int32_t n_devices, const int32_t* device_ids) 
     if (n_devices == 0) n_devices = visible;
     if (n_devices < 0 || n_devices > visible) return fail(RTC_ERR_INVALID, "bad device count");
     release(s);
+    s->shard_ppm = {};
     Flattened f;
     int rc;
     if (s->bvh_builder == 1) {  // the tree of a big scene is built on the first device of the commit
@@ -1520,6 +1652,13 @@ int rtc_render_ppm(RtcScene* s, int32_t depth, char* ppm, size_t capacity, size_
 int rtc_render_views_ppm(RtcScene* s, int32_t depth, uint32_t n_views, const RtcView* views, char* ppm, size_t capacity,
                          size_t* view_offsets, RtcStats* stats) {
     return render_views_ppm_impl(s, depth, n_views, views, ppm, capacity, view_offsets, stats);
+}
+int rtc_render_shard_ppm_rows(RtcScene* s, int32_t depth, int32_t shard, int32_t n_shards, uint64_t* row_bytes, RtcStats* stats) {
+    return render_shard_ppm_rows_impl(s, depth, shard, n_shards, row_bytes, stats);
+}
+int rtc_write_shard_ppm(RtcScene* s, int32_t shard, int32_t n_shards, const uint64_t* row_bytes, char* ppm, size_t capacity,
+                        size_t* ppm_bytes) {
+    return write_shard_ppm_impl(s, shard, n_shards, row_bytes, ppm, capacity, ppm_bytes);
 }
 
 int rtc_trace_rays(RtcScene* s, uint32_t n, const float* origins, const float* directions, int32_t depth, float* out_rgb,

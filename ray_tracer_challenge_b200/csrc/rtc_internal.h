@@ -195,6 +195,13 @@ struct RtcScene {
     // commit statistics
     int n_bvh_nodes = 0, n_linear = 0, n_xforms = 0;
     float reach = 0.f;  // Flattened::reach of the commit: rtc_render_views refuses camera origins beyond it in tree scenes
+    // rtc_render_shard_ppm_rows -> rtc_write_shard_ppm: the shard the last phase 1 encoded (n_shards 0: none) and the byte
+    // lengths it computed for the shard's rows in frame-row order.  Any render, rtc_set_* / rtc_map_* or commit clears it.
+    // (The slot's h_ppm_rows cannot serve: ppm_layout turns it into offsets in place.)
+    struct ShardPpm {
+        int shard = -1, n_shards = 0;
+        std::vector<unsigned long long> rows;
+    } shard_ppm;
 };
 
 namespace rtc {
@@ -264,6 +271,21 @@ inline void ppm_layout(uint32_t height, int n_dev, size_t header, unsigned long 
         }
     }
     L.total = at;
+}
+// rtc_write_shard_ppm's scan: ppm_layout of one frame cut into n_shards shards, from the byte lengths of all its rows in
+// frame-row order (row_bytes, every shard's rtc_render_shard_ppm_rows put together by the callers).  shard_rows[i] receives
+// shard i's rows in its band order — its frame rows in increasing order — and, after the scan, their offsets in shard i's
+// text.  Every process lays out the whole frame on its own; only shard 0 passes header_text and text, so the header is
+// written once.  Shared with the host harness (tests/emu/emu_ppm.cpp: emu_ppm_shards).
+inline void ppm_layout_frame_rows(uint32_t height, int n_shards, size_t header, const uint64_t* row_bytes,
+                                  std::vector<std::vector<unsigned long long>>& shard_rows, PpmLayout& L,
+                                  const char* header_text = nullptr, char* text = nullptr) {
+    shard_rows.assign(n_shards, {});
+    for (int i = 0; i < n_shards; i++) shard_rows[i].reserve(ppm_device_rows(height, i, n_shards));
+    for (uint32_t y = 0; y < height; y++) shard_rows[y / kBandRows % n_shards].push_back(row_bytes[y]);
+    std::vector<unsigned long long*> rows(n_shards);
+    for (int i = 0; i < n_shards; i++) rows[i] = shard_rows[i].data();
+    ppm_layout(height, n_shards, header, rows.data(), L, 1, header_text, text);
 }
 
 // A tree builder other than the host's binned SAH (rtc_lbvh.cu: the device LBVH).  In: the padded boxes of the bounded

@@ -219,6 +219,13 @@ extern "C" {
     /// is `ppm[view_offsets[v]..view_offsets[v + 1]]`; `capacity >= n_views * rtc_ppm_bound(w, h)`, `n_views + 1` offsets.
     pub fn rtc_render_views_ppm(scene: *mut RtcScene, depth: i32, n_views: u32, views: *const RtcView, ppm: *mut c_char,
                                 capacity: usize, view_offsets: *mut usize, stats: *mut RtcStats) -> c_int;
+    /// One shard's text of a frame shared by several processes, in two phases with the callers' exchange of `row_bytes`
+    /// (`height` entries, frame-row order) in between: phase 1 renders the shard and writes its rows' lengths, phase 2 writes
+    /// its bands' text at their offsets in `ppm` (shard 0 also the header); `*ppm_bytes` is the whole text's length.
+    pub fn rtc_render_shard_ppm_rows(scene: *mut RtcScene, depth: i32, shard: i32, n_shards: i32, row_bytes: *mut u64,
+                                     stats: *mut RtcStats) -> c_int;
+    pub fn rtc_write_shard_ppm(scene: *mut RtcScene, shard: i32, n_shards: i32, row_bytes: *const u64, ppm: *mut c_char,
+                               capacity: usize, ppm_bytes: *mut usize) -> c_int;
     pub fn rtc_trace_rays(scene: *mut RtcScene, n: u32, origins: *const f32, directions: *const f32, depth: i32,
                           out_rgb: *mut f32, out_t: *mut f32, out_prim: *mut i32) -> c_int;
     pub fn rtc_shard_bands(height: u32, shard: i32, n_shards: i32, first_rows: *mut u32) -> c_int;
