@@ -304,6 +304,29 @@ typedef struct RtcView {
  *     rtc_set_camera keeps its meaning (it invalidates the commit). */
 int rtc_render_views(RtcScene*, int32_t depth, uint32_t n_views, const RtcView* views, float* rgb_f32, uint8_t* rgb_u8,
                      RtcStats* stats);
+/* Anti-aliased Camera::render: n x n samples per pixel (n = samples_per_axis), box-filtered.  The samples of the committed
+ * W x H canvas are pixels the reference itself renders: those of Camera::render at n W x n H with the same field of view
+ * and transform (the sample camera C_n: Camera::new(n W, n H, fov, transform), camera.rs:23-56 — the committed half_width,
+ * half_height and transform_inverse, pixel_size = (half_width * 2) / (float)(n W); C_1 is the committed camera).
+ * rgb_f32 / rgb_u8: width * height * 3 each, as rtc_render's; either may be NULL (NULL, NULL = leave the frame on the device).
+ *   - Pixel (x, y), x < width - 1 and y < height - 1: sample (i, j), i, j in [0, n), is color_at of C_n's ray for pixel
+ *     (n x + i, n y + j); with generated jitter its generator key is that pixel's in the n W x n H frame,
+ *     (n y + j) * (n W) + (n x + i).  Per channel in f32: s = sample (0, 0), then s = s + sample (i, j) with j the outer
+ *     and i the inner loop, then s / (float)(n * n).  The 8-bit value is Canvas::scale_color of that mean.  The last row and
+ *     column are zero in both planes (camera.rs:80-81).
+ *   - So n = 1 gives rtc_render's planes bit for bit, and n >= 2 the box filter of rtc_render's frame of the scene
+ *     committed with C_n (whose own last row and column are never used), for every kernel build and option.  The samples
+ *     are reduced on the device: the n W x n H frame is never stored.
+ *   - The arguments are checked before the scene's state, all with RTC_ERR_INVALID: a NULL scene; n outside [1, 16]; a
+ *     sample canvas rtc_set_camera would refuse ((n W) * (n H) > 2^31 / 3); a depth outside [0, 23].  Then an uncommitted
+ *     scene is RTC_ERR_STATE.
+ *   - Destinations and devices as rtc_render_views' for one view: pinned or pageable host memory, each committed device
+ *     rendering its interleaved bands of output rows (rtc_shard_bands' rule).  A tree scene whose ray trees branch renders
+ *     with one persistent streaming launch, whatever RTC_OPT_WAVEFRONT says.
+ *   - stats: primary_rays = n * n * (width - 1) * (height - 1) over the devices' shares, launches = the launches made,
+ *     kernel_ms covers the render kernels.  There is no detailed variant.
+ *   - Nothing of rtc_render's state changes: the committed camera, its frame on the device and its learnt tile order. */
+int rtc_render_samples(RtcScene*, int32_t depth, uint32_t samples_per_axis, float* rgb_f32, uint8_t* rgb_u8, RtcStats* stats);
 /* Camera::render followed by Canvas::to_ppm (canvas.rs:58-96), the last step of every demo, with the text written on the
  * device.  rtc_ppm_bound is host arithmetic: the header's length plus width * height * 3 * 4 bytes (three digits and a
  * separator per value), an upper bound on the text of any frame of that size.

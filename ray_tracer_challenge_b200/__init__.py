@@ -106,6 +106,7 @@ _HOST_EXTRAS = {
     "sg_trace_rays": (_I, [_V, _I, C.c_uint32, _FP, _FP, _I, _I, _FP, _FP, _IP]),
     "sg_flatten": (_I, [_V, _I, _IP, C.POINTER(RtcPrim), C.POINTER(RtcNode), C.POINTER(C.c_int32), _IP]),
     "sg_render_prepared_views": (_I, [_V, _I, _I, _I, _IP, _I, _FP, _U8P, C.POINTER(SgStats)]),
+    "sg_render_prepared_samples": (_I, [_V, _I, _I, _I, _I, _FP, _U8P, C.POINTER(SgStats)]),
     "sg_camera_render_views": (_I, [_V, _IP, _I, _I, _I, _FP, _U8P, C.POINTER(SgStats)]),
     "sg_camera_view": (_I, [_V, _I, C.POINTER(RtcView)]),
     "sg_farthest_camera": (_I, [_V, _IP, _I]),
@@ -210,6 +211,22 @@ class PreparedScene:
             u8.ctypes.data_as(_U8P) if u8 is not None else None, C.byref(stats)))
         self.last_stats = api.last_rtc_stats()
         return _canvases(api, n, h, w, rgb, u8)
+
+    def render_samples(self, samples, depth=DEFAULT_RAY_RECURSION_DEPTH, want_rgb=True, want_u8=True, out_rgb=None, out_u8=None,
+                       fma=False):
+        """rtc_render_samples: the committed scene anti-aliased with samples x samples samples per pixel, each sample a pixel
+        of the reference's render at samples times the canvas size, box-filtered on the device (samples = 1 is render()'s
+        frame).  Buffers may be caller-supplied (e.g. pinned); want_* = False leaves the frame on the device."""
+        w, h = self.camera.width_pixels, self.camera.height_pixels
+        rgb, u8 = _view_planes(1, h, w, want_rgb, want_u8, None if out_rgb is None else out_rgb[None],
+                               None if out_u8 is None else out_u8[None])
+        stats = SgStats()
+        api = self.api
+        api.check(api.lib.sg_render_prepared_samples(
+            api.ctx, self.handle, int(depth), int(samples), int(fma), _api.fptr(rgb) if rgb is not None else None,
+            u8.ctypes.data_as(_U8P) if u8 is not None else None, C.byref(stats)))
+        self.last_stats = api.last_rtc_stats()
+        return Canvas(w, h, rgb[0] if rgb is not None else None, u8[0] if u8 is not None else None, api=api)
 
     def render_ppm(self, depth=DEFAULT_RAY_RECURSION_DEPTH, out=None, fma=False) -> str:
         """rtc_render_ppm: the committed scene rendered and its frame's `Canvas::to_ppm` text (canvas.rs:58-96) written on the
@@ -351,7 +368,19 @@ class HostApi(_api.Api):
             camera.last_rtc_stats = api.last_rtc_stats()
             return buf[:n].tobytes().decode("ascii")
 
+        def render_b200_samples(camera, world, samples, reflection_recursion_depth=DEFAULT_RAY_RECURSION_DEPTH, want_u8=True):
+            """Camera::render_b200_samples — render_b200 anti-aliased with samples x samples samples per pixel
+            (rtc_render_samples): flatten, commit, render, release."""
+            prepared = PreparedScene(api, camera, world)
+            try:
+                canvas = prepared.render_samples(samples, reflection_recursion_depth, want_u8=want_u8)
+            finally:
+                prepared.release()
+            camera.last_rtc_stats = prepared.last_stats
+            return canvas
+
         self.Camera.render_b200 = render_b200
+        self.Camera.render_b200_samples = render_b200_samples
         self.Camera.render_b200_u8 = render_b200_u8
         self.Camera.render_b200_ppm = render_b200_ppm
         self.Camera.render = render_b200

@@ -650,6 +650,17 @@ int sg_render_prepared_views(sg_ctx* c, int h, int depth, int n, const int* cams
     to_sg_stats(c->last_stats, stats);
     return rc ? fail(rtc_last_error()) : 0;
 }
+// rtc_render_samples on a prepared scene: n x n samples per pixel of its canvas, frames as sg_render_prepared's
+int sg_render_prepared_samples(sg_ctx* c, int h, int depth, int samples_per_axis, int fma, float* out_rgb, uint8_t* out_u8,
+                               sg_stats* stats) {
+    if (h < 0 || h >= (int)c->prepared.size() || !c->prepared[h]) return fail("bad prepared handle");
+    if (samples_per_axis < 0) return fail("negative samples_per_axis");
+    RtcScene* scene = c->prepared[h]->scene;
+    if (rtc_set_option(scene, RTC_OPT_FMA_CONTRACTION, fma ? 1 : 0)) return fail(rtc_last_error());
+    const int rc = rtc_render_samples(scene, depth, (uint32_t)samples_per_axis, out_rgb, out_u8, &c->last_stats);
+    to_sg_stats(c->last_stats, stats);
+    return rc ? fail(rtc_last_error()) : 0;
+}
 // rtc_render_views_ppm on a prepared scene: n cameras (handles) of its canvas size, their texts one after the other in out,
 // view i's at offsets[i] (n + 1 offsets).  Returns the total length, or -1.
 int64_t sg_render_prepared_views_ppm(sg_ctx* c, int h, int depth, int n, const int* cams, int fma, char* out, int64_t capacity,

@@ -186,13 +186,15 @@ struct KernelBuild {
     decltype(&fast::launch_trace) trace;
     decltype(&fast::launch_wave) wave;
     decltype(&fast::launch_views) views;
+    decltype(&fast::launch_samples) samples;
 };
 const KernelBuild& kernel_build(bool strict_fp, bool csg_sweep) {
-    static const KernelBuild builds[4] = {{fast::launch_render, fast::launch_trace, fast::launch_wave, fast::launch_views},
-                                          {strict::launch_render, strict::launch_trace, strict::launch_wave, strict::launch_views},
-                                          {fast_sweep::launch_render, fast_sweep::launch_trace, fast_sweep::launch_wave, fast_sweep::launch_views},
-                                          {strict_sweep::launch_render, strict_sweep::launch_trace, strict_sweep::launch_wave,
-                                           strict_sweep::launch_views}};
+    static const KernelBuild builds[4] = {
+        {fast::launch_render, fast::launch_trace, fast::launch_wave, fast::launch_views, fast::launch_samples},
+        {strict::launch_render, strict::launch_trace, strict::launch_wave, strict::launch_views, strict::launch_samples},
+        {fast_sweep::launch_render, fast_sweep::launch_trace, fast_sweep::launch_wave, fast_sweep::launch_views, fast_sweep::launch_samples},
+        {strict_sweep::launch_render, strict_sweep::launch_trace, strict_sweep::launch_wave, strict_sweep::launch_views,
+         strict_sweep::launch_samples}};
     return builds[(strict_fp ? 1 : 0) + (csg_sweep ? 2 : 0)];
 }
 
@@ -818,9 +820,11 @@ struct ViewsText {
     size_t* view_offsets;
 };
 
-// rtc_render_views (text == nullptr) and rtc_render_views_ppm, from the scene's state on: the arguments are checked
+// rtc_render_views (text == nullptr), rtc_render_views_ppm and rtc_render_samples (samples > 0: n_views == 1, views[0] the
+// sample camera, and the samples kernels with that many samples per axis), from the scene's state on: the arguments are
+// checked
 int render_views_body(RtcScene* s, int depth, uint32_t n_views, const RtcView* views, float* rgb, uint8_t* u8, RtcStats* stats,
-                      const ViewsText* text, const char* fn) {
+                      const ViewsText* text, const char* fn, int samples = 0) {
     if (!s->committed) return fail(RTC_ERR_STATE, std::string(fn) + " before rtc_scene_commit");
     // The tree's boxes are padded for ray origins up to the commit's reach (rtc_commit.cu: "pad"): a camera farther out
     // could lose hits the reference reports.  Small and tree-less scenes test every item exactly: any view goes.
@@ -955,7 +959,11 @@ int render_views_body(RtcScene* s, int depth, uint32_t n_views, const RtcView* v
                     F.stream_counter = slot->d_stream_counter, F.stream_blocks = stream_blocks(slot->sm_count);
                     CUDA_TRY(cudaMemsetAsync(slot->d_stream_counter, 0, sizeof(unsigned), lane));
                 }
-                kernel_build(s->strict_fp, r.csg_sweep).views(r.scene, r.small, F, slot->d_views + L.v0, (int)(L.v1 - L.v0), slot->d_counters, lane);
+                if (samples)
+                    kernel_build(s->strict_fp, r.csg_sweep).samples(r.scene, r.small, F, slot->h_views[0], samples, slot->d_counters, lane);
+                else
+                    kernel_build(s->strict_fp, r.csg_sweep).views(r.scene, r.small, F, slot->d_views + L.v0, (int)(L.v1 - L.v0),
+                                                                  slot->d_counters, lane);
                 CUDA_TRY(cudaGetLastError());
                 st.launches++;
                 const int idx = launches_on[i];
@@ -1025,7 +1033,8 @@ int render_views_body(RtcScene* s, int depth, uint32_t n_views, const RtcView* v
         uint64_t rows = 0;  // camera.rs:80-81, per view, of this device's bands
         for (int b = i; b < total_bands; b += n_shards)
             rows += (uint64_t)std::max(0, std::min<int>((int)s->height - 1, (b + 1) * kBandRows) - b * kBandRows);
-        add_counters(st, *slot->h_counters, (uint64_t)n_views * rows * (uint64_t)(s->width - 1),
+        const uint64_t per_pixel = samples ? (uint64_t)samples * samples : 1;  // primary rays of one output pixel
+        add_counters(st, *slot->h_counters, per_pixel * n_views * rows * (uint64_t)(s->width - 1),
                      s->light_is_rect ? (uint64_t)s->u_steps * s->v_steps : 1);
     }
     if (text) text->view_offsets[n_views] = text_at;
@@ -1042,6 +1051,22 @@ int render_views_impl(RtcScene* s, int depth, uint32_t n_views, const RtcView* v
     if (int rc = check_views(n_views, views, "rtc_render_views")) return rc;
     if (int rc = check_depth(depth)) return rc;
     return render_views_body(s, depth, n_views, views, rgb, u8, stats, nullptr, "rtc_render_views");
+}
+
+// rtc_render_samples ------------------------------------------------------------------------------------------------------
+constexpr uint32_t kMaxSamplesPerAxis = 16;
+
+int render_samples_impl(RtcScene* s, int depth, uint32_t n, float* rgb, uint8_t* u8, RtcStats* stats) {
+    // the arguments first (no device needed), then the scene's state
+    if (!s) return fail(RTC_ERR_INVALID, "null scene");
+    if (n < 1 || n > kMaxSamplesPerAxis)
+        return fail(RTC_ERR_INVALID, "rtc_render_samples: samples_per_axis must be in [1, " + std::to_string(kMaxSamplesPerAxis) + "]");
+    if ((uint64_t)n * s->width * ((uint64_t)n * s->height) > (1ull << 31) / 3)
+        return fail(RTC_ERR_INVALID, "rtc_render_samples: the sample canvas (samples_per_axis * width) x (samples_per_axis * height) is "
+                                     "bigger than rtc_set_camera allows");
+    if (int rc = check_depth(depth)) return rc;
+    const RtcView c = sample_camera(s, n);  // the committed camera's origin: within the commit's reach
+    return render_views_body(s, depth, 1, &c, rgb, u8, stats, nullptr, "rtc_render_samples", (int)n);
 }
 
 // rtc_render_ppm ---------------------------------------------------------------------------------------------------------
@@ -1642,6 +1667,9 @@ int rtc_render_detailed(RtcScene* s, int32_t depth, float* rgb, uint8_t* u8, Rtc
 }
 int rtc_render_views(RtcScene* s, int32_t depth, uint32_t n_views, const RtcView* views, float* rgb, uint8_t* u8, RtcStats* stats) {
     return render_views_impl(s, depth, n_views, views, rgb, u8, stats);
+}
+int rtc_render_samples(RtcScene* s, int32_t depth, uint32_t samples_per_axis, float* rgb, uint8_t* u8, RtcStats* stats) {
+    return render_samples_impl(s, depth, samples_per_axis, rgb, u8, stats);
 }
 size_t rtc_ppm_bound(uint32_t width, uint32_t height) {
     return ppm_header(width, height).size() + (size_t)width * height * 3 * 4;

@@ -213,6 +213,16 @@ inline bool streams_pixels(const RtcScene* s, const SmallScene& small) {
 }
 // DevFrame::converge: the warp vote before every ray when the ray trees branch, unless RTC_CONVERGE forces it
 inline int frame_converge(const RtcScene* s) { return s->converge < 0 ? (int)s->has_branching_materials : s->converge; }
+// The sample camera C_n of rtc_render_samples, shared with the host harness of the kernels: Camera::new(n W, n H, fov,
+// transform) (camera.rs:23-56).  n W / n H is the same real number as W / H, so the aspect and the half-sizes are the
+// committed ones; only pixel_size is derived again.  C_1 is the committed camera.
+inline RtcView sample_camera(const RtcScene* s, uint32_t n) {
+    RtcView c;
+    c.half_width = s->half_w, c.half_height = s->half_h;
+    c.pixel_size = n == 1 ? s->pixel_size : (s->half_w * 2.0f) / (float)(n * s->width);
+    memcpy(c.transform_inverse, s->cam_inv, sizeof(c.transform_inverse));
+    return c;
+}
 // DevFrame::stream_blocks: render_stream's persistent grid, the resident blocks of its launch bounds (RTC_STREAM_MINBLOCKS)
 inline int stream_blocks(int sm_count) { return sm_count * 6; }
 

@@ -5,11 +5,12 @@
 #include "rtc_types.h"
 
 namespace rtc {
-// The kernel a launch function runs for its inputs.  launch_render, launch_views and launch_trace (rtc_kernels.cu) switch
-// on it, and so does the host harness of the kernels (tests/emu/emu_kernels.cpp), which thus runs the kernel the GPU runs.
+// The kernel a launch function runs for its inputs.  launch_render, launch_views, launch_samples and launch_trace
+// (rtc_kernels.cu) switch on it, and so does the host harness of the kernels (tests/emu/emu_kernels.cpp), which thus runs the kernel the GPU runs.
 struct KernelVariant {
-    bool stream;  // render_stream / render_stream_views: a tree scene whose lanes draw pixels from F.stream_counter
-    // otherwise the template flags of render_tiles / render_tiles_views / trace_rays
+    bool stream;  // render_stream / render_stream_views / render_stream_samples: a tree scene whose lanes draw pixels from
+                  // F.stream_counter
+    // otherwise the template flags of render_tiles / render_tiles_views / render_tiles_samples / trace_rays
     bool stats, small, converge, drawn, lean;
 };
 constexpr int variant_code(bool stats, bool small, bool converge, bool drawn, bool lean) {
@@ -46,6 +47,11 @@ void launch_render(const DevScene& S, const SmallScene& SS, const DevFrame& F, D
 // frame at F.rgb / F.u8 + v * width * height * 3; a tree scene with F.stream_counter set renders them as one pixel stream.
 void launch_views(const DevScene& S, const SmallScene& SS, const DevFrame& F, const DevView* views, int n_views, DevCounters* counters,
                   cudaStream_t stream);
+// n x n samples per pixel of the committed canvas (rtc_render_samples): the bands of F, each output pixel the box filter of
+// the pixels (n x + i, n y + j) of `camera`, the reference's Camera::new at n width x n height; a tree scene with
+// F.stream_counter set renders them as one pixel stream.
+void launch_samples(const DevScene& S, const SmallScene& SS, const DevFrame& F, const DevView& camera, int samples_per_axis,
+                    DevCounters* counters, cudaStream_t stream);
 void launch_trace(const DevScene& S, const SmallScene& SS, int n, const float* origins, const float* directions, int depth,
                   float* out_rgb, float* out_t, int* out_pos, DevCounters* counters, cudaStream_t stream);
 void launch_fma_peak(float* out, int blocks, int iters, cudaStream_t stream);
@@ -59,6 +65,8 @@ void launch_render(const DevScene& S, const SmallScene& SS, const DevFrame& F, D
                    cudaStream_t stream);
 void launch_views(const DevScene& S, const SmallScene& SS, const DevFrame& F, const DevView* views, int n_views, DevCounters* counters,
                   cudaStream_t stream);
+void launch_samples(const DevScene& S, const SmallScene& SS, const DevFrame& F, const DevView& camera, int samples_per_axis,
+                    DevCounters* counters, cudaStream_t stream);
 void launch_trace(const DevScene& S, const SmallScene& SS, int n, const float* origins, const float* directions, int depth,
                   float* out_rgb, float* out_t, int* out_pos, DevCounters* counters, cudaStream_t stream);
 void launch_wave(const DevScene& S, const SmallScene& SS, const DevFrame& F, const WavePoolRaw& pool, DevCounters* counters, int blocks,
@@ -70,6 +78,8 @@ void launch_render(const DevScene& S, const SmallScene& SS, const DevFrame& F, D
                    cudaStream_t stream);
 void launch_views(const DevScene& S, const SmallScene& SS, const DevFrame& F, const DevView* views, int n_views, DevCounters* counters,
                   cudaStream_t stream);
+void launch_samples(const DevScene& S, const SmallScene& SS, const DevFrame& F, const DevView& camera, int samples_per_axis,
+                    DevCounters* counters, cudaStream_t stream);
 void launch_trace(const DevScene& S, const SmallScene& SS, int n, const float* origins, const float* directions, int depth,
                   float* out_rgb, float* out_t, int* out_pos, DevCounters* counters, cudaStream_t stream);
 void launch_wave(const DevScene& S, const SmallScene& SS, const DevFrame& F, const WavePoolRaw& pool, DevCounters* counters, int blocks,
@@ -80,6 +90,8 @@ void launch_render(const DevScene& S, const SmallScene& SS, const DevFrame& F, D
                    cudaStream_t stream);
 void launch_views(const DevScene& S, const SmallScene& SS, const DevFrame& F, const DevView* views, int n_views, DevCounters* counters,
                   cudaStream_t stream);
+void launch_samples(const DevScene& S, const SmallScene& SS, const DevFrame& F, const DevView& camera, int samples_per_axis,
+                    DevCounters* counters, cudaStream_t stream);
 void launch_trace(const DevScene& S, const SmallScene& SS, int n, const float* origins, const float* directions, int depth,
                   float* out_rgb, float* out_t, int* out_pos, DevCounters* counters, cudaStream_t stream);
 void launch_wave(const DevScene& S, const SmallScene& SS, const DevFrame& F, const WavePoolRaw& pool, DevCounters* counters, int blocks,

@@ -542,6 +542,29 @@ impl Camera {
         canvas
     }
 
+    /// `render_b200` anti-aliased: each pixel is the mean of `samples_per_axis`² samples, the pixels of the reference's
+    /// `Camera::new(n * hsize, n * vsize, fov, transform).render(world, depth)` (n = samples_per_axis) that fall in it,
+    /// summed row by row in f32.  The samples are reduced on the device (`rtc_render_samples`); 1 is `render_b200`.
+    pub fn render_b200_samples(&self, world: World, reflection_recursion_depth: i16, samples_per_axis: u32) -> Canvas {
+        let (w, h) = (self.width_pixels as usize, self.height_pixels as usize);
+        let mut rgb = vec![0f32; w * h * 3];
+        unsafe {
+            let scene = self.commit_b200(&world);
+            let mut stats: sys::RtcStats = std::mem::zeroed();
+            check(sys::rtc_render_samples(scene, reflection_recursion_depth as i32, samples_per_axis, rgb.as_mut_ptr(),
+                                          std::ptr::null_mut(), &mut stats));
+            sys::rtc_scene_destroy(scene);
+        }
+        let mut canvas = Canvas::new(w, h);
+        for y in 0..h {
+            for x in 0..w {
+                let i = (y * w + x) * 3;
+                canvas.write_pixel(x, y, Color::new(rgb[i], rgb[i + 1], rgb[i + 2]));
+            }
+        }
+        canvas
+    }
+
     /// The demos' flow — `camera.render(world, depth).to_ppm()` (e.g. demos/src/bin/soft_shadows.rs:84-87) — without
     /// the f32 plane ever leaving the device: `camera.render_b200_u8(world, depth).to_ppm()`.
     pub fn render_b200_u8(&self, world: World, reflection_recursion_depth: i16) -> CanvasU8 {

@@ -211,6 +211,10 @@ extern "C" {
     pub fn rtc_render_detailed(scene: *mut RtcScene, depth: i32, rgb_f32: *mut f32, rgb_u8: *mut u8, stats: *mut RtcStats) -> c_int;
     pub fn rtc_render_views(scene: *mut RtcScene, depth: i32, n_views: u32, views: *const RtcView, rgb_f32: *mut f32, rgb_u8: *mut u8,
                             stats: *mut RtcStats) -> c_int;
+    /// `Camera::render` anti-aliased: `samples_per_axis`² samples per pixel, the pixels of the reference's render at
+    /// `samples_per_axis` times the canvas size, box-filtered on the device; 1 gives `rtc_render`'s planes.
+    pub fn rtc_render_samples(scene: *mut RtcScene, depth: i32, samples_per_axis: u32, rgb_f32: *mut f32, rgb_u8: *mut u8,
+                              stats: *mut RtcStats) -> c_int;
     /// `Canvas::to_ppm` of the rendered frame, its text written on the device; `capacity >= rtc_ppm_bound(w, h)`.
     pub fn rtc_ppm_bound(width: u32, height: u32) -> usize;
     pub fn rtc_render_ppm(scene: *mut RtcScene, depth: i32, ppm: *mut c_char, capacity: usize, ppm_bytes: *mut usize,
