@@ -404,6 +404,31 @@ int rtc_write_shard_ppm(RtcScene*, int32_t shard, int32_t n_shards, const uint64
  *     largest chunk and 16 bytes per row of a chunk (its row lengths, on the device and pinned on the host). */
 int rtc_render_views_ppm(RtcScene*, int32_t depth, uint32_t n_views, const RtcView* views, char* ppm, size_t capacity,
                          size_t* view_offsets, RtcStats* stats);
+/* Anti-aliased batches: rtc_render_samples for every view of an rtc_render_views batch, as frames or as PPM text.
+ *   - Pixels: view v's planes (f32 and 8-bit) are bit for bit what rtc_render_samples(n) returns for the scene committed with
+ *     view v's camera, for every kernel build and option.  View v's sample camera has the view's half_width, half_height and
+ *     transform_inverse, and pixel_size = the view's own when n = 1, else (half_width * 2) / (float)(n W).  A sample's
+ *     generated-jitter key is its index in that view's own n W x n H frame; the f32 sum order and the zero last row and column
+ *     are rtc_render_samples'.  So n = 1 gives rtc_render_views' planes bit for bit.  rgb_f32 / rgb_u8 are view-major as in
+ *     rtc_render_views; NULL, NULL leaves the frames on the device.
+ *   - Text: rtc_render_views_samples_ppm lays out its texts and view_offsets as rtc_render_views_ppm does; view v's text is
+ *     byte for byte Canvas::to_ppm of view v's 8-bit plane above.
+ *   - The arguments are checked before the scene's state, in this order, all with RTC_ERR_INVALID: a NULL scene; every check
+ *     rtc_render_views makes on n_views and views; samples_per_axis outside [1, 16]; a sample canvas rtc_set_camera would
+ *     refuse (rtc_render_samples' rule); a depth outside [0, 23]; for the text call, ppm or view_offsets NULL, or a capacity
+ *     below n_views * rtc_ppm_bound of the committed canvas (a product that overflows size_t too).  Then an uncommitted scene
+ *     is RTC_ERR_STATE, and a view beyond the committed reach of a tree scene is refused as rtc_render_views refuses it.
+ *   - Chunks, slices, staging, devices and destinations are rtc_render_views' and rtc_render_views_ppm's (RTC_VIEW_ARENA_BYTES,
+ *     the 256 MiB cap on a pageable destination's staged text).  A tree scene whose ray trees branch renders each chunk with
+ *     one persistent streaming launch, whatever RTC_OPT_WAVEFRONT says.  The samples are reduced on the device: no view's
+ *     n W x n H frame is stored.
+ *   - stats: primary_rays = n * n * n_views * (width - 1) * (height - 1) over the devices' shares; the other fields are the
+ *     views calls' (the text call's total_ms covers the whole call).
+ *   - Nothing of rtc_render's state changes: the committed camera, its frame on the device and its learnt tile order. */
+int rtc_render_views_samples(RtcScene*, int32_t depth, uint32_t n_views, const RtcView* views, uint32_t samples_per_axis,
+                             float* rgb_f32, uint8_t* rgb_u8, RtcStats* stats);
+int rtc_render_views_samples_ppm(RtcScene*, int32_t depth, uint32_t n_views, const RtcView* views, uint32_t samples_per_axis,
+                                 char* ppm, size_t capacity, size_t* view_offsets, RtcStats* stats);
 /* World::color_at (world.rs:88-101) for caller-supplied rays: origins / directions are n*3 f32; out_rgb n*3;
  * out_t (optional) the hit distance or -1; out_prim (optional) the hit primitive index or -1. */
 int rtc_trace_rays(RtcScene*, uint32_t n, const float* origins, const float* directions, int32_t depth,

@@ -118,6 +118,12 @@ _HOST_EXTRAS = {
                                                  C.POINTER(SgStats)]),
     "sg_camera_render_views_ppm": (C.c_int64, [_V, _IP, _I, _I, _I, C.c_void_p, C.c_int64, C.POINTER(C.c_size_t),
                                                C.POINTER(SgStats)]),
+    "sg_render_prepared_views_samples": (_I, [_V, _I, _I, _I, _IP, _I, _I, _FP, _U8P, C.POINTER(SgStats)]),
+    "sg_render_prepared_views_samples_ppm": (C.c_int64, [_V, _I, _I, _I, _IP, _I, _I, C.c_void_p, C.c_int64, C.POINTER(C.c_size_t),
+                                                         C.POINTER(SgStats)]),
+    "sg_camera_render_views_samples": (_I, [_V, _IP, _I, _I, _I, _I, _FP, _U8P, C.POINTER(SgStats)]),
+    "sg_camera_render_views_samples_ppm": (C.c_int64, [_V, _IP, _I, _I, _I, _I, C.c_void_p, C.c_int64, C.POINTER(C.c_size_t),
+                                                       C.POINTER(SgStats)]),
     "rtc_ppm_bound": (C.c_size_t, [C.c_uint32, C.c_uint32]),  # librtc_b200.so, reached through the host library
 }
 
@@ -227,6 +233,41 @@ class PreparedScene:
             u8.ctypes.data_as(_U8P) if u8 is not None else None, C.byref(stats)))
         self.last_stats = api.last_rtc_stats()
         return Canvas(w, h, rgb[0] if rgb is not None else None, u8[0] if u8 is not None else None, api=api)
+
+    def render_views_samples(self, cameras, samples, depth=DEFAULT_RAY_RECURSION_DEPTH, want_rgb=True, want_u8=True, out_rgb=None,
+                             out_u8=None, fma=False):
+        """rtc_render_views_samples: render_views' batch anti-aliased as render_samples does it — view i is
+        render_samples(samples) of this scene committed with cameras[i].  Returns one Canvas per camera, views into one
+        (n, h, w, 3) array per plane; want_* = False leaves the frames on the device.  The reach rule is render_views'."""
+        cameras = list(cameras)
+        n, w, h = len(cameras), self.camera.width_pixels, self.camera.height_pixels
+        rgb, u8 = _view_planes(n, h, w, want_rgb, want_u8, out_rgb, out_u8)
+        stats = SgStats()
+        api = self.api
+        api.check(api.lib.sg_render_prepared_views_samples(
+            api.ctx, self.handle, int(depth), n, _handles(cameras), int(samples), int(fma),
+            _api.fptr(rgb) if rgb is not None else None, u8.ctypes.data_as(_U8P) if u8 is not None else None, C.byref(stats)))
+        self.last_stats = api.last_rtc_stats()
+        return _canvases(api, n, h, w, rgb, u8)
+
+    def render_views_samples_ppm(self, cameras, samples, depth=DEFAULT_RAY_RECURSION_DEPTH, out=None, fma=False) -> list:
+        """rtc_render_views_samples_ppm: render_views_samples' batch with each view's `Canvas::to_ppm` text written on the
+        device.  Returns one str per camera; `out` as render_views_ppm's."""
+        cameras = list(cameras)
+        n, w, h = len(cameras), self.camera.width_pixels, self.camera.height_pixels
+        api = self.api
+        buf = _ppm_buffer(api, w, h, out, max(n, 1))
+        offsets = (C.c_size_t * (n + 1))()
+        stats = SgStats()
+        api.check(api.lib.sg_render_prepared_views_samples_ppm(api.ctx, self.handle, int(depth), n, _handles(cameras), int(samples),
+                                                               int(fma), buf.ctypes.data, buf.nbytes, offsets, C.byref(stats)))
+        self.last_stats = api.last_rtc_stats()
+        return _ppm_texts(buf, list(offsets))
+
+    def render_samples_ppm(self, samples, depth=DEFAULT_RAY_RECURSION_DEPTH, out=None, fma=False) -> str:
+        """`render_samples(samples).to_ppm()` with the text written on the device: the committed camera rendered as a one-view
+        rtc_render_views_samples_ppm batch.  `out` as render_ppm's."""
+        return self.render_views_samples_ppm([self.camera], samples, depth, out, fma)[0]
 
     def render_ppm(self, depth=DEFAULT_RAY_RECURSION_DEPTH, out=None, fma=False) -> str:
         """rtc_render_ppm: the committed scene rendered and its frame's `Canvas::to_ppm` text (canvas.rs:58-96) written on the
@@ -379,8 +420,21 @@ class HostApi(_api.Api):
             camera.last_rtc_stats = prepared.last_stats
             return canvas
 
+        def render_b200_samples_ppm(camera, world, samples, reflection_recursion_depth=DEFAULT_RAY_RECURSION_DEPTH, out=None) -> str:
+            """The anti-aliased demo flow, `camera.render_b200_samples(world, samples).to_ppm()`, in one call: flatten,
+            commit, render with samples x samples samples per pixel and write the PPM text on the device
+            (rtc_render_views_samples_ppm of one view), release.  `out` as PreparedScene.render_ppm's."""
+            prepared = PreparedScene(api, camera, world)
+            try:
+                text = prepared.render_samples_ppm(samples, reflection_recursion_depth, out)
+            finally:
+                prepared.release()
+            camera.last_rtc_stats = prepared.last_stats
+            return text
+
         self.Camera.render_b200 = render_b200
         self.Camera.render_b200_samples = render_b200_samples
+        self.Camera.render_b200_samples_ppm = render_b200_samples_ppm
         self.Camera.render_b200_u8 = render_b200_u8
         self.Camera.render_b200_ppm = render_b200_ppm
         self.Camera.render = render_b200
@@ -434,6 +488,37 @@ class HostApi(_api.Api):
         stats = SgStats()
         self.check(self.lib.sg_camera_render_views_ppm(self.ctx, _handles(cameras), n, world.handle, int(depth), buf.ctypes.data,
                                                        buf.nbytes, offsets, C.byref(stats)))
+        self.last_views_stats = self.last_rtc_stats()
+        return _ppm_texts(buf, list(offsets))
+
+    def render_views_samples(self, world, cameras, samples, depth=DEFAULT_RAY_RECURSION_DEPTH, want_u8=True):
+        """The one-shot anti-aliased batch: render_views' flatten and commit, then rtc_render_views_samples.  Canvas i is
+        `cameras[i].render_b200_samples(world, samples, depth)`."""
+        cameras = list(cameras)
+        if not cameras:
+            raise ValueError("render_views_samples needs at least one camera")
+        n, w, h = len(cameras), cameras[0].width_pixels, cameras[0].height_pixels
+        rgb, u8 = _view_planes(n, h, w, True, want_u8, None, None)
+        stats = SgStats()
+        self.check(self.lib.sg_camera_render_views_samples(self.ctx, _handles(cameras), n, world.handle, int(depth), int(samples),
+                                                           _api.fptr(rgb), u8.ctypes.data_as(_U8P) if u8 is not None else None,
+                                                           C.byref(stats)))
+        self.last_views_stats = self.last_rtc_stats()
+        return _canvases(self, n, h, w, rgb, u8)
+
+    def render_views_samples_ppm(self, world, cameras, samples, depth=DEFAULT_RAY_RECURSION_DEPTH, out=None) -> list:
+        """The one-shot anti-aliased batch in text: render_views' flatten and commit, then rtc_render_views_samples_ppm.
+        Returns `cameras[i].render_b200_samples(world, samples, depth).to_ppm()` for each camera; `out` as
+        PreparedScene.render_views_ppm's."""
+        cameras = list(cameras)
+        if not cameras:
+            raise ValueError("render_views_samples_ppm needs at least one camera")
+        n, w, h = len(cameras), cameras[0].width_pixels, cameras[0].height_pixels
+        buf = _ppm_buffer(self, w, h, out, n)
+        offsets = (C.c_size_t * (n + 1))()
+        stats = SgStats()
+        self.check(self.lib.sg_camera_render_views_samples_ppm(self.ctx, _handles(cameras), n, world.handle, int(depth), int(samples),
+                                                               buf.ctypes.data, buf.nbytes, offsets, C.byref(stats)))
         self.last_views_stats = self.last_rtc_stats()
         return _ppm_texts(buf, list(offsets))
 

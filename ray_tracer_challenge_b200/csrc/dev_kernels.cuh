@@ -395,6 +395,150 @@ __global__ void __launch_bounds__(kBlockThreads, min_blocks(RTC_STREAM_MINBLOCKS
     flush_counters<false>(r, k, counters);
 }
 
+// K1e render_tiles_views_samples: rtc_render_views_samples, render_tiles_samples for a batch of views.  blockIdx.z is a
+// view of the launch: the block reads its sample camera from the view table (one warp-uniform load per sample) and writes
+// view z's frame, which follows view z - 1's.  A sample's jitter key is its index in its own view's n W x n H frame.  The
+// body restates render_tiles_samples' rather than sharing it, for the reason render_tiles_views gives: a shared inlined
+// body lets ptxas allocate the existing kernels differently.
+template <bool SMALL, bool CONVERGE, bool DRAWN, bool LEAN>
+__global__ void __launch_bounds__(kBlockThreads, samples_min_blocks(SMALL, CONVERGE, LEAN))
+    render_tiles_views_samples(const __grid_constant__ DevScene S, const __grid_constant__ SmallScene SS, const DevFrame F,
+                               DevCounters* counters, const DevView* views, int n) {
+    if (SMALL) stage_small_scene(S, SS);
+    const Env E{S, SS};
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int band = F.shard + (F.band_begin + (int)blockIdx.y) * F.n_shards, bx = blockIdx.x;
+    const int x = bx * kTileW + (warp % kWarpsX) * 8 + (lane & 7);
+    const int y = band * kBandRows + (warp / kWarpsX) * 4 + (lane >> 3);
+    const DevView* C = views + blockIdx.z;  // warp-uniform
+    Ctr<false> k;
+    Rays r;
+    const bool rendered = x < S.width - 1 && y < S.height - 1;  // camera.rs:80-81
+    const unsigned big_w = (unsigned)n * (unsigned)S.width;      // the sample frame's width: the jitter key's row stride
+    V3 sum = mk(0.f, 0.f, 0.f);
+    for (int s = 0; s < n * n; s++) {  // warp-uniform trip count: the converging build votes in every color_at
+        const int j = s / n, i = s - j * n;
+        const int sx = n * x + i, sy = n * y + j;
+        V3 o = mk(0.f, 0.f, 0.f), d = mk(0.f, 0.f, 1.f);
+        if (rendered) ray_for_pixel(*C, sx, sy, o, d);
+        V3 c = mk(0.f, 0.f, 0.f);
+        if (CONVERGE || rendered)
+            c = color_at<false, SMALL, CONVERGE, DRAWN, LEAN>(E, rendered, o, d, F.depth, (unsigned)sy * big_w + (unsigned)sx, r, k,
+                                                             nullptr, nullptr);
+        sum = s == 0 ? c : sum + c;
+    }
+    const V3 c = rendered ? sample_mean(sum, n) : mk(0.f, 0.f, 0.f);
+    // Canvas::write_pixel + scale_color as in render_tiles: warp-transposed streaming stores where the rows allow them
+    const size_t view0 = (size_t)blockIdx.z * ((size_t)S.width * S.height * 3);
+    __shared__ __align__(16) float s_rgb[kBlockThreads * 3];
+    __shared__ __align__(16) unsigned char s_u8[kBlockThreads * 3];
+    const int wx0 = bx * kTileW + (warp % kWarpsX) * 8, wy0 = band * kBandRows + (warp / kWarpsX) * 4;  // warp-uniform
+    if ((S.width & 7) == 0 && wx0 + 8 <= S.width && wy0 + 4 <= S.height) {
+        float* w_rgb = s_rgb + warp * 96;
+        unsigned char* w_u8 = s_u8 + warp * 96;
+        w_rgb[lane * 3] = c.x, w_rgb[lane * 3 + 1] = c.y, w_rgb[lane * 3 + 2] = c.z;
+        w_u8[lane * 3] = scale_color(c.x), w_u8[lane * 3 + 1] = scale_color(c.y), w_u8[lane * 3 + 2] = scale_color(c.z);
+        __syncwarp();
+        const size_t px0 = (size_t)wy0 * S.width + wx0;
+        if (F.rgb && lane < 24) {
+            const int row = lane / 6, q = lane - row * 6;
+            __stcs(reinterpret_cast<float4*>(F.rgb + view0 + (px0 + (size_t)row * S.width) * 3) + q, reinterpret_cast<const float4*>(w_rgb)[lane]);
+        }
+        if (F.u8 && lane >= 20) {
+            const int u = lane - 20, row = u / 3, q = u - row * 3;
+            __stcs(reinterpret_cast<uint2*>(F.u8 + view0 + (px0 + (size_t)row * S.width) * 3) + q, reinterpret_cast<const uint2*>(w_u8)[u]);
+        }
+    } else if (x < S.width && y < S.height) {
+        const size_t idx = view0 + ((size_t)y * S.width + x) * 3;
+        if (F.rgb) F.rgb[idx] = c.x, F.rgb[idx + 1] = c.y, F.rgb[idx + 2] = c.z;
+        if (F.u8) F.u8[idx] = scale_color(c.x), F.u8[idx + 1] = scale_color(c.y), F.u8[idx + 2] = scale_color(c.z);
+    }
+    flush_counters<false>(r, k, counters);
+}
+
+// The pixel stream of rtc_render_views_samples: SamplePixelStream over views x bands x 8x4 blocks, the view outermost as in
+// ViewPixelStream.  A lane keeps its pixel's view (its sample camera and its frame's offset) until the pixel's last sample.
+struct ViewSamplePixelStream {
+    static constexpr bool kStream = true;
+    const DevScene& S;
+    const DevFrame& F;
+    unsigned* counter;      // next unclaimed stream index of this launch
+    unsigned total;         // stream indices of this launch
+    int blocks_x;           // 8-pixel blocks across the frame
+    const DevView* views;   // the launch's sample cameras
+    unsigned view_blocks;   // 8x4 blocks of one view in this launch
+    int n;                  // samples per axis
+    bool done = false;      // warp-uniform: the counter has run past the end
+    bool pending = false;   // the claimed pixel has samples left to trace
+    int x = 0, y = 0;       // the claimed pixel
+    int next = 0;           // its sample in flight (finish) or to start (refill)
+    const DevView* cam = nullptr;  // its view's sample camera
+    size_t out = 0;         // where its view starts in the frame planes (elements)
+    V3 sum = mk(0.f, 0.f, 0.f);
+    __device__ __forceinline__ bool exhausted() const { return done; }
+    __device__ __forceinline__ void start(V3& ro, V3& rd, unsigned& pixel) {
+        const int j = next / n, i = next - j * n;
+        const int sx = n * x + i, sy = n * y + j;
+        pixel = (unsigned)sy * ((unsigned)n * (unsigned)S.width) + (unsigned)sx;  // the view's sample frame's jitter key
+        ray_for_pixel(*cam, sx, sy, ro, rd);
+    }
+    __device__ __forceinline__ void store(int px, int py, V3 c) {  // Canvas::write_pixel + scale_color (canvas.rs:26-43)
+        const size_t i = out + ((size_t)py * S.width + px) * 3;
+        if (F.rgb) F.rgb[i] = c.x, F.rgb[i + 1] = c.y, F.rgb[i + 2] = c.z;
+        if (F.u8) F.u8[i] = scale_color(c.x), F.u8[i + 1] = scale_color(c.y), F.u8[i + 2] = scale_color(c.z);
+    }
+    __device__ __forceinline__ bool refill(bool& running, V3& ro, V3& rd, unsigned& pixel) {
+        bool started = false;
+        if (!running && pending) start(ro, rd, pixel), running = started = true;
+        const unsigned idle = __ballot_sync(0xffffffffu, !running);
+        if (done || (__popc(idle) < kRefillLanes && idle != 0xffffffffu)) return started;
+        const int lane = threadIdx.x & 31, leader = __ffs(idle) - 1;
+        unsigned base = 0;
+        if (lane == leader) base = atomicAdd(counter, (unsigned)__popc(idle));
+        base = __shfl_sync(0xffffffffu, base, leader);
+        if (base + (unsigned)__popc(idle) >= total) done = true;
+        if (running) return started;
+        const unsigned idx = base + (unsigned)__popc(idle & ((1u << lane) - 1u));
+        if (idx >= total) return false;
+        const unsigned within = idx & 31u, view = (idx >> 5) / view_blocks, block = (idx >> 5) - view * view_blocks;
+        const unsigned per_band = (unsigned)blocks_x * 2u;
+        const unsigned band_i = block / per_band, b = block - band_i * per_band;
+        const int band = F.shard + (F.band_begin + (int)band_i) * F.n_shards;
+        const int px = (int)(b >> 1) * 8 + (int)(within & 7u), py = band * kBandRows + (int)(b & 1u) * 4 + (int)(within >> 3);
+        if (px >= S.width || py >= S.height) return false;
+        out = (size_t)view * ((size_t)S.width * S.height * 3);
+        if (px >= S.width - 1 || py >= S.height - 1) {  // camera.rs:80-81: never rendered, stays black (canvas.rs:23)
+            store(px, py, mk(0.f, 0.f, 0.f));
+            return false;
+        }
+        x = px, y = py, next = 0, pending = true, cam = views + view;
+        start(ro, rd, pixel);
+        running = true;
+        return true;
+    }
+    __device__ __forceinline__ void finish(unsigned, V3 c) {
+        sum = next == 0 ? c : sum + c;
+        if (++next == n * n) {
+            pending = false;
+            store(x, y, sample_mean(sum, n));
+        }
+    }
+};
+
+__global__ void __launch_bounds__(kBlockThreads, min_blocks(RTC_STREAM_MINBLOCKS))
+    render_stream_views_samples(const __grid_constant__ DevScene S, const __grid_constant__ SmallScene SS, const DevFrame F,
+                                DevCounters* counters, const DevView* views, int n_views, int n) {
+    const Env E{S, SS};
+    const int blocks_x = (S.width + 7) / 8;
+    const unsigned view_blocks = (unsigned)F.n_bands * (unsigned)blocks_x * 2u;
+    ViewSamplePixelStream src{S, F, F.stream_counter, (unsigned)n_views * view_blocks * 32u, blocks_x, views, view_blocks, n};
+    Ctr<false> k;
+    Rays r;
+    color_at<false, false, true, false, false, ViewSamplePixelStream>(E, false, mk(0.f, 0.f, 0.f), mk(0.f, 0.f, 1.f), F.depth, 0u, r,
+                                                                      k, nullptr, nullptr, src);
+    flush_counters<false>(r, k, counters);
+}
+
 // ---- the wavefront renderer's kernels (dev_wave.cuh) --------------------------------------------------------------------
 #ifndef RTC_WAVE_TRACE_MINBLOCKS
 #define RTC_WAVE_TRACE_MINBLOCKS 8
@@ -449,7 +593,7 @@ __global__ void __launch_bounds__(kBlockThreads) trace_rays(const __grid_constan
 }
 
 // The instantiations frame_variant (rtc_launch.h) can select, X(STATS, SMALL, CONVERGE, DRAWN, LEAN): render_tiles takes all
-// of them, render_tiles_views and render_tiles_samples those without STATS.  The *_sweep builds have no lean kernel.
+// of them, render_tiles_views, render_tiles_samples and render_tiles_views_samples those without STATS.  The *_sweep builds have no lean kernel.
 #ifndef RTC_CSG_SWEEP_BUILD
 constexpr bool kHasLean = true;
 #define RTC_LEAN_TILE_VARIANTS(X) X(false, true, false, true, true) X(false, true, false, false, true)

@@ -675,6 +675,36 @@ int64_t sg_render_prepared_views_ppm(sg_ctx* c, int h, int depth, int n, const i
     to_sg_stats(c->last_stats, stats);
     return rc ? fail(rtc_last_error()) : (int64_t)offsets[n];
 }
+// rtc_render_views_samples on a prepared scene: n cameras (handles) of its canvas size, samples_per_axis^2 samples per pixel,
+// frames view-major in out_rgb / out_u8
+int sg_render_prepared_views_samples(sg_ctx* c, int h, int depth, int n, const int* cams, int samples_per_axis, int fma, float* out_rgb,
+                                     uint8_t* out_u8, sg_stats* stats) {
+    if (h < 0 || h >= (int)c->prepared.size() || !c->prepared[h]) return fail("bad prepared handle");
+    if (samples_per_axis < 0) return fail("negative samples_per_axis");
+    RtcScene* scene = c->prepared[h]->scene;
+    std::vector<RtcView> views;
+    if (camera_views(c, cams, n, c->prepared[h]->width, c->prepared[h]->height, views)) return -1;
+    if (rtc_set_option(scene, RTC_OPT_FMA_CONTRACTION, fma ? 1 : 0)) return fail(rtc_last_error());
+    const int rc = rtc_render_views_samples(scene, depth, (uint32_t)n, views.data(), (uint32_t)samples_per_axis, out_rgb, out_u8,
+                                            &c->last_stats);
+    to_sg_stats(c->last_stats, stats);
+    return rc ? fail(rtc_last_error()) : 0;
+}
+// ... and its text form (rtc_render_views_samples_ppm): offsets and the return value as sg_render_prepared_views_ppm's
+int64_t sg_render_prepared_views_samples_ppm(sg_ctx* c, int h, int depth, int n, const int* cams, int samples_per_axis, int fma,
+                                             char* out, int64_t capacity, size_t* offsets, sg_stats* stats) {
+    if (h < 0 || h >= (int)c->prepared.size() || !c->prepared[h]) return fail("bad prepared handle");
+    if (capacity < 0) return fail("negative capacity");
+    if (samples_per_axis < 0) return fail("negative samples_per_axis");
+    RtcScene* scene = c->prepared[h]->scene;
+    std::vector<RtcView> views;
+    if (camera_views(c, cams, n, c->prepared[h]->width, c->prepared[h]->height, views)) return -1;
+    if (rtc_set_option(scene, RTC_OPT_FMA_CONTRACTION, fma ? 1 : 0)) return fail(rtc_last_error());
+    const int rc = rtc_render_views_samples_ppm(scene, depth, (uint32_t)n, views.data(), (uint32_t)samples_per_axis, out,
+                                                (size_t)capacity, offsets, &c->last_stats);
+    to_sg_stats(c->last_stats, stats);
+    return rc ? fail(rtc_last_error()) : (int64_t)offsets[n];
+}
 // The one-shot batch: flatten, commit with the camera whose origin is farthest out, run `render` on the scene and the
 // cameras' views, release.  The world is consumed once.
 static int views_one_shot(sg_ctx* c, const int* cams, int n, int w, sg_stats* stats,
@@ -716,6 +746,26 @@ int64_t sg_camera_render_views_ppm(sg_ctx* c, const int* cams, int n, int w, int
     if (capacity < 0) return fail("negative capacity");
     const int rc = views_one_shot(c, cams, n, w, stats, [&](RtcScene* scene, const std::vector<RtcView>& views) {
         return rtc_render_views_ppm(scene, depth, (uint32_t)n, views.data(), out, (size_t)capacity, offsets, &c->last_stats);
+    });
+    return rc ? -1 : (int64_t)offsets[n];
+}
+// The one-shot anti-aliased batch (sg_camera_render_views with samples_per_axis^2 samples per pixel) ...
+int sg_camera_render_views_samples(sg_ctx* c, const int* cams, int n, int w, int depth, int samples_per_axis, float* out_rgb,
+                                   uint8_t* out_u8, sg_stats* stats) {
+    if (samples_per_axis < 0) return fail("negative samples_per_axis");
+    return views_one_shot(c, cams, n, w, stats, [&](RtcScene* scene, const std::vector<RtcView>& views) {
+        return rtc_render_views_samples(scene, depth, (uint32_t)n, views.data(), (uint32_t)samples_per_axis, out_rgb, out_u8,
+                                        &c->last_stats);
+    });
+}
+// ... and its text form: offsets and the return value as sg_camera_render_views_ppm's
+int64_t sg_camera_render_views_samples_ppm(sg_ctx* c, const int* cams, int n, int w, int depth, int samples_per_axis, char* out,
+                                           int64_t capacity, size_t* offsets, sg_stats* stats) {
+    if (capacity < 0) return fail("negative capacity");
+    if (samples_per_axis < 0) return fail("negative samples_per_axis");
+    const int rc = views_one_shot(c, cams, n, w, stats, [&](RtcScene* scene, const std::vector<RtcView>& views) {
+        return rtc_render_views_samples_ppm(scene, depth, (uint32_t)n, views.data(), (uint32_t)samples_per_axis, out, (size_t)capacity,
+                                            offsets, &c->last_stats);
     });
     return rc ? -1 : (int64_t)offsets[n];
 }

@@ -187,14 +187,18 @@ struct KernelBuild {
     decltype(&fast::launch_wave) wave;
     decltype(&fast::launch_views) views;
     decltype(&fast::launch_samples) samples;
+    decltype(&fast::launch_views_samples) views_samples;
 };
 const KernelBuild& kernel_build(bool strict_fp, bool csg_sweep) {
     static const KernelBuild builds[4] = {
-        {fast::launch_render, fast::launch_trace, fast::launch_wave, fast::launch_views, fast::launch_samples},
-        {strict::launch_render, strict::launch_trace, strict::launch_wave, strict::launch_views, strict::launch_samples},
-        {fast_sweep::launch_render, fast_sweep::launch_trace, fast_sweep::launch_wave, fast_sweep::launch_views, fast_sweep::launch_samples},
+        {fast::launch_render, fast::launch_trace, fast::launch_wave, fast::launch_views, fast::launch_samples,
+         fast::launch_views_samples},
+        {strict::launch_render, strict::launch_trace, strict::launch_wave, strict::launch_views, strict::launch_samples,
+         strict::launch_views_samples},
+        {fast_sweep::launch_render, fast_sweep::launch_trace, fast_sweep::launch_wave, fast_sweep::launch_views, fast_sweep::launch_samples,
+         fast_sweep::launch_views_samples},
         {strict_sweep::launch_render, strict_sweep::launch_trace, strict_sweep::launch_wave, strict_sweep::launch_views,
-         strict_sweep::launch_samples}};
+         strict_sweep::launch_samples, strict_sweep::launch_views_samples}};
     return builds[(strict_fp ? 1 : 0) + (csg_sweep ? 2 : 0)];
 }
 
@@ -820,11 +824,12 @@ struct ViewsText {
     size_t* view_offsets;
 };
 
-// rtc_render_views (text == nullptr), rtc_render_views_ppm and rtc_render_samples (samples > 0: n_views == 1, views[0] the
-// sample camera, and the samples kernels with that many samples per axis), from the scene's state on: the arguments are
-// checked
+// rtc_render_views (text == nullptr) and rtc_render_views_ppm, and with samples > 0 samples per axis
+// rtc_render_views_samples(_ppm) and rtc_render_samples (single: n_views == 1, views[0] the committed camera, rendered by
+// rtc_render_samples' own kernels), from the scene's state on: the arguments are checked.  With samples the view table holds
+// the views' sample cameras (sample_camera).
 int render_views_body(RtcScene* s, int depth, uint32_t n_views, const RtcView* views, float* rgb, uint8_t* u8, RtcStats* stats,
-                      const ViewsText* text, const char* fn, int samples = 0) {
+                      const ViewsText* text, const char* fn, int samples = 0, bool single = false) {
     if (!s->committed) return fail(RTC_ERR_STATE, std::string(fn) + " before rtc_scene_commit");
     // The tree's boxes are padded for ray origins up to the commit's reach (rtc_commit.cu: "pad"): a camera farther out
     // could lose hits the reference reports.  Small and tree-less scenes test every item exactly: any view goes.
@@ -889,9 +894,10 @@ int render_views_body(RtcScene* s, int depth, uint32_t n_views, const RtcView* v
         r.small.plane_cells = r.plane_cells_eligible && r.small.cell_masks;
         if (int rc = ensure_views(slot, n_views, frame_px * 15 * chunk)) return rc;
         for (uint32_t v = 0; v < n_views; v++) {  // the view table, uploaded once per call on the render stream
+            const RtcView w = samples ? sample_camera(views[v], s->width, (uint32_t)samples) : views[v];
             DevView& d = slot->h_views[v];
-            rows3(views[v].transform_inverse, d.cam_inv);
-            d.half_w = views[v].half_width, d.half_h = views[v].half_height, d.pixel_size = views[v].pixel_size, d.pad = 0.f;
+            rows3(w.transform_inverse, d.cam_inv);
+            d.half_w = w.half_width, d.half_h = w.half_height, d.pixel_size = w.pixel_size, d.pad = 0.f;
         }
         CUDA_TRY(cudaMemcpyAsync(slot->d_views, slot->h_views, n_views * sizeof(DevView), cudaMemcpyHostToDevice, slot->stream));
         CUDA_TRY(cudaMemsetAsync(slot->d_counters, 0, sizeof(DevCounters), slot->stream));
@@ -959,8 +965,11 @@ int render_views_body(RtcScene* s, int depth, uint32_t n_views, const RtcView* v
                     F.stream_counter = slot->d_stream_counter, F.stream_blocks = stream_blocks(slot->sm_count);
                     CUDA_TRY(cudaMemsetAsync(slot->d_stream_counter, 0, sizeof(unsigned), lane));
                 }
-                if (samples)
+                if (single)
                     kernel_build(s->strict_fp, r.csg_sweep).samples(r.scene, r.small, F, slot->h_views[0], samples, slot->d_counters, lane);
+                else if (samples)
+                    kernel_build(s->strict_fp, r.csg_sweep).views_samples(r.scene, r.small, F, slot->d_views + L.v0, (int)(L.v1 - L.v0),
+                                                                          samples, slot->d_counters, lane);
                 else
                     kernel_build(s->strict_fp, r.csg_sweep).views(r.scene, r.small, F, slot->d_views + L.v0, (int)(L.v1 - L.v0),
                                                                   slot->d_counters, lane);
@@ -1056,17 +1065,46 @@ int render_views_impl(RtcScene* s, int depth, uint32_t n_views, const RtcView* v
 // rtc_render_samples ------------------------------------------------------------------------------------------------------
 constexpr uint32_t kMaxSamplesPerAxis = 16;
 
+// n samples per axis of the committed canvas: n in [1, 16], and a sample canvas rtc_set_camera would take
+int check_samples(const RtcScene* s, uint32_t n, const char* fn) {
+    if (n < 1 || n > kMaxSamplesPerAxis)
+        return fail(RTC_ERR_INVALID, std::string(fn) + ": samples_per_axis must be in [1, " + std::to_string(kMaxSamplesPerAxis) + "]");
+    if ((uint64_t)n * s->width * ((uint64_t)n * s->height) > (1ull << 31) / 3)
+        return fail(RTC_ERR_INVALID, std::string(fn) + ": the sample canvas (samples_per_axis * width) x (samples_per_axis * height) is "
+                                                       "bigger than rtc_set_camera allows");
+    return 0;
+}
+
 int render_samples_impl(RtcScene* s, int depth, uint32_t n, float* rgb, uint8_t* u8, RtcStats* stats) {
     // the arguments first (no device needed), then the scene's state
     if (!s) return fail(RTC_ERR_INVALID, "null scene");
-    if (n < 1 || n > kMaxSamplesPerAxis)
-        return fail(RTC_ERR_INVALID, "rtc_render_samples: samples_per_axis must be in [1, " + std::to_string(kMaxSamplesPerAxis) + "]");
-    if ((uint64_t)n * s->width * ((uint64_t)n * s->height) > (1ull << 31) / 3)
-        return fail(RTC_ERR_INVALID, "rtc_render_samples: the sample canvas (samples_per_axis * width) x (samples_per_axis * height) is "
-                                     "bigger than rtc_set_camera allows");
+    if (int rc = check_samples(s, n, "rtc_render_samples")) return rc;
     if (int rc = check_depth(depth)) return rc;
-    const RtcView c = sample_camera(s, n);  // the committed camera's origin: within the commit's reach
-    return render_views_body(s, depth, 1, &c, rgb, u8, stats, nullptr, "rtc_render_samples", (int)n);
+    const RtcView c = sample_camera(s, 1);  // the committed camera: within the commit's reach
+    return render_views_body(s, depth, 1, &c, rgb, u8, stats, nullptr, "rtc_render_samples", (int)n, true);
+}
+
+// rtc_render_views_samples (text == nullptr) and rtc_render_views_samples_ppm: the arguments in the header's order (no device
+// needed), then the scene's state
+int render_views_samples_impl(RtcScene* s, int depth, uint32_t n_views, const RtcView* views, uint32_t n, float* rgb, uint8_t* u8,
+                              const ViewsText* text, RtcStats* stats) {
+    const char* fn = text ? "rtc_render_views_samples_ppm" : "rtc_render_views_samples";
+    if (!s) return fail(RTC_ERR_INVALID, "null scene");
+    if (int rc = check_views(n_views, views, fn)) return rc;
+    if (int rc = check_samples(s, n, fn)) return rc;
+    if (int rc = check_depth(depth)) return rc;
+    if (text) {
+        if (!text->ppm || !text->view_offsets) return fail(RTC_ERR_INVALID, std::string(fn) + ": ppm and view_offsets must be non-null");
+        const size_t bound = rtc_ppm_bound(s->width, s->height);
+        if (bound > SIZE_MAX / n_views) return fail(RTC_ERR_INVALID, std::string(fn) + ": n_views * rtc_ppm_bound overflows size_t");
+        if (text->capacity < bound * n_views)
+            return fail(RTC_ERR_INVALID, std::string(fn) + ": capacity " + std::to_string(text->capacity) +
+                                             " is below n_views * rtc_ppm_bound = " + std::to_string(bound * n_views));
+    }
+    const auto t0 = std::chrono::steady_clock::now();
+    const int rc = render_views_body(s, depth, n_views, views, rgb, u8, stats, text, fn, (int)n);
+    if (!rc && text && stats) stats->total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    return rc;
 }
 
 // rtc_render_ppm ---------------------------------------------------------------------------------------------------------
@@ -1670,6 +1708,15 @@ int rtc_render_views(RtcScene* s, int32_t depth, uint32_t n_views, const RtcView
 }
 int rtc_render_samples(RtcScene* s, int32_t depth, uint32_t samples_per_axis, float* rgb, uint8_t* u8, RtcStats* stats) {
     return render_samples_impl(s, depth, samples_per_axis, rgb, u8, stats);
+}
+int rtc_render_views_samples(RtcScene* s, int32_t depth, uint32_t n_views, const RtcView* views, uint32_t samples_per_axis, float* rgb,
+                             uint8_t* u8, RtcStats* stats) {
+    return render_views_samples_impl(s, depth, n_views, views, samples_per_axis, rgb, u8, nullptr, stats);
+}
+int rtc_render_views_samples_ppm(RtcScene* s, int32_t depth, uint32_t n_views, const RtcView* views, uint32_t samples_per_axis,
+                                 char* ppm, size_t capacity, size_t* view_offsets, RtcStats* stats) {
+    const ViewsText text{ppm, capacity, view_offsets};
+    return render_views_samples_impl(s, depth, n_views, views, samples_per_axis, nullptr, nullptr, &text, stats);
 }
 size_t rtc_ppm_bound(uint32_t width, uint32_t height) {
     return ppm_header(width, height).size() + (size_t)width * height * 3 * 4;

@@ -215,13 +215,18 @@ inline bool streams_pixels(const RtcScene* s, const SmallScene& small) {
 inline int frame_converge(const RtcScene* s) { return s->converge < 0 ? (int)s->has_branching_materials : s->converge; }
 // The sample camera C_n of rtc_render_samples, shared with the host harness of the kernels: Camera::new(n W, n H, fov,
 // transform) (camera.rs:23-56).  n W / n H is the same real number as W / H, so the aspect and the half-sizes are the
-// committed ones; only pixel_size is derived again.  C_1 is the committed camera.
-inline RtcView sample_camera(const RtcScene* s, uint32_t n) {
-    RtcView c;
-    c.half_width = s->half_w, c.half_height = s->half_h;
-    c.pixel_size = n == 1 ? s->pixel_size : (s->half_w * 2.0f) / (float)(n * s->width);
-    memcpy(c.transform_inverse, s->cam_inv, sizeof(c.transform_inverse));
+// committed ones; only pixel_size is derived again.  C_1 is the committed camera.  The RtcView overload is the same for one
+// view of a batch (rtc_render_views_samples) of a width-pixel canvas.
+inline RtcView sample_camera(const RtcView& view, uint32_t width, uint32_t n) {
+    RtcView c = view;
+    if (n != 1) c.pixel_size = (view.half_width * 2.0f) / (float)(n * width);
     return c;
+}
+inline RtcView sample_camera(const RtcScene* s, uint32_t n) {
+    RtcView v;
+    v.half_width = s->half_w, v.half_height = s->half_h, v.pixel_size = s->pixel_size;
+    memcpy(v.transform_inverse, s->cam_inv, sizeof(v.transform_inverse));
+    return sample_camera(v, s->width, n);
 }
 // DevFrame::stream_blocks: render_stream's persistent grid, the resident blocks of its launch bounds (RTC_STREAM_MINBLOCKS)
 inline int stream_blocks(int sm_count) { return sm_count * 6; }

@@ -5,8 +5,9 @@
 // K1 render_tiles : Camera::render (camera.rs:76-91) — one thread per pixel, 128-thread blocks covering a
 //                   16x8 pixel tile as four 8x4 warps so that a warp's rays stay coherent; writes the f32
 //                   RGB canvas and the 8-bit canvas (canvas.rs:39-43) in the same pass.
-//                   render_tiles_views / render_tiles_samples: the same for a batch of views, and for n x n samples
-//                   per pixel (rtc_render_samples); render_stream* the pixel-stream forms for branching tree scenes.
+//                   render_tiles_views / render_tiles_samples / render_tiles_views_samples: the same for a batch of
+//                   views, for n x n samples per pixel (rtc_render_samples), and for both at once
+//                   (rtc_render_views_samples); render_stream* the pixel-stream forms for branching tree scenes.
 // K4 trace_rays   : World::color_at for caller-supplied rays (the unit-test probe).
 // K5 fma_peak     : dependent-FMA micro-benchmark for the measured FP32 roofline denominator.
 // Each is compiled once more with -DRTC_CSG_SWEEP_BUILD, as `fast_sweep` / `strict_sweep`: the builds that evaluate CSGs
@@ -117,6 +118,32 @@ void launch_samples(const DevScene& S, const SmallScene& SS, const DevFrame& F, 
 #undef RTC_LAUNCH_SAMPLES
 #undef RTC_LAUNCH_SAMPLES_true
 #undef RTC_LAUNCH_SAMPLES_false
+    }
+}
+
+// A batch of views with n x n samples per pixel (rtc_render_views_samples): launch_samples' kernel choice, views[v] view v's
+// sample camera, view z of the grid view v's frame as in launch_views
+void launch_views_samples(const DevScene& S, const SmallScene& SS, const DevFrame& F, const DevView* views, int n_views, int n,
+                          DevCounters* counters, cudaStream_t stream) {
+    dim3 grid((S.width + kTileW - 1) / kTileW, F.n_bands, n_views);
+    if (grid.x == 0 || grid.y == 0 || grid.z == 0) return;
+    const KernelVariant v = frame_variant(S, SS, F, false, kHasLean);
+    if (v.stream) {
+        render_stream_views_samples<<<F.stream_blocks, kBlockThreads, 0, stream>>>(S, SS, F, counters, views, n_views, n);
+        return;
+    }
+    const int smem = dynamic_smem(v);
+    switch (variant_code(v)) {
+#define RTC_LAUNCH_VIEWS_SAMPLES(ST, SM, CV, DR, LE) RTC_LAUNCH_VIEWS_SAMPLES_##ST(SM, CV, DR, LE)
+#define RTC_LAUNCH_VIEWS_SAMPLES_true(SM, CV, DR, LE)  // the counting pass has no samples kernel
+#define RTC_LAUNCH_VIEWS_SAMPLES_false(SM, CV, DR, LE)                                                                         \
+    case variant_code(false, SM, CV, DR, LE):                                                                                 \
+        render_tiles_views_samples<SM, CV, DR, LE><<<grid, kBlockThreads, smem, stream>>>(S, SS, F, counters, views, n); \
+        break;
+        RTC_TILE_VARIANTS(RTC_LAUNCH_VIEWS_SAMPLES)
+#undef RTC_LAUNCH_VIEWS_SAMPLES
+#undef RTC_LAUNCH_VIEWS_SAMPLES_true
+#undef RTC_LAUNCH_VIEWS_SAMPLES_false
     }
 }
 

@@ -5,12 +5,14 @@
 #include "rtc_types.h"
 
 namespace rtc {
-// The kernel a launch function runs for its inputs.  launch_render, launch_views, launch_samples and launch_trace
-// (rtc_kernels.cu) switch on it, and so does the host harness of the kernels (tests/emu/emu_kernels.cpp), which thus runs the kernel the GPU runs.
+// The kernel a launch function runs for its inputs.  launch_render, launch_views, launch_samples, launch_views_samples and
+// launch_trace (rtc_kernels.cu) switch on it, and so does the host harness of the kernels (tests/emu/emu_kernels.cpp), which
+// thus runs the kernel the GPU runs.
 struct KernelVariant {
-    bool stream;  // render_stream / render_stream_views / render_stream_samples: a tree scene whose lanes draw pixels from
-                  // F.stream_counter
-    // otherwise the template flags of render_tiles / render_tiles_views / render_tiles_samples / trace_rays
+    bool stream;  // render_stream / render_stream_views / render_stream_samples / render_stream_views_samples: a tree scene
+                  // whose lanes draw pixels from F.stream_counter
+    // otherwise the template flags of render_tiles / render_tiles_views / render_tiles_samples / render_tiles_views_samples /
+    // trace_rays
     bool stats, small, converge, drawn, lean;
 };
 constexpr int variant_code(bool stats, bool small, bool converge, bool drawn, bool lean) {
@@ -50,8 +52,12 @@ void launch_views(const DevScene& S, const SmallScene& SS, const DevFrame& F, co
 // n x n samples per pixel of the committed canvas (rtc_render_samples): the bands of F, each output pixel the box filter of
 // the pixels (n x + i, n y + j) of `camera`, the reference's Camera::new at n width x n height; a tree scene with
 // F.stream_counter set renders them as one pixel stream.
+// launch_views_samples: the same for a batch of views (rtc_render_views_samples), cameras[v] view v's sample camera and its
+// frame at F.rgb / F.u8 + v * width * height * 3, as launch_views lays them out.
 void launch_samples(const DevScene& S, const SmallScene& SS, const DevFrame& F, const DevView& camera, int samples_per_axis,
                     DevCounters* counters, cudaStream_t stream);
+void launch_views_samples(const DevScene& S, const SmallScene& SS, const DevFrame& F, const DevView* cameras, int n_views,
+                          int samples_per_axis, DevCounters* counters, cudaStream_t stream);
 void launch_trace(const DevScene& S, const SmallScene& SS, int n, const float* origins, const float* directions, int depth,
                   float* out_rgb, float* out_t, int* out_pos, DevCounters* counters, cudaStream_t stream);
 void launch_fma_peak(float* out, int blocks, int iters, cudaStream_t stream);
@@ -67,6 +73,8 @@ void launch_views(const DevScene& S, const SmallScene& SS, const DevFrame& F, co
                   cudaStream_t stream);
 void launch_samples(const DevScene& S, const SmallScene& SS, const DevFrame& F, const DevView& camera, int samples_per_axis,
                     DevCounters* counters, cudaStream_t stream);
+void launch_views_samples(const DevScene& S, const SmallScene& SS, const DevFrame& F, const DevView* cameras, int n_views,
+                          int samples_per_axis, DevCounters* counters, cudaStream_t stream);
 void launch_trace(const DevScene& S, const SmallScene& SS, int n, const float* origins, const float* directions, int depth,
                   float* out_rgb, float* out_t, int* out_pos, DevCounters* counters, cudaStream_t stream);
 void launch_wave(const DevScene& S, const SmallScene& SS, const DevFrame& F, const WavePoolRaw& pool, DevCounters* counters, int blocks,
@@ -80,6 +88,8 @@ void launch_views(const DevScene& S, const SmallScene& SS, const DevFrame& F, co
                   cudaStream_t stream);
 void launch_samples(const DevScene& S, const SmallScene& SS, const DevFrame& F, const DevView& camera, int samples_per_axis,
                     DevCounters* counters, cudaStream_t stream);
+void launch_views_samples(const DevScene& S, const SmallScene& SS, const DevFrame& F, const DevView* cameras, int n_views,
+                          int samples_per_axis, DevCounters* counters, cudaStream_t stream);
 void launch_trace(const DevScene& S, const SmallScene& SS, int n, const float* origins, const float* directions, int depth,
                   float* out_rgb, float* out_t, int* out_pos, DevCounters* counters, cudaStream_t stream);
 void launch_wave(const DevScene& S, const SmallScene& SS, const DevFrame& F, const WavePoolRaw& pool, DevCounters* counters, int blocks,
@@ -92,6 +102,8 @@ void launch_views(const DevScene& S, const SmallScene& SS, const DevFrame& F, co
                   cudaStream_t stream);
 void launch_samples(const DevScene& S, const SmallScene& SS, const DevFrame& F, const DevView& camera, int samples_per_axis,
                     DevCounters* counters, cudaStream_t stream);
+void launch_views_samples(const DevScene& S, const SmallScene& SS, const DevFrame& F, const DevView* cameras, int n_views,
+                          int samples_per_axis, DevCounters* counters, cudaStream_t stream);
 void launch_trace(const DevScene& S, const SmallScene& SS, int n, const float* origins, const float* directions, int depth,
                   float* out_rgb, float* out_t, int* out_pos, DevCounters* counters, cudaStream_t stream);
 void launch_wave(const DevScene& S, const SmallScene& SS, const DevFrame& F, const WavePoolRaw& pool, DevCounters* counters, int blocks,

@@ -645,6 +645,63 @@ impl Camera {
             .collect()
     }
 
+    /// `render_b200_views` anti-aliased: canvas i is `cameras[i].render_b200_samples(world, depth, samples_per_axis)`, every
+    /// view of the batch from one commit and one `rtc_render_views_samples` call.
+    pub fn render_b200_views_samples(cameras: &[Camera], world: World, reflection_recursion_depth: i16, samples_per_axis: u32)
+                                     -> Vec<Canvas> {
+        let (far, w, h, views) = Camera::batch_views(cameras);
+        let mut rgb = vec![0f32; views.len() * w * h * 3];
+        unsafe {
+            let scene = cameras[far].commit_b200(&world);
+            let mut stats: sys::RtcStats = std::mem::zeroed();
+            check(sys::rtc_render_views_samples(scene, reflection_recursion_depth as i32, views.len() as u32, views.as_ptr(),
+                                                samples_per_axis, rgb.as_mut_ptr(), std::ptr::null_mut(), &mut stats));
+            sys::rtc_scene_destroy(scene);
+        }
+        rgb.chunks(w * h * 3)
+            .map(|frame| {
+                let mut canvas = Canvas::new(w, h);
+                for y in 0..h {
+                    for x in 0..w {
+                        let i = (y * w + x) * 3;
+                        canvas.write_pixel(x, y, Color::new(frame[i], frame[i + 1], frame[i + 2]));
+                    }
+                }
+                canvas
+            })
+            .collect()
+    }
+
+    /// `render_b200_views_samples` then `Canvas::to_ppm` of every view, the texts written on the device
+    /// (`rtc_render_views_samples_ppm`).  String i is `cameras[i].render_b200_samples(world, depth, samples_per_axis).to_ppm()`.
+    pub fn render_b200_views_samples_ppm(cameras: &[Camera], world: World, reflection_recursion_depth: i16, samples_per_axis: u32)
+                                         -> Vec<String> {
+        let (far, w, h, views) = Camera::batch_views(cameras);
+        let capacity = views.len() * unsafe { sys::rtc_ppm_bound(w as u32, h as u32) };
+        let mut text = vec![0u8; capacity];
+        let mut offsets = vec![0usize; views.len() + 1];
+        unsafe {
+            let scene = cameras[far].commit_b200(&world);
+            let mut stats: sys::RtcStats = std::mem::zeroed();
+            check(sys::rtc_render_views_samples_ppm(scene, reflection_recursion_depth as i32, views.len() as u32, views.as_ptr(),
+                                                    samples_per_axis, text.as_mut_ptr() as *mut std::os::raw::c_char, capacity,
+                                                    offsets.as_mut_ptr(), &mut stats));
+            sys::rtc_scene_destroy(scene);
+        }
+        offsets
+            .windows(2)
+            .map(|o| String::from_utf8(text[o[0]..o[1]].to_vec()).expect("PPM text is ASCII"))
+            .collect()
+    }
+
+    /// The anti-aliased demo flow in one call: `camera.render_b200_samples_ppm(world, depth, n)` is
+    /// `camera.render_b200_samples(world, depth, n).to_ppm()`, with the text written on the device.
+    pub fn render_b200_samples_ppm(&self, world: World, reflection_recursion_depth: i16, samples_per_axis: u32) -> String {
+        Camera::render_b200_views_samples_ppm(std::slice::from_ref(self), world, reflection_recursion_depth, samples_per_axis)
+            .pop()
+            .expect("one view")
+    }
+
     /// A batch's views and the camera it commits with: the one whose origin is farthest out, so that the tree's reach
     /// covers every view.  Every camera must have one canvas size.
     fn batch_views(cameras: &[Camera]) -> (usize, usize, usize, Vec<sys::RtcView>) {

@@ -223,6 +223,13 @@ extern "C" {
     /// is `ppm[view_offsets[v]..view_offsets[v + 1]]`; `capacity >= n_views * rtc_ppm_bound(w, h)`, `n_views + 1` offsets.
     pub fn rtc_render_views_ppm(scene: *mut RtcScene, depth: i32, n_views: u32, views: *const RtcView, ppm: *mut c_char,
                                 capacity: usize, view_offsets: *mut usize, stats: *mut RtcStats) -> c_int;
+    /// `rtc_render_samples` for every view of an `rtc_render_views` batch: view v is the anti-aliased frame of the scene
+    /// committed with view v's camera, `samples_per_axis`² samples per pixel, frames view-major as `rtc_render_views`'.
+    pub fn rtc_render_views_samples(scene: *mut RtcScene, depth: i32, n_views: u32, views: *const RtcView, samples_per_axis: u32,
+                                    rgb_f32: *mut f32, rgb_u8: *mut u8, stats: *mut RtcStats) -> c_int;
+    /// `rtc_render_views_samples` then `Canvas::to_ppm` of every view, texts and offsets laid out as `rtc_render_views_ppm`'s.
+    pub fn rtc_render_views_samples_ppm(scene: *mut RtcScene, depth: i32, n_views: u32, views: *const RtcView, samples_per_axis: u32,
+                                        ppm: *mut c_char, capacity: usize, view_offsets: *mut usize, stats: *mut RtcStats) -> c_int;
     /// One shard's text of a frame shared by several processes, in two phases with the callers' exchange of `row_bytes`
     /// (`height` entries, frame-row order) in between: phase 1 renders the shard and writes its rows' lengths, phase 2 writes
     /// its bands' text at their offsets in `ppm` (shard 0 also the header); `*ppm_bytes` is the whole text's length.
