@@ -358,7 +358,8 @@ int rtc_render_ppm(RtcScene*, int32_t depth, char* ppm, size_t capacity, size_t*
  *     (rtc_shard_bands) are written, the others are not touched — so the ranks can write into one shared array, or into zeroed
  *     private ones summed by an all-reduce.  stats are rtc_render_shard's, with total_ms covering the whole phase.
  *   - Phase 2, rtc_write_shard_ppm: given every row's length (all shards' entries), writes the text of the shard's bands at
- *     their offsets in ppm; shard 0 also writes the header.  *ppm_bytes receives the whole text's length, the same on every
+ *     their offsets in ppm; shard 0 also writes the header.  It encodes the 8-bit plane its phase 1 left on the device
+ *     (rtc_render_shard_samples_ppm_rows' anti-aliased one, below, as well).  *ppm_bytes receives the whole text's length, the same on every
  *     shard.  A shard writes only [band_at, band_at + band_bytes) of each of its bands (and shard 0 the header): no other byte
  *     of ppm, so the ranks can write into one shared buffer without locking.  No stats.
  *   - The bytes: the union of every shard's writes is byte for byte rtc_render_ppm's text of the same scene — Canvas::to_ppm of
@@ -380,6 +381,35 @@ int rtc_render_ppm(RtcScene*, int32_t depth, char* ppm, size_t capacity, size_t*
 int rtc_render_shard_ppm_rows(RtcScene*, int32_t depth, int32_t shard, int32_t n_shards, uint64_t* row_bytes, RtcStats* stats);
 int rtc_write_shard_ppm(RtcScene*, int32_t shard, int32_t n_shards, const uint64_t* row_bytes, char* ppm, size_t capacity,
                         size_t* ppm_bytes);
+/* rtc_render_samples for one shard of a frame shared by several processes (one process per GPU): rtc_render_shard's split of
+ * an anti-aliased frame, as frames or as PPM text.
+ *   - Pixels, rtc_render_shard_samples: only the bands b with b % n_shards == shard (rtc_shard_bands) are rendered and written
+ *     into the full-size buffers (width * height * 3 each, as rtc_render_samples'); no other row is touched.  The union over
+ *     all shards is rtc_render_samples(n)'s planes bit for bit, in f32 and in 8 bits, for every kernel build and option: pixels
+ *     are independent and a sample's generated-jitter key is its index in the n W x n H frame, which a shard does not change.
+ *     NULL, NULL leaves the shard's bands on the device.
+ *   - Text, rtc_render_shard_samples_ppm_rows: phase 1 of rtc_render_shard_ppm_rows' two phases for that anti-aliased shard —
+ *     the shard render above with the frame left on the device, then the byte length of every row the shard owns, written
+ *     into row_bytes exactly as rtc_render_shard_ppm_rows writes it.  Phase 2 is rtc_write_shard_ppm, unchanged: it encodes
+ *     the plane the last phase 1 of either kind left.  The union of the shards' writes is byte for byte
+ *     rtc_render_views_samples_ppm's text of the committed camera (Canvas::to_ppm of rtc_render_samples' 8-bit plane).  Phase
+ *     state and the own-row check are rtc_write_shard_ppm's: any render (rtc_render_shard and rtc_render_samples included),
+ *     rtc_set_* / rtc_map_* or commit in between voids phase 1.
+ *   - The arguments are checked before the scene's state, in this order, all with RTC_ERR_INVALID: a NULL scene; (text call)
+ *     row_bytes NULL; n_shards < 1 or shard outside [0, n_shards); samples_per_axis outside [1, 16] or a sample canvas
+ *     rtc_set_camera would refuse (rtc_render_samples' rule); a depth outside [0, 23].  Then an uncommitted scene is
+ *     RTC_ERR_STATE, and so is a scene committed on more than one device (rtc_render_shard's rule).
+ *   - The render is rtc_render_samples' one-view path — slices, pinned and pageable destinations (staged through the
+ *     device's pinned frames), one persistent streaming launch for a tree scene whose ray trees branch — over the shard's
+ *     bands only.  Nothing of rtc_render's state changes.
+ *   - stats: primary_rays = n * n * (width - 1) * (the shard's rows below height - 1); launches and kernel_ms as
+ *     rtc_render_samples'; for the text call total_ms covers the whole phase.
+ *   - Device memory kept with the device for later calls: rtc_render_samples' frame in the view arena, and rtc_render_ppm's
+ *     text buffers. */
+int rtc_render_shard_samples(RtcScene*, int32_t depth, uint32_t samples_per_axis, int32_t shard, int32_t n_shards,
+                             float* rgb_f32, uint8_t* rgb_u8, RtcStats* stats);
+int rtc_render_shard_samples_ppm_rows(RtcScene*, int32_t depth, uint32_t samples_per_axis, int32_t shard, int32_t n_shards,
+                                      uint64_t* row_bytes, RtcStats* stats);
 /* rtc_render_views followed by Canvas::to_ppm of every view, with the text written on the device.
  *   - ppm receives the views' texts one after the other, no terminating NUL: view v's text is ppm[view_offsets[v] ..
  *     view_offsets[v + 1]).  view_offsets has n_views + 1 entries: view_offsets[0] = 0, view_offsets[n_views] the total.

@@ -106,13 +106,14 @@ _HOST_EXTRAS = {
     "sg_trace_rays": (_I, [_V, _I, C.c_uint32, _FP, _FP, _I, _I, _FP, _FP, _IP]),
     "sg_flatten": (_I, [_V, _I, _IP, C.POINTER(RtcPrim), C.POINTER(RtcNode), C.POINTER(C.c_int32), _IP]),
     "sg_render_prepared_views": (_I, [_V, _I, _I, _I, _IP, _I, _FP, _U8P, C.POINTER(SgStats)]),
-    "sg_render_prepared_samples": (_I, [_V, _I, _I, _I, _I, _FP, _U8P, C.POINTER(SgStats)]),
+    "sg_render_prepared_samples": (_I, [_V, _I, _I, _I, _I, _I, _I, _FP, _U8P, C.POINTER(SgStats)]),
     "sg_camera_render_views": (_I, [_V, _IP, _I, _I, _I, _FP, _U8P, C.POINTER(SgStats)]),
     "sg_camera_view": (_I, [_V, _I, C.POINTER(RtcView)]),
     "sg_farthest_camera": (_I, [_V, _IP, _I]),
     "sg_camera_render_ppm": (C.c_int64, [_V, _I, _I, _I, C.c_void_p, C.c_int64, C.POINTER(SgStats)]),
     "sg_render_prepared_ppm": (C.c_int64, [_V, _I, _I, _I, C.c_void_p, C.c_int64, C.POINTER(SgStats)]),
     "sg_render_prepared_shard_ppm_rows": (_I, [_V, _I, _I, _I, _I, _I, C.c_void_p, C.POINTER(SgStats)]),
+    "sg_render_prepared_shard_samples_ppm_rows": (_I, [_V, _I, _I, _I, _I, _I, _I, C.c_void_p, C.POINTER(SgStats)]),
     "sg_write_prepared_shard_ppm": (C.c_int64, [_V, _I, _I, _I, C.c_void_p, C.c_void_p, C.c_int64]),
     "sg_render_prepared_views_ppm": (C.c_int64, [_V, _I, _I, _I, _IP, _I, C.c_void_p, C.c_int64, C.POINTER(C.c_size_t),
                                                  C.POINTER(SgStats)]),
@@ -219,18 +220,20 @@ class PreparedScene:
         return _canvases(api, n, h, w, rgb, u8)
 
     def render_samples(self, samples, depth=DEFAULT_RAY_RECURSION_DEPTH, want_rgb=True, want_u8=True, out_rgb=None, out_u8=None,
-                       fma=False):
+                       fma=False, shard=0, n_shards=0):
         """rtc_render_samples: the committed scene anti-aliased with samples x samples samples per pixel, each sample a pixel
         of the reference's render at samples times the canvas size, box-filtered on the device (samples = 1 is render()'s
-        frame).  Buffers may be caller-supplied (e.g. pinned); want_* = False leaves the frame on the device."""
+        frame).  Buffers may be caller-supplied (e.g. pinned); want_* = False leaves the frame on the device.  shard /
+        n_shards as render's: n_shards >= 1 renders and writes only that shard's bands (rtc_render_shard_samples; a scene
+        committed on one device), the other rows of the buffers untouched."""
         w, h = self.camera.width_pixels, self.camera.height_pixels
         rgb, u8 = _view_planes(1, h, w, want_rgb, want_u8, None if out_rgb is None else out_rgb[None],
                                None if out_u8 is None else out_u8[None])
         stats = SgStats()
         api = self.api
         api.check(api.lib.sg_render_prepared_samples(
-            api.ctx, self.handle, int(depth), int(samples), int(fma), _api.fptr(rgb) if rgb is not None else None,
-            u8.ctypes.data_as(_U8P) if u8 is not None else None, C.byref(stats)))
+            api.ctx, self.handle, int(depth), int(samples), int(shard), int(n_shards), int(fma),
+            _api.fptr(rgb) if rgb is not None else None, u8.ctypes.data_as(_U8P) if u8 is not None else None, C.byref(stats)))
         self.last_stats = api.last_rtc_stats()
         return Canvas(w, h, rgb[0] if rgb is not None else None, u8[0] if u8 is not None else None, api=api)
 
@@ -282,17 +285,24 @@ class PreparedScene:
         self.last_stats = api.last_rtc_stats()
         return buf[:n].tobytes().decode("ascii")
 
-    def render_shard_ppm_rows(self, shard, n_shards, row_bytes, depth=DEFAULT_RAY_RECURSION_DEPTH, fma=False):
+    def render_shard_ppm_rows(self, shard, n_shards, row_bytes, depth=DEFAULT_RAY_RECURSION_DEPTH, fma=False, samples=0):
         """rtc_render_shard_ppm_rows, the first phase of one shard's text of a frame shared by several processes: renders the
         shard's bands (rtc_render_shard, the frame left on the device) and writes the byte length of each of their rows'
         text into `row_bytes` (a uint64 array of one entry per frame row; the other shards' entries are not touched).  The
-        callers then exchange the entries (multi.render_ppm_shared does it through shared memory) and call write_shard_ppm."""
+        callers then exchange the entries (multi.render_ppm_shared does it through shared memory) and call write_shard_ppm.
+        samples >= 1 renders the shard anti-aliased instead (rtc_render_shard_samples_ppm_rows): the texts then make up
+        render_samples_ppm(samples)'s."""
         h = self.camera.height_pixels
         api = self.api
         row_bytes = _row_bytes(row_bytes, h)
         stats = SgStats()
-        api.check(api.lib.sg_render_prepared_shard_ppm_rows(api.ctx, self.handle, int(depth), int(shard), int(n_shards), int(fma),
-                                                            row_bytes.ctypes.data, C.byref(stats)))
+        if samples:
+            api.check(api.lib.sg_render_prepared_shard_samples_ppm_rows(api.ctx, self.handle, int(depth), int(samples), int(shard),
+                                                                        int(n_shards), int(fma), row_bytes.ctypes.data,
+                                                                        C.byref(stats)))
+        else:
+            api.check(api.lib.sg_render_prepared_shard_ppm_rows(api.ctx, self.handle, int(depth), int(shard), int(n_shards),
+                                                                int(fma), row_bytes.ctypes.data, C.byref(stats)))
         self.last_stats = api.last_rtc_stats()
 
     def write_shard_ppm(self, shard, n_shards, row_bytes, out) -> int:

@@ -650,14 +650,29 @@ int sg_render_prepared_views(sg_ctx* c, int h, int depth, int n, const int* cams
     to_sg_stats(c->last_stats, stats);
     return rc ? fail(rtc_last_error()) : 0;
 }
-// rtc_render_samples on a prepared scene: n x n samples per pixel of its canvas, frames as sg_render_prepared's
-int sg_render_prepared_samples(sg_ctx* c, int h, int depth, int samples_per_axis, int fma, float* out_rgb, uint8_t* out_u8,
-                               sg_stats* stats) {
+// rtc_render_samples on a prepared scene: n x n samples per pixel of its canvas, frames as sg_render_prepared's; shard and
+// n_shards as sg_render_prepared's (n_shards >= 1: rtc_render_shard_samples)
+int sg_render_prepared_samples(sg_ctx* c, int h, int depth, int samples_per_axis, int shard, int n_shards, int fma, float* out_rgb,
+                               uint8_t* out_u8, sg_stats* stats) {
     if (h < 0 || h >= (int)c->prepared.size() || !c->prepared[h]) return fail("bad prepared handle");
     if (samples_per_axis < 0) return fail("negative samples_per_axis");
     RtcScene* scene = c->prepared[h]->scene;
     if (rtc_set_option(scene, RTC_OPT_FMA_CONTRACTION, fma ? 1 : 0)) return fail(rtc_last_error());
-    const int rc = rtc_render_samples(scene, depth, (uint32_t)samples_per_axis, out_rgb, out_u8, &c->last_stats);
+    const int rc = n_shards >= 1 ? rtc_render_shard_samples(scene, depth, (uint32_t)samples_per_axis, shard, n_shards, out_rgb,
+                                                            out_u8, &c->last_stats)
+                                 : rtc_render_samples(scene, depth, (uint32_t)samples_per_axis, out_rgb, out_u8, &c->last_stats);
+    to_sg_stats(c->last_stats, stats);
+    return rc ? fail(rtc_last_error()) : 0;
+}
+// Phase 1 of an anti-aliased shard's text (rtc_render_shard_samples_ppm_rows); phase 2 is sg_write_prepared_shard_ppm
+int sg_render_prepared_shard_samples_ppm_rows(sg_ctx* c, int h, int depth, int samples_per_axis, int shard, int n_shards, int fma,
+                                              uint64_t* row_bytes, sg_stats* stats) {
+    if (h < 0 || h >= (int)c->prepared.size() || !c->prepared[h]) return fail("bad prepared handle");
+    if (samples_per_axis < 0) return fail("negative samples_per_axis");
+    RtcScene* scene = c->prepared[h]->scene;
+    if (rtc_set_option(scene, RTC_OPT_FMA_CONTRACTION, fma ? 1 : 0)) return fail(rtc_last_error());
+    const int rc = rtc_render_shard_samples_ppm_rows(scene, depth, (uint32_t)samples_per_axis, shard, n_shards, row_bytes,
+                                                     &c->last_stats);
     to_sg_stats(c->last_stats, stats);
     return rc ? fail(rtc_last_error()) : 0;
 }

@@ -827,9 +827,12 @@ struct ViewsText {
 // rtc_render_views (text == nullptr) and rtc_render_views_ppm, and with samples > 0 samples per axis
 // rtc_render_views_samples(_ppm) and rtc_render_samples (single: n_views == 1, views[0] the committed camera, rendered by
 // rtc_render_samples' own kernels), from the scene's state on: the arguments are checked.  With samples the view table holds
-// the views' sample cameras (sample_camera).
+// the views' sample cameras (sample_camera).  shard0 / n_shards_ext as render_impl's: n_shards_ext 0 splits the views over the
+// committed devices; n_shards_ext >= 1 (one committed device) renders only the bands of shard0 of a frame shared by several
+// processes (rtc_render_shard_samples).
 int render_views_body(RtcScene* s, int depth, uint32_t n_views, const RtcView* views, float* rgb, uint8_t* u8, RtcStats* stats,
-                      const ViewsText* text, const char* fn, int samples = 0, bool single = false) {
+                      const ViewsText* text, const char* fn, int samples = 0, bool single = false, int shard0 = 0,
+                      int n_shards_ext = 0) {
     if (!s->committed) return fail(RTC_ERR_STATE, std::string(fn) + " before rtc_scene_commit");
     // The tree's boxes are padded for ray origins up to the commit's reach (rtc_commit.cu: "pad"): a camera farther out
     // could lose hits the reference reports.  Small and tree-less scenes test every item exactly: any view goes.
@@ -848,7 +851,9 @@ int render_views_body(RtcScene* s, int depth, uint32_t n_views, const RtcView* v
             }
     s->shard_ppm = {};  // any render voids a pending rtc_write_shard_ppm (include/rtc_b200.h)
     auto t0 = std::chrono::steady_clock::now();
-    const int ndev = (int)s->replicas.size(), n_shards = ndev;
+    const int ndev = (int)s->replicas.size();
+    const bool external = n_shards_ext > 0;
+    const int n_shards = external ? n_shards_ext : ndev;
     const int total_bands = ((int)s->height + kBandRows - 1) / kBandRows;
     const bool copy_out = rgb || u8;
     const size_t frame_px = (size_t)s->width * s->height;
@@ -917,7 +922,7 @@ int render_views_body(RtcScene* s, int depth, uint32_t n_views, const RtcView* v
         for (int i = 0; i < ndev; i++) {
             Replica& r = s->replicas[i];
             DeviceSlot* slot = r.slot;
-            const int shard = i;
+            const int shard = external ? shard0 : i;
             const int nb = shard < total_bands ? (total_bands - shard + n_shards - 1) / n_shards : 0;
             CUDA_TRY(cudaSetDevice(slot->device));
             float* d_rgb = reinterpret_cast<float*>(slot->d_view_frames);
@@ -1040,7 +1045,7 @@ int render_views_body(RtcScene* s, int depth, uint32_t n_views, const RtcView* v
         if (!text) CUDA_TRY(cudaEventElapsedTime(&ms, slot->ev0, slot->ev1));
         st.kernel_ms = std::max(st.kernel_ms, (double)ms);
         uint64_t rows = 0;  // camera.rs:80-81, per view, of this device's bands
-        for (int b = i; b < total_bands; b += n_shards)
+        for (int b = external ? shard0 : i; b < total_bands; b += n_shards)
             rows += (uint64_t)std::max(0, std::min<int>((int)s->height - 1, (b + 1) * kBandRows) - b * kBandRows);
         const uint64_t per_pixel = samples ? (uint64_t)samples * samples : 1;  // primary rays of one output pixel
         add_counters(st, *slot->h_counters, per_pixel * n_views * rows * (uint64_t)(s->width - 1),
@@ -1337,8 +1342,21 @@ int check_shard_scene(const RtcScene* s, const char* fn) {
     return 0;
 }
 
-// Phase 1: rtc_render_shard with the frame left on the device, then (a) for the shard's rows.  Their lengths go to row_bytes
-// (frame-row order; no other entry is touched) and are kept for phase 2's own-row check.
+// The end of phase 1, behind a shard render that left its frame on the device: (a) for the shard's rows of `plane` (the
+// device's 8-bit plane of that render).  Their lengths go to row_bytes (frame-row order; no other entry is touched) and are
+// kept, with the plane, for phase 2.
+int shard_ppm_rows(RtcScene* s, const unsigned char* plane, int shard, int n_shards, uint64_t* row_bytes) {
+    std::vector<PpmRows> rows;
+    if (int rc = ppm_row_lengths(s, &plane, 1, 0, shard, n_shards, rows)) return rc;
+    const unsigned long long* lengths = s->replicas[0].slot->h_ppm_rows;
+    s->shard_ppm.rows.assign(lengths, lengths + rows[0].n_rows);  // band order: the shard's frame rows in increasing order
+    s->shard_ppm.shard = shard, s->shard_ppm.n_shards = n_shards, s->shard_ppm.plane = plane;
+    for (uint32_t y = 0, k = 0; y < s->height; y++)
+        if ((int)(y / kBandRows % n_shards) == shard) row_bytes[y] = lengths[k++];
+    return 0;
+}
+
+// Phase 1: rtc_render_shard with the frame left on the device, then shard_ppm_rows.
 int render_shard_ppm_rows_impl(RtcScene* s, int depth, int shard, int n_shards, uint64_t* row_bytes, RtcStats* stats) {
     const char* fn = "rtc_render_shard_ppm_rows";
     if (!s) return fail(RTC_ERR_INVALID, "null scene");
@@ -1353,15 +1371,39 @@ int render_shard_ppm_rows_impl(RtcScene* s, int depth, int shard, int n_shards, 
         if (stats) *stats = st;
         return rc;
     }
-    const unsigned char* frame = s->replicas[0].slot->d_u8;
-    std::vector<PpmRows> rows;
-    if (int rc = ppm_row_lengths(s, &frame, 1, 0, shard, n_shards, rows)) return rc;
-    const unsigned long long* lengths = s->replicas[0].slot->h_ppm_rows;
-    s->shard_ppm.rows.assign(lengths, lengths + rows[0].n_rows);  // band order: the shard's frame rows in increasing order
-    s->shard_ppm.shard = shard, s->shard_ppm.n_shards = n_shards;
-    for (uint32_t y = 0, k = 0; y < s->height; y++)
-        if ((int)(y / kBandRows % n_shards) == shard) row_bytes[y] = lengths[k++];
+    if (int rc = shard_ppm_rows(s, s->replicas[0].slot->d_u8, shard, n_shards, row_bytes)) return rc;
     st.total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    if (stats) *stats = st;
+    return 0;
+}
+
+// rtc_render_shard_samples (row_bytes == nullptr) and rtc_render_shard_samples_ppm_rows: rtc_render_samples' one-view path
+// for the bands of one shard of a frame shared by several processes.  The arguments in the header's order (no device
+// needed), then the scene's state.
+int render_shard_samples_impl(RtcScene* s, int depth, uint32_t n, int shard, int n_shards, float* rgb, uint8_t* u8,
+                              bool text, uint64_t* row_bytes, RtcStats* stats) {
+    const char* fn = text ? "rtc_render_shard_samples_ppm_rows" : "rtc_render_shard_samples";
+    if (!s) return fail(RTC_ERR_INVALID, "null scene");
+    if (text && !row_bytes) return fail(RTC_ERR_INVALID, std::string(fn) + ": row_bytes must be non-null");
+    if (int rc = check_shard(shard, n_shards, fn)) return rc;
+    if (int rc = check_samples(s, n, fn)) return rc;
+    if (int rc = check_depth(depth)) return rc;
+    if (int rc = check_shard_scene(s, fn)) return rc;
+    const auto t0 = std::chrono::steady_clock::now();
+    RtcStats st;
+    memset(&st, 0, sizeof(st));
+    const RtcView c = sample_camera(s, 1);  // the committed camera: within the commit's reach
+    if (int rc = render_views_body(s, depth, 1, &c, rgb, u8, &st, nullptr, fn, (int)n, true, shard, n_shards)) {
+        if (stats) *stats = st;
+        return rc;
+    }
+    if (text) {
+        // one view is a chunk of one: its 8-bit plane follows its f32 plane in the view arena (render_views_body)
+        const unsigned char* plane =
+            reinterpret_cast<const unsigned char*>(s->replicas[0].slot->d_view_frames) + (size_t)s->width * s->height * 12;
+        if (int rc = shard_ppm_rows(s, plane, shard, n_shards, row_bytes)) return rc;
+        st.total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    }
     if (stats) *stats = st;
     return 0;
 }
@@ -1409,7 +1451,7 @@ int write_shard_ppm_impl(RtcScene* s, int shard, int n_shards, const uint64_t* r
     const std::vector<unsigned long long>& own = shard_rows[shard];
     if (int rc = ensure_ppm_rows(slot, std::max<size_t>(own.size(), 1))) return rc;
     if (!own.empty()) memcpy(slot->h_ppm_rows, own.data(), own.size() * sizeof(unsigned long long));
-    const std::vector<PpmRows> rows{PpmRows{slot->d_u8, (int)s->width, shard, n_shards, (int)own.size()}};
+    const std::vector<PpmRows> rows{PpmRows{s->shard_ppm.plane, (int)s->width, shard, n_shards, (int)own.size()}};
     if (int rc = ppm_write_copy(s, rows, L, ppm)) return rc;
     CUDA_TRY(cudaSetDevice(slot->device));
     CUDA_TRY(cudaStreamSynchronize(slot->stream));
@@ -1730,6 +1772,14 @@ int rtc_render_views_ppm(RtcScene* s, int32_t depth, uint32_t n_views, const Rtc
 }
 int rtc_render_shard_ppm_rows(RtcScene* s, int32_t depth, int32_t shard, int32_t n_shards, uint64_t* row_bytes, RtcStats* stats) {
     return render_shard_ppm_rows_impl(s, depth, shard, n_shards, row_bytes, stats);
+}
+int rtc_render_shard_samples(RtcScene* s, int32_t depth, uint32_t samples_per_axis, int32_t shard, int32_t n_shards, float* rgb,
+                             uint8_t* u8, RtcStats* stats) {
+    return render_shard_samples_impl(s, depth, samples_per_axis, shard, n_shards, rgb, u8, false, nullptr, stats);
+}
+int rtc_render_shard_samples_ppm_rows(RtcScene* s, int32_t depth, uint32_t samples_per_axis, int32_t shard, int32_t n_shards,
+                                      uint64_t* row_bytes, RtcStats* stats) {
+    return render_shard_samples_impl(s, depth, samples_per_axis, shard, n_shards, nullptr, nullptr, true, row_bytes, stats);
 }
 int rtc_write_shard_ppm(RtcScene* s, int32_t shard, int32_t n_shards, const uint64_t* row_bytes, char* ppm, size_t capacity,
                         size_t* ppm_bytes) {

@@ -195,11 +195,13 @@ struct RtcScene {
     // commit statistics
     int n_bvh_nodes = 0, n_linear = 0, n_xforms = 0;
     float reach = 0.f;  // Flattened::reach of the commit: rtc_render_views refuses camera origins beyond it in tree scenes
-    // rtc_render_shard_ppm_rows -> rtc_write_shard_ppm: the shard the last phase 1 encoded (n_shards 0: none) and the byte
-    // lengths it computed for the shard's rows in frame-row order.  Any render, rtc_set_* / rtc_map_* or commit clears it.
-    // (The slot's h_ppm_rows cannot serve: ppm_layout turns it into offsets in place.)
+    // rtc_render_shard_ppm_rows / rtc_render_shard_samples_ppm_rows -> rtc_write_shard_ppm: the shard the last phase 1 encoded
+    // (n_shards 0: none), the device's 8-bit plane it encoded (the slot's d_u8, or the samples render's in the view arena) and
+    // the byte lengths it computed for the shard's rows in frame-row order.  Any render, rtc_set_* / rtc_map_* or commit clears
+    // it.  (The slot's h_ppm_rows cannot serve: ppm_layout turns it into offsets in place.)
     struct ShardPpm {
         int shard = -1, n_shards = 0;
+        const unsigned char* plane = nullptr;
         std::vector<unsigned long long> rows;
     } shard_ppm;
 };

@@ -1,7 +1,8 @@
 """Host plumbing for one frame rendered by several processes (one per GPU, `torchrun`): a canvas in POSIX shared
 memory that every rank writes its bands into — the "simple host gather" of SURVEY.md §8e, with no copy and no
-collective on the data path — the same for the frame's PPM text (SharedText, render_ppm_shared), plus the two scalar
-reductions the benchmark needs (torch.distributed is plumbing here, not the product)."""
+collective on the data path (render_samples_shared for an anti-aliased frame) — the same for the frame's PPM text
+(SharedText, render_ppm_shared), plus the two scalar reductions the benchmark needs (torch.distributed is plumbing here,
+not the product)."""
 from __future__ import annotations
 
 from multiprocessing import shared_memory
@@ -116,12 +117,21 @@ def open_shared_text(dist, rank: int, name: str, width: int, height: int) -> Sha
     return text
 
 
-def render_ppm_shared(dist, rank: int, world_size: int, prepared, text: SharedText, depth: int = 5) -> int:
+def render_samples_shared(dist, rank: int, world_size: int, prepared, canvas: SharedCanvas, samples: int, depth: int = 5):
+    """One anti-aliased frame (samples x samples samples per pixel) rendered by world_size ranks of one node into `canvas`,
+    rank r writing the bands of shard r of `prepared` (a PreparedScene committed on one device) into both planes, then a
+    barrier: canvas.rgb / canvas.u8 then hold render_samples(samples)'s frame."""
+    prepared.render_samples(samples, depth, out_rgb=canvas.rgb, out_u8=canvas.u8, shard=rank, n_shards=world_size)
+    dist.barrier()
+
+
+def render_ppm_shared(dist, rank: int, world_size: int, prepared, text: SharedText, depth: int = 5, samples: int = 0) -> int:
     """One frame's `Canvas::to_ppm` text written by world_size ranks of one node, rank r rendering shard r of `prepared`
     (a PreparedScene committed on one device): phase 1 into text.row_bytes, a barrier (every row's length is then in
     place), phase 2 into text.buf, a barrier.  Returns the text's length on every rank: text.text(length) is the frame's
-    text.  The exchange is shared memory; torch.distributed only provides the barriers."""
-    prepared.render_shard_ppm_rows(rank, world_size, text.row_bytes, depth)
+    text.  The exchange is shared memory; torch.distributed only provides the barriers.  samples >= 1: the anti-aliased
+    frame's text, render_samples_ppm(samples)'s."""
+    prepared.render_shard_ppm_rows(rank, world_size, text.row_bytes, depth, samples=samples)
     dist.barrier()
     length = prepared.write_shard_ppm(rank, world_size, text.row_bytes, text.buf)
     dist.barrier()

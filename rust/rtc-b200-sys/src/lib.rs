@@ -237,6 +237,14 @@ extern "C" {
                                      stats: *mut RtcStats) -> c_int;
     pub fn rtc_write_shard_ppm(scene: *mut RtcScene, shard: i32, n_shards: i32, row_bytes: *const u64, ppm: *mut c_char,
                                capacity: usize, ppm_bytes: *mut usize) -> c_int;
+    /// `rtc_render_samples` for one shard of a frame shared by several processes: only the bands `b % n_shards == shard` are
+    /// rendered and written into the full-size buffers; the shards together give `rtc_render_samples`' planes bit for bit.
+    pub fn rtc_render_shard_samples(scene: *mut RtcScene, depth: i32, samples_per_axis: u32, shard: i32, n_shards: i32,
+                                    rgb_f32: *mut f32, rgb_u8: *mut u8, stats: *mut RtcStats) -> c_int;
+    /// Phase 1 of an anti-aliased shard's text: `rtc_render_shard_samples` with the frame left on the device, then its rows'
+    /// lengths as `rtc_render_shard_ppm_rows` writes them; phase 2 is `rtc_write_shard_ppm`.
+    pub fn rtc_render_shard_samples_ppm_rows(scene: *mut RtcScene, depth: i32, samples_per_axis: u32, shard: i32, n_shards: i32,
+                                             row_bytes: *mut u64, stats: *mut RtcStats) -> c_int;
     pub fn rtc_trace_rays(scene: *mut RtcScene, n: u32, origins: *const f32, directions: *const f32, depth: i32,
                           out_rgb: *mut f32, out_t: *mut f32, out_prim: *mut i32) -> c_int;
     pub fn rtc_shard_bands(height: u32, shard: i32, n_shards: i32, first_rows: *mut u32) -> c_int;
